@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — frames/s of the disparity -> voxel-cloud hot path (BASELINE.json metric) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ...] [--dump-outputs DIR]
 
 A "step" is one reconstruction cycle of the reference (pose.cpp:361-434 + :527-531): seq_len = 50 accepted
 frames go through createAndTransformPtCloud (validity mask, Q reprojection, rigid transform, per-frame
@@ -305,6 +305,7 @@ def run_ours(args, rank, world, local_rank):
         counts = P.createCycleClouds(fr_host[s] if host else fr_dev[s], dt, device_pointers=not host)
         if world > 1:
             exchange()
+        stats["counts"] = counts
         stats["n_vox"] = int(counts.sum())
         stats["n_part"] = P.lastCyclePartials()
         stats["engine"] = P.lastCycleEngine()
@@ -320,7 +321,8 @@ def run_ours(args, rank, world, local_rank):
                 out = P.downsamplePtCloud(out_pin.numpy().view(abi.POINT))
             stats["n_out"] = len(out)
         else:
-            _, stats["n_out"] = P.downsamplePtCloudDevice()
+            stats["out_dev"] = P.downsamplePtCloudDevice()
+            stats["n_out"] = stats["out_dev"][1]
 
     def barrier():
         if world > 1:
@@ -391,12 +393,31 @@ def run_ours(args, rank, world, local_rank):
             dt_s = float(t.item())
         return nbytes / dt_s / 1e9, dt_s * 1e3
 
+    def last_step_outputs():
+        """What the last step of the timed device-resident leg returned to its caller: the per-frame counts and the combined
+        cloud, or with --dont_downsample (nothing is downsampled) the points the cycle appended.  The combined cloud is read
+        from the context's device result buffer, valid until the next call on the context (the leg ends with nothing but a
+        read of the launch counter)."""
+        out = {"frame_counts": stats["counts"]}
+        if nd:
+            out["cycle_points"] = P.lastCyclePoints()
+            return out
+        ptr, n = stats["out_dev"]
+        out["cloud"] = np.zeros(0, abi.POINT)
+        if n:
+            class DevArr:
+                __cuda_array_interface__ = {"shape": (n * abi.POINT.itemsize,), "typestr": "|u1", "data": (ptr, False), "version": 2}
+            out["cloud"] = torch.as_tensor(DevArr(), device=dev).cpu().numpy().view(abi.POINT)
+        return out
+
     h2d_gbs, h2d_ms = h2d_ceiling()
     timed(host=False)  # untimed pass: every buffer reaches its steady-state size
     clocks = ClockSampler(local_rank)
     clocks.start()
     ms, wall, launches = timed(host=False)
     clk = clocks.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_step_outputs(), rank, world)
     cells_after_value = P.cloudSize()
     ms_e2e_ev, ms_e2e, _ = timed(host=True)   # end to end = wall time of the region (copy stream included)
     d2h = stats["n_out"] * 16 + F * 4
@@ -605,6 +626,35 @@ def run_reference(args, rank, world):
             "e2e": {"value": fps, "unit": "frames/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
 
 
+# points of one dump over all ranks (each rank writes at most DUMP_MAX_POINTS // world): 12 B of xyz + 8 B of rgb + 8 B of
+# sample index each, so a dump stays under 64 MB
+DUMP_MAX_POINTS = 1_500_000
+
+
+def dump_outputs(out_dir, arrays, rank=0, world=1):
+    """Writes every array as <out_dir>/<name>.npy (<name>_rank<r>.npy when several ranks share the directory): counts as
+    float64; a point cloud as <name>_xyz (n x 3 float32) and <name>_rgb (n float64: the whole packed 32-bit colour word,
+    0x00RRGGBB).  A cloud of more than DUMP_MAX_POINTS // world points is cut to a fixed sample (seed 0, ascending, so two
+    builds that agree pick the same points) whose indices go to <name>_index (float64)."""
+    suffix = f"_rank{rank}" if world > 1 else ""
+    max_points = DUMP_MAX_POINTS // world
+    os.makedirs(out_dir, exist_ok=True)
+
+    def save(name, a):
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), a)
+
+    for name, a in arrays.items():
+        if a.dtype != abi.POINT:
+            save(name, a.astype(np.float64))
+            continue
+        if len(a) > max_points:
+            idx = np.sort(np.random.default_rng(0).choice(len(a), max_points, replace=False))
+            save(name + "_index", idx.astype(np.float64))
+            a = a[idx]
+        save(name + "_xyz", np.stack([a["x"], a["y"], a["z"]], 1).astype(np.float32))
+        save(name + "_rgb", a["rgb"].astype(np.float64))
+
+
 def emit(res, real_stdout):
     os.write(real_stdout, (json.dumps(res) + "\n").encode())
 
@@ -625,7 +675,14 @@ def main():
     ap.add_argument("--merge-mode", default="fused", choices=sorted(MERGE_MODES))
     ap.add_argument("--parity-steps", type=int, default=-1,
                     help="cycles compared with the CPU oracle after the timed regions (default 2; 1 at 4K; 0 = off)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (per-frame counts, combined cloud) "
+                         "as DIR/<name>.npy, to compare two builds on identical inputs")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     global MERGE_MODE
     MERGE_MODE = args.merge_mode
     if args.parity_steps < 0:

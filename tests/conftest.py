@@ -16,3 +16,15 @@ def pytest_configure(config):
 @pytest.fixture(scope="session")
 def golden_dir():
     return os.path.join(ROOT, "tests", "golden")
+
+
+@pytest.fixture(scope="session")
+def real(golden_dir):
+    """The reference's three real frames (disparity + labels) and what it logged for them, plus a seeded synthetic colour
+    plane: colours only travel with the points, nothing compares them with the reference."""
+    import numpy as np
+
+    from online_3d_reconstruction_b200 import synth
+    g = dict(np.load(os.path.join(golden_dir, "real_frames.npz")))
+    g["bgr"] = synth.make_frame_images(np.random.default_rng(1248), 720, 1280)[1]
+    return g

@@ -4,8 +4,9 @@ where /root/reference exists; the GPU box only sees the committed .npz files).
     python tests/golden/make_golden.py
 
 Sources (relative to /root/reference/build):
-  disparities/{1248,1249,1251}.png, segmentlabels/{same}.png, images/1248.png  real 1280x720 frames
+  disparities/{1248,1249,1251}.png, segmentlabels/{same}.png  real 1280x720 frames (no colour plane)
   output/log.txt:39-46,64          valid-pixel counts + variances the reference logged for them
+  images/1248.png                  input of the median / bilateral crops below
   output/medianBlurred_{15,31}.png cv::medianBlur outputs of images/1248.png written by the reference
   output/bilateralFiltered_{15,31}.png cv::bilateralFilter(img, k, 2k, k/2) outputs written by the reference
   cloud.ply                        a combined-grid VoxelGrid output of the reference (voxel_size 0.05)
@@ -29,9 +30,10 @@ def main():
     nums = [1248, 1249, 1251]
     disp = np.stack([cv2.imread(R + f"disparities/{n}.png", cv2.IMREAD_GRAYSCALE) for n in nums])
     labels = np.stack([cv2.imread(R + f"segmentlabels/{n}.png", cv2.IMREAD_GRAYSCALE) for n in nums])
-    bgr1248 = cv2.imread(R + "images/1248.png")
+    # no colour plane: the logged numbers depend on disparities and labels only, and a 720p photo alone would put the file
+    # over 1 MB (the tests draw a seeded synthetic colour plane instead)
     np.savez_compressed(
-        os.path.join(OUT, "real_frames.npz"), img_nums=np.array(nums), disp=disp, labels=labels, bgr1248=bgr1248,
+        os.path.join(OUT, "real_frames.npz"), img_nums=np.array(nums), disp=disp, labels=labels,
         # log.txt:39,40,42 "index i disp_img_var V plane_fitted_disp_img_var P"; :45,46,64 "point_clout_pts"
         disp_img_var=np.array([2.27913, 2.64813, 2.08488]),
         plane_fitted_disp_img_var=np.array([1.63692, 1.49152, 1.64115]),

@@ -6,6 +6,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -39,6 +40,49 @@ def test_both_arms_print_one_config_object_and_every_workload_builds():
         ny, nx = abi.scan_dims(p)
         assert ny > 0 and nx > 0
     assert bench.static_config("config2_semidense_720p", 8)["frames_per_step"] == 50   # per GPU: weak scaling
+
+
+def _cloud(rng, n):
+    pts = np.zeros(n, abi.POINT)
+    pts["x"], pts["y"], pts["z"] = rng.normal(size=(3, n)).astype(np.float32)
+    pts["rgb"] = rng.integers(0, 1 << 32, n, dtype=np.uint32)   # every bit of the colour word, the top byte too
+    return pts
+
+
+def test_dump_outputs_writes_float_arrays_and_a_fixed_sample(tmp_path, monkeypatch):
+    """--dump-outputs: counts as float64, a cloud as xyz float32 and the whole colour word as float64; a cloud larger than the
+    cap becomes the same ascending sample on every run, with its indices."""
+    monkeypatch.setattr(bench, "DUMP_MAX_POINTS", 1000)
+    pts = _cloud(np.random.default_rng(3), 5000)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"frame_counts": np.array([3, 0, 7], np.uint32), "cloud": pts})
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["cloud_index.npy", "cloud_rgb.npy", "cloud_xyz.npy", "frame_counts.npy"]
+    out = {}
+    for f in files:
+        a, b = np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)
+        assert a.dtype in (np.float32, np.float64) and np.array_equal(a, b), f
+        out[f[:-4]] = a
+    idx = out["cloud_index"].astype(np.int64)
+    assert len(idx) == 1000 and np.all(np.diff(idx) > 0)
+    assert np.array_equal(out["cloud_xyz"], np.stack([pts["x"][idx], pts["y"][idx], pts["z"][idx]], 1))
+    assert np.array_equal(out["cloud_rgb"].astype(np.uint32), pts["rgb"][idx])
+    assert out["frame_counts"].tolist() == [3, 0, 7]
+
+
+@pytest.mark.parametrize("world", [1, 3])
+def test_dump_outputs_of_all_ranks_stay_under_64_mb(tmp_path, world):
+    """Every rank writes its shard into the same directory: with each shard larger than its share of the cap, the files of all
+    ranks together stay under 64 MB."""
+    rng = np.random.default_rng(4)
+    n = bench.DUMP_MAX_POINTS // world + 100_000
+    for r in range(world):
+        bench.dump_outputs(str(tmp_path), {"frame_counts": np.arange(50, dtype=np.uint32), "cloud": _cloud(rng, n)}, r, world)
+    files = os.listdir(tmp_path)
+    assert len(files) == 4 * world
+    assert sum(os.path.getsize(tmp_path / f) for f in files) < 64e6
+    xyz = [np.load(tmp_path / f, mmap_mode="r") for f in files if "cloud_xyz" in f]
+    assert len(xyz) == world and all(len(a) == bench.DUMP_MAX_POINTS // world for a in xyz)
 
 
 @pytest.mark.timeout(600)

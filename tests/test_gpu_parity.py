@@ -39,11 +39,6 @@ def _eq(a, b):
         raise AssertionError(f"{len(np.unique(bad))} of {len(a)} records differ; first at {bad[0]}: {a[bad[0]]} vs {b[bad[0]]}")
 
 
-@pytest.fixture(scope="module")
-def real(golden_dir):
-    return np.load(os.path.join(golden_dir, "real_frames.npz"))
-
-
 # ---------------------------------------------------------------------------------------------- masks
 @pytest.mark.parametrize("J", [1, 3, 15])
 @pytest.mark.parametrize("geom", [SMALL, SMALL4])
@@ -65,10 +60,10 @@ def test_mask_counts_match_reference_log_720p(real):
         for i in range(3):
             coef, f64 = ob.plane_fit(p, real["labels"][i], real["disp"][i])
             keep = []
-            fr = abi.make_frame(None, real["bgr1248"], np.eye(4), labels=real["labels"][i], plane_coef=coef, keep=keep)
+            fr = abi.make_frame(None, real["bgr"], np.eye(4), labels=real["labels"][i], plane_coef=coef, keep=keep)
             m = P.validityMask(fr, abi.DISP_F64)
             assert int(m.sum()) == int(real["point_cloud_pts"][i])
-            fr64 = abi.make_frame(f64, real["bgr1248"], np.eye(4), keep=keep)
+            fr64 = abi.make_frame(f64, real["bgr"], np.eye(4), keep=keep)
             pts = P.createAndTransformPtCloud(fr64, abi.DISP_F64)
             exp = ob.create_and_transform_pt_cloud(p, fr64, abi.DISP_F64)
             _eq(pts, exp)
@@ -167,7 +162,7 @@ def test_real_frame_720p_dense(real):
     keep = []
     p = abi.make_params(jump_pixels=1, voxel_size=0.05)
     T = synth.trajectory(np.random.default_rng(3), 1)[0]
-    fr = abi.make_frame(real["disp"][0], real["bgr1248"], T, keep=keep)
+    fr = abi.make_frame(real["disp"][0], real["bgr"], T, keep=keep)
     exp = ob.create_and_transform_pt_cloud(p, fr, abi.DISP_U8)
     with Pose(p) as P:
         got = P.createAndTransformPtCloud(fr)

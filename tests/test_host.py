@@ -3,6 +3,8 @@ mirror matches the C layout, host pose composition matches the oracle, the gener
 import ctypes as C
 import os
 import re
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -40,18 +42,17 @@ def test_ctypes_layout_matches_c():
 
 
 def test_no_cpu_fallback_without_device(L):
-    """Without a GPU the product must fail loudly, not compute on the CPU."""
-    try:
-        import torch
-        if torch.cuda.is_available():
-            pytest.skip("a GPU is present")
-    except ImportError:
-        pass
-    p = abi.make_params()
-    h = C.c_void_p()
-    rc = L.o3r_create(C.byref(p), C.byref(h))
-    assert rc == abi.O3R_ERR_CUDA and not h.value
-    assert b"no CPU fallback" in L.o3r_last_error(None)
+    """Without a GPU the product must fail loudly, not compute on the CPU.  The check runs in a child process that sees
+    no device, so it also runs on a machine that has one."""
+    code = ("import ctypes as C, sys; sys.path.insert(0, sys.argv[1])\n"
+            "from online_3d_reconstruction_b200 import abi, lib\n"
+            "L = lib.load(); p = abi.make_params(); h = C.c_void_p()\n"
+            "rc = L.o3r_create(C.byref(p), C.byref(h))\n"
+            "assert rc == abi.O3R_ERR_CUDA and not h.value, rc\n"
+            "assert b'no CPU fallback' in L.o3r_last_error(None), L.o3r_last_error(None)\n")
+    r = subprocess.run([sys.executable, "-c", code, ROOT], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True, timeout=120)
+    assert r.returncode == 0, r.stdout + r.stderr
 
 
 def test_invalid_params_rejected(L):

@@ -11,11 +11,6 @@ import oracle_binding as ob
 from online_3d_reconstruction_b200 import abi
 
 
-@pytest.fixture(scope="module")
-def real(golden_dir):
-    return np.load(os.path.join(golden_dir, "real_frames.npz"))
-
-
 def test_disp_variance_matches_reference_log(real):
     """getVariance on raw u8 disparity == build/output/log.txt:39-42 (6 significant figures)."""
     p = abi.make_params(jump_pixels=1)
@@ -28,7 +23,7 @@ def test_plane_fit_variance_and_mask_count_match_reference_log(real):
     """createPlaneFittedDisparityImages + getVariance(planeFitted) and the valid-pixel count of
     createSingleImgPtCloud (jump_pixels=1, --use_segment_labels) == log.txt:39-46,64."""
     p = abi.make_params(jump_pixels=1, voxel_size=0.05, use_segment_labels=True)
-    bgr = real["bgr1248"]
+    bgr = real["bgr"]
     for i in range(3):
         coef, f64 = ob.plane_fit(p, real["labels"][i], real["disp"][i])
         v = ob.get_variance(p, f64, True)
@@ -59,8 +54,8 @@ def test_plane_fit_against_opencv_gemm_and_svd_inverse(real, golden_dir):
         assert coef.shape == cv.shape
         assert np.max(np.abs(coef - cv) / np.abs(cv)) < 1e-9
         keep = []
-        fa = abi.make_frame(None, real["bgr1248"], np.eye(4), labels=real["labels"][i], plane_coef=coef, keep=keep)
-        fb = abi.make_frame(None, real["bgr1248"], np.eye(4), labels=real["labels"][i], plane_coef=cv, keep=keep)
+        fa = abi.make_frame(None, real["bgr"], np.eye(4), labels=real["labels"][i], plane_coef=coef, keep=keep)
+        fb = abi.make_frame(None, real["bgr"], np.eye(4), labels=real["labels"][i], plane_coef=cv, keep=keep)
         pa = ob.create_single_img_pt_cloud(p, fa, abi.DISP_F64)
         pb = ob.create_single_img_pt_cloud(p, fb, abi.DISP_F64)
         assert len(pa) == len(pb) == int(real["point_cloud_pts"][i])
