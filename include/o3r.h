@@ -271,25 +271,6 @@ typedef struct o3r_cell {
     uint32_t pad;
 } o3r_cell;                  /* 40 bytes */
 
-/* Pre-reduce the last batch on the combined grid and bucket the partial cells by
- * owner = hash64(key) % world.  `send` is a DEVICE buffer of `cap` cells; counts[world] (host)
- * receives the cells per owner, bucket r starting at sum(counts[0..r)).  ACCUMULATE mode,
- * contexts created with defer_merge (see o3r_set_defer_merge). */
-int o3r_exchange_pack(o3r_ctx* ctx, int world, o3r_cell* send_dev, size_t cap, uint32_t* counts);
-
-/* Merge `n` received partial cells (DEVICE buffer, any order) into the resident shard. */
-int o3r_exchange_merge(o3r_ctx* ctx, const o3r_cell* recv_dev, size_t n);
-
-/* The same exchange without host round trips.  o3r_exchange_pack_dev queues the pack on the context's stream and
- * returns at once; `info_dev` (DEVICE, world + 8 u32) receives the cells per owner, then the cycle's combined-grid cell
- * range {imin, jmin, kmin, imax, jmax, kmax} as int32 (min > max when the batch was empty), then the cell count and a
- * pad word — the header the ranks all-gather (on the same stream) to size the payload exchange.  `cap` must be at least
- * o3r_exchange_bound(ctx), the host-known bound of the cells the pack can emit.  o3r_exchange_merge_bb takes the union
- * of the gathered cell ranges, so the merge does not have to reduce (and wait for) the range of the received cells. */
-size_t o3r_exchange_bound(o3r_ctx* ctx);
-int o3r_exchange_pack_dev(o3r_ctx* ctx, int world, o3r_cell* send_dev, size_t cap, uint32_t* info_dev);
-int o3r_exchange_merge_bb(o3r_ctx* ctx, const o3r_cell* recv_dev, size_t n, const int bb[6]);
-
 /* Parity probe for O3R_MERGE_ACCUMULATE_FUSED: when set, the fused engine also stores every per-frame voxel centroid of
  * the batch, in no particular order, and o3r_last_batch_points returns that multiset. */
 int o3r_set_keep_frame_voxels(o3r_ctx* ctx, int keep);
@@ -308,17 +289,14 @@ int o3r_set_keep_frame_voxels(o3r_ctx* ctx, int keep);
  * colours exactly, centroids within float reassociation (1e-5 relative).
  * NCCL is loaded at run time (libnccl.so.2); o3r_comm_unique_id + o3r_comm_init create a communicator of the library's own
  * (the id travels by whatever channel the host has: MPI, a file, torch.distributed), o3r_comm_attach adopts an existing
- * ncclComm_t.  Both switch the context to deferred merging (o3r_set_defer_merge). */
+ * ncclComm_t.  While a communicator is attached, o3r_frames_cloud* leaves the merge to o3r_exchange_cycle; after
+ * o3r_comm_destroy the context merges its cycles itself again. */
 #define O3R_COMM_ID_BYTES 128
 int o3r_comm_unique_id(void* id_out /* O3R_COMM_ID_BYTES, rank 0 */);
 int o3r_comm_init(o3r_ctx* ctx, int world, int rank, const void* id, size_t slot_cells);   /* collective */
 int o3r_comm_attach(o3r_ctx* ctx, void* nccl_comm, int world, int rank, size_t slot_cells);
 int o3r_comm_destroy(o3r_ctx* ctx);
 int o3r_exchange_cycle(o3r_ctx* ctx);                                                     /* collective, asynchronous */
-
-/* When set, o3r_frames_cloud* keeps the batch's per-frame clouds but does not merge them into the
- * resident cloud; the caller runs o3r_exchange_pack / o3r_exchange_merge instead. */
-int o3r_set_defer_merge(o3r_ctx* ctx, int defer);
 
 /* ---- introspection ----------------------------------------------------------------------------- */
 

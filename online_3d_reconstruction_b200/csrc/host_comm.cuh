@@ -129,7 +129,6 @@ int comm_setup(o3r_ctx* ctx, int world, int rank, size_t slot_cells) {
     CU(ctx->x_send.ensure(bytes));
     CU(ctx->x_recv.ensure(bytes));
     CU(ctx->x_list.ensure((size_t)world * slot_cells * sizeof(o3r_cell)));
-    ctx->defer_merge = 1;   // cycles are merged by o3r_exchange_cycle from now on
     return O3R_OK;
 }
 

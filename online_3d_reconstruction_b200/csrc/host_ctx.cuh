@@ -105,7 +105,6 @@ struct o3r_ctx {
     uint32_t npix = 0;
     int canon = 0;
     float leaf_f = 0, inv_f = 0, leaf_c = 0, inv_c = 0, inv_cz = 0;
-    int defer_merge = 0;
     DevBuf lut_r, lut_z;
     // input staging (host-pointer entry points)
     // double-buffered: a prefetch of the next cycle's inputs fills one set while the kernels read the other
@@ -188,7 +187,6 @@ struct o3r_ctx {
     bool keep_frame_voxels = false;   // parity probe: the bucket engine also writes every per-frame voxel centroid (any order)
     size_t last_partials = 0;
     bool last_has_partials = false;
-    uint32_t n_cyc = 0;
     // ... or points (RETAIN / dont_downsample)
     DevBuf cloud;
     size_t n_cloud = 0;

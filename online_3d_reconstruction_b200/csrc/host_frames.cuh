@@ -606,7 +606,7 @@ int frames_cloud_impl(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_typ
     ctx->last_total = ctx->last_off[n];
     if (frame_counts)
         for (int i = 0; i < n; ++i) frame_counts[i] = ctx->last_off[i + 1] - ctx->last_off[i];
-    if (!opt.merge || ctx->defer_merge) return O3R_OK;
+    if (!opt.merge || ctx->comm) return O3R_OK;   // with a communicator, o3r_exchange_cycle merges the cycle
     const float4* outp = ctx->last_is_vox ? ctx->vox.as<float4>() : ctx->pts.as<float4>();
     if (ctx->retain()) return cloud_append_dev(ctx, outp, ctx->last_total);
     const int* bbp = ctx->last_has_cellbb ? ctx->last_cellbb : nullptr;

@@ -85,13 +85,12 @@ int refresh_nres(o3r_ctx* ctx, bool block) {
     return O3R_OK;
 }
 
-// Builds the cycle's cell list (ckey/cacc/crgb, n_cyc) from items, continuing from the resident sums when
+// Builds the cycle's cell list (ckey/cacc/crgb, count in counters[CNT_CYC]) from items, continuing from the resident sums when
 // `use_resident`.  `bb` = {imin,jmin,kmin,imax,jmax,kmax} of the items' combined-grid cells when the caller already
 // knows it (host), else null.  Leaves h_counters[CNT_CYC], [CNT_NEW] valid.
 template <typename Items>
 int acc_build_cycle(o3r_ctx* ctx, const Items& items, size_t n, bool use_resident, const int* bb) {
     uint32_t* cnt = ctx->counters.as<uint32_t>();
-    ctx->n_cyc = 0;
     ctx->n_cyc_ub = 0;
     ctx->h_counters[CNT_CYC] = ctx->h_counters[CNT_NEW] = 0;
     if (n == 0) return O3R_OK;
@@ -127,7 +126,6 @@ int acc_build_cycle(o3r_ctx* ctx, const Items& items, size_t n, bool use_residen
 // on the device (n = the host's bound).  The radix plan skips the digits that are constant over the batch.
 template <typename Items>
 int acc_build_cycle_abs(o3r_ctx* ctx, const Items& items, size_t n, bool use_resident, const uint32_t* n_dev) {
-    ctx->n_cyc = 0;
     ctx->n_cyc_ub = 0;
     ctx->h_counters[CNT_CYC] = ctx->h_counters[CNT_NEW] = 0;
     if (n == 0) return O3R_OK;

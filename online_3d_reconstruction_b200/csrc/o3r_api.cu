@@ -207,12 +207,6 @@ int o3r_set_keep_frame_voxels(o3r_ctx* ctx, int keep) {
     return O3R_OK;
 }
 
-int o3r_set_defer_merge(o3r_ctx* ctx, int defer) {
-    if (!ctx) return O3R_ERR_INVALID;
-    ctx->defer_merge = defer != 0;
-    return O3R_OK;
-}
-
 void* o3r_host_alloc(size_t bytes) {
     void* p = nullptr;
     if (cudaMallocHost(&p, bytes) != cudaSuccess) return nullptr;
@@ -554,117 +548,6 @@ int o3r_blur_u8(o3r_ctx* ctx, const uint8_t* src, size_t src_step, int rows, int
     return O3R_OK;
 }
 
-// Pre-reduces the last batch on the combined grid and buckets the partial cells by owner.  Nothing here waits for the GPU:
-// launches are sized by the host's bound of the cycle's cell count, the exact count stays on the device.
-// info (device, world + 8 words, may be null): counts per owner, the cycle's cell range, the cell count.
-static int exchange_pack_impl(o3r_ctx* ctx, int world, o3r_cell* send_dev, size_t cap, uint32_t* info_dev, uint32_t** ocnt_out) {
-    if (ctx->retain()) return ctx->fail(O3R_ERR_UNSUPPORTED, "exchange needs O3R_MERGE_ACCUMULATE");
-    uint32_t* cnt = ctx->counters.as<uint32_t>();
-    CU(ctx->okeys.ensure((size_t)kMaxPasses * kRsBins * 4 + sizeof(SortPlan)));
-    uint32_t* ocnt = ctx->okeys.as<uint32_t>();   // laid out like ghist: the owner histogram is pass 0's
-    if (ocnt_out) *ocnt_out = ocnt;
-    ZERO(ocnt, (size_t)kMaxPasses * kRsBins * 4);
-    const int none[6] = {0x7fffffff, 0x7fffffff, 0x7fffffff, (int)0x80000000, (int)0x80000000, (int)0x80000000};
-    const int* bbp = ctx->last_has_cellbb ? ctx->last_cellbb : nullptr;
-    if (!ctx->last_is_vox || ctx->last_total == 0) {   // nothing to send: header only
-        ctx->n_cyc_ub = 0;
-        ZERO(cnt + CNT_CYC, 4);
-        if (info_dev)
-            LAUNCH(k_pack_cells, 1, kThreads, 0, cnt + CNT_CYC, (const uint32_t*)nullptr, (const uint64_t*)nullptr, (const float4*)nullptr,
-                   (const uint4*)nullptr, send_dev, ocnt, (uint32_t)world, none[0], none[1], none[2], none[3], none[4], none[5], info_dev);
-        return O3R_OK;
-    }
-    int rc;
-    if (ctx->last_has_partials) {
-        AccItemsCells items{ctx->partials.as<o3r_cell>(), nullptr, nullptr};
-        rc = acc_build_cycle(ctx, items, ctx->last_partials, false, bbp);
-    } else {
-        AccItemsPts items{ctx->vox.as<float4>(), nullptr, nullptr};
-        rc = acc_build_cycle(ctx, items, ctx->last_total, false, bbp);
-    }
-    if (rc) return rc;
-    const size_t nub = ctx->n_cyc_ub;
-    if (cap < nub) return ctx->fail(O3R_ERR_CAPACITY, "send buffer smaller than o3r_exchange_bound()");
-    // one stable radix pass on the owner id buckets the (key-sorted) cells by destination rank
-    SortU32 sb;
-    rc = carve_sort_u32(ctx, nub, sb);
-    if (rc) return rc;
-    SortPlan* plan = reinterpret_cast<SortPlan*>(ocnt + kMaxPasses * kRsBins);
-    SortPlan pl;
-    memset(&pl, 0, sizeof(pl));
-    pl.active_mask = 1; pl.final_parity = 1; pl.n_active = 1; pl.n_passes = 1; pl.bits[0] = 8;
-    { int rcu = upload_small(ctx, plan, &pl, sizeof(pl)); if (rcu) return rcu; }
-    CU(ctx->seg2.ensure(16));
-    const uint32_t g = std::min<uint32_t>(std::max(1u, cdiv(nub, kThreads)), 148 * 8);
-    LAUNCH(k_owner, g, kThreads, 0, cnt + CNT_CYC, ctx->ckey.as<uint64_t>(), (uint32_t)world, sb.k0, sb.v0, ocnt, ctx->seg2.as<uint32_t>());
-    rc = sort_pairs<uint32_t>(ctx, sb.k0, sb.k1, sb.v0, sb.v1, ctx->seg2.as<uint32_t>(), 1, std::max<size_t>(nub, 1), plan, 1, 0, ocnt,
-                              0 /* raw owner counts: they are also the exchange header */);
-    if (rc) return rc;
-    const int* bb = bbp ? bbp : none;
-    LAUNCH(k_pack_cells, g, kThreads, 0, cnt + CNT_CYC, sb.v1, ctx->ckey.as<uint64_t>(), ctx->cacc.as<float4>(), ctx->crgb.as<uint4>(),
-           send_dev, ocnt, (uint32_t)world, bb[0], bb[1], bb[2], bb[3], bb[4], bb[5], info_dev);
-    return O3R_OK;
-}
-
-size_t o3r_exchange_bound(o3r_ctx* ctx) {
-    if (!ctx) return 0;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    if (!ctx->last_is_vox || ctx->last_total == 0) return 0;
-    // cells the next pack can emit: no more than the batch has records, no more than its cell range holds
-    size_t n = ctx->last_has_partials ? ctx->last_partials : ctx->last_total;
-    if (ctx->last_has_cellbb) {
-        const int* b = ctx->last_cellbb;
-        const double cells = ((double)b[3] - b[0] + 1) * ((double)b[4] - b[1] + 1) * ((double)b[5] - b[2] + 1);
-        if (cells > 0 && cells < (double)n) n = (size_t)cells;
-    }
-    return n;
-}
-
-int o3r_exchange_pack_dev(o3r_ctx* ctx, int world, o3r_cell* send_dev, size_t cap, uint32_t* info_dev) {
-    if (!ctx || world < 1 || world > 256 || !info_dev) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    return exchange_pack_impl(ctx, world, send_dev, cap, info_dev, nullptr);
-}
-
-int o3r_exchange_pack(o3r_ctx* ctx, int world, o3r_cell* send_dev, size_t cap, uint32_t* counts) {
-    if (!ctx || world < 1 || world > 256 || !counts) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    uint32_t* ocnt = nullptr;
-    int rc = exchange_pack_impl(ctx, world, send_dev, cap, nullptr, &ocnt);
-    if (rc) return rc;
-    CU(cudaMemcpyAsync(counts, ocnt, (size_t)world * 4, cudaMemcpyDeviceToHost, ctx->st));
-    CU(cudaMemcpyAsync(ctx->h_counters + CNT_CYC, ctx->counters.as<uint32_t>() + CNT_CYC, 4, cudaMemcpyDeviceToHost, ctx->st));
-    CU(cudaStreamSynchronize(ctx->st));
-    ctx->n_cyc = ctx->h_counters[CNT_CYC];
-    return O3R_OK;
-}
-
-static int exchange_merge_impl(o3r_ctx* ctx, const o3r_cell* recv_dev, size_t n, const int* bb) {
-    if (ctx->retain()) return ctx->fail(O3R_ERR_UNSUPPORTED, "exchange needs O3R_MERGE_ACCUMULATE");
-    if (n == 0) return O3R_OK;
-    AccItemsCells items{recv_dev, nullptr, nullptr};
-    int rc = acc_build_cycle(ctx, items, n, true, bb);
-    if (rc) return rc;
-    return acc_apply_cycle(ctx);
-}
-
-int o3r_exchange_merge(o3r_ctx* ctx, const o3r_cell* recv_dev, size_t n) {
-    if (!ctx || (n && !recv_dev)) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    return exchange_merge_impl(ctx, recv_dev, n, nullptr);
-}
-
-int o3r_exchange_merge_bb(o3r_ctx* ctx, const o3r_cell* recv_dev, size_t n, const int bb[6]) {
-    if (!ctx || (n && !recv_dev) || !bb) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    return exchange_merge_impl(ctx, recv_dev, n, bb);
-}
-
-
 // ---- the exchange inside the library: communicator + one call per cycle (SURVEY 8e) --------------------------------------
 int o3r_comm_unique_id(void* id_out) {
     if (!id_out) return O3R_ERR_INVALID;
@@ -716,6 +599,7 @@ int o3r_comm_destroy(o3r_ctx* ctx) {
     NcclApi* N = nccl_api();
     if (ctx->comm && ctx->comm_owned) NC(N->CommDestroy((ncclComm_t)ctx->comm));
     ctx->comm = nullptr; ctx->comm_owned = false; ctx->world = 1; ctx->rank = 0;
+    ctx->x_send.release(); ctx->x_recv.release(); ctx->x_list.release();
     return O3R_OK;
 }
 

@@ -864,33 +864,6 @@ __global__ void __launch_bounds__(kThreads) k_owner(const uint32_t* __restrict__
         if (s_cnt[r]) atomicAdd(&counts[r], s_cnt[r]);
 }
 
-// also publishes the exchange header: counts per owner, then the cycle's cell range (6 int32), then 2 pad words
-__global__ void __launch_bounds__(kThreads) k_pack_cells(const uint32_t* __restrict__ n_cyc_ptr, const uint32_t* __restrict__ order,
-                                                         const uint64_t* __restrict__ ckey, const float4* __restrict__ cacc,
-                                                         const uint4* __restrict__ crgb, o3r_cell* __restrict__ out,
-                                                         const uint32_t* __restrict__ counts, uint32_t world, int b0, int b1,
-                                                         int b2, int b3, int b4, int b5, uint32_t* __restrict__ info) {
-    const uint32_t n_cyc = *n_cyc_ptr;
-    if (blockIdx.x == 0 && info) {
-        for (uint32_t r = threadIdx.x; r < world; r += kThreads) info[r] = counts[r];
-        if (threadIdx.x == 0) {
-            const int bb[6] = {b0, b1, b2, b3, b4, b5};
-            for (int a = 0; a < 6; ++a) info[world + a] = (uint32_t)bb[a];
-            info[world + 6] = n_cyc; info[world + 7] = 0u;
-        }
-    }
-    for (uint32_t i = blockIdx.x * kThreads + threadIdx.x; i < n_cyc; i += gridDim.x * kThreads) {
-        const uint32_t h = order[i];
-        const float4 a = cacc[h];
-        const uint4 c = crgb[h];
-        o3r_cell r;
-        r.key = ckey[h];
-        r.sx = a.x; r.sy = a.y; r.sz = a.z; r.n = __float_as_uint(a.w);
-        r.sr = c.x; r.sg = c.y; r.sb = c.z; r.pad = 0;
-        out[i] = r;
-    }
-}
-
 // rigid transform of a resident point cloud in place (pose.cpp:353)
 __global__ void __launch_bounds__(kThreads) k_transform_pts(float4* __restrict__ pts, size_t n, const float* __restrict__ Tm) {
     __shared__ float T[12];

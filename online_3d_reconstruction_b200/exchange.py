@@ -1,19 +1,8 @@
-"""Multi-GPU plumbing for the combined-grid merge (SURVEY §8e): one process per GPU, frames sharded
-f mod P, partial cells hash-partitioned by owner and exchanged with an all-to-all-v.
-
-The data path is libo3r.so (o3r_exchange_pack buckets the cycle's partial cells by owner on the GPU,
-o3r_exchange_merge folds received cells into the resident shard); this module only moves the buckets:
-counts by all_gather, payload by grouped isend/irecv (ncclGroupStart ... ncclSend/ncclRecv ... on NCCL,
-the same calls on gloo for the CPU tests).
+"""Host mirrors of the multi-GPU split (SURVEY §8e): one process per GPU, frames sharded f mod P, and each
+combined-grid cell owned by the rank hash64(key) mod P names.  The exchange itself runs inside libo3r.so
+(o3r_comm_init / o3r_exchange_cycle); this module lets a caller or a test compute the same split on the host.
 """
 import numpy as np
-import torch
-import torch.distributed as dist
-
-from . import abi
-
-CELL_BYTES = abi.CELL.itemsize
-_M64 = (1 << 64) - 1
 
 
 def hash64(x):
@@ -35,120 +24,3 @@ def owner_of(keys, world):
 def shard_frames(n_frames, rank, world):
     """Indices of the cycle's frames this rank reconstructs (frame f -> rank f mod P)."""
     return list(range(rank, n_frames, world))
-
-
-def exchange_cells(send, counts, group=None):
-    """All-to-all-v of o3r_cell records.
-
-    send:   flat uint8 tensor holding this rank's cells bucketed by destination rank (bucket r starts at
-            sum(counts[:r]) cells), on the device of the process group's backend.
-    counts: cells per destination rank (len == world size).
-    Returns (recv uint8 tensor, n_recv): the cells this rank owns, grouped by source rank in rank order.
-    """
-    world, rank = dist.get_world_size(group), dist.get_rank(group)
-    counts = [int(c) for c in counts]
-    assert len(counts) == world
-    mine = torch.tensor(counts, dtype=torch.int64, device=send.device)
-    allc = [torch.empty_like(mine) for _ in range(world)]
-    dist.all_gather(allc, mine, group=group)
-    recv_counts = [int(allc[src][rank]) for src in range(world)]   # one host sync: the split sizes
-    n_recv = sum(recv_counts)
-    recv = torch.empty(max(n_recv, 1) * CELL_BYTES, dtype=torch.uint8, device=send.device)
-    s_off = np.concatenate([[0], np.cumsum(counts)]) * CELL_BYTES
-    r_off = np.concatenate([[0], np.cumsum(recv_counts)]) * CELL_BYTES
-    ops = []
-    for peer in range(world):
-        if peer == rank:
-            continue
-        if recv_counts[peer]:
-            ops.append(dist.P2POp(dist.irecv, recv[r_off[peer]:r_off[peer + 1]], peer, group))
-        if counts[peer]:
-            ops.append(dist.P2POp(dist.isend, send[s_off[peer]:s_off[peer + 1]], peer, group))
-    if counts[rank]:
-        recv[r_off[rank]:r_off[rank + 1]].copy_(send[s_off[rank]:s_off[rank + 1]])
-    if ops:
-        for w in dist.batch_isend_irecv(ops):
-            w.wait()
-    return recv, n_recv
-
-
-def exchange_by_header(send, info, group=None):
-    """The transport half of a cycle's exchange: all-gather of the ranks' headers, ONE host read of the gathered
-    headers, grouped send/recv of the buckets.
-
-    send: uint8 tensor with this rank's cells bucketed by destination rank (as o3r_exchange_pack_dev leaves them).
-    info: int32 tensor of world + 8 words on the same device (o3r.h): cells per destination rank, the rank's
-          combined-grid cell range {imin, jmin, kmin, imax, jmax, kmax} (min > max when it sent nothing), cell count, pad.
-    Returns (recv uint8 tensor, n_recv, bb, n_sent): the cells this rank owns grouped by source rank, and the union of
-    the ranks' cell ranges (None when nobody sent anything).
-    """
-    world, rank = dist.get_world_size(group), dist.get_rank(group)
-    gathered = [torch.empty_like(info) for _ in range(world)]
-    dist.all_gather(gathered, info, group=group)
-    g = torch.stack(gathered).cpu().numpy().reshape(world, world + 8)   # the one host sync of the exchange
-    counts = [int(c) for c in g[rank, :world]]
-    recv_counts = [int(g[src, rank]) for src in range(world)]
-    bbs = g[:, world:world + 6]
-    valid = bbs[:, 0] <= bbs[:, 3]
-    bb = None
-    if valid.any():
-        bb = [int(v) for v in bbs[valid, :3].min(axis=0)] + [int(v) for v in bbs[valid, 3:].max(axis=0)]
-    n_recv = sum(recv_counts)
-    recv = torch.empty(max(n_recv, 1) * CELL_BYTES, dtype=torch.uint8, device=send.device)
-    s_off = np.concatenate([[0], np.cumsum(counts)]) * CELL_BYTES
-    r_off = np.concatenate([[0], np.cumsum(recv_counts)]) * CELL_BYTES
-    ops = []
-    for peer in range(world):
-        if peer == rank:
-            continue
-        if recv_counts[peer]:
-            ops.append(dist.P2POp(dist.irecv, recv[r_off[peer]:r_off[peer + 1]], peer, group))
-        if counts[peer]:
-            ops.append(dist.P2POp(dist.isend, send[s_off[peer]:s_off[peer + 1]], peer, group))
-    if counts[rank]:
-        recv[r_off[rank]:r_off[rank + 1]].copy_(send[s_off[rank]:s_off[rank + 1]])
-    if ops:
-        for w in dist.batch_isend_irecv(ops):
-            w.wait()
-    return recv, n_recv, bb, sum(counts)
-
-
-def exchange_cycle(P, send, info, group=None):
-    """One cycle's exchange with a single host round trip: pack on the GPU (queued), exchange_by_header, merge on the
-    GPU (queued).
-
-    P:    the rank's Pose (defer-merge mode); call this with torch's current stream set to P's stream
-          (`with torch.cuda.stream(torch.cuda.ExternalStream(P.stream()))`) so that the library's kernels and the
-          collectives are ordered without extra synchronisation.
-    send: uint8 device tensor of at least P.exchangeBound() cells; info: int32 device tensor of world + 8 words.
-    Returns the number of cells this rank sent.
-    """
-    world = dist.get_world_size(group)
-    P.exchangePackDevice(world, send.data_ptr(), send.numel() // CELL_BYTES, info.data_ptr())
-    recv, n_recv, bb, n_sent = exchange_by_header(send, info, group)
-    if n_recv:
-        P.exchangeMerge(recv.data_ptr(), n_recv, bb)
-    P._exchange_keepalive = recv     # the merge kernels are only queued: keep the buffer until the next cycle
-    return n_sent
-
-
-def merge_cells_host(cells):
-    """Reference merge of partial cells on the host (tests): sort by key, add partials in order."""
-    cells = np.asarray(cells, dtype=abi.CELL)
-    order = np.argsort(cells["key"], kind="stable")
-    c = cells[order]
-    keys, start = np.unique(c["key"], return_index=True)
-    out = np.zeros(len(keys), dtype=abi.CELL)
-    out["key"] = keys
-    for f in ("n", "sr", "sg", "sb"):
-        out[f] = np.add.reduceat(c[f].astype(np.uint64), start).astype(np.uint32)
-    for f in ("sx", "sy", "sz"):
-        acc = np.zeros(len(keys), dtype=np.float32)
-        end = np.append(start[1:], len(c))
-        for i, (a, b) in enumerate(zip(start, end)):   # float sums strictly in order
-            s = np.float32(0)
-            for v in c[f][a:b]:
-                s = np.float32(s + v)
-            acc[i] = s
-        out[f] = acc
-    return out

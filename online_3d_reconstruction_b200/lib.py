@@ -16,8 +16,8 @@ SYMBOLS = [
     "o3r_frame_cloud", "o3r_frames_cloud", "o3r_frames_cloud_dev", "o3r_frames_prefetch", "o3r_frames_prefetch_cancel", "o3r_last_batch_points",
     "o3r_cloud_transform", "o3r_cloud_append", "o3r_cloud_downsample", "o3r_cloud_downsample_dev", "o3r_cloud_size",
     "o3r_cloud_clear",
-    "o3r_voxel_grid", "o3r_blur_u8", "o3r_frame_mask", "o3r_disp_variance", "o3r_plane_fit", "o3r_sor", "o3r_last_batch_partials", "o3r_exchange_bound", "o3r_exchange_pack_dev", "o3r_exchange_merge_bb",
-    "o3r_exchange_pack", "o3r_exchange_merge", "o3r_set_defer_merge", "o3r_set_keep_frame_voxels", "o3r_last_batch_engine",
+    "o3r_voxel_grid", "o3r_blur_u8", "o3r_frame_mask", "o3r_disp_variance", "o3r_plane_fit", "o3r_sor", "o3r_last_batch_partials",
+    "o3r_set_keep_frame_voxels", "o3r_last_batch_engine",
     "o3r_comm_unique_id", "o3r_comm_init", "o3r_comm_attach", "o3r_comm_destroy", "o3r_exchange_cycle",
     "o3r_launch_count", "o3r_stream", "o3r_sync", "o3r_profile", "o3r_profile_read",
 ]
@@ -73,13 +73,6 @@ def load():
     L.o3r_sor.argtypes = [vp, vp, sz, C.c_int, C.c_double, vp, vp, C.POINTER(C.c_double)]
     L.o3r_disp_variance.argtypes = [vp, vp, sz, C.POINTER(C.c_double)]
     L.o3r_plane_fit.argtypes = [vp, vp, sz, vp, sz, vp, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_double)]
-    L.o3r_exchange_pack.argtypes = [vp, C.c_int, vp, sz, vp]
-    L.o3r_exchange_merge.argtypes = [vp, vp, sz]
-    L.o3r_exchange_bound.argtypes = [vp]
-    L.o3r_exchange_bound.restype = C.c_size_t
-    L.o3r_exchange_pack_dev.argtypes = [vp, C.c_int, vp, sz, vp]
-    L.o3r_exchange_merge_bb.argtypes = [vp, vp, sz, C.POINTER(C.c_int)]
-    L.o3r_set_defer_merge.argtypes = [vp, C.c_int]
     L.o3r_set_keep_frame_voxels.argtypes = [vp, C.c_int]
     L.o3r_last_batch_engine.argtypes = [vp]
     L.o3r_comm_unique_id.argtypes = [vp]

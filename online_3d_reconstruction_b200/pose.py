@@ -222,22 +222,7 @@ class Pose:
                                           coef.ctypes.data, 255, C.byref(n), C.byref(v)))
         return coef[:n.value].copy(), v.value
 
-    # -- multi-GPU exchange (device buffers are torch tensors owned by the caller) -----------------------------
-    def setDeferMerge(self, defer):
-        self._check(self._L.o3r_set_defer_merge(self._h, int(defer)))
-
-    def exchangePack(self, world, send_ptr, cap):
-        counts = np.zeros(world, dtype=np.uint32)
-        self._check(self._L.o3r_exchange_pack(self._h, world, send_ptr, cap, counts.ctypes.data))
-        return counts
-
-    def exchangeMerge(self, recv_ptr, n, bb=None):
-        if bb is None:
-            self._check(self._L.o3r_exchange_merge(self._h, recv_ptr, n))
-        else:
-            self._check(self._L.o3r_exchange_merge_bb(self._h, recv_ptr, n, (C.c_int * 6)(*[int(b) for b in bb])))
-
-    # the exchange inside the library (NCCL bound at run time): see include/o3r.h
+    # -- multi-GPU exchange inside the library (NCCL bound at run time): see include/o3r.h ----------------------
     @staticmethod
     def commUniqueId():
         """rank 0: the 128-byte NCCL id every rank passes to commInit (send it over any host channel)."""
@@ -256,10 +241,3 @@ class Pose:
     def exchangeCycle(self):
         """Collective, asynchronous: partial cells of the last cycle -> owners (grouped ncclSend/ncclRecv) -> merge."""
         self._check(self._L.o3r_exchange_cycle(self._h))
-
-    def exchangeBound(self):
-        return int(self._L.o3r_exchange_bound(self._h))
-
-    def exchangePackDevice(self, world, send_ptr, cap, info_ptr):
-        """Queues the pack on the context's stream; info_ptr = device buffer of world + 8 u32 (see o3r.h)."""
-        self._check(self._L.o3r_exchange_pack_dev(self._h, world, send_ptr, cap, info_ptr))

@@ -16,7 +16,7 @@ for p in (ROOT, os.path.join(ROOT, "tests")):
         sys.path.insert(0, p)
 
 import oracle_binding as ob  # noqa: E402
-from online_3d_reconstruction_b200 import abi, synth  # noqa: E402
+from online_3d_reconstruction_b200 import abi, exchange, synth  # noqa: E402
 from online_3d_reconstruction_b200.pose import Pose  # noqa: E402
 
 
@@ -58,6 +58,9 @@ def main():
                 single = S.downsamplePtCloud()
             union = np.concatenate(shards)
             ku, ks = keys_of(union, voxel), keys_of(single, voxel)
+            # every rank holds exactly the cells the host mirror of the device's owner hash assigns to it
+            assert np.array_equal(exchange.owner_of(ku, world), np.repeat(np.arange(world), [len(s) for s in shards])), \
+                "a cell sits on a rank the owner hash does not name"
             order = np.argsort(ku, kind="stable")
             union, ku = union[order], ku[order]
             assert len(np.unique(ku)) == len(ku), "ownership is not disjoint"

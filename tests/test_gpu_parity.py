@@ -3,7 +3,7 @@
 Bar (north_star): validity masks, voxel keys, per-voxel counts, colours and output ORDER bit-exact;
 coordinates / centroids within 1e-5 relative.  On one GPU the implementation is designed to be
 bit-exact for coordinates and centroids too (stable sort + in-order sums), and the tests assert that;
-the 1e-5 tolerance is only needed across ranks (test_exchange_two_ranks).
+the 1e-5 tolerance is only needed across ranks (tests/test_gpu_multirank.py).
 """
 import os
 
@@ -11,7 +11,7 @@ import numpy as np
 import pytest
 
 import oracle_binding as ob
-from online_3d_reconstruction_b200 import abi, exchange, synth
+from online_3d_reconstruction_b200 import abi, synth
 from online_3d_reconstruction_b200.pose import Pose
 
 pytestmark = pytest.mark.gpu
@@ -649,78 +649,3 @@ def test_full_resolution_properties_720p():
         assert not passthrough and np.all(counts == 1)
         _eq(again, sh)
 
-
-# -------------------------------------------------------------------------------------------- multi-GPU
-@pytest.mark.parametrize("api", ["sync", "dev"])
-@pytest.mark.parametrize("mode", [abi.MERGE_ACCUMULATE, abi.MERGE_ACCUMULATE_TILED])
-def test_exchange_two_ranks_equals_single_rank(mode, api):
-    """SURVEY §8e on one device: two contexts act as two ranks (frames f mod 2), exchange hash-partitioned
-    partial cells, and the union of their shards must equal the single-rank result: keys, counts and colours
-    exactly, centroids within 1e-5 (cross-rank partial sums reassociate)."""
-    torch = pytest.importorskip("torch")
-    keep = []
-    geom = SMALL4
-    p = abi.make_params(jump_pixels=1, voxel_size=0.05, min_points_per_voxel=1, merge_mode=mode, **geom)
-    cycles = [_frames(80, 6, geom["rows"], geom["cols"], keep=keep), _frames(81, 6, geom["rows"], geom["cols"], keep=keep, traj_start=6)]
-    with Pose(p) as S:
-        for frames in cycles:
-            S.createCycleClouds(frames)
-        single = S.downsamplePtCloud()
-    W = 2
-    ranks = [Pose(p) for _ in range(W)]
-    try:
-        for r in ranks:
-            r.setDeferMerge(True)
-        for frames in cycles:
-            sends, counts, bbs = [], [], []
-            for r, P in enumerate(ranks):
-                P.createCycleClouds(frames[r::W])
-                buf = torch.empty(len(frames) * P.max_points_per_frame * abi.CELL.itemsize // W + 64, dtype=torch.uint8, device="cuda")
-                if api == "sync":
-                    c = P.exchangePack(W, buf.data_ptr(), buf.numel() // abi.CELL.itemsize)
-                else:   # the round-trip-free entry points: header on the device, cell range passed to the merge
-                    assert 0 < P.exchangeBound() <= buf.numel() // abi.CELL.itemsize
-                    info = torch.zeros(W + 8, dtype=torch.int32, device="cuda")
-                    P.exchangePackDevice(W, buf.data_ptr(), buf.numel() // abi.CELL.itemsize, info.data_ptr())
-                    P.sync()
-                    h = info.cpu().numpy()
-                    c = h[:W].astype(np.uint32)
-                    assert int(h[W + 6]) == int(c.sum()) <= P.exchangeBound()
-                    bbs.append(h[W:W + 6])
-                sends.append(buf)
-                counts.append(c)
-            bb = None
-            if bbs:
-                bb = list(np.min([b[:3] for b in bbs], axis=0)) + list(np.max([b[3:] for b in bbs], axis=0))
-            for s, buf in enumerate(sends):   # the device buckets by the same hash the host mirror computes
-                sent = buf[:int(counts[s].sum()) * abi.CELL.itemsize].cpu().numpy().view(abi.CELL)
-                own = exchange.owner_of(sent["key"], W)
-                assert np.array_equal(own, np.repeat(np.arange(W), counts[s]))
-            for r, P in enumerate(ranks):
-                parts = []
-                for s in range(W):
-                    off = int(counts[s][:r].sum()) * abi.CELL.itemsize
-                    parts.append(sends[s][off:off + int(counts[s][r]) * abi.CELL.itemsize])
-                recv = torch.cat(parts)
-                torch.cuda.synchronize()
-                P.exchangeMerge(recv.data_ptr(), recv.numel() // abi.CELL.itemsize, bb)
-        shards = [P.downsamplePtCloud() for P in ranks]
-    finally:
-        for r in ranks:
-            r.close()
-    union = np.concatenate(shards)
-    leaf = (0.05, 0.05, 1000.0)
-    def keys_of(a):
-        sh = a.copy()
-        sh["z"] += np.float32(500)
-        return np.array([ob.cell_key(q["x"], q["y"], q["z"], leaf) for q in sh], dtype=np.uint64)
-    ku, ks = keys_of(union), keys_of(single)
-    order = np.argsort(ku, kind="stable")
-    union, ku = union[order], ku[order]
-    assert len(np.unique(ku)) == len(ku)            # disjoint ownership
-    assert np.array_equal(ku, ks)
-    assert np.array_equal(union["rgb"], single["rgb"])
-    for f, shift in (("x", 0.0), ("y", 0.0), ("z", 500.0)):
-        a, b = union[f].astype(np.float64) + shift, single[f].astype(np.float64) + shift
-        assert np.all(np.abs(a - b) <= 1e-5 * np.abs(b)), f
-    assert min(len(s) for s in shards) > 0.3 * len(single) / W
