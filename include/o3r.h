@@ -290,7 +290,26 @@ int o3r_set_keep_frame_voxels(o3r_ctx* ctx, int keep);
  * NCCL is loaded at run time (libnccl.so.2); o3r_comm_unique_id + o3r_comm_init create a communicator of the library's own
  * (the id travels by whatever channel the host has: MPI, a file, torch.distributed), o3r_comm_attach adopts an existing
  * ncclComm_t.  While a communicator is attached, o3r_frames_cloud* leaves the merge to o3r_exchange_cycle; after
- * o3r_comm_destroy the context merges its cycles itself again. */
+ * o3r_comm_destroy the context merges its cycles itself again.
+ *
+ * O3R_MERGE_RETAIN (ICP on) and dont_downsample shard differently: the points stay on the rank that made them.
+ *   - o3r_comm_init / o3r_comm_attach need an empty resident cloud (O3R_ERR_INVALID otherwise); slot_cells is checked but
+ *     not used, no slot buffers are allocated.
+ *   - Every o3r_frames_cloud* call appends the rank's frames (f mod world == rank, in order) to its local cloud and counts
+ *     as one cycle, so all ranks make the same number of calls; n = 0 is a cycle in which this rank has no frame.
+ *   - o3r_cloud_transform stays local: every rank applies the same T at the same point of the call sequence.
+ *   - o3r_exchange_cycle is a no-op returning O3R_OK; o3r_cloud_append returns O3R_ERR_UNSUPPORTED (appended points have
+ *     no place in the global frame order); o3r_cloud_size and o3r_cloud_clear stay local (all ranks clear together).
+ *   - o3r_cloud_downsample / o3r_cloud_downsample_dev are collectives: the global bbox is all-reduced, every point travels
+ *     once to the owner of its combined-grid cell (hash64(absolute cell key) mod world) with an order tag (cycle, global
+ *     frame), and the owner sums its cells' points in cloud_big order.  Each rank returns the cells it owns, ascending
+ *     voxel index, min_points_per_voxel applied; the union ordered by key is the single-GPU output bit for bit, centroids
+ *     included.  On a pass-through grid (PCL's int32 guard on the GLOBAL bbox) and with dont_downsample every rank returns
+ *     its own points, which, interleaved back in frame order, are the single-GPU output.  The result is kept until the local
+ *     cloud changes (frames, transform, clear): a second call (the cap = 0 query, then the fill) does not communicate.
+ *     A rank that fails takes part in every agreement step, so all ranks return an error and none is left waiting.
+ *     Limits: fewer than 2^32 points per rank and per owner; bits(cycles) + bits(frames per cycle) <= 32 (the order tag),
+ *     beyond which every rank returns O3R_ERR_UNSUPPORTED; clear the cloud to start the count again. */
 #define O3R_COMM_ID_BYTES 128
 int o3r_comm_unique_id(void* id_out /* O3R_COMM_ID_BYTES, rank 0 */);
 int o3r_comm_init(o3r_ctx* ctx, int world, int rank, const void* id, size_t slot_cells);   /* collective */

@@ -87,6 +87,7 @@ struct NcclApi {
     ncclResult_t (*GroupEnd)() = nullptr;
     ncclResult_t (*Send)(const void*, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
     ncclResult_t (*Recv)(void*, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
+    ncclResult_t (*AllReduce)(const void*, void*, size_t, ncclDataType_t, ncclRedOp_t, ncclComm_t, cudaStream_t) = nullptr;
     const char* (*GetErrorString)(ncclResult_t) = nullptr;
     std::string err;
 };
@@ -108,6 +109,7 @@ NcclApi* nccl_api() {
         api.GroupEnd = reinterpret_cast<decltype(api.GroupEnd)>(sym("ncclGroupEnd"));
         api.Send = reinterpret_cast<decltype(api.Send)>(sym("ncclSend"));
         api.Recv = reinterpret_cast<decltype(api.Recv)>(sym("ncclRecv"));
+        api.AllReduce = reinterpret_cast<decltype(api.AllReduce)>(sym("ncclAllReduce"));
         api.GetErrorString = reinterpret_cast<decltype(api.GetErrorString)>(sym("ncclGetErrorString"));
     });
     return &api;
@@ -123,7 +125,16 @@ NcclApi* nccl_api() {
 int comm_setup(o3r_ctx* ctx, int world, int rank, size_t slot_cells) {
     if (world < 1 || world > 256 || rank < 0 || rank >= world || slot_cells == 0 || slot_cells >= (1ull << 31))
         return ctx->fail(O3R_ERR_INVALID, "bad communicator arguments");
-    if (ctx->retain()) return ctx->fail(O3R_ERR_UNSUPPORTED, "the exchange needs an accumulating merge mode");
+    if (ctx->retain()) {   // RETAIN / dont_downsample: the points stay where they are made (host_retain.cuh); no slots
+        if (ctx->n_cloud) return ctx->fail(O3R_ERR_INVALID, "a sharded retained cloud starts empty: attach the communicator before the first cycle");
+        CU(ctx->rt_agree.ensure(((size_t)16 + 4 * (size_t)world + 4) * 4));
+        CU(ctx->seg2.ensure(16));   // (these four are what the downsample's agreement steps touch: they never fail later)
+        CU(ctx->bbox.ensure(6 * 4));
+        CU(ctx->grids.ensure(sizeof(GridParams)));
+        ctx->world = world; ctx->rank = rank; ctx->slot_cap = (uint32_t)slot_cells;
+        ctx->rt_reset();
+        return O3R_OK;
+    }
     ctx->world = world; ctx->rank = rank; ctx->slot_cap = (uint32_t)slot_cells;
     const size_t bytes = (size_t)world * (slot_cells + 1) * sizeof(o3r_cell);
     CU(ctx->x_send.ensure(bytes));

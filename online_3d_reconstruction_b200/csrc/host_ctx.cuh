@@ -184,6 +184,16 @@ struct o3r_ctx {
     uint32_t slot_cap = 0;            // cells per (source, destination) slot
     DevBuf x_send, x_recv, x_list;
     bool x_pending_check = false;
+    // ... and its RETAIN form (host_retain.cuh): the points stay on the rank that made them; per appended frame its first point
+    // in the local cloud, its cycle and its global frame index (the order tag of cloud_big order); the last collective result
+    struct RtFrame { size_t first; uint32_t cycle, frame; };
+    std::vector<RtFrame> rt_frames;
+    uint32_t rt_cycles = 0;           // o3r_frames_cloud* calls since the communicator came (or the last clear)
+    bool rt_valid = false;            // rt_out holds the result for the current local cloud
+    size_t rt_m = 0;
+    size_t rt_ftab_n = 0;             // frame records already in rt_ftab
+    DevBuf rt_agree, rt_ftab, rt_tags, rt_send, rt_recv, rt_pts, rt_out;
+    void rt_reset() { rt_frames.clear(); rt_cycles = 0; rt_valid = false; rt_m = 0; rt_ftab_n = 0; }
     bool keep_frame_voxels = false;   // parity probe: the bucket engine also writes every per-frame voxel centroid (any order)
     size_t last_partials = 0;
     bool last_has_partials = false;

@@ -198,6 +198,10 @@ int frames_cloud_impl(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_typ
     ctx->busy_set = -1;
     auto now = [] { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
     const double tr0 = now();
+    // sharded RETAIN: every call is one cycle of the order tag, whatever it holds (n = 0: this rank has no frame in it)
+    const bool rt_shard = opt.merge && ctx->comm && ctx->retain();
+    const uint32_t rt_cycle = ctx->rt_cycles;
+    if (rt_shard) { ++ctx->rt_cycles; ctx->rt_valid = false; }
     if (n <= 0) { ctx->last_n = 0; ctx->last_total = 0; return O3R_OK; }
     if (n > 65535) return ctx->fail(O3R_ERR_INVALID, "too many frames in one batch");
     if (disp_type < 0 || disp_type > 3) return ctx->fail(O3R_ERR_INVALID, "bad disp_type");
@@ -606,9 +610,18 @@ int frames_cloud_impl(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_typ
     ctx->last_total = ctx->last_off[n];
     if (frame_counts)
         for (int i = 0; i < n; ++i) frame_counts[i] = ctx->last_off[i + 1] - ctx->last_off[i];
-    if (!opt.merge || ctx->comm) return O3R_OK;   // with a communicator, o3r_exchange_cycle merges the cycle
+    if (!opt.merge || (ctx->comm && !ctx->retain())) return O3R_OK;   // with a communicator, o3r_exchange_cycle merges the cycle
     const float4* outp = ctx->last_is_vox ? ctx->vox.as<float4>() : ctx->pts.as<float4>();
-    if (ctx->retain()) return cloud_append_dev(ctx, outp, ctx->last_total);
+    if (ctx->retain()) {
+        const size_t base = ctx->n_cloud;
+        const int rca = cloud_append_dev(ctx, outp, ctx->last_total);
+        if (rca) return rca;
+        if (rt_shard)   // rank r's frame i is the cycle's frame i * world + r
+            for (int i = 0; i < n; ++i)
+                if (ctx->last_off[i + 1] > ctx->last_off[i])
+                    ctx->rt_frames.push_back({base + ctx->last_off[i], rt_cycle, (uint32_t)i * (uint32_t)ctx->world + (uint32_t)ctx->rank});
+        return O3R_OK;
+    }
     const int* bbp = ctx->last_has_cellbb ? ctx->last_cellbb : nullptr;
     if ((use_bucket || use_tile) && ctx->last_partials == 0) return O3R_OK;   // nothing valid in the whole batch
     const int rcm = ctx->last_has_partials ? acc_merge_cells(ctx, ctx->partials.as<o3r_cell>(), ctx->last_partials, bbp)

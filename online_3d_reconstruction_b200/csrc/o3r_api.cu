@@ -6,6 +6,7 @@
 #include "host_sor.cuh"
 #include "host_frames.cuh"
 #include "host_comm.cuh"
+#include "host_retain.cuh"
 
 
 // =====================================================================================================================
@@ -138,7 +139,8 @@ void o3r_destroy(o3r_ctx* ctx) {
                       &ctx->res_acc[0], &ctx->res_acc[1], &ctx->res_rgb[0], &ctx->res_rgb[1], &ctx->ckey, &ctx->cacc,
                       &ctx->crgb, &ctx->partials, &ctx->pr_status, &ctx->bk_frames, &ctx->bk_counts, &ctx->bk_nl, &ctx->bk_pts, &ctx->bk_pos,
                       &ctx->bk_status, &ctx->bk_misc, &ctx->bk_stray, &ctx->tv_tiles, &ctx->tv_misc, &ctx->tv_scratch, &ctx->x_send, &ctx->x_recv, &ctx->x_list, &ctx->sor_hard, &ctx->sor_pts, &ctx->sor_off, &ctx->sor_dist, &ctx->sor_grids,
-                      &ctx->sor_pgrids, &ctx->sor_rows, &ctx->sor_thr, &ctx->sor_skeys, &ctx->sor_svals, &ctx->sor_cnt, &ctx->sor_cntoff, &ctx->new_cnt, &ctx->new_off, &ctx->new_keys, &ctx->okeys, &ctx->cloud};
+                      &ctx->sor_pgrids, &ctx->sor_rows, &ctx->sor_thr, &ctx->sor_skeys, &ctx->sor_svals, &ctx->sor_cnt, &ctx->sor_cntoff, &ctx->new_cnt, &ctx->new_off, &ctx->new_keys, &ctx->okeys, &ctx->cloud,
+                      &ctx->rt_agree, &ctx->rt_ftab, &ctx->rt_tags, &ctx->rt_send, &ctx->rt_recv, &ctx->rt_pts, &ctx->rt_out};
     for (DevBuf* b : bufs) b->release();
     for (auto& r : ctx->prof) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
     for (auto e : ctx->ev_pool) cudaEventDestroy(e);
@@ -306,6 +308,7 @@ int o3r_cloud_transform(o3r_ctx* ctx, const float T[16]) {
     if (!ctx->retain())
         return ctx->fail(O3R_ERR_UNSUPPORTED,
                          "o3r_cloud_transform needs O3R_MERGE_RETAIN: accumulated cells cannot be re-binned");
+    ctx->rt_valid = false;   // (on every rank of a sharded cloud, even one without points: the ranks stay in step)
     if (ctx->n_cloud == 0) return O3R_OK;
     CU(ctx->tmat.ensure(64));
     { int rcu = upload_small(ctx, ctx->tmat.p, T, 48); if (rcu) return rcu; }
@@ -318,6 +321,8 @@ int o3r_cloud_append(o3r_ctx* ctx, const o3r_point* pts, size_t n) {
     if (!ctx || (n && !pts)) return O3R_ERR_INVALID;
     std::lock_guard<std::mutex> lk(ctx->mu);
     CU(cudaSetDevice(ctx->p.device));
+    if (ctx->comm && ctx->retain())
+        return ctx->fail(O3R_ERR_UNSUPPORTED, "o3r_cloud_append on a sharded retained cloud: appended points have no place in the frame order");
     if (n == 0) return O3R_OK;
     if (ctx->retain()) {
         CU(ctx->cloud.ensure((ctx->n_cloud + n) * 16, ctx->st, ctx->n_cloud * 16));
@@ -352,6 +357,7 @@ int o3r_cloud_clear(o3r_ctx* ctx) {
     CU(cudaSetDevice(ctx->p.device));
     CU(cudaStreamSynchronize(ctx->st));
     ctx->n_cloud = 0; ctx->n_res_ub = 0; ctx->n_res_exact = true;
+    ctx->rt_reset();
     ZERO(ctx->counters.as<uint32_t>() + CNT_NRES, 4);
     return O3R_OK;
 }
@@ -402,6 +408,7 @@ static int cloud_downsample_dev(o3r_ctx* ctx, const float4** res, size_t* m, boo
         return O3R_OK;
     }
     uint32_t* cnt = ctx->counters.as<uint32_t>();
+    if (ctx->retain() && ctx->comm) return retain_downsample_sharded(ctx, res, m);   // collective (host_retain.cuh)
     if (ctx->retain()) {  // one-shot pcl::VoxelGrid over cloud_big, exactly pose_functions.cpp:1654-1709
         if (ctx->n_cloud == 0) return O3R_OK;
         CU(ctx->ckey.ensure(ctx->n_cloud * 16));   // result points (<= n_cloud)
@@ -600,6 +607,9 @@ int o3r_comm_destroy(o3r_ctx* ctx) {
     if (ctx->comm && ctx->comm_owned) NC(N->CommDestroy((ncclComm_t)ctx->comm));
     ctx->comm = nullptr; ctx->comm_owned = false; ctx->world = 1; ctx->rank = 0;
     ctx->x_send.release(); ctx->x_recv.release(); ctx->x_list.release();
+    ctx->rt_reset();
+    DevBuf* rt_bufs[] = {&ctx->rt_agree, &ctx->rt_ftab, &ctx->rt_tags, &ctx->rt_send, &ctx->rt_recv, &ctx->rt_pts, &ctx->rt_out};
+    for (DevBuf* b : rt_bufs) b->release();
     return O3R_OK;
 }
 
@@ -607,6 +617,7 @@ int o3r_exchange_cycle(o3r_ctx* ctx) {
     if (!ctx) return O3R_ERR_INVALID;
     std::lock_guard<std::mutex> lk(ctx->mu);
     CU(cudaSetDevice(ctx->p.device));
+    if (ctx->comm && ctx->retain()) return O3R_OK;   // RETAIN: the points stay where they were made; o3r_cloud_downsample exchanges
     return exchange_cycle_impl(ctx);
 }
 

@@ -24,3 +24,22 @@ def owner_of(keys, world):
 def shard_frames(n_frames, rank, world):
     """Indices of the cycle's frames this rank reconstructs (frame f -> rank f mod P)."""
     return list(range(rank, n_frames, world))
+
+
+def unshard_points(shards, counts, world):
+    """Sharded RETAIN: the ranks' own points (pass-through grid, dont_downsample) -> the single-GPU cloud_big order.
+
+    shards[r] = rank r's points in its local order; counts[r] = its per-cycle arrays of per-frame point counts (what
+    createCycleClouds returned, an empty array for a cycle without frames).  Cycle by cycle, global frame f = i*world + r
+    is rank r's i-th frame of that cycle, so the frames are taken in order f = 0, 1, ... from rank f mod world."""
+    at = [0] * world
+    parts = []
+    for s in range(len(counts[0])):
+        n_frames = sum(len(counts[r][s]) for r in range(world))
+        for f in range(n_frames):
+            r, i = f % world, f // world
+            c = int(counts[r][s][i])
+            parts.append(shards[r][at[r]:at[r] + c])
+            at[r] += c
+    assert all(at[r] == len(shards[r]) for r in range(world)), "counts do not cover the shards"
+    return np.concatenate(parts) if parts else np.zeros(0, dtype=shards[0].dtype)
