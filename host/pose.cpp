@@ -341,6 +341,17 @@ int Pose::run() {
     const double app_start_time = now_s();
     o3r_ctx* ctx = make_ctx(*this, O3R_MERGE_ACCUMULATE, seq_len);
     if (!ctx) return 1;
+    // --preview (pose.cpp:638-674 shows a downsampled copy of cloud_big every cycle): the headless equivalent keeps a
+    // key-sorted copy of the combined grid, updated each cycle from the cells that cycle changed, and rewrites preview.ply
+    const bool do_preview = preview && !dont_downsample;
+    if (preview && dont_downsample)
+        cout << "--preview needs the combined grid, which --dont_downsample skips: no preview.ply is written" << endl;
+    if (do_preview && o3r_cloud_track_changes(ctx, 1) != O3R_OK) {
+        cerr << "o3r_cloud_track_changes: " << o3r_last_error(ctx) << endl; o3r_destroy(ctx); return 1;
+    }
+    std::map<uint64_t, o3r_point> preview_map;
+    vector<o3r_point> chg_pts;
+    vector<uint64_t> chg_keys;
     vector<o3r_point> hexPos_MAVLink, hexPos_FM;
     vector<int> accepted_nums;
     int current_idx = 0, cycle = 0;
@@ -422,6 +433,20 @@ int Pose::run() {
         const double t4 = now_s();
         cout << "\n\nPoint Cloud Creation time: " << (t4 - t2) << " sec" << endl;
         log_file << "\nPoint Cloud Creation time:\t\t\t" << (t4 - t2) << " sec" << endl;
+        if (do_preview) {
+            size_t m = 0;
+            int rc = o3r_cloud_changes(ctx, nullptr, nullptr, nullptr, 0, &m);
+            chg_pts.resize(std::max<size_t>(m, 1)); chg_keys.resize(std::max<size_t>(m, 1));
+            if (!rc) rc = o3r_cloud_changes(ctx, chg_pts.data(), chg_keys.data(), nullptr, chg_pts.size(), &m);
+            if (rc) { cerr << "o3r_cloud_changes: " << o3r_last_error(ctx) << endl; o3r_destroy(ctx); return 1; }
+            for (size_t i = 0; i < m; ++i) preview_map[chg_keys[i]] = chg_pts[i];
+            vector<o3r_point> view;
+            view.reserve(preview_map.size());
+            for (const auto& kv : preview_map) view.push_back(kv.second);
+            host::save_ply_binary(folder + "preview.ply", view.data(), view.size());
+            for (ostream* o : {(ostream*)&cout, (ostream*)&log_file})
+                *o << "Preview cells changed/total: " << m << "/" << preview_map.size() << endl;
+        }
         cycle++;
         cout << "\nCycle time: " << (now_s() - t0) << " sec" << endl;
         log_file << "Cycle time:\t\t\t\t\t" << (now_s() - t0) << " sec" << endl;

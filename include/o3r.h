@@ -218,6 +218,35 @@ int o3r_cloud_downsample_dev(o3r_ctx* ctx, const o3r_point** dev_out, size_t* n_
 int o3r_cloud_size(o3r_ctx* ctx, size_t* n);
 int o3r_cloud_clear(o3r_ctx* ctx);
 
+/* Change tracking of the resident cloud (O3R_MERGE_ACCUMULATE, _TILED, _FUSED; with or without a communicator): a
+ * consumer that keeps a copy of the combined grid (a viewer, a link to a ground station, the next pipeline stage) reads
+ * after each cycle only the cells that cycle touched instead of the whole map.  Upserting the records by key into a
+ * key-sorted map keeps that map equal to o3r_cloud_downsample's output, order included.
+ *   - Tracking.  enable = 1 starts tracking, or restarts it when it is on; the next o3r_cloud_changes then returns every
+ *     cell the downsample would emit (the full state: how a consumer that joins late or reconnects starts).  enable = 0
+ *     stops tracking and frees its buffers.  Tracking is off by default; while it is off it costs nothing.  While it is
+ *     on, every merged cycle adds four small kernel launches and nothing is read back.
+ *   - Records.  A call returns every cell whose point count grew since the last consuming call and whose count is
+ *     >= min_points_per_voxel, and no other cell (except the full state after an enable), in ascending cell key (=
+ *     ascending voxel index).  Each record is bit-identical to that cell's record in o3r_cloud_downsample.  keys (the
+ *     absolute cell key, as o3r_voxel_grid reports it) and counts (points in the cell) are optional; either may be NULL.
+ *   - Query, then fill.  out = NULL with cap = 0 queries *n_out and consumes nothing (a second query returns the same
+ *     records).  A call that delivers the records and returns O3R_OK consumes them; O3R_ERR_CAPACITY consumes nothing and
+ *     still reports *n_out.  A merge, clear or enable between the query and the fill makes the fill return the grown set.
+ *     The query's result is kept until the tracked state changes, so query-then-fill computes it once.
+ *   - o3r_cloud_changes_dev: the records stay in device buffers owned by the context, valid until the next call on it;
+ *     the call consumes on return.  Any of the three pointers may be NULL.
+ *   - o3r_cloud_clear empties the pending set; tracking stays as it was (a consumer that clears the cloud clears its map).
+ *   - With a communicator each rank returns the changes of the cells it owns; the union over ranks is the global change
+ *     set.  After an exchange slot overflow o3r_cloud_changes fails with O3R_ERR_CAPACITY (the next o3r_cloud_downsample
+ *     still reports the overflow too).
+ *   - O3R_MERGE_RETAIN and dont_downsample: O3R_ERR_UNSUPPORTED from all three calls (every transform moves every point,
+ *     so there is no cheap change set).  o3r_cloud_changes[_dev] with tracking off: O3R_ERR_INVALID. */
+int o3r_cloud_track_changes(o3r_ctx* ctx, int enable);
+int o3r_cloud_changes(o3r_ctx* ctx, o3r_point* out, uint64_t* keys, uint32_t* counts, size_t cap, size_t* n_out);
+int o3r_cloud_changes_dev(o3r_ctx* ctx, const o3r_point** dev_out, const uint64_t** dev_keys,
+                          const uint32_t** dev_counts, size_t* n_out);
+
 /* ---- stand-alone stages (parity probes; same kernels as above) ------------------------------- */
 
 /* pcl::VoxelGrid<PointXYZRGB>::filter on a host cloud: leaf (lx,ly,lz) as PCL's setLeafSize floats,

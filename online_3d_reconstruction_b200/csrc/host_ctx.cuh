@@ -78,8 +78,8 @@ struct FillQueue {
 };
 
 enum { CNT_PTS = 0, CNT_VOX = 1, CNT_CYC = 2, CNT_NEW = 3, CNT_EMIT = 4, CNT_NEWSCAN = 5, CNT_BASE = 6, CNT_NRES = 7, CNT_ZERO = 8, CNT_PART = 9, CNT_PARTCHUNK = 10,
-       CNT_XFLAG = 11, CNT_XRECV = 12,
-       CNT_CELLBB = 16, CNT_N = 32 };
+       CNT_XFLAG = 11, CNT_XRECV = 12, CNT_CHG0 = 13 /* and 14: the pending set's count, one per buffer */,
+       CNT_CELLBB = 16, CNT_CHGOUT = 22, CNT_CHGERR = 23, CNT_N = 32 };
 
 }  // namespace
 
@@ -194,6 +194,17 @@ struct o3r_ctx {
     size_t rt_ftab_n = 0;             // frame records already in rt_ftab
     DevBuf rt_agree, rt_ftab, rt_tags, rt_send, rt_recv, rt_pts, rt_out;
     void rt_reset() { rt_frames.clear(); rt_cycles = 0; rt_valid = false; rt_m = 0; rt_ftab_n = 0; }
+    // change tracking of the resident cloud (host_changes.cuh): the pending set D (sorted unique absolute cell keys,
+    // double-buffered, count in counters[CNT_CHG0 + chg_cur], host upper bound chg_ub) or "everything" after an enable;
+    // the last emitted result (chg_m records in chg_out / chg_okeys / chg_ocnt), valid until the tracked state changes
+    bool chg_on = false, chg_all = false, chg_valid = false;
+    int chg_cur = 0;
+    size_t chg_ub = 0, chg_m = 0;
+    DevBuf chg_keys[2], chg_cnt, chg_off, chg_part, chg_pos, chg_out, chg_okeys, chg_ocnt;
+    void chg_release() {
+        DevBuf* b[] = {&chg_keys[0], &chg_keys[1], &chg_cnt, &chg_off, &chg_part, &chg_pos, &chg_out, &chg_okeys, &chg_ocnt};
+        for (DevBuf* x : b) x->release();
+    }
     bool keep_frame_voxels = false;   // parity probe: the bucket engine also writes every per-frame voxel centroid (any order)
     size_t last_partials = 0;
     bool last_has_partials = false;

@@ -6,6 +6,9 @@
 
 namespace {
 
+int chg_reserve(o3r_ctx* ctx, size_t n_cyc_ub);   // change tracking (host_changes.cuh)
+int chg_cycle(o3r_ctx* ctx, size_t n_cyc_ub);
+
 // ---- engine 2: merge `n` items (points or partial cells) into the resident accumulators --------------------------
 inline int bits_for(long long range) { int b = 0; while ((1ll << b) <= range) ++b; return b; }
 
@@ -161,6 +164,7 @@ int acc_apply_cycle(o3r_ctx* ctx) {
         CU(ctx->res_rgb[nxt].ensure(cells * 16));
     }
     CU(ctx->new_keys.ensure(n_cyc_ub * 8));
+    { int rc = chg_reserve(ctx, n_cyc_ub); if (rc) return rc; }
     if (tr.on) fprintf(stderr, "[o3r trace] n_res_ub %zu n_cyc_ub %zu\n", ctx->n_res_ub, n_cyc_ub);
     tr.mark("ensures");
     LAUNCH(k_acc_update, tiles, kThreads, 0, cnt + CNT_CYC, ctx->cacc.as<float4>(), ctx->crgb.as<uint4>(),
@@ -184,7 +188,7 @@ int acc_apply_cycle(o3r_ctx* ctx) {
     CU(cudaMemcpyAsync(ctx->h_nres, cnt + CNT_NRES, 4, cudaMemcpyDeviceToHost, ctx->st));
     CU(cudaEventRecord(ctx->ev_nres, ctx->st));
     tr.mark("launches");
-    return O3R_OK;
+    return chg_cycle(ctx, n_cyc_ub);
 }
 
 int acc_merge_points(o3r_ctx* ctx, const float4* pts, size_t n, const int* bb) {

@@ -7,6 +7,7 @@
 #include "host_frames.cuh"
 #include "host_comm.cuh"
 #include "host_retain.cuh"
+#include "host_changes.cuh"
 
 
 // =====================================================================================================================
@@ -142,6 +143,7 @@ void o3r_destroy(o3r_ctx* ctx) {
                       &ctx->sor_pgrids, &ctx->sor_rows, &ctx->sor_thr, &ctx->sor_skeys, &ctx->sor_svals, &ctx->sor_cnt, &ctx->sor_cntoff, &ctx->new_cnt, &ctx->new_off, &ctx->new_keys, &ctx->okeys, &ctx->cloud,
                       &ctx->rt_agree, &ctx->rt_ftab, &ctx->rt_tags, &ctx->rt_send, &ctx->rt_recv, &ctx->rt_pts, &ctx->rt_out};
     for (DevBuf* b : bufs) b->release();
+    ctx->chg_release();
     for (auto& r : ctx->prof) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
     for (auto e : ctx->ev_pool) cudaEventDestroy(e);
     if (ctx->h_counters) cudaFreeHost(ctx->h_counters);
@@ -359,6 +361,7 @@ int o3r_cloud_clear(o3r_ctx* ctx) {
     ctx->n_cloud = 0; ctx->n_res_ub = 0; ctx->n_res_exact = true;
     ctx->rt_reset();
     ZERO(ctx->counters.as<uint32_t>() + CNT_NRES, 4);
+    if (ctx->chg_on) chg_reset(ctx, false);
     return O3R_OK;
 }
 
@@ -487,6 +490,60 @@ int o3r_cloud_downsample_dev(o3r_ctx* ctx, const o3r_point** dev_out, size_t* n_
     if (pending) { rc = downsample_finish(ctx, n_out); if (rc) return rc; }
     else CU(cudaStreamSynchronize(ctx->st));
     if (dev_out) *dev_out = reinterpret_cast<const o3r_point*>(res);
+    return O3R_OK;
+}
+
+int o3r_cloud_track_changes(o3r_ctx* ctx, int enable) {
+    if (!ctx) return O3R_ERR_INVALID;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    CU(cudaSetDevice(ctx->p.device));
+    { int rc = chg_check_mode(ctx); if (rc) return rc; }
+    if (!enable) {
+        CU(cudaStreamSynchronize(ctx->st));   // (queued unions may still read or write the buffers)
+        ctx->chg_on = ctx->chg_all = ctx->chg_valid = false;
+        ctx->chg_ub = ctx->chg_m = 0;
+        ctx->chg_release();
+        return O3R_OK;
+    }
+    ctx->chg_on = true;
+    chg_reset(ctx, true);   // the next read returns the full state
+    return O3R_OK;
+}
+
+int o3r_cloud_changes(o3r_ctx* ctx, o3r_point* out, uint64_t* keys, uint32_t* counts, size_t cap, size_t* n_out) {
+    if (!ctx || !n_out) return O3R_ERR_INVALID;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    CU(cudaSetDevice(ctx->p.device));
+    *n_out = 0;
+    int rc = chg_compute(ctx);
+    if (rc) return rc;
+    const size_t m = ctx->chg_m;
+    *n_out = m;
+    if (!out && cap == 0) return O3R_OK;   // size query: nothing consumed
+    if (cap < m) return ctx->fail(O3R_ERR_CAPACITY, "output buffer too small");
+    if (m) {
+        if (out) CU(cudaMemcpyAsync(out, ctx->chg_out.p, m * 16, cudaMemcpyDeviceToHost, ctx->st));
+        if (keys) CU(cudaMemcpyAsync(keys, ctx->chg_okeys.p, m * 8, cudaMemcpyDeviceToHost, ctx->st));
+        if (counts) CU(cudaMemcpyAsync(counts, ctx->chg_ocnt.p, m * 4, cudaMemcpyDeviceToHost, ctx->st));
+        CU(cudaStreamSynchronize(ctx->st));
+    }
+    chg_reset(ctx, false);   // delivered: nothing is pending any more
+    return O3R_OK;
+}
+
+int o3r_cloud_changes_dev(o3r_ctx* ctx, const o3r_point** dev_out, const uint64_t** dev_keys, const uint32_t** dev_counts,
+                          size_t* n_out) {
+    if (!ctx || !n_out) return O3R_ERR_INVALID;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    CU(cudaSetDevice(ctx->p.device));
+    *n_out = 0;
+    int rc = chg_compute(ctx);
+    if (rc) return rc;
+    *n_out = ctx->chg_m;
+    if (dev_out) *dev_out = ctx->chg_out.as<const o3r_point>();
+    if (dev_keys) *dev_keys = ctx->chg_okeys.as<const uint64_t>();
+    if (dev_counts) *dev_counts = ctx->chg_ocnt.as<const uint32_t>();
+    chg_reset(ctx, false);   // (the records stay in the context's buffers until the next call)
     return O3R_OK;
 }
 

@@ -802,6 +802,15 @@ __global__ void __launch_bounds__(kThreads) k_acc_emit_cnt(const uint32_t* __res
     if (threadIdx.x == 0) cnt[t] = s_c;
 }
 
+// one cell's output record from its accumulators {sx, sy, sz + 500, n} and colour sums: the one place this arithmetic lives
+// (k_acc_emit and the change set's k_chg_emit both call it, so their records cannot drift apart)
+__device__ __forceinline__ float4 acc_centroid(const float4 a, const uint4 c) {
+    const float fn = (float)__float_as_uint(a.w);
+    const uint32_t rgb = ((uint32_t)__fdiv_rn((float)c.x, fn) << 16) | ((uint32_t)__fdiv_rn((float)c.y, fn) << 8) |
+                         (uint32_t)__fdiv_rn((float)c.z, fn);
+    return make_float4(__fdiv_rn(a.x, fn), __fdiv_rn(a.y, fn), __fsub_rn(__fdiv_rn(a.z, fn), 500.0f), __uint_as_float(rgb));
+}
+
 __global__ void __launch_bounds__(kThreads) k_acc_emit(const uint32_t* __restrict__ n_res_ptr, const float4* __restrict__ res_acc,
                                                        const uint4* __restrict__ res_rgb, uint32_t min_points,
                                                        const uint32_t* __restrict__ off, float4* __restrict__ out) {
@@ -820,13 +829,7 @@ __global__ void __launch_bounds__(kThreads) k_acc_emit(const uint32_t* __restric
     for (int j = 0; j < 4; ++j) {
         if (!(flags & (1u << j))) continue;
         const uint32_t i = t * kTileV + threadIdx.x * 4 + j;
-        const float4 a = res_acc[i];
-        const uint4 c = res_rgb[i];
-        const float fn = (float)__float_as_uint(a.w);
-        const uint32_t rgb = ((uint32_t)__fdiv_rn((float)c.x, fn) << 16) | ((uint32_t)__fdiv_rn((float)c.y, fn) << 8) |
-                             (uint32_t)__fdiv_rn((float)c.z, fn);
-        out[o++] = make_float4(__fdiv_rn(a.x, fn), __fdiv_rn(a.y, fn), __fsub_rn(__fdiv_rn(a.z, fn), 500.0f),
-                               __uint_as_float(rgb));
+        out[o++] = acc_centroid(res_acc[i], res_rgb[i]);
     }
 }
 

@@ -178,6 +178,33 @@ class Pose:
         self._check(self._L.o3r_cloud_downsample_dev(self._h, C.byref(ptr), C.byref(n)))
         return ptr.value, n.value
 
+    def trackCloudChanges(self, enable=True):
+        """Change tracking of the resident cloud (accumulate modes) on / off.  Enabling (or re-enabling) makes the next
+        cloudChanges() return the full state; disabling frees the tracking buffers."""
+        self._check(self._L.o3r_cloud_track_changes(self._h, int(enable)))
+
+    def cloudChanges(self):
+        """The cells whose point count grew since the last call (every cell after trackCloudChanges), count >=
+        min_points_per_voxel, ascending cell key -> (points, keys u64, counts u32).  Upserting them by key into a
+        key-sorted map keeps it equal to downsamplePtCloud(), bit for bit.  Consumes the changes."""
+        n = C.c_size_t(0)
+        self._check(self._L.o3r_cloud_changes(self._h, None, None, None, 0, C.byref(n)))
+        cap = max(1, n.value)
+        out = np.empty(cap, dtype=abi.POINT)
+        keys = np.empty(cap, dtype=np.uint64)
+        counts = np.empty(cap, dtype=np.uint32)
+        self._check(self._L.o3r_cloud_changes(self._h, out.ctypes.data, keys.ctypes.data, counts.ctypes.data, cap,
+                                              C.byref(n)))
+        k = n.value
+        return out[:k], keys[:k], counts[:k]
+
+    def cloudChangesDevice(self):
+        """Same as cloudChanges but the records stay in device memory owned by the context (valid until the next call on
+        it) -> (points pointer, keys pointer, counts pointer, n).  Consumes the changes."""
+        pts, keys, counts, n = C.c_void_p(), C.c_void_p(), C.c_void_p(), C.c_size_t(0)
+        self._check(self._L.o3r_cloud_changes_dev(self._h, C.byref(pts), C.byref(keys), C.byref(counts), C.byref(n)))
+        return pts.value, keys.value, counts.value, n.value
+
     # -- stand-alone stages --------------------------------------------------------------------------------
     def voxelGrid(self, pts, leaf, min_points=0):
         """pcl::VoxelGrid on a host cloud -> (points, keys u64, counts u32, passthrough)."""
