@@ -1,11 +1,24 @@
 // host_bucket.cuh — host side of the fused bucket engine (bucket.cuh): per-frame bucket grids from a conservative bound of
-// the frame's world bbox, buffer sizing, the launch sequence of one chunk of frames
+// the frame's world bbox, buffer sizing, the launch sequence of one chunk of frames, the read-back and the verdict on it, and
+// the steps both fused engines share (host_tile.cuh includes this file)
 // (host side of libo3r.so; included by o3r_api.cu, one translation unit)
 #pragma once
 
 #include "host_merge.cuh"
 
 namespace {
+
+// what a fused engine makes of its batch once the read-back has landed
+enum class Verdict { ACCEPT, RERUN, NEXT_ENGINE };
+
+// the batch's fills and sizing common to both fused engines (after the engine's own buffers are sized)
+int fused_prepare(o3r_ctx* ctx, size_t cap_batch) {
+    if (ctx->keep_frame_voxels) CU(ctx->vox.ensure(cap_batch * 16));
+    FILL(ctx->counters.as<uint32_t>() + CNT_CELLBB, 24, FILL_CELLBB);
+    ZERO(ctx->counters.as<uint32_t>() + CNT_PART, 8);
+    ctx->tiled_now = false;
+    return O3R_OK;
+}
 
 constexpr int kBkStrayCap = 8192;   // stray records per chunk (a couple per frame in practice)
 
@@ -91,7 +104,18 @@ bool bk_plan(const o3r_ctx* ctx, const o3r_frame* frames, int n, int chunk, int 
     return true;
 }
 
-// sizes the engine's buffers for a batch
+// misc layout: [0..1] flags (upstream, reduce), [2..3] totals {points, non-empty buckets}, [4] scan ticket, [5] reduce ticket,
+// [6] stray count, [7] debug voxel count (batch-wide), [64..64+n) per-frame voxel counts, then n bytes of per-frame pass-through flags
+struct BkMisc {
+    uint32_t *flags, *totals, *t_scan, *t_reduce, *dbg_cnt, *stray_cnt, *fvox;
+    uint8_t* pass;
+};
+BkMisc bk_misc(o3r_ctx* ctx, int n) {
+    uint32_t* m = ctx->bk_misc.as<uint32_t>();
+    return BkMisc{m, m + 2, m + 4, m + 5, m + 7, m + 6, m + 64, reinterpret_cast<uint8_t*>(m + 64 + n)};
+}
+
+// sizes the engine's buffers for a batch and queues its fills
 int bk_prepare(o3r_ctx* ctx, const BkPlan& pl, int n, size_t cap_batch, size_t cap_chunk) {
     CU(ctx->bk_frames.ensure((size_t)n * sizeof(BkFrame)));
     { int rcu = upload_small(ctx, ctx->bk_frames.p, pl.fr.data(), (size_t)n * sizeof(BkFrame)); if (rcu) return rcu; }
@@ -107,18 +131,12 @@ int bk_prepare(o3r_ctx* ctx, const BkPlan& pl, int n, size_t cap_batch, size_t c
     const size_t part_ub = std::min(cap_batch, pl.total_nb) + (size_t)kBkStrayCap * pl.chunk_nb.size();
     CU(ctx->partials.ensure(std::max<size_t>(part_ub, 1) * sizeof(o3r_cell)));
     CU(ctx->bbox.ensure((size_t)n * 6 * 4));
+    const int rc = fused_prepare(ctx, cap_batch);
+    if (rc) return rc;
+    const BkMisc M = bk_misc(ctx, n);
+    ZERO(M.flags, 8);
+    ZERO(M.dbg_cnt, 4);
     return O3R_OK;
-}
-
-// misc layout: [0..1] flags (upstream, reduce), [2..3] totals {points, non-empty buckets}, [4] scan ticket, [5] reduce ticket,
-// [6] stray count, [7] debug voxel count (batch-wide), [64..64+n) per-frame voxel counts, then n bytes of per-frame pass-through flags
-struct BkMisc {
-    uint32_t *flags, *totals, *t_scan, *t_reduce, *dbg_cnt, *stray_cnt, *fvox;
-    uint8_t* pass;
-};
-BkMisc bk_misc(o3r_ctx* ctx, int n) {
-    uint32_t* m = ctx->bk_misc.as<uint32_t>();
-    return BkMisc{m, m + 2, m + 4, m + 5, m + 7, m + 6, m + 64, reinterpret_cast<uint8_t*>(m + 64 + n)};
 }
 
 // one chunk of frames [f0, f0 + nc) through hist -> scan -> scatter -> reduce; partial cells are appended to ctx->partials at
@@ -133,15 +151,10 @@ int bk_run_chunk(o3r_ctx* ctx, const AParams& P, const BkPlan& pl, int ci, int f
     const uint32_t scan_tiles = cdiv(nb, kBkScanTile);
     const size_t nl_ub = std::min(nb, cap_chunk);
     unsigned long long* st_scan = ctx->bk_status.as<unsigned long long>();
-    {
-        ZeroBatch Z;
-        Z.add(ctx->bk_counts.p, nb * 4);
-        Z.add(ctx->bk_status.p, ((size_t)scan_tiles + 1) * 8);
-        Z.add(M.totals, 20);   // totals, both tickets, stray count
-        Z.add(cnt + CNT_PARTCHUNK, 4);
-        int rcz = zero_batch(ctx, Z);
-        if (rcz) return rcz;
-    }
+    ZERO(ctx->bk_counts.p, nb * 4);
+    ZERO(ctx->bk_status.p, ((size_t)scan_tiles + 1) * 8);
+    ZERO(M.totals, 20);   // totals, both tickets, stray count
+    ZERO(cnt + CNT_PARTCHUNK, 4);
     const dim3 grid(P.tiles_per_frame, nc);
     uint32_t* bbox = ctx->bbox.as<uint32_t>() + (size_t)f0 * 6;
     FILL(bbox, (size_t)(nc) * 24, FILL_BBOX);
@@ -151,7 +164,7 @@ int bk_run_chunk(o3r_ctx* ctx, const AParams& P, const BkPlan& pl, int ci, int f
            ctx->bk_nl.as<uint4>(), st_scan, M.t_scan, M.totals, M.flags);
     LAUNCH_N("k_bk_scatter", (k_bk_scatter<DT>), grid, kThreads, 0, P, fr, bk, M.pass + f0, ctx->inv_f,
              ctx->bk_counts.as<uint32_t>(), ctx->bk_pts.as<float4>(), ctx->bk_pos.as<unsigned long long>(), M.flags);
-    const uint32_t rgrid = std::max(1u, std::min<uint32_t>(cdiv(nl_ub, kRdG), (uint32_t)ctx->bk_reduce_ctas));
+    const uint32_t rgrid = std::max(1u, std::min<uint32_t>(cdiv(nl_ub, kRdG), 148 * 4));
     float4* dbg = ctx->keep_frame_voxels ? ctx->vox.as<float4>() : nullptr;
     LAUNCH(k_bk_reduce, rgrid, kThreads, bk_reduce_smem(), ctx->bk_pts.as<float4>(), ctx->bk_pos.as<unsigned long long>(),
            ctx->bk_nl.as<uint4>(), M.totals, ctx->inv_c, ctx->inv_cz, ctx->partials.as<o3r_cell>(),
@@ -161,6 +174,24 @@ int bk_run_chunk(o3r_ctx* ctx, const AParams& P, const BkPlan& pl, int ci, int f
            ctx->bk_stray.as<o3r_cell>(), cnt + CNT_PARTCHUNK, M.flags);
     LAUNCH(k_add_u32, 1, 32, 0, cnt + CNT_PART, cnt + CNT_PARTCHUNK);
     return O3R_OK;
+}
+
+// queues the copies of the per-frame voxel COUNTS (h_offs[1..n]) and the two overflow flag words (h_offs[n+1..n+2])
+int bk_read_back(o3r_ctx* ctx, int n) {
+    const BkMisc M = bk_misc(ctx, n);
+    CU(cudaMemcpyAsync(ctx->h_offs + 1, M.fvox, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->st));
+    CU(cudaMemcpyAsync(ctx->h_offs + n + 1, M.flags, 8, cudaMemcpyDeviceToHost, ctx->st));
+    return O3R_OK;
+}
+
+// on the landed read-back: a bucket too full / a point outside the grid bound sends this batch and the context's later ones
+// to the sort engine
+Verdict bk_verdict(o3r_ctx* ctx, int n) {
+    const uint32_t* h = ctx->h_offs;
+    if (!(h[n + 1] | h[n + 2])) return Verdict::ACCEPT;
+    if (trace_on()) fprintf(stderr, "[o3r trace] bucket engine overflow flags %u %u: falling back to the sort engine\n", h[n + 1], h[n + 2]);
+    ctx->bucket_off = true;
+    return Verdict::NEXT_ENGINE;
 }
 
 }  // namespace

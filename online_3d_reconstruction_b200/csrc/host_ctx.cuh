@@ -11,6 +11,7 @@
 #include <cstring>
 #include <mutex>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "blur.cuh"
@@ -30,9 +31,11 @@ namespace {
 std::string g_create_err;
 
 inline double now_ms() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
+// O3R_TRACE set: host-side phase times go to stderr
+inline bool trace_on() { static const bool on = getenv("O3R_TRACE") != nullptr; return on; }
 struct Tr {
     bool on; double t; const char* where;
-    explicit Tr(const char* w) : on(getenv("O3R_TRACE") != nullptr), t(now_ms()), where(w) {}
+    explicit Tr(const char* w) : on(trace_on()), t(now_ms()), where(w) {}
     void mark(const char* what) { if (!on) return; const double n = now_ms(); fprintf(stderr, "[o3r trace] %s/%s %.3f ms\n", where, what, n - t); t = n; }
 };
 
@@ -80,6 +83,9 @@ struct FillQueue {
 enum { CNT_PTS = 0, CNT_VOX = 1, CNT_CYC = 2, CNT_NEW = 3, CNT_EMIT = 4, CNT_NEWSCAN = 5, CNT_BASE = 6, CNT_NRES = 7, CNT_ZERO = 8, CNT_PART = 9, CNT_PARTCHUNK = 10,
        CNT_XFLAG = 11, CNT_XRECV = 12, CNT_CHG0 = 13 /* and 14: the pending set's count, one per buffer */,
        CNT_CELLBB = 16, CNT_CHGOUT = 22, CNT_CHGERR = 23, CNT_N = 32 };
+
+// engine of the merged path that served a batch; the values are what o3r_last_batch_engine returns
+enum class Engine { SORT = 0, BUCKET = 1, TILE = 2 };
 
 }  // namespace
 
@@ -166,10 +172,8 @@ struct o3r_ctx {
     // FUSED mode (bucket.cuh): per-frame bucket grids, bucket counters / cursors, non-empty bucket list, binned points + scan
     // positions, look-back words, flags / totals / tickets / per-frame counts
     DevBuf bk_frames, bk_counts, bk_nl, bk_pts, bk_pos, bk_status, bk_misc, bk_stray;
-    int bk_reduce_ctas = 148 * 4;
     bool bucket_off = false;          // a batch overflowed the engine's limits: the sort engine serves this context from then on
-    bool last_bucketed = false;       // the last batch ran through the bucket / tile engine (no per-frame clouds were materialised)
-    int last_engine = 0;              // 0 sort, 1 bucket, 2 tile
+    Engine last_engine = Engine::SORT;   // not SORT: the last batch materialised no per-frame clouds
     // FUSED mode, tile engine (tile.cuh): look-back words; flags / ticket / per-frame counts / pass-through guesses
     DevBuf tv_tiles, tv_misc, tv_scratch;   // per-tile {count, scratch position, offset}; flags / counters; records in arrival order
     size_t tv_scratch_cap = 0, tv_part_cap = 0;   // records the scratch list / the batch's partial list hold (grown on overflow)
@@ -325,17 +329,17 @@ int fill_queue(o3r_ctx* ctx, void* dst, size_t bytes, int kind) {
 }
 #define ZERO(ptr, bytes) do { int rcz_ = fill_queue(ctx, (ptr), (bytes), FILL_ZERO); if (rcz_) return rcz_; } while (0)
 #define FILL(ptr, bytes, kind) do { int rcz_ = fill_queue(ctx, (ptr), (bytes), (kind)); if (rcz_) return rcz_; } while (0)
-// (kept for the call sites that collect several regions themselves)
-struct ZeroBatch {
-    struct R { void* p; size_t bytes; } r[8];
-    int n = 0;
-    void add(void* p, size_t bytes) { if (bytes) { r[n].p = p; r[n].bytes = bytes; ++n; } }
-};
-int zero_batch(o3r_ctx* ctx, const ZeroBatch& B) {
-    for (int i = 0; i < B.n; ++i) { int rc = fill_queue(ctx, B.r[i].p, B.r[i].bytes, FILL_ZERO); if (rc) return rc; }
-    return O3R_OK;
-}
 inline size_t disp_elem(int t) { return t == O3R_DISP_U8 ? 1 : t == O3R_DISP_U16 ? 2 : t == O3R_DISP_F32 ? 4 : 8; }
+// calls f(std::integral_constant<int, DT>) for the runtime disparity type: the one place it becomes a template argument
+template <typename F>
+int with_disp_type(int disp_type, F&& f) {
+    switch (disp_type) {
+        case O3R_DISP_U8: return f(std::integral_constant<int, O3R_DISP_U8>());
+        case O3R_DISP_U16: return f(std::integral_constant<int, O3R_DISP_U16>());
+        case O3R_DISP_F32: return f(std::integral_constant<int, O3R_DISP_F32>());
+        default: return f(std::integral_constant<int, O3R_DISP_F64>());
+    }
+}
 
 int read_counters(o3r_ctx* ctx) {
     CU(cudaMemcpyAsync(ctx->h_counters, ctx->counters.p, CNT_N * 4, cudaMemcpyDeviceToHost, ctx->st));

@@ -189,15 +189,21 @@ int flush_deferred_prefetch(o3r_ctx* ctx) {
     return O3R_OK;
 }
 
+// the O3R_TRACE line of a FUSED batch: the engine it starts with and the context state that chose it
+void trace_fused_engine(const o3r_ctx* ctx, Engine e, const AParams& P, const BatchOpts& opt) {
+    fprintf(stderr, "[o3r trace] fused: engine %s (want_keys %d merge %d tile_off %d bucket_off %d canon %d vec %d R %d)\n",
+            e == Engine::TILE ? "tile" : e == Engine::BUCKET ? "bucket" : "sort", P.want_keys, (int)opt.merge, (int)ctx->tv_off,
+            (int)ctx->bucket_off, ctx->canon, P.vec, ctx->tv_R);
+}
+
 // The batched per-frame path.  `frames` hold host pointers (host_inputs: every frame is copied to device staging
 // on the copy stream, chunk by chunk, overlapping the previous chunk's kernels) or device pointers.
 int frames_cloud_impl(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_type, uint32_t* frame_counts,
                       const BatchOpts& opt, bool host_inputs) {
     const o3r_params& p = ctx->p;
-    static const bool trace = getenv("O3R_TRACE") != nullptr;
+    const bool trace = trace_on();
     ctx->busy_set = -1;
-    auto now = [] { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
-    const double tr0 = now();
+    const double tr0 = now_ms();
     // sharded RETAIN: every call is one cycle of the order tag, whatever it holds (n = 0: this rank has no frame in it)
     const bool rt_shard = opt.merge && ctx->comm && ctx->retain();
     const uint32_t rt_cycle = ctx->rt_cycles;
@@ -348,20 +354,9 @@ int frames_cloud_impl(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_typ
     BkPlan bkp;
     TvPlan tvp;
     const bool fused_ok = ctx->fused() && P.want_keys && opt.merge && !opt.mask_only && !(p.sor_mean_k > 0 && J > 0);
-    bool use_tile = fused_ok && !ctx->tv_off && tv_plan(ctx, P, frames, n, tvp);
-    bool use_bucket = !use_tile && fused_ok && !ctx->bucket_off && bk_plan(ctx, frames, n, chunk, disp_type, label_mode, bkp);
-    std::vector<uint8_t> tv_guess;   // per frame: PCL's overflow guard as the tile kernel will assume it
-    int tv_R = 0;
-    if (use_tile) {
-        tv_guess.assign(n, (uint8_t)(ctx->tv_guess >= 0 ? ctx->tv_guess : (tvp.guess_pass ? 1 : 0)));
-        if (ctx->tv_R < 0) {   // smallest window that covers the nominal depth range (disparities up to 2 min_disparity)
-            const double w_need = std::fabs(p.Q[14] * 2.0 * p.min_disparity + p.Q[15]);
-            ctx->tv_R = kTvMaxR;
-            for (int r = 1; r <= kTvMaxR; ++r)
-                if (tvp.wlim(r) >= w_need) { ctx->tv_R = r; break; }
-        }
-    }
-    if (trace && ctx->fused()) fprintf(stderr, "[o3r trace] fused: engine %s (want_keys %d merge %d tile_off %d bucket_off %d canon %d vec %d R %d)\n", use_tile ? "tile" : use_bucket ? "bucket" : "sort", P.want_keys, (int)opt.merge, (int)ctx->tv_off, (int)ctx->bucket_off, ctx->canon, P.vec, ctx->tv_R);
+    auto bucket_ok = [&] { return fused_ok && !ctx->bucket_off && bk_plan(ctx, frames, n, chunk, disp_type, label_mode, bkp); };
+    Engine engine = fused_ok && tv_begin(ctx, P, frames, n, tvp) ? Engine::TILE : bucket_ok() ? Engine::BUCKET : Engine::SORT;
+    if (trace && ctx->fused()) trace_fused_engine(ctx, engine, P, opt);
     bool inputs_resident = false;   // second attempt: the staging buffers already hold every frame
     double tr1 = 0, tr2 = 0;
     for (;;) {
@@ -373,26 +368,10 @@ int frames_cloud_impl(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_typ
         SortU32 sb{nullptr, nullptr, nullptr, nullptr};
         if (!opt.mask_only) {
             CU(ctx->vox_off.ensure((size_t)(n + 1) * 4));
-            if (use_tile) {
-                bool all_pass = true;
-                for (uint8_t g : tv_guess) all_pass = all_pass && g;
-                tv_R = all_pass ? 0 : ctx->tv_R;
-                int rc = tv_prepare(ctx, tvp, n, chunk, cap_batch, tv_guess);
+            if (engine != Engine::SORT) {
+                const int rc = engine == Engine::TILE ? tv_prepare(ctx, tvp, n, chunk, cap_batch)
+                                                      : bk_prepare(ctx, bkp, n, cap_batch, cap_chunk);
                 if (rc) return rc;
-                if (ctx->keep_frame_voxels) CU(ctx->vox.ensure(cap_batch * 16));
-                FILL(cnt + CNT_CELLBB, 24, FILL_CELLBB);
-                ZERO(cnt + CNT_PART, 8);
-                ctx->tiled_now = false;
-            } else if (use_bucket) {
-                int rc = bk_prepare(ctx, bkp, n, cap_batch, cap_chunk);
-                if (rc) return rc;
-                if (ctx->keep_frame_voxels) CU(ctx->vox.ensure(cap_batch * 16));
-                const BkMisc M = bk_misc(ctx, n);
-                ZERO(M.flags, 8);
-                ZERO(M.dbg_cnt, 4);
-                FILL(cnt + CNT_CELLBB, 24, FILL_CELLBB);
-                ZERO(cnt + CNT_PART, 8);
-                ctx->tiled_now = false;
             } else if (P.want_keys) {
                 CU(ctx->pts.ensure(cap_chunk * 16));
                 CU(ctx->vox.ensure(cap_batch * 16));
@@ -443,39 +422,20 @@ int frames_cloud_impl(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_typ
                         LAUNCH_N("k_blur_box", (k_blur<O3R_BLUR_BOX>), g, kBlurRows, sm, bj, p.rows, p.cols, p.blur_kernel, rx0, ry0, rx1, ry1);
                 }
             }
-            int rc;
-            if (use_tile) {   // planes -> partial cells of the chunk, per-frame voxel counts, exact bboxes
-                switch (disp_type) {
-                    case O3R_DISP_U8: rc = tv_run_chunk<O3R_DISP_U8>(ctx, P, tvp, tv_R, f0, nc, n); break;
-                    case O3R_DISP_U16: rc = tv_run_chunk<O3R_DISP_U16>(ctx, P, tvp, tv_R, f0, nc, n); break;
-                    case O3R_DISP_F32: rc = tv_run_chunk<O3R_DISP_F32>(ctx, P, tvp, tv_R, f0, nc, n); break;
-                    default: rc = tv_run_chunk<O3R_DISP_F64>(ctx, P, tvp, tv_R, f0, nc, n); break;
-                }
-                if (rc) return rc;
-                continue;
-            }
-            if (use_bucket) {   // hist -> scan -> scatter -> reduce: partial cells of the chunk, per-frame voxel counts
-                const int ci = f0 / chunk;
-                switch (disp_type) {
-                    case O3R_DISP_U8: rc = bk_run_chunk<O3R_DISP_U8>(ctx, P, bkp, ci, f0, nc, n, cap_chunk); break;
-                    case O3R_DISP_U16: rc = bk_run_chunk<O3R_DISP_U16>(ctx, P, bkp, ci, f0, nc, n, cap_chunk); break;
-                    case O3R_DISP_F32: rc = bk_run_chunk<O3R_DISP_F32>(ctx, P, bkp, ci, f0, nc, n, cap_chunk); break;
-                    default: rc = bk_run_chunk<O3R_DISP_F64>(ctx, P, bkp, ci, f0, nc, n, cap_chunk); break;
-                }
-                if (rc) return rc;
-                continue;
-            }
-            // stage A: V1 mode writes the chunk scratch; dont_downsample mode writes the batch buffer at the running base
+            // tile engine: planes -> partial cells of the chunk, per-frame voxel counts, exact bboxes; bucket engine: the same through
+            // hist -> scan -> scatter -> reduce; sort engine: stage A, whose V1 mode writes the chunk scratch and whose
+            // dont_downsample mode writes the batch buffer at the running base
             float4* pts_out = ctx->pts.as<float4>();
             const uint32_t* base_a = P.want_keys ? nullptr : cnt + CNT_BASE;
             uint32_t* goff_a = P.want_keys ? nullptr : goff + f0;
-            switch (disp_type) {
-                case O3R_DISP_U8: rc = launch_stage_a<O3R_DISP_U8>(ctx, P, fr, nc, opt, pts_out, sb.k0, base_a, goff_a); break;
-                case O3R_DISP_U16: rc = launch_stage_a<O3R_DISP_U16>(ctx, P, fr, nc, opt, pts_out, sb.k0, base_a, goff_a); break;
-                case O3R_DISP_F32: rc = launch_stage_a<O3R_DISP_F32>(ctx, P, fr, nc, opt, pts_out, sb.k0, base_a, goff_a); break;
-                default: rc = launch_stage_a<O3R_DISP_F64>(ctx, P, fr, nc, opt, pts_out, sb.k0, base_a, goff_a); break;
-            }
+            int rc = with_disp_type(disp_type, [&](auto dt) {
+                constexpr int DT = decltype(dt)::value;
+                if (engine == Engine::TILE) return tv_run_chunk<DT>(ctx, P, tvp, f0, nc, n);
+                if (engine == Engine::BUCKET) return bk_run_chunk<DT>(ctx, P, bkp, f0 / chunk, f0, nc, n, cap_chunk);
+                return launch_stage_a<DT>(ctx, P, fr, nc, opt, pts_out, sb.k0, base_a, goff_a);
+            });
             if (rc) return rc;
+            if (engine != Engine::SORT) continue;
             if (opt.mask_only) { ctx->busy_set = -1; return O3R_OK; }   // (single frame; the last batch's state is untouched)
             const float4* vg_pts = ctx->pts.as<float4>();
             const uint32_t* vg_off = ctx->frame_off.as<uint32_t>();
@@ -521,16 +481,9 @@ int frames_cloud_impl(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_typ
             ctx->h_offs_cap = std::max<size_t>(offs_words, 256);
             CU(cudaMallocHost((void**)&ctx->h_offs, ctx->h_offs_cap * 4));
         }
-        if (use_tile) {   // per-frame voxel COUNTS (h_offs[1..n]), the flag word (h_offs[n+1]), the guard's actual verdicts
-            const TvMisc M = tv_misc(ctx, n);
-            CU(cudaMemcpyAsync(ctx->h_offs + 1, M.fvox, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->st));
-            CU(cudaMemcpyAsync(ctx->h_offs + n + 1, M.flags, 4, cudaMemcpyDeviceToHost, ctx->st));
-            CU(cudaMemcpyAsync(ctx->h_offs + n + 2, M.max_cursor, 4, cudaMemcpyDeviceToHost, ctx->st));
-            CU(cudaMemcpyAsync(ctx->h_offs + n + 3, M.actual, (size_t)n, cudaMemcpyDeviceToHost, ctx->st));
-        } else if (use_bucket) {   // per-frame voxel COUNTS (h_offs[1..n]) and the two overflow flag words (h_offs[n+1..n+2])
-            const BkMisc M = bk_misc(ctx, n);
-            CU(cudaMemcpyAsync(ctx->h_offs + 1, M.fvox, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->st));
-            CU(cudaMemcpyAsync(ctx->h_offs + n + 1, M.flags, 8, cudaMemcpyDeviceToHost, ctx->st));
+        if (engine != Engine::SORT) {   // per-frame counts and the engine's flags
+            const int rc = engine == Engine::TILE ? tv_read_back(ctx, n) : bk_read_back(ctx, n);
+            if (rc) return rc;
         } else {
             CU(cudaMemcpyAsync(ctx->h_offs, goff, (size_t)(n + 1) * 4, cudaMemcpyDeviceToHost, ctx->st));
         }
@@ -543,64 +496,30 @@ int frames_cloud_impl(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_typ
             int rcf = flush_deferred_prefetch(ctx);
             if (rcf) return rcf;
         }
-        ctx->last_has_partials = ctx->last_is_vox && ((ctx->tiled() && ctx->tiled_now) || use_bucket || use_tile);
+        ctx->last_has_partials = ctx->last_is_vox && ((ctx->tiled() && ctx->tiled_now) || engine != Engine::SORT);
         if (ctx->last_has_partials)
             CU(cudaMemcpyAsync(ctx->h_counters + CNT_PART, cnt + CNT_PART, 4, cudaMemcpyDeviceToHost, ctx->st));
-        tr1 = now();
+        tr1 = now_ms();
         CU(cudaStreamSynchronize(ctx->st));
-        tr2 = now();
-        if (use_tile) {
-            const uint32_t fl = ctx->h_offs[n + 1];
-            const uint8_t* actual = reinterpret_cast<const uint8_t*>(ctx->h_offs + n + 3);
-            if (fl) {
-                if (trace) fprintf(stderr, "[o3r trace] tile engine flags %u (R %d)\n", fl, tv_R);
+        tr2 = now_ms();
+        if (engine != Engine::SORT) {
+            const Verdict v = engine == Engine::TILE ? tv_verdict(ctx, tvp, n) : bk_verdict(ctx, n);
+            if (v != Verdict::ACCEPT) {   // rerun from the staging buffers, with this engine or the next one
                 inputs_resident = true;
-                bool retry = true;
-                if (fl & TV_FLAG_SPACE) {   // a record list was too short: what the batch needs is known now (+ 25 %)
-                    ctx->tv_scratch_cap = std::max(ctx->tv_scratch_cap, (size_t)ctx->h_offs[n + 2] + ctx->h_offs[n + 2] / 4 + 1024);
-                    ctx->tv_part_cap = std::max(ctx->tv_part_cap, (size_t)ctx->h_counters[CNT_PART] + ctx->h_counters[CNT_PART] / 4 + 1024);
-                }
-                if (fl & TV_FLAG_PASS) tv_guess.assign(actual, actual + n);   // the bboxes are exact: so is this
-                else if (fl & TV_FLAG_RANGE) {   // a disparity beyond the window's reach: widen it
-                    if (tv_R < kTvMaxR) ctx->tv_R = tv_R + 1; else retry = false;
-                }
-                if (!retry) {   // no window is wide enough: next engine
-                    ctx->tv_off = true;
-                    use_tile = false;
-                    use_bucket = !ctx->bucket_off && bk_plan(ctx, frames, n, chunk, disp_type, label_mode, bkp);
-                }
+                if (v == Verdict::NEXT_ENGINE) engine = engine == Engine::TILE && bucket_ok() ? Engine::BUCKET : Engine::SORT;
                 continue;
             }
-            ctx->tv_guess = actual[n - 1];
-            {   // A combined grid fine against the sideways scatter of the points leaves one record per 1-3 points: a 40-byte record per
-                // 16-byte point is then a loss, and the sort engine's direct merge of the points serves the context from here on.
-                size_t total_vox = 0;
-                for (int i = 0; i < n; ++i) total_vox += ctx->h_offs[i + 1];
-                if ((size_t)ctx->h_counters[CNT_PART] * 4 > total_vox && total_vox > 0) ctx->tv_off = ctx->bucket_off = true;
-            }
-            ctx->h_offs[0] = 0;
-            for (int i = 0; i < n; ++i) ctx->h_offs[i + 1] += ctx->h_offs[i];
-        }
-        if (use_bucket) {
-            if (ctx->h_offs[n + 1] | ctx->h_offs[n + 2]) {   // a bucket too full / a point outside the grid bound: sort engine from now on
-                if (trace) fprintf(stderr, "[o3r trace] bucket engine overflow flags %u %u: falling back to the sort engine\n", ctx->h_offs[n + 1], ctx->h_offs[n + 2]);
-                ctx->bucket_off = true;
-                use_bucket = false;
-                inputs_resident = true;
-                continue;
-            }
-            ctx->h_offs[0] = 0;
+            ctx->h_offs[0] = 0;   // per-frame counts -> offsets
             for (int i = 0; i < n; ++i) ctx->h_offs[i + 1] += ctx->h_offs[i];
         }
         break;
     }
-    ctx->last_bucketed = use_bucket || use_tile;
-    ctx->last_engine = use_tile ? 2 : use_bucket ? 1 : 0;
+    ctx->last_engine = engine;
     ctx->busy_set = -1;
     ctx->last_partials = ctx->last_has_partials ? ctx->h_counters[CNT_PART] : 0;
     // The tile pre-reduction pays only when it reduces: a 40-byte partial replaces a 16-byte voxel in the merge.  On grids
     // finer than the point spacing (e.g. 4K at voxel_size 0.01) nearly every voxel is its own cell: merge the voxels then.
-    if (ctx->last_has_partials && !use_bucket && !use_tile) {
+    if (ctx->last_has_partials && engine == Engine::SORT) {
         ctx->tiled_poor = ctx->last_partials * 2 > ctx->h_offs[n];
         if (ctx->tiled_poor) { ctx->last_has_partials = false; ctx->last_partials = 0; }
     }
@@ -623,10 +542,10 @@ int frames_cloud_impl(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_typ
         return O3R_OK;
     }
     const int* bbp = ctx->last_has_cellbb ? ctx->last_cellbb : nullptr;
-    if ((use_bucket || use_tile) && ctx->last_partials == 0) return O3R_OK;   // nothing valid in the whole batch
+    if (engine != Engine::SORT && ctx->last_partials == 0) return O3R_OK;   // nothing valid in the whole batch
     const int rcm = ctx->last_has_partials ? acc_merge_cells(ctx, ctx->partials.as<o3r_cell>(), ctx->last_partials, bbp)
                                            : acc_merge_points(ctx, outp, ctx->last_total, bbp);
-    if (trace) fprintf(stderr, "[o3r trace] frames_cloud: enqueue %.3f ms, sync wait %.3f ms, merge enqueue %.3f ms\n", tr1 - tr0, tr2 - tr1, now() - tr2);
+    if (trace) fprintf(stderr, "[o3r trace] frames_cloud: enqueue %.3f ms, sync wait %.3f ms, merge enqueue %.3f ms\n", tr1 - tr0, tr2 - tr1, now_ms() - tr2);
     return rcm;
 }
 

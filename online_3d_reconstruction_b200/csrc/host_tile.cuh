@@ -1,5 +1,5 @@
-// host_tile.cuh — host side of the fused tile engine (tile.cuh): the window bound, the pass-through guess, buffer sizing and
-// the launch sequence of one chunk of frames
+// host_tile.cuh — host side of the fused tile engine (tile.cuh): the window bound, the pass-through guess, buffer sizing,
+// the launch sequence of one chunk of frames, the read-back and the verdict on it (reruns, engine policy)
 // (host side of libo3r.so; included by o3r_api.cu, one translation unit)
 #pragma once
 
@@ -8,11 +8,14 @@
 
 namespace {
 
+// a batch's plan: the tiling and the window bound, and the pass-through guesses and window radius of the current attempt
 struct TvPlan {
     int ntx = 0, nty = 0;
     size_t tiles_per_frame = 0;
     double L = 0;                    // pixels per unit of |q14 d + q15| that two points of one leaf can lie apart (tile.cuh, header)
     bool guess_pass = false;         // the guard's verdict on a nominal frame (first batch of a context)
+    std::vector<uint8_t> guess;      // per frame: PCL's overflow guard as the tile kernel will assume it
+    int R = 0;                       // 0: every frame is guessed to pass through (no window)
     double wlim(int R) const { return (double)(R + 1) / L; }
 };
 
@@ -83,6 +86,19 @@ bool tv_plan(const o3r_ctx* ctx, const AParams& P, const o3r_frame* frames, int 
     return true;
 }
 
+// false = the engine does not serve this batch; otherwise the first guesses and (once per context) the window radius
+bool tv_begin(o3r_ctx* ctx, const AParams& P, const o3r_frame* frames, int n, TvPlan& pl) {
+    if (ctx->tv_off || !tv_plan(ctx, P, frames, n, pl)) return false;
+    pl.guess.assign(n, (uint8_t)(ctx->tv_guess >= 0 ? ctx->tv_guess : (pl.guess_pass ? 1 : 0)));
+    if (ctx->tv_R < 0) {   // smallest window that covers the nominal depth range (disparities up to 2 min_disparity)
+        const double w_need = std::fabs(ctx->p.Q[14] * 2.0 * ctx->p.min_disparity + ctx->p.Q[15]);
+        ctx->tv_R = kTvMaxR;
+        for (int r = 1; r <= kTvMaxR; ++r)
+            if (pl.wlim(r) >= w_need) { ctx->tv_R = r; break; }
+    }
+    return true;
+}
+
 // misc layout (u32 words): [0] flags, [1] ticket, [2] debug voxel count, [3] scratch cursor, [4] largest cursor of the batch,
 // [16 .. 16 + n) per-frame voxel counts, then n bytes of guessed and n bytes of actual pass-through flags
 struct TvMisc {
@@ -97,7 +113,8 @@ TvMisc tv_misc(o3r_ctx* ctx, int n) {
 
 // The record lists are sized from what the previous batches needed (the device reports overflow, the host grows and reruns):
 // a tile can emit up to kTvItems records, a typical one a few dozen.
-int tv_prepare(o3r_ctx* ctx, const TvPlan& pl, int n, int chunk, size_t cap_batch, const std::vector<uint8_t>& guess) {
+int tv_prepare(o3r_ctx* ctx, TvPlan& pl, int n, int chunk, size_t cap_batch) {
+    pl.R = std::all_of(pl.guess.begin(), pl.guess.end(), [](uint8_t g) { return g != 0; }) ? 0 : ctx->tv_R;
     const size_t tiles_chunk = pl.tiles_per_frame * (size_t)chunk, tiles_batch = pl.tiles_per_frame * (size_t)n;
     CU(ctx->tv_tiles.ensure(3 * (tiles_chunk + 4) * 4));
     CU(ctx->tv_misc.ensure((16 + (size_t)n) * 4 + 2 * (size_t)n + 16));
@@ -111,40 +128,36 @@ int tv_prepare(o3r_ctx* ctx, const TvPlan& pl, int n, int chunk, size_t cap_batc
     CU(ctx->partials.ensure(ctx->tv_part_cap * sizeof(o3r_cell)));
     const TvMisc M = tv_misc(ctx, n);
     ZERO(M.flags, (16 + (size_t)n) * 4);
-    return upload_small(ctx, M.guess, guess.data(), (size_t)n);
+    const int rc = upload_small(ctx, M.guess, pl.guess.data(), (size_t)n);
+    if (rc) return rc;
+    return fused_prepare(ctx, cap_batch);
 }
 
 template <int DT, int R>
 int tv_launch(o3r_ctx* ctx, const AParams& P, const TvArgs& A, uint32_t n_tiles) {
     const uint32_t bit = 1u << (DT * (kTvMaxR + 1) + R);
-    static const size_t extra = getenv("O3R_TV_EXTRA_SMEM") ? (size_t)atoi(getenv("O3R_TV_EXTRA_SMEM")) : 0;   // occupancy experiments
     if (!(ctx->tv_attr & bit)) {   // (the attribute is per function and device)
-        CU(cudaFuncSetAttribute(k_tv<DT, R>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(tv_smem<R>() + extra)));
+        CU(cudaFuncSetAttribute(k_tv<DT, R>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tv_smem<R>()));
         cudaFuncSetAttribute(k_tv<DT, R>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
         ctx->tv_attr |= bit;
     }
-    LAUNCH_N("k_tv", (k_tv<DT, R>), n_tiles, kTvThreads, tv_smem<R>() + extra, P, A);
+    LAUNCH_N("k_tv", (k_tv<DT, R>), n_tiles, kTvThreads, tv_smem<R>(), P, A);
     return O3R_OK;
 }
 
 // one chunk of frames [f0, f0 + nc): the fused kernel + the guard check; partial cells are appended to ctx->partials at the
 // device-side base cnt[CNT_PART] (advanced here)
 template <int DT>
-int tv_run_chunk(o3r_ctx* ctx, const AParams& P, const TvPlan& pl, int R, int f0, int nc, int n) {
+int tv_run_chunk(o3r_ctx* ctx, const AParams& P, const TvPlan& pl, int f0, int nc, int n) {
     uint32_t* cnt = ctx->counters.as<uint32_t>();
     const TvMisc M = tv_misc(ctx, n);
     const uint32_t n_tiles = (uint32_t)(pl.tiles_per_frame * (size_t)nc);
     uint32_t* tile_cnt = ctx->tv_tiles.as<uint32_t>();
     uint32_t* tile_at = tile_cnt + (pl.tiles_per_frame * (size_t)nc + 4);
     uint32_t* tile_off = tile_at + (pl.tiles_per_frame * (size_t)nc + 4);
-    {
-        ZeroBatch Z;
-        Z.add(M.ticket, 4);
-        Z.add(M.cursor, 4);
-        Z.add(cnt + CNT_PARTCHUNK, 4);
-        int rcz = zero_batch(ctx, Z);
-        if (rcz) return rcz;
-    }
+    ZERO(M.ticket, 4);
+    ZERO(M.cursor, 4);
+    ZERO(cnt + CNT_PARTCHUNK, 4);
     uint32_t* bbox = ctx->bbox.as<uint32_t>() + (size_t)f0 * 6;
     FILL(bbox, (size_t)(nc) * 24, FILL_BBOX);
     TvArgs A;
@@ -152,7 +165,7 @@ int tv_run_chunk(o3r_ctx* ctx, const AParams& P, const TvPlan& pl, int R, int f0
     A.frame_pass = M.guess + f0;
     A.ntx = pl.ntx; A.nty = pl.nty; A.n_frames = nc;
     A.inv_f = ctx->inv_f; A.icx = ctx->inv_c; A.icz = ctx->inv_cz;
-    A.wlim = R > 0 ? pl.wlim(R) : INFINITY;
+    A.wlim = pl.R > 0 ? pl.wlim(pl.R) : INFINITY;
     {   // the largest u8 disparity that keeps |q14 d + q15| below the bound
         int dl = -1;
         for (int d = 0; d < 256; ++d)
@@ -172,7 +185,7 @@ int tv_run_chunk(o3r_ctx* ctx, const AParams& P, const TvPlan& pl, int R, int f0
     A.dbg_vox = ctx->keep_frame_voxels ? ctx->vox.as<float4>() : nullptr;
     A.dbg_cnt = M.dbg_cnt;
     int rc;
-    switch (R) {
+    switch (pl.R) {
         case 0: rc = tv_launch<DT, 0>(ctx, P, A, n_tiles); break;
         case 1: rc = tv_launch<DT, 1>(ctx, P, A, n_tiles); break;
         case 2: rc = tv_launch<DT, 2>(ctx, P, A, n_tiles); break;
@@ -187,6 +200,45 @@ int tv_run_chunk(o3r_ctx* ctx, const AParams& P, const TvPlan& pl, int R, int f0
            M.flags, nc, bbox, ctx->inv_f, M.guess + f0, M.actual + f0);
     LAUNCH(k_add_u32, 1, 32, 0, cnt + CNT_PART, cnt + CNT_PARTCHUNK);
     return O3R_OK;
+}
+
+// queues the copies of the per-frame voxel COUNTS (h_offs[1..n]), the flag word (h_offs[n+1]), the largest scratch cursor
+// (h_offs[n+2]) and the guard's actual verdicts (n bytes from h_offs[n+3])
+int tv_read_back(o3r_ctx* ctx, int n) {
+    const TvMisc M = tv_misc(ctx, n);
+    CU(cudaMemcpyAsync(ctx->h_offs + 1, M.fvox, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->st));
+    CU(cudaMemcpyAsync(ctx->h_offs + n + 1, M.flags, 4, cudaMemcpyDeviceToHost, ctx->st));
+    CU(cudaMemcpyAsync(ctx->h_offs + n + 2, M.max_cursor, 4, cudaMemcpyDeviceToHost, ctx->st));
+    CU(cudaMemcpyAsync(ctx->h_offs + n + 3, M.actual, (size_t)n, cudaMemcpyDeviceToHost, ctx->st));
+    return O3R_OK;
+}
+
+// on the landed read-back (and the partial count in h_counters[CNT_PART]).  A raised flag reruns the batch with what the device
+// found out; when no window is wide enough, this batch and the context's later ones go to the next engine.
+Verdict tv_verdict(o3r_ctx* ctx, TvPlan& pl, int n) {
+    const uint32_t* h = ctx->h_offs;
+    const uint32_t fl = h[n + 1];
+    const uint8_t* actual = reinterpret_cast<const uint8_t*>(h + n + 3);
+    if (fl) {
+        if (trace_on()) fprintf(stderr, "[o3r trace] tile engine flags %u (R %d)\n", fl, pl.R);
+        if (fl & TV_FLAG_SPACE) {   // a record list was too short: what the batch needs is known now (+ 25 %)
+            ctx->tv_scratch_cap = std::max(ctx->tv_scratch_cap, (size_t)h[n + 2] + h[n + 2] / 4 + 1024);
+            ctx->tv_part_cap = std::max(ctx->tv_part_cap, (size_t)ctx->h_counters[CNT_PART] + ctx->h_counters[CNT_PART] / 4 + 1024);
+        }
+        if (fl & TV_FLAG_PASS) pl.guess.assign(actual, actual + n);   // the bboxes are exact: so is this
+        else if (fl & TV_FLAG_RANGE) {   // a disparity beyond the window's reach: widen it
+            if (pl.R >= kTvMaxR) { ctx->tv_off = true; return Verdict::NEXT_ENGINE; }
+            ctx->tv_R = pl.R + 1;
+        }
+        return Verdict::RERUN;
+    }
+    ctx->tv_guess = actual[n - 1];
+    // A combined grid fine against the sideways scatter of the points leaves one record per 1-3 points: a 40-byte record per
+    // 16-byte point is then a loss, and the sort engine's direct merge of the points serves the context from here on.
+    size_t total_vox = 0;
+    for (int i = 0; i < n; ++i) total_vox += h[i + 1];
+    if ((size_t)ctx->h_counters[CNT_PART] * 4 > total_vox && total_vox > 0) ctx->tv_off = ctx->bucket_off = true;
+    return Verdict::ACCEPT;
 }
 
 }  // namespace

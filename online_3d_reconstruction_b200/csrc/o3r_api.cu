@@ -87,24 +87,13 @@ int o3r_create(const o3r_params* params, o3r_ctx** out_ctx) {
     if (e != cudaSuccess) return bail(e, "smem attr");
     // shared-memory carve-out per kernel (percent of the 228 KB array; the rest is L1).  Measured on B200:
     // the run-reduce kernels gather points, so they want L1 as much as occupancy.
-    {
-        auto env_or = [](const char* name, int dflt) { const char* v = getenv(name); return v ? atoi(v) : dflt; };
-        const int cv_vg = env_or("O3R_CARVEOUT_VG", 50), cv_acc = env_or("O3R_CARVEOUT_ACC", 50),
-                  cv_sort = env_or("O3R_CARVEOUT_SORT", 100), cv_emit = env_or("O3R_CARVEOUT_EMIT", -1);
-        cudaFuncSetAttribute(k_vg_reduce_w, cudaFuncAttributePreferredSharedMemoryCarveout, cv_vg);
-        cudaFuncSetAttribute(k_acc_reduce<uint32_t, AccItemsPts>, cudaFuncAttributePreferredSharedMemoryCarveout, cv_acc);
-        cudaFuncSetAttribute(k_acc_reduce<uint64_t, AccItemsPts>, cudaFuncAttributePreferredSharedMemoryCarveout, cv_acc);
-        cudaFuncSetAttribute(k_acc_reduce<uint32_t, AccItemsCells>, cudaFuncAttributePreferredSharedMemoryCarveout, cv_acc);
-        cudaFuncSetAttribute(k_acc_reduce<uint64_t, AccItemsCells>, cudaFuncAttributePreferredSharedMemoryCarveout, cv_acc);
-        cudaFuncSetAttribute(k_rs_onesweep<uint32_t>, cudaFuncAttributePreferredSharedMemoryCarveout, cv_sort);
-        cudaFuncSetAttribute(k_rs_onesweep<uint64_t>, cudaFuncAttributePreferredSharedMemoryCarveout, cv_sort);
-        if (cv_emit >= 0) {
-            cudaFuncSetAttribute(k_emit<O3R_DISP_U8>, cudaFuncAttributePreferredSharedMemoryCarveout, cv_emit);
-            cudaFuncSetAttribute(k_emit<O3R_DISP_U16>, cudaFuncAttributePreferredSharedMemoryCarveout, cv_emit);
-            cudaFuncSetAttribute(k_emit<O3R_DISP_F32>, cudaFuncAttributePreferredSharedMemoryCarveout, cv_emit);
-            cudaFuncSetAttribute(k_emit<O3R_DISP_F64>, cudaFuncAttributePreferredSharedMemoryCarveout, cv_emit);
-        }
-    }
+    cudaFuncSetAttribute(k_vg_reduce_w, cudaFuncAttributePreferredSharedMemoryCarveout, 50);
+    cudaFuncSetAttribute(k_acc_reduce<uint32_t, AccItemsPts>, cudaFuncAttributePreferredSharedMemoryCarveout, 50);
+    cudaFuncSetAttribute(k_acc_reduce<uint64_t, AccItemsPts>, cudaFuncAttributePreferredSharedMemoryCarveout, 50);
+    cudaFuncSetAttribute(k_acc_reduce<uint32_t, AccItemsCells>, cudaFuncAttributePreferredSharedMemoryCarveout, 50);
+    cudaFuncSetAttribute(k_acc_reduce<uint64_t, AccItemsCells>, cudaFuncAttributePreferredSharedMemoryCarveout, 50);
+    cudaFuncSetAttribute(k_rs_onesweep<uint32_t>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+    cudaFuncSetAttribute(k_rs_onesweep<uint64_t>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
     e = cudaFuncSetAttribute(k_bk_reduce, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bk_reduce_smem());
     if (e != cudaSuccess) return bail(e, "smem attr");
     // the bucket kernels stage through shared memory and want their 4-5 CTAs per SM: largest carve-out
@@ -113,7 +102,6 @@ int o3r_create(const o3r_params* params, o3r_ctx** out_ctx) {
     cudaFuncSetAttribute(k_bk_scatter<O3R_DISP_U16>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
     cudaFuncSetAttribute(k_bk_scatter<O3R_DISP_F32>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
     cudaFuncSetAttribute(k_bk_scatter<O3R_DISP_F64>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-    if (const char* v = getenv("O3R_BK_CTAS")) ctx->bk_reduce_ctas = std::max(1, atoi(v));
     cudaFuncSetAttribute(k_blur<O3R_BLUR_MEDIAN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)blur_smem(kBlurMaxK, O3R_BLUR_MEDIAN));
     cudaFuncSetAttribute(k_blur<O3R_BLUR_BOX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)blur_smem(kBlurMaxK, O3R_BLUR_BOX));
     *out_ctx = ctx;
@@ -160,7 +148,7 @@ void o3r_destroy(o3r_ctx* ctx) {
 
 uint64_t o3r_launch_count(const o3r_ctx* ctx) { return ctx ? ctx->launches : 0; }
 size_t o3r_last_batch_partials(const o3r_ctx* ctx) { return (ctx && ctx->last_has_partials) ? ctx->last_partials : 0; }
-int o3r_last_batch_engine(const o3r_ctx* ctx) { return ctx ? ctx->last_engine : 0; }
+int o3r_last_batch_engine(const o3r_ctx* ctx) { return ctx ? (int)ctx->last_engine : 0; }
 void* o3r_stream(o3r_ctx* ctx) { return ctx ? (void*)ctx->st : nullptr; }
 
 int o3r_sync(o3r_ctx* ctx) {
@@ -297,7 +285,7 @@ int o3r_last_batch_points(o3r_ctx* ctx, o3r_point* out, size_t cap, size_t* n_ou
     if (!ctx) return O3R_ERR_INVALID;
     std::lock_guard<std::mutex> lk(ctx->mu);
     CU(cudaSetDevice(ctx->p.device));
-    if (ctx->last_bucketed && !ctx->keep_frame_voxels)
+    if (ctx->last_engine != Engine::SORT && !ctx->keep_frame_voxels)
         return ctx->fail(O3R_ERR_UNSUPPORTED, "O3R_MERGE_ACCUMULATE_FUSED does not materialise the per-frame clouds (see o3r_set_keep_frame_voxels)");
     const float4* src = ctx->last_is_vox ? ctx->vox.as<float4>() : ctx->pts.as<float4>();
     return copy_out(ctx, src, ctx->last_total, out, cap, n_out);
@@ -336,7 +324,7 @@ int o3r_cloud_append(o3r_ctx* ctx, const o3r_point* pts, size_t n) {
     CU(ctx->vox.ensure(n * 16));
     CU(cudaMemcpyAsync(ctx->vox.p, pts, n * 16, cudaMemcpyHostToDevice, ctx->st));
     ctx->last_n = 0; ctx->last_total = 0; ctx->last_has_cellbb = false;   // the batch buffer was overwritten
-    ctx->last_has_partials = false; ctx->last_partials = 0; ctx->last_bucketed = false; ctx->last_engine = 0;
+    ctx->last_has_partials = false; ctx->last_partials = 0; ctx->last_engine = Engine::SORT;
     const int rc = acc_merge_points(ctx, ctx->vox.as<float4>(), n, nullptr);
     if (rc) return rc;
     CU(cudaStreamSynchronize(ctx->st));   // (a page-locked `pts` is read asynchronously) the caller may reuse or free it now

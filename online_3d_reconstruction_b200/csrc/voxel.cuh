@@ -538,10 +538,6 @@ __global__ void k_add_base(uint32_t* base, const uint32_t* total, uint32_t* goff
     if (threadIdx.x == 0) { *base += *total; *goff_end = *base; }
 }
 
-__global__ void k_set_total(uint32_t* dst, const uint32_t* total) {
-    if (threadIdx.x == 0) *dst = *total;
-}
-
 // compact keys of the cycle's items + whole-array digit histograms for the plan's digit layout
 template <typename KeyT, typename Items>
 __global__ void __launch_bounds__(kThreads) k_acc_key(Items items, uint32_t n, float ix, float iz, KeyCodec kc,

@@ -132,7 +132,7 @@ class Pose:
         return out[:n.value]
 
     def lastCycleEngine(self):
-        """1 when the last cycle ran through the fused bucket engine, 0 for the sort engine."""
+        """Engine of the last cycle: 2 = the fused tile engine, 1 = the fused bucket engine, 0 = the sort engine."""
         return int(self._L.o3r_last_batch_engine(self._h))
 
     def setKeepFrameVoxels(self, keep):
