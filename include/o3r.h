@@ -56,7 +56,12 @@ enum { O3R_BLUR_MEDIAN = 0, O3R_BLUR_BOX = 1, O3R_BLUR_BILATERAL = 2 };
 /* how the global cloud is kept (SURVEY §8a row M) */
 enum {
     O3R_MERGE_ACCUMULATE = 0, /* per-cell accumulators keyed by the combined-grid key, merged every
-                                 cycle; o3r_cloud_transform is unsupported                         */
+                                 cycle; o3r_cloud_transform is unsupported.  Colour sums are exact
+                                 uint32 (PCL folds floats: the colours differ once a cell's channel
+                                 sum passes 2^24, ~65 800 points).  PCL's int32 guard is NOT emulated on
+                                 the combined grid: a map wider than 2^31 combined cells still gets
+                                 cells where the reference would return cloud_big unchanged.  Cells are
+                                 limited to +-(2^20 - 1) per axis                                   */
     O3R_MERGE_RETAIN     = 1, /* cloud_big kept as points (pose.cpp:434); o3r_cloud_transform
                                  applies tf_icp in place (pose.cpp:353); one-shot voxelisation     */
     O3R_MERGE_ACCUMULATE_TILED = 2, /* as ACCUMULATE, but every 1024 consecutive per-frame voxels are first
@@ -199,7 +204,9 @@ int o3r_last_batch_points(o3r_ctx* ctx, o3r_point* out, size_t cap, size_t* n_ou
 int o3r_cloud_transform(o3r_ctx* ctx, const float T[16]);
 
 /* Replaces: cloud_big->insert(end, ...) pose.cpp:434 for points produced elsewhere
- * (e.g. the --downsample tool reading a PLY, pose.cpp:71-77).  Host pointer. */
+ * (e.g. the --downsample tool reading a PLY, pose.cpp:71-77).  Host pointer.  In the accumulate modes a point
+ * outside +-(2^20 - 1) combined-grid cells on any axis, or with a NaN / inf coordinate, makes the call return
+ * O3R_ERR_INVALID without merging any of the n points. */
 int o3r_cloud_append(o3r_ctx* ctx, const o3r_point* pts, size_t n);
 
 /* Replaces: PointCloud::Ptr Pose::downsamplePtCloud(PointCloud::Ptr&, bool combinedPtCloud=true)

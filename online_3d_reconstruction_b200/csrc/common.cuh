@@ -88,12 +88,14 @@ __device__ __forceinline__ void xform(const float* T, float x, float y, float z,
     oz = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(T[8], x), __fmul_rn(T[9], y)), __fmul_rn(T[10], z)), T[11]);
 }
 
-// pcl::VoxelGrid leaf index (relative to min_b), PCL 1.8 voxel_grid.hpp first pass
+// pcl::VoxelGrid leaf index (relative to min_b), PCL 1.8 voxel_grid.hpp first pass.  PCL computes it in int and lets it
+// wrap when div0*div1*div2 exceeds INT32_MAX (see make_grid); uint32 arithmetic gives the same bits without the
+// undefined signed overflow.
 __device__ __forceinline__ uint32_t vg_rel_idx(const GridParams& G, float x, float y, float z) {
     const int i0 = (int)(__fsub_rn(floorf(__fmul_rn(x, G.inv[0])), (float)G.min_b[0]));
     const int i1 = (int)(__fsub_rn(floorf(__fmul_rn(y, G.inv[1])), (float)G.min_b[1]));
     const int i2 = (int)(__fsub_rn(floorf(__fmul_rn(z, G.inv[2])), (float)G.min_b[2]));
-    return (uint32_t)(i0 + i1 * G.mul1 + i2 * G.mul2);
+    return (uint32_t)i0 + (uint32_t)i1 * (uint32_t)G.mul1 + (uint32_t)i2 * (uint32_t)G.mul2;
 }
 
 // 64-bit absolute cell key: (k+2^20)<<42 | (j+2^20)<<21 | (i+2^20)
@@ -130,7 +132,7 @@ __device__ __forceinline__ GridParams make_grid(const uint32_t* bb, float ix, fl
         div[a] = max_b - G.min_b[a] + 1;
     }
     G.mul1 = div[0];
-    G.mul2 = div[0] * div[1];
+    G.mul2 = (int)((uint32_t)div[0] * (uint32_t)div[1]);   // (wraps as PCL's int product does)
     const long long cells = (long long)div[0] * div[1] * div[2];
     // PCL's index is a 32-bit int: when div0*div1*div2 exceeds it (the guard above uses the slightly smaller d = (int64)((max - min) * inv) + 1)
     // the index wraps, here exactly as in PCL, and all 32 bits are live

@@ -378,7 +378,8 @@ int frames_cloud_impl(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_typ
                 int rc = carve_sort_u32(ctx, cap_chunk, sb);
                 if (rc) return rc;
                 if (!ctx->retain()) FILL(cnt + CNT_CELLBB, 24, FILL_CELLBB);
-                ctx->tiled_now = ctx->tiled() && !(ctx->tiled_poor && (ctx->tiled_batches % 16) != 0);
+                // (a chunk that could hold 2^30 per-frame voxels goes around it: k_cell_prereduce's look-back word counts 30 bits)
+                ctx->tiled_now = ctx->tiled() && !(ctx->tiled_poor && (ctx->tiled_batches % 16) != 0) && cap_chunk < kRsWideSeg;
                 ++ctx->tiled_batches;
                 if (ctx->tiled_now) {   // worst case one partial per item; never reached in practice (~1/8)
                     CU(ctx->partials.ensure(cap_batch * sizeof(o3r_cell)));

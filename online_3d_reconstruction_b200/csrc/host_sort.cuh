@@ -8,23 +8,38 @@ namespace {
 
 // ---- radix sort driver -----------------------------------------------------------------------------------------
 // The caller provides ghist [n_seg][passes][256] (already filled) and plan.
+// Segments that can reach kRsWideSeg items publish their look-back prefixes in 64-bit status words: a digit's inclusive
+// prefix would overflow the 30 count bits of the 32-bit word.
+template <typename KeyT, typename StT>
+int sort_pairs_t(o3r_ctx* ctx, KeyT* k0, KeyT* k1, uint32_t* v0, uint32_t* v1, const uint32_t* seg_off, int n_seg,
+                 size_t per_seg_cap, const SortPlan* plan, int passes, int iota_first, const uint32_t* ghist,
+                 int ghist_is_prefix) {
+    const uint32_t tiles_ub = std::max(1u, cdiv(per_seg_cap, kRsTile));
+    const size_t st_words = (size_t)n_seg * tiles_ub * kRsBins;
+    // status words for every pass + one ticket per pass, cleared with one memset
+    const size_t bytes = st_words * passes * sizeof(StT) + 64 * 4;
+    CU(ctx->hist.ensure(bytes));
+    ZERO(ctx->hist.p, bytes);
+    StT* status = ctx->hist.as<StT>();
+    uint32_t* tickets = reinterpret_cast<uint32_t*>(status + st_words * passes);
+    const uint32_t grid = tiles_ub * (uint32_t)n_seg;
+    const char* name = sizeof(StT) == 4 ? (sizeof(KeyT) == 4 ? "k_rs_onesweep_u32" : "k_rs_onesweep_u64")
+                                        : (sizeof(KeyT) == 4 ? "k_rs_onesweep_u32_wide" : "k_rs_onesweep_u64_wide");
+    for (int p = 0; p < passes; ++p)
+        LAUNCH_N(name, (k_rs_onesweep<KeyT, StT>), grid, kThreads, rs_scatter_smem<KeyT>(), k0, k1, v0, v1, seg_off, plan,
+                 p, tiles_ub, ghist, status + st_words * p, tickets + p, iota_first, ghist_is_prefix);
+    return O3R_OK;
+}
+
 template <typename KeyT>
 int sort_pairs(o3r_ctx* ctx, KeyT* k0, KeyT* k1, uint32_t* v0, uint32_t* v1, const uint32_t* seg_off, int n_seg,
                size_t per_seg_cap, const SortPlan* plan, int passes, int iota_first, const uint32_t* ghist,
                int ghist_is_prefix = 1) {
-    const uint32_t tiles_ub = std::max(1u, cdiv(per_seg_cap, kRsTile));
-    const size_t st_words = (size_t)n_seg * tiles_ub * kRsBins;
-    // status words for every pass + one ticket per pass, cleared with one memset
-    CU(ctx->hist.ensure((st_words * passes + 64) * 4));
-    ZERO(ctx->hist.p, (st_words * passes + 64) * 4);
-    uint32_t* status = ctx->hist.as<uint32_t>();
-    uint32_t* tickets = status + st_words * passes;
-    const uint32_t grid = tiles_ub * (uint32_t)n_seg;
-    for (int p = 0; p < passes; ++p)
-        LAUNCH_N(sizeof(KeyT) == 4 ? "k_rs_onesweep_u32" : "k_rs_onesweep_u64", (k_rs_onesweep<KeyT>), grid, kThreads,
-                 rs_scatter_smem<KeyT>(), k0, k1, v0, v1, seg_off, plan, p, tiles_ub, ghist,
-                 status + st_words * p, tickets + p, iota_first, ghist_is_prefix);
-    return O3R_OK;
+    if (per_seg_cap >= kRsWideSeg)
+        return sort_pairs_t<KeyT, uint64_t>(ctx, k0, k1, v0, v1, seg_off, n_seg, per_seg_cap, plan, passes, iota_first, ghist,
+                                            ghist_is_prefix);
+    return sort_pairs_t<KeyT, uint32_t>(ctx, k0, k1, v0, v1, seg_off, n_seg, per_seg_cap, plan, passes, iota_first, ghist,
+                                        ghist_is_prefix);
 }
 
 // ---- engine 1: VoxelGrid on segments whose leaf indices already sit in sortbuf keys0 ----------------------------

@@ -79,10 +79,17 @@ int o3r_create(const o3r_params* params, o3r_ctx** out_ctx) {
     cudaMemcpyAsync(ctx->lut_r.p, lr, sizeof(lr), cudaMemcpyHostToDevice, ctx->st);
     cudaMemcpyAsync(ctx->lut_z.p, lz, sizeof(lz), cudaMemcpyHostToDevice, ctx->st);
     if ((e = cudaStreamSynchronize(ctx->st)) != cudaSuccess) return bail(e, "init sync");
-    e = cudaFuncSetAttribute(k_rs_onesweep<uint64_t>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    // the radix pass: both key widths, each with the 32-bit and the wide (64-bit) look-back word
+    e = cudaFuncSetAttribute(k_rs_onesweep<uint64_t, uint32_t>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                              (int)rs_scatter_smem<uint64_t>());
     if (e != cudaSuccess) return bail(e, "smem attr (is this an sm_100a device?)");
-    e = cudaFuncSetAttribute(k_rs_onesweep<uint32_t>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    e = cudaFuncSetAttribute(k_rs_onesweep<uint32_t, uint32_t>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             (int)rs_scatter_smem<uint32_t>());
+    if (e != cudaSuccess) return bail(e, "smem attr");
+    e = cudaFuncSetAttribute(k_rs_onesweep<uint64_t, uint64_t>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             (int)rs_scatter_smem<uint64_t>());
+    if (e != cudaSuccess) return bail(e, "smem attr");
+    e = cudaFuncSetAttribute(k_rs_onesweep<uint32_t, uint64_t>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                              (int)rs_scatter_smem<uint32_t>());
     if (e != cudaSuccess) return bail(e, "smem attr");
     // shared-memory carve-out per kernel (percent of the 228 KB array; the rest is L1).  Measured on B200:
@@ -92,8 +99,10 @@ int o3r_create(const o3r_params* params, o3r_ctx** out_ctx) {
     cudaFuncSetAttribute(k_acc_reduce<uint64_t, AccItemsPts>, cudaFuncAttributePreferredSharedMemoryCarveout, 50);
     cudaFuncSetAttribute(k_acc_reduce<uint32_t, AccItemsCells>, cudaFuncAttributePreferredSharedMemoryCarveout, 50);
     cudaFuncSetAttribute(k_acc_reduce<uint64_t, AccItemsCells>, cudaFuncAttributePreferredSharedMemoryCarveout, 50);
-    cudaFuncSetAttribute(k_rs_onesweep<uint32_t>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-    cudaFuncSetAttribute(k_rs_onesweep<uint64_t>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+    cudaFuncSetAttribute(k_rs_onesweep<uint32_t, uint32_t>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+    cudaFuncSetAttribute(k_rs_onesweep<uint64_t, uint32_t>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+    cudaFuncSetAttribute(k_rs_onesweep<uint32_t, uint64_t>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+    cudaFuncSetAttribute(k_rs_onesweep<uint64_t, uint64_t>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
     e = cudaFuncSetAttribute(k_bk_reduce, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bk_reduce_smem());
     if (e != cudaSuccess) return bail(e, "smem attr");
     // the bucket kernels stage through shared memory and want their 4-5 CTAs per SM: largest carve-out

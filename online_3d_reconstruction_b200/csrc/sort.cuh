@@ -220,7 +220,8 @@ __global__ void __launch_bounds__(kThreads) k_rs_ghist(const KeyT* __restrict__ 
 // ---- one radix pass in one kernel: stable in-tile rank, decoupled look-back for the tile's digit offsets ---------
 // ("onesweep"): every tile publishes its per-digit counts in status[seg][tile][1024] (2 flag bits + 30 count
 // bits in one word), then each thread walks back over the predecessors' words of ITS digit(s) until it
-// meets an inclusive prefix.  Tiles take their index from an atomic ticket so a predecessor is always resident
+// meets an inclusive prefix.  A digit's inclusive prefix counts up to the whole segment: segments that can reach
+// 2^30 items use the 64-bit status word instead (StT = uint64_t: 2 flag bits + 62 count bits).  Tiles take their index from an atomic ticket so a predecessor is always resident
 // or finished before anyone waits on it.
 // Dynamic shared memory: pairs[4096] (key, value) | cnt[kWarps][bins] u16 | gbase[bins] u32 | scan
 template <typename KeyT>
@@ -235,6 +236,8 @@ constexpr size_t rs_scatter_smem() {
 }
 
 constexpr uint32_t kStLocal = 1u << 30, kStGlobal = 2u << 30, kStMask = (1u << 30) - 1u;
+// segments of at least this many items sort with 64-bit look-back words
+constexpr size_t kRsWideSeg = (size_t)1 << 30;
 
 // flag + payload live in ONE word, so relaxed gpu-scope accesses are enough (no fence, no system scope)
 __device__ __forceinline__ uint32_t ld_volatile_u32(const uint32_t* p) {
@@ -245,13 +248,25 @@ __device__ __forceinline__ uint32_t ld_volatile_u32(const uint32_t* p) {
 __device__ __forceinline__ void st_volatile_u32(uint32_t* p, uint32_t v) {
     asm volatile("st.relaxed.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
 }
+__device__ __forceinline__ uint32_t ld_status(const uint32_t* p) { return ld_volatile_u32(p); }
+__device__ __forceinline__ void st_status(uint32_t* p, uint32_t v) { st_volatile_u32(p, v); }
+__device__ __forceinline__ uint64_t ld_status(const uint64_t* p) {
+    uint64_t v;
+    asm volatile("ld.relaxed.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
+    return v;
+}
+__device__ __forceinline__ void st_status(uint64_t* p, uint64_t v) {
+    asm volatile("st.relaxed.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
+}
 
-template <typename KeyT>
+template <typename KeyT, typename StT>
 __global__ void __launch_bounds__(kThreads, sizeof(KeyT) == 4 ? O3R_RS_MINB : (O3R_RS_MINB > 3 ? 3 : O3R_RS_MINB)) k_rs_onesweep(
     KeyT* __restrict__ keys0, KeyT* __restrict__ keys1, uint32_t* __restrict__ vals0, uint32_t* __restrict__ vals1,
     const uint32_t* __restrict__ seg_off, const SortPlan* __restrict__ plan, int pass, uint32_t tiles_ub,
-    const uint32_t* __restrict__ ghist, uint32_t* __restrict__ status, uint32_t* __restrict__ ticket, int iota_first,
+    const uint32_t* __restrict__ ghist, StT* __restrict__ status, uint32_t* __restrict__ ticket, int iota_first,
     int ghist_is_prefix) {
+    constexpr int kFlagShift = (int)sizeof(StT) * 8 - 2;
+    constexpr StT kLocal = (StT)1 << kFlagShift, kGlobal = (StT)2 << kFlagShift, kCountMask = kLocal - 1;
     extern __shared__ __align__(16) unsigned char rs_smem[];
     RsPair<KeyT>* s_pairs = reinterpret_cast<RsPair<KeyT>*>(rs_smem);
     uint16_t* cnt = reinterpret_cast<uint16_t*>(rs_smem + (size_t)kRsTile * sizeof(RsPair<KeyT>));   // [kWarps][1024]
@@ -399,14 +414,14 @@ __global__ void __launch_bounds__(kThreads, sizeof(KeyT) == 4 ? O3R_RS_MINB : (O
     // publish, look back (padding only ever inflates the highest digit)
     uint32_t prefix[kRsBpt];
     {
-        uint32_t* st = status + ((size_t)s * tiles_ub + t) * kRsBins + b0;
+        StT* st = status + ((size_t)s * tiles_ub + t) * kRsBins + b0;
 #pragma unroll
         for (int q = 0; q < kRsBpt; ++q) {
             prefix[q] = 0;
             if ((uint32_t)(b0 + q) < nb) {
                 uint32_t real = run[q];
                 if ((uint32_t)(b0 + q) == nb - 1u) real -= (kRsTile - ntile);
-                st_volatile_u32(st + q, (t == 0 ? kStGlobal : kStLocal) | real);
+                st_status(st + q, (t == 0 ? kGlobal : kLocal) | (StT)real);
             }
         }
         if (t > 0) {
@@ -418,26 +433,26 @@ __global__ void __launch_bounds__(kThreads, sizeof(KeyT) == 4 ? O3R_RS_MINB : (O
                 // The tiles of a segment start together, so most predecessors are still LOCAL when a tile looks back and
                 // the walk is long: kLb status words are loaded per step (independent loads, one L2 round trip).
                 constexpr int kLb = 8;
-                const uint32_t* pst = st + q - kRsBins;
-                uint32_t pf = 0;
+                const StT* pst = st + q - kRsBins;
+                StT pf = 0;
                 bool done = false;
                 for (uint32_t back = t; back > 0 && !done;) {
                     const uint32_t m = min(back, (uint32_t)kLb);
-                    uint32_t v[kLb];
+                    StT v[kLb];
 #pragma unroll
-                    for (int j = 0; j < kLb; ++j) v[j] = (uint32_t)j < m ? ld_volatile_u32(pst - (size_t)j * kRsBins) : kStGlobal;
+                    for (int j = 0; j < kLb; ++j) v[j] = (uint32_t)j < m ? ld_status(pst - (size_t)j * kRsBins) : kGlobal;
 #pragma unroll
                     for (int j = 0; j < kLb; ++j) {
                         if (done) continue;
-                        while ((v[j] >> 30) == 0u) { __nanosleep(32); v[j] = ld_volatile_u32(pst - (size_t)j * kRsBins); }
-                        pf += v[j] & kStMask;
-                        if ((v[j] >> 30) == 2u) done = true;
+                        while ((v[j] >> kFlagShift) == 0u) { __nanosleep(32); v[j] = ld_status(pst - (size_t)j * kRsBins); }
+                        pf += v[j] & kCountMask;
+                        if ((v[j] >> kFlagShift) == 2u) done = true;
                     }
                     back -= m;
                     pst -= (size_t)m * kRsBins;
                 }
-                prefix[q] = pf;
-                st_volatile_u32(st + q, kStGlobal | (pf + real));
+                prefix[q] = (uint32_t)pf;   // < 2^32: a segment holds fewer than 2^32 items
+                st_status(st + q, kGlobal | (pf + real));
             }
         }
     }

@@ -10,6 +10,8 @@
 //   STARTS from the resident accumulator of that cell, so the resident sums equal what a one-shot
 //   voxelisation of the whole history would have produced (pose.cpp:434 + :527-531).
 #pragma once
+#include <type_traits>
+
 #include "common.cuh"
 #include "sort.cuh"
 
@@ -202,7 +204,7 @@ __global__ void __launch_bounds__(kThreads) k_vg_reduce(VgArgs A, const uint32_t
 // waited for is always resident or finished.  Every run is emitted (no min-points filter here).
 struct RunCarry {
     float sx, sy, sz;
-    uint32_t n, r, g, b, slot, tag, first;
+    uint32_t n, r, g, b, slot, tag, first;   // r, g, b: the policy's colour sums as 32-bit words (col_bits)
     uint32_t pad;
     uint32_t flag;
 };  // 48 bytes
@@ -217,11 +219,29 @@ struct RunSmem {
     uint32_t ticket;
 };
 
-// Sequential sum of staged items [a, e).  Only the three FADD chains are serial; the shared-memory loads of the
+// Colour sums: CT = float folds the channels as floats in run order (CentroidPoint, engine 1); CT = uint32_t keeps exact
+// integer sums (engine 2's accumulators).  The two agree while a channel sum stays below 2^24.
+template <typename CT>
+__device__ __forceinline__ void col_add(CT& s, uint32_t v) {
+    if constexpr (std::is_same<CT, float>::value) s = __fadd_rn(s, (float)v);
+    else s += v;
+}
+template <typename CT>
+__device__ __forceinline__ uint32_t col_bits(CT s) {   // a colour sum as the 32-bit word a RunCarry holds
+    if constexpr (std::is_same<CT, float>::value) return __float_as_uint(s);
+    else return s;
+}
+template <typename CT>
+__device__ __forceinline__ CT col_from_bits(uint32_t w) {
+    if constexpr (std::is_same<CT, float>::value) return __uint_as_float(w);
+    else return w;
+}
+
+// Sequential sum of staged items [a, e).  Only the FADD chains are serial; the shared-memory loads of the
 // next batch are issued before the current batch is added.
-template <typename KeyT, bool PACKED>
+template <typename KeyT, bool PACKED, typename CT>
 __device__ __forceinline__ void run_sum(const RunSmem<KeyT, PACKED>& S, uint32_t a, uint32_t e, float& sx, float& sy,
-                                        float& sz, uint32_t& cn, uint32_t& cr, uint32_t& cg, uint32_t& cb) {
+                                        float& sz, uint32_t& cn, CT& cr, CT& cg, CT& cb) {
     constexpr int B = 4;
     uint32_t i = a;
     if (PACKED) {
@@ -237,7 +257,7 @@ __device__ __forceinline__ void run_sum(const RunSmem<KeyT, PACKED>& S, uint32_t
                 for (int u = 0; u < B; ++u) {
                     sx = __fadd_rn(sx, p[u].x); sy = __fadd_rn(sy, p[u].y); sz = __fadd_rn(sz, p[u].z);
                     const uint32_t w = __float_as_uint(p[u].w);
-                    cr += (w >> 16) & 255u; cg += (w >> 8) & 255u; cb += w & 255u;
+                    col_add(cr, (w >> 16) & 255u); col_add(cg, (w >> 8) & 255u); col_add(cb, w & 255u);
                     p[u] = q[u];
                 }
                 cn += B;
@@ -246,7 +266,7 @@ __device__ __forceinline__ void run_sum(const RunSmem<KeyT, PACKED>& S, uint32_t
             for (int u = 0; u < B; ++u) {
                 sx = __fadd_rn(sx, p[u].x); sy = __fadd_rn(sy, p[u].y); sz = __fadd_rn(sz, p[u].z);
                 const uint32_t w = __float_as_uint(p[u].w);
-                cr += (w >> 16) & 255u; cg += (w >> 8) & 255u; cb += w & 255u;
+                col_add(cr, (w >> 16) & 255u); col_add(cg, (w >> 8) & 255u); col_add(cb, w & 255u);
             }
             cn += B;
         }
@@ -254,7 +274,7 @@ __device__ __forceinline__ void run_sum(const RunSmem<KeyT, PACKED>& S, uint32_t
             const float4 p = S.a[i];
             sx = __fadd_rn(sx, p.x); sy = __fadd_rn(sy, p.y); sz = __fadd_rn(sz, p.z);
             const uint32_t w = __float_as_uint(p.w);
-            cn += 1; cr += (w >> 16) & 255u; cg += (w >> 8) & 255u; cb += w & 255u;
+            cn += 1; col_add(cr, (w >> 16) & 255u); col_add(cg, (w >> 8) & 255u); col_add(cb, w & 255u);
         }
     } else {
         for (; i + 4 <= e; i += 4) {
@@ -265,14 +285,14 @@ __device__ __forceinline__ void run_sum(const RunSmem<KeyT, PACKED>& S, uint32_t
 #pragma unroll
             for (int u = 0; u < 4; ++u) {
                 sx = __fadd_rn(sx, p[u].x); sy = __fadd_rn(sy, p[u].y); sz = __fadd_rn(sz, p[u].z);
-                cn += __float_as_uint(p[u].w); cr += q[u].x; cg += q[u].y; cb += q[u].z;
+                cn += __float_as_uint(p[u].w); col_add(cr, q[u].x); col_add(cg, q[u].y); col_add(cb, q[u].z);
             }
         }
         for (; i < e; ++i) {
             const float4 p = S.a[i];
             const uint4 q = S.c[i];
             sx = __fadd_rn(sx, p.x); sy = __fadd_rn(sy, p.y); sz = __fadd_rn(sz, p.z);
-            cn += __float_as_uint(p.w); cr += q.x; cg += q.y; cb += q.z;
+            cn += __float_as_uint(p.w); col_add(cr, q.x); col_add(cg, q.y); col_add(cb, q.z);
         }
     }
 }
@@ -346,12 +366,13 @@ __device__ __forceinline__ void run_reduce_tile(const KeyT* __restrict__ keys, u
         const bool tail = rI == H - 1 && more;
         const KeyT key = (Pol::kNeedsKey || tail) ? keys[wbase + a] : (KeyT)0;
         float sx = 0.f, sy = 0.f, sz = 0.f;
-        uint32_t cn = 0, cr = 0, cg = 0, cb = 0, tag = 0;
+        uint32_t cn = 0, tag = 0;
+        typename Pol::ColT cr = 0, cg = 0, cb = 0;
         pol.start(wbase + a, sx, sy, sz, cn, cr, cg, cb, tag);
         const uint32_t first_v = wbase + a;   // position of the run's first element
         run_sum(S, a, e, sx, sy, sz, cn, cr, cg, cb);
         if (tail && keys[wbase + wn] == key)   // still open at the tile end: hand it on
-            carry_publish(carry, sx, sy, sz, cn, cr, cg, cb, slot0 + rI, tag, first_v);
+            carry_publish(carry, sx, sy, sz, cn, col_bits(cr), col_bits(cg), col_bits(cb), slot0 + rI, tag, first_v);
         else
             pol.emit(slot0 + rI, key, sx, sy, sz, cn, cr, cg, cb, tag, first_v);
     }
@@ -362,22 +383,26 @@ __device__ __forceinline__ void run_reduce_tile(const KeyT* __restrict__ keys, u
         while (ld_volatile_u32(&pc->flag) == 0u) __nanosleep(64);
         __threadfence();
         float sx = __ldcg(&pc->sx), sy = __ldcg(&pc->sy), sz = __ldcg(&pc->sz);
-        uint32_t cn = __ldcg(&pc->n), cr = __ldcg(&pc->r), cg = __ldcg(&pc->g), cb = __ldcg(&pc->b);
+        uint32_t cn = __ldcg(&pc->n);
+        using CT = typename Pol::ColT;
+        CT cr = col_from_bits<CT>(__ldcg(&pc->r)), cg = col_from_bits<CT>(__ldcg(&pc->g)), cb = col_from_bits<CT>(__ldcg(&pc->b));
         const uint32_t slot = __ldcg(&pc->slot), tag = __ldcg(&pc->tag), first_v = __ldcg(&pc->first);
         run_sum(S, 0u, lead, sx, sy, sz, cn, cr, cg, cb);
         const KeyT key = keys[wbase];
         if (H == 0 && more && keys[wbase + wn] == key)
-            carry_publish(carry, sx, sy, sz, cn, cr, cg, cb, slot, tag, first_v);
+            carry_publish(carry, sx, sy, sz, cn, col_bits(cr), col_bits(cg), col_bits(cb), slot, tag, first_v);
         else
             pol.emit(slot, key, sx, sy, sz, cn, cr, cg, cb, tag, first_v);
     }
 }
 
-// engine 1 policy: CentroidPoint of a VoxelGrid leaf.  Optionally tracks the range of combined-grid cells the
-// emitted centroids fall in (so the merge can sort compact keys).
+// engine 1 policy: CentroidPoint of a VoxelGrid leaf (coordinate and colour channels folded as floats in run order, as
+// k_vg_reduce and PCL do).  Optionally tracks the range of combined-grid cells the emitted centroids fall in (so the
+// merge can sort compact keys).
 struct VgPol {
     static constexpr bool kNeedsKey = false;
     static constexpr bool kPacked = true;
+    using ColT = float;
     const float4* spts;   // the segment's points when they are already in sorted order (null: gather pts[vals[pos]])
     const float4* pts; const uint32_t* vals;
     float4* out; int z_shift; bool verbatim;
@@ -387,10 +412,10 @@ struct VgPol {
         a = spts ? __ldcs(spts + pos) : pts[vals[pos]];
         if (z_shift) a.z = __fadd_rn(a.z, 500.0f);
     }
-    __device__ __forceinline__ void start(uint32_t, float&, float&, float&, uint32_t&, uint32_t&, uint32_t&, uint32_t&,
+    __device__ __forceinline__ void start(uint32_t, float&, float&, float&, uint32_t&, float&, float&, float&,
                                           uint32_t&) const {}   // sums start at zero
-    __device__ __forceinline__ void emit(uint32_t slot, uint32_t, float sx, float sy, float sz, uint32_t n, uint32_t r,
-                                         uint32_t g, uint32_t b, uint32_t, uint32_t first) {
+    __device__ __forceinline__ void emit(uint32_t slot, uint32_t, float sx, float sy, float sz, uint32_t n, float r,
+                                         float g, float b, uint32_t, uint32_t first) {
         float4 o;
         if (verbatim) {   // PCL: output = *input_
             o = spts ? spts[first] : pts[vals[first]];
@@ -398,8 +423,8 @@ struct VgPol {
             const float fn = (float)n;
             float cz = __fdiv_rn(sz, fn);
             if (z_shift) cz = __fsub_rn(cz, 500.0f);
-            const uint32_t rgb = ((uint32_t)__fdiv_rn((float)r, fn) << 16) | ((uint32_t)__fdiv_rn((float)g, fn) << 8) |
-                                 (uint32_t)__fdiv_rn((float)b, fn);
+            const uint32_t rgb = ((uint32_t)__fdiv_rn(r, fn) << 16) | ((uint32_t)__fdiv_rn(g, fn) << 8) |
+                                 (uint32_t)__fdiv_rn(b, fn);
             o = make_float4(__fdiv_rn(sx, fn), __fdiv_rn(sy, fn), cz, __uint_as_float(rgb));
         }
         out[slot] = o;
@@ -497,6 +522,10 @@ struct AccItemsPts {   // items are points of weight 1 (z gets +500)
         i = (int)floorf(__fmul_rn(p.x, ix)); j = (int)floorf(__fmul_rn(p.y, ix));
         k = (int)floorf(__fmul_rn(__fadd_rn(p.z, 500.0f), iz));
     }
+    __device__ __forceinline__ bool finite(uint32_t v) const {
+        const float4 p = pts[v];
+        return isfinite(p.x) && isfinite(p.y) && isfinite(p.z);
+    }
 };
 struct AccItemsCells {  // items are partial cells received from other ranks
     const o3r_cell* cells;
@@ -514,15 +543,18 @@ struct AccItemsCells {  // items are partial cells received from other ranks
         const int B = 1 << 20;
         i = (int)(key & 0x1fffffu) - B; j = (int)((key >> 21) & 0x1fffffu) - B; k = (int)(key >> 42) - B;
     }
+    __device__ __forceinline__ bool finite(uint32_t) const { return true; }
 };
 
-// range of combined-grid cells of n items (only when the range was not tracked upstream)
+// range of combined-grid cells of n items (only when the range was not tracked upstream).  A NaN coordinate converts to
+// cell 0, so a non-finite item widens the range to INT_MIN instead, which the host refuses like any cell beyond +-2^20.
 template <typename Items>
 __global__ void __launch_bounds__(kThreads) k_acc_cellbb(Items items, uint32_t n, float ix, float iz, int* __restrict__ cellbb) {
     int mn[3] = {0x7fffffff, 0x7fffffff, 0x7fffffff}, mx[3] = {(int)0x80000000, (int)0x80000000, (int)0x80000000};
     for (uint32_t v = blockIdx.x * kThreads + threadIdx.x; v < n; v += gridDim.x * kThreads) {
         int c[3];
         items.cell(v, ix, iz, c[0], c[1], c[2]);
+        if (!items.finite(v)) c[0] = (int)0x80000000;
 #pragma unroll
         for (int a = 0; a < 3; ++a) { mn[a] = min(mn[a], c[a]); mx[a] = max(mx[a], c[a]); }
     }
@@ -633,10 +665,12 @@ __global__ void __launch_bounds__(kThreads) k_acc_heads(AccArgs<KeyT> A, uint32_
 
 // engine 2 policy: look the cell up in the resident shard and continue its sums in input order.
 // Emits the cycle's cell list (sorted by key): ckey (absolute), cacc = {sx, sy, sz, n}, crgb = {sr, sg, sb, found_pos + 1}.
+// Colour sums are exact uint32 (they differ from a float fold once a channel sum passes 2^24; DESIGN §2).
 template <typename KeyT, typename Items>
 struct AccPol {
     static constexpr bool kNeedsKey = true;
     static constexpr bool kPacked = Items::kPacked;
+    using ColT = uint32_t;
     Items items;
     KeyCodec kc;
     const uint32_t* tags;   // per element position: resident position + 1 of a head's cell, 0 = new cell

@@ -479,14 +479,16 @@ int orc_voxel_grid(const o3r_point* pts, size_t n, float lx, float ly, float lz,
         max_b[a] = (int)std::floor(mx[a] * inv[a]);
         div_b[a] = max_b[a] - min_b[a] + 1;
     }
-    const int mul[3] = {1, div_b[0], div_b[0] * div_b[1]};
+    /* PCL's divb_mul_ and index are int and wrap once div_b[0]*div_b[1]*div_b[2] exceeds INT32_MAX (the guard above uses the
+       slightly smaller (max - min) * inv); uint32 arithmetic gives the same bits without the undefined signed overflow */
+    const uint32_t mul[3] = {1u, (uint32_t)div_b[0], (uint32_t)div_b[0] * (uint32_t)div_b[1]};
     struct IdxPt { unsigned idx; unsigned pt; };
     std::vector<IdxPt> iv(n);
     for (size_t i = 0; i < n; ++i) {
         const int i0 = (int)(std::floor(pts[i].x * inv[0]) - (float)min_b[0]);
         const int i1 = (int)(std::floor(pts[i].y * inv[1]) - (float)min_b[1]);
         const int i2 = (int)(std::floor(pts[i].z * inv[2]) - (float)min_b[2]);
-        iv[i].idx = (unsigned)(i0 * mul[0] + i1 * mul[1] + i2 * mul[2]);
+        iv[i].idx = (uint32_t)i0 * mul[0] + (uint32_t)i1 * mul[1] + (uint32_t)i2 * mul[2];
         iv[i].pt = (unsigned)i;
     }
     /* PCL uses std::sort (order inside a voxel unspecified); the oracle fixes it to input order. */
