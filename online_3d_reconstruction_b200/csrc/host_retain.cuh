@@ -39,22 +39,10 @@ int rt_engine1(o3r_ctx* ctx, const float4* pts, size_t n, size_t* m) {
     *m = 0;
     if (n == 0) return O3R_OK;
     CU(ctx->rt_out.ensure(n * 16));
-    CU(ctx->vox_off.ensure(2 * 4));
     const uint32_t seg_h[2] = {0u, (uint32_t)n};
     { int rcu = upload_small(ctx, ctx->seg2.p, seg_h, 8); if (rcu) return rcu; }
-    const uint32_t* seg = ctx->seg2.as<uint32_t>();
-    SortU32 sb;
-    int rc = carve_sort_u32(ctx, n, sb);
-    if (rc) return rc;
-    LAUNCH(k_vg_key, dim3(std::min<uint32_t>(cdiv(n, kThreads), 148 * 16), 1), kThreads, 0, pts, seg, ctx->grids.as<GridParams>(), 1,
-           sb.k0);
-    rc = vg_sorted_reduce(ctx, sb, pts, seg, 1, n, ctx->grids.as<GridParams>(), ctx->inv_c, ctx->inv_c, ctx->inv_cz,
-                          ctx->p.min_points_per_voxel, 1, ctx->rt_out.as<float4>(), ctx->vox_off.as<uint32_t>(), nullptr, nullptr);
-    if (rc) return rc;
-    rc = read_counters(ctx);
-    if (rc) return rc;
-    *m = ctx->h_counters[CNT_VOX];
-    return O3R_OK;
+    return vg_one_segment(ctx, pts, ctx->seg2.as<uint32_t>(), n, ctx->inv_c, ctx->inv_c, ctx->inv_cz,
+                          ctx->p.min_points_per_voxel, 1, ctx->rt_out.as<float4>(), nullptr, nullptr, m);
 }
 
 // step 1, local part: the z-shifted bbox of the local cloud and the words of the first agreement

@@ -70,7 +70,8 @@ int sort_segments_plan(o3r_ctx* ctx, const SortU32& sb, const uint32_t* seg_off,
     return O3R_OK;
 }
 
-// sorts + reduces; out/out_off sized by the caller.  CNT_VOX receives the total.
+// sorts + reduces; out/out_off sized by the caller.  CNT_VOX receives the total.  track_cells / out_base only serve the
+// unfiltered reduction (min_points <= 1, no keys / counts).
 int vg_sorted_reduce(o3r_ctx* ctx, const SortU32& sb, const float4* pts, const uint32_t* seg_off, int n_seg,
                      size_t per_seg_cap, const GridParams* grids, float ix, float iy, float iz, uint32_t min_points,
                      int z_shift, float4* out, uint32_t* out_off, uint64_t* out_keys, uint32_t* out_counts,
@@ -78,7 +79,6 @@ int vg_sorted_reduce(o3r_ctx* ctx, const SortU32& sb, const float4* pts, const u
     int rcs = sort_segments_plan(ctx, sb, seg_off, n_seg, per_seg_cap, grids);
     if (rcs) return rcs;
     SortPlan* plan = ctx->plan_all.as<SortPlan>();
-    const bool fast = min_points <= 1 && !out_keys && !out_counts;
     int rc = sort_pairs<uint32_t>(ctx, sb.k0, sb.k1, sb.v0, sb.v1, seg_off, n_seg, per_seg_cap, plan, 4, 1,
                                   ctx->ghist.as<uint32_t>());
     if (rc) return rc;
@@ -96,16 +96,33 @@ int vg_sorted_reduce(o3r_ctx* ctx, const SortU32& sb, const float4* pts, const u
     LAUNCH(k_vg_heads, grid, kThreads, 0, A, ctx->head_cnt.as<uint32_t>());
     LAUNCH(k_scan_u32, 1, kScanThreads, 0, ctx->head_cnt.as<uint32_t>(), ctx->head_off.as<uint32_t>(), (uint32_t)nt,
            cnt + CNT_VOX);
-    if (fast) {
-        const size_t wbytes = 64 + (nt + 1) * sizeof(RunCarry);
-        CU(ctx->runwork.ensure(wbytes));
-        ZERO(ctx->runwork.p, wbytes);
-        LAUNCH(k_vg_reduce_w, (uint32_t)nt, kThreads, 0, A, ctx->head_off.as<uint32_t>(), cnt + CNT_VOX, out, out_off,
-               n_seg, ctx->runwork.as<uint32_t>(), reinterpret_cast<RunCarry*>(ctx->runwork.as<char>() + 64),
-               track_cells ? 1 : 0, ctx->inv_c, ctx->inv_cz, reinterpret_cast<int*>(cnt + CNT_CELLBB), out_base);
-    } else
-        LAUNCH(k_vg_reduce, grid, kThreads, 0, A, ctx->head_off.as<uint32_t>(), cnt + CNT_VOX, out, out_off, n_seg,
-               out_keys, out_counts);
+    const size_t wbytes = 64 + (nt + 1) * sizeof(RunCarry);
+    CU(ctx->runwork.ensure(wbytes));
+    ZERO(ctx->runwork.p, wbytes);
+    const bool full = min_points > 1 || out_keys || out_counts;
+    LAUNCH_N(full ? "k_vg_reduce_w_full" : "k_vg_reduce_w", (full ? k_vg_reduce_w<true> : k_vg_reduce_w<false>),
+             (uint32_t)nt, kThreads, 0, A, ctx->head_off.as<uint32_t>(), cnt + CNT_VOX, out, out_off, n_seg,
+             ctx->runwork.as<uint32_t>(), reinterpret_cast<RunCarry*>(ctx->runwork.as<char>() + 64), track_cells ? 1 : 0,
+             ctx->inv_c, ctx->inv_cz, reinterpret_cast<int*>(cnt + CNT_CELLBB), out_base, out_keys, out_counts);
+    return O3R_OK;
+}
+
+// engine 1 over the one segment [0, n) of pts, whose bounds are already in `seg` and whose grid is in ctx->grids: leaf
+// indices, sort, reduction into `out` (and `out_keys` / `out_counts` when given).  Waits for the stream; *m = records.
+int vg_one_segment(o3r_ctx* ctx, const float4* pts, const uint32_t* seg, size_t n, float ix, float iy, float iz,
+                   uint32_t min_points, int z_shift, float4* out, uint64_t* out_keys, uint32_t* out_counts, size_t* m) {
+    CU(ctx->vox_off.ensure(2 * 4));
+    SortU32 sb;
+    int rc = carve_sort_u32(ctx, n, sb);
+    if (rc) return rc;
+    const GridParams* grids = ctx->grids.as<GridParams>();
+    LAUNCH(k_vg_key, dim3(std::min<uint32_t>(cdiv(n, kThreads), 148 * 16), 1), kThreads, 0, pts, seg, grids, z_shift, sb.k0);
+    rc = vg_sorted_reduce(ctx, sb, pts, seg, 1, n, grids, ix, iy, iz, min_points, z_shift, out, ctx->vox_off.as<uint32_t>(),
+                          out_keys, out_counts);
+    if (rc) return rc;
+    rc = read_counters(ctx);
+    if (rc) return rc;
+    *m = ctx->h_counters[CNT_VOX];
     return O3R_OK;
 }
 

@@ -94,7 +94,8 @@ int o3r_create(const o3r_params* params, o3r_ctx** out_ctx) {
     if (e != cudaSuccess) return bail(e, "smem attr");
     // shared-memory carve-out per kernel (percent of the 228 KB array; the rest is L1).  Measured on B200:
     // the run-reduce kernels gather points, so they want L1 as much as occupancy.
-    cudaFuncSetAttribute(k_vg_reduce_w, cudaFuncAttributePreferredSharedMemoryCarveout, 50);
+    cudaFuncSetAttribute(k_vg_reduce_w<false>, cudaFuncAttributePreferredSharedMemoryCarveout, 50);
+    cudaFuncSetAttribute(k_vg_reduce_w<true>, cudaFuncAttributePreferredSharedMemoryCarveout, 50);
     cudaFuncSetAttribute(k_acc_reduce<uint32_t, AccItemsPts>, cudaFuncAttributePreferredSharedMemoryCarveout, 50);
     cudaFuncSetAttribute(k_acc_reduce<uint64_t, AccItemsPts>, cudaFuncAttributePreferredSharedMemoryCarveout, 50);
     cudaFuncSetAttribute(k_acc_reduce<uint32_t, AccItemsCells>, cudaFuncAttributePreferredSharedMemoryCarveout, 50);
@@ -367,33 +368,23 @@ static int voxel_grid_dev(o3r_ctx* ctx, const float4* pts, size_t n, float ix, f
                           int z_shift, float4* out, uint64_t* out_keys, uint32_t* out_counts, size_t* n_out,
                           int* passthrough) {
     if (n >= (1ull << 32)) return ctx->fail(O3R_ERR_INVALID, "cloud too large for 32-bit indices");
-    uint32_t* cnt = ctx->counters.as<uint32_t>();
     CU(ctx->seg2.ensure(16));
     const uint32_t seg_h[2] = {0u, (uint32_t)n};
     { int rcu = upload_small(ctx, ctx->seg2.p, seg_h, 8); if (rcu) return rcu; }
     const uint32_t* seg = ctx->seg2.as<uint32_t>();
     CU(ctx->bbox.ensure(6 * 4));
     CU(ctx->grids.ensure(sizeof(GridParams)));
-    CU(ctx->vox_off.ensure(2 * 4));
-    SortU32 sb;
-    int rc = carve_sort_u32(ctx, n, sb);
-    if (rc) return rc;
-    const uint32_t tiles = cdiv(n, kTileV);
     FILL(ctx->bbox.as<uint32_t>(), (size_t)(1) * 24, FILL_BBOX);
-    LAUNCH(k_bbox_pts, dim3(tiles, 1), kThreads, 0, pts, seg, z_shift, ctx->bbox.as<uint32_t>());
+    LAUNCH(k_bbox_pts, dim3(cdiv(n, kTileV), 1), kThreads, 0, pts, seg, z_shift, ctx->bbox.as<uint32_t>());
     LAUNCH(k_grid_params, 1, 32, 0, 1, ctx->bbox.as<uint32_t>(), ix, iy, iz, ctx->grids.as<GridParams>());
-    LAUNCH(k_vg_key, dim3(std::min<uint32_t>(cdiv(n, kThreads), 148 * 16), 1), kThreads, 0, pts, seg,
-           ctx->grids.as<GridParams>(), z_shift, sb.k0);
-    rc = vg_sorted_reduce(ctx, sb, pts, seg, 1, n, ctx->grids.as<GridParams>(), ix, iy, iz, min_points, z_shift, out,
-                          ctx->vox_off.as<uint32_t>(), out_keys, out_counts);
+    int rc = vg_one_segment(ctx, pts, seg, n, ix, iy, iz, min_points, z_shift, out, out_keys, out_counts, n_out);
     if (rc) return rc;
-    GridParams g;
-    CU(cudaMemcpyAsync(&g, ctx->grids.p, sizeof(g), cudaMemcpyDeviceToHost, ctx->st));
-    rc = read_counters(ctx);
-    if (rc) return rc;
-    (void)cnt;
-    *n_out = ctx->h_counters[CNT_VOX];
-    if (passthrough) *passthrough = g.passthrough;
+    if (passthrough) {
+        GridParams g;
+        CU(cudaMemcpyAsync(&g, ctx->grids.p, sizeof(g), cudaMemcpyDeviceToHost, ctx->st));
+        CU(cudaStreamSynchronize(ctx->st));
+        *passthrough = g.passthrough;
+    }
     return O3R_OK;
 }
 

@@ -121,78 +121,6 @@ __global__ void __launch_bounds__(kThreads) k_vg_heads(VgArgs A, uint32_t* __res
     if (threadIdx.x == 0) head_cnt[(size_t)s * A.tiles_ub + t] = s_c;
 }
 
-__global__ void __launch_bounds__(kThreads) k_vg_reduce(VgArgs A, const uint32_t* __restrict__ head_off,
-                                                        const uint32_t* __restrict__ head_total,
-                                                        float4* __restrict__ out, uint32_t* __restrict__ seg_out_off,
-                                                        int n_seg, uint64_t* __restrict__ out_keys,
-                                                        uint32_t* __restrict__ out_counts) {
-    __shared__ uint32_t s_scan[34];
-    const int s = blockIdx.y;
-    const uint32_t t = blockIdx.x;
-    if (t == 0 && threadIdx.x == 0) {
-        seg_out_off[s] = head_off[(size_t)s * A.tiles_ub];
-        if (s == n_seg - 1) seg_out_off[n_seg] = *head_total;
-    }
-    const uint32_t beg = A.seg_off[s], n = A.seg_off[s + 1] - beg;
-    if (t * kTileV >= n) return;
-    const int par = A.plan[s].final_parity;
-    const bool ident = A.plan[s].n_active == 0;   // nothing was sorted (pass-through / single-cell segment)
-    const uint32_t* keys = (par ? A.keys1 : A.keys0) + beg;
-    const uint32_t* vals = (par ? A.vals1 : A.vals0) + beg;
-    uint32_t flags = 0;
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-        const uint32_t pos = t * kTileV + threadIdx.x * 4 + j;
-        if (pos < n && vg_emits(keys, pos, n, A.min_points)) flags |= 1u << j;
-    }
-    uint32_t tot;
-    uint32_t o = head_off[(size_t)s * A.tiles_ub + t] + block_excl_scan((uint32_t)__popc(flags), s_scan, tot);
-    if (!flags) return;
-    const bool verbatim = A.grids && A.grids[s].passthrough;  // PCL: output = *input_
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-        if (!(flags & (1u << j))) continue;
-        const uint32_t pos = t * kTileV + threadIdx.x * 4 + j;
-        const uint32_t k = keys[pos];
-        if (verbatim) {
-            const float4 p = A.pts[ident ? beg + pos : vals[pos]];
-            out[o] = p;
-            if (out_keys) out_keys[o] = abs_cell_key(p.x, p.y, A.z_shift ? __fadd_rn(p.z, 500.0f) : p.z, A.lx_inv, A.ly_inv, A.lz_inv);
-            if (out_counts) out_counts[o] = 1;
-            ++o;
-            continue;
-        }
-        // CentroidPoint<PointXYZRGB>: float sums in run order, divide by (float)n; colour sums as floats
-        float sx = 0.f, sy = 0.f, sz = 0.f, sr = 0.f, sg = 0.f, sb = 0.f;
-        uint32_t cnt = 0;
-        float4 first = make_float4(0.f, 0.f, 0.f, 0.f);
-        for (uint32_t q = pos; q < n && keys[q] == k; ++q) {
-            const float4 p = A.pts[ident ? beg + q : vals[q]];
-            const float z = A.z_shift ? __fadd_rn(p.z, 500.0f) : p.z;
-            if (cnt == 0) first = make_float4(p.x, p.y, z, 0.f);
-            const uint32_t c = __float_as_uint(p.w);
-            sx = __fadd_rn(sx, p.x); sy = __fadd_rn(sy, p.y); sz = __fadd_rn(sz, z);
-            sr = __fadd_rn(sr, (float)((c >> 16) & 255u));
-            sg = __fadd_rn(sg, (float)((c >> 8) & 255u));
-            sb = __fadd_rn(sb, (float)(c & 255u));
-            ++cnt;
-        }
-        const float fn = (float)cnt;
-        float cz = __fdiv_rn(sz, fn);
-        if (A.z_shift) cz = __fsub_rn(cz, 500.0f);
-        const uint32_t rgb = ((uint32_t)__fdiv_rn(sr, fn) << 16) | ((uint32_t)__fdiv_rn(sg, fn) << 8) |
-                             (uint32_t)__fdiv_rn(sb, fn);
-        out[o] = make_float4(__fdiv_rn(sx, fn), __fdiv_rn(sy, fn), cz, __uint_as_float(rgb));
-        if (out_keys) out_keys[o] = abs_cell_key(first.x, first.y, first.z, A.lx_inv, A.ly_inv, A.lz_inv);
-        if (out_counts) out_counts[o] = cnt;
-        ++o;
-    }
-}
-
-// passthrough segments keep their points verbatim (PCL: output = *input_); the identity keys already make
-// every element its own run, so k_vg_reduce reproduces them — except that a centroid of one point is
-// sum/1 = the point and uint32(c/1) = c, i.e. bit-identical.  Nothing extra to do.
-
 // ---- CTA-cooperative run reduction (shared by both engines) --------------------------------------------------------
 // A CTA owns kTileV consecutive sorted elements.  All threads stage the tile's items into shared memory
 // (coalesced key/value loads, gathered item loads), then ONE thread per run adds the run's items strictly in
@@ -201,7 +129,10 @@ __global__ void __launch_bounds__(kThreads) k_vg_reduce(VgArgs A, const uint32_t
 // A run that crosses a tile boundary is handed on: the tile where it is still open publishes its partial sums
 // (RunCarry, flag last), the next tile's carry thread waits for them, continues with its leading elements and
 // either emits the run or hands it on again.  Tiles take their index from an atomic ticket, so the tile being
-// waited for is always resident or finished.  Every run is emitted (no min-points filter here).
+// waited for is always resident or finished.  Every run is emitted, unless the policy filters (Pol::kFilter): then only
+// the runs it passes get an output slot, numbered in run order, and a dropped run carries kNoSlot to its emit.
+constexpr uint32_t kNoSlot = 0xffffffffu;
+
 struct RunCarry {
     float sx, sy, sz;
     uint32_t n, r, g, b, slot, tag, first;   // r, g, b: the policy's colour sums as 32-bit words (col_bits)
@@ -217,6 +148,11 @@ struct RunSmem {
     uint16_t hpos[kTileV + 2];
     uint32_t scan[34];
     uint32_t ticket;
+};
+// filtering policies also keep each run's output rank in the tile (0xffff: no slot)
+template <typename KeyT, bool PACKED>
+struct RunSmemRanked : RunSmem<KeyT, PACKED> {
+    uint16_t hslot[kTileV];
 };
 
 // Colour sums: CT = float folds the channels as floats in run order (CentroidPoint, engine 1); CT = uint32_t keeps exact
@@ -306,9 +242,9 @@ __device__ __forceinline__ void carry_publish(RunCarry* c, float sx, float sy, f
 }
 
 // `carry` points at this tile's RunCarry; carry[-1] is the previous tile of the same segment.
-template <typename KeyT, typename Pol>
+template <typename KeyT, typename Pol, typename Smem>
 __device__ __forceinline__ void run_reduce_tile(const KeyT* __restrict__ keys, uint32_t n, uint32_t t, uint32_t slot0,
-                                                Pol& pol, RunSmem<KeyT, Pol::kPacked>& S, RunCarry* __restrict__ carry) {
+                                                Pol& pol, Smem& S, RunCarry* __restrict__ carry) {
     const int tid = threadIdx.x;
     const uint32_t wbase = t * kTileV;
     const uint32_t wn = min((uint32_t)kTileV, n - wbase);
@@ -354,12 +290,27 @@ __device__ __forceinline__ void run_reduce_tile(const KeyT* __restrict__ keys, u
     }
     uint32_t H;
     uint32_t hoff = block_excl_scan((uint32_t)__popc(flags), S.scan, H);
+    if constexpr (Pol::kFilter) {   // output rank of each run among the tile's runs the policy passes: a second scan
+        uint32_t emits = 0;
+#pragma unroll
+        for (int j = 0; j < 4; ++j)
+            if ((flags & (1u << j)) && pol.emits(keys, wbase + tid * 4 + j, n)) emits |= 1u << j;
+        uint32_t E, h = hoff;
+        uint32_t r = block_excl_scan((uint32_t)__popc(emits), S.scan, E);
+#pragma unroll
+        for (int j = 0; j < 4; ++j)
+            if (flags & (1u << j)) S.hslot[h++] = (emits & (1u << j)) ? (uint16_t)r++ : (uint16_t)0xffffu;
+    }
 #pragma unroll
     for (int j = 0; j < 4; ++j)
         if (flags & (1u << j)) S.hpos[hoff++] = (uint16_t)(tid * 4 + j);
     if (tid == 0) S.hpos[H] = (uint16_t)wn;
     __syncthreads();
     const bool more = wbase + wn < n;              // the segment continues after this tile
+    auto slot_of = [&](uint32_t rI) {   // output slot of the tile's run rI
+        if constexpr (Pol::kFilter) return S.hslot[rI] == 0xffffu ? kNoSlot : slot0 + S.hslot[rI];
+        else return slot0 + rI;
+    };
     // ---- one thread per run whose head lies in the tile
     for (uint32_t rI = tid; rI < H; rI += kThreads) {
         const uint32_t a = S.hpos[rI], e = S.hpos[rI + 1];
@@ -372,9 +323,9 @@ __device__ __forceinline__ void run_reduce_tile(const KeyT* __restrict__ keys, u
         const uint32_t first_v = wbase + a;   // position of the run's first element
         run_sum(S, a, e, sx, sy, sz, cn, cr, cg, cb);
         if (tail && keys[wbase + wn] == key)   // still open at the tile end: hand it on
-            carry_publish(carry, sx, sy, sz, cn, col_bits(cr), col_bits(cg), col_bits(cb), slot0 + rI, tag, first_v);
+            carry_publish(carry, sx, sy, sz, cn, col_bits(cr), col_bits(cg), col_bits(cb), slot_of(rI), tag, first_v);
         else
-            pol.emit(slot0 + rI, key, sx, sy, sz, cn, cr, cg, cb, tag, first_v);
+            pol.emit(slot_of(rI), key, sx, sy, sz, cn, cr, cg, cb, tag, first_v);
     }
     // ---- the run handed over by the previous tile: its elements are the tile's leading ones
     const uint32_t lead = H ? S.hpos[0] : wn;
@@ -397,27 +348,38 @@ __device__ __forceinline__ void run_reduce_tile(const KeyT* __restrict__ keys, u
 }
 
 // engine 1 policy: CentroidPoint of a VoxelGrid leaf (coordinate and colour channels folded as floats in run order, as
-// k_vg_reduce and PCL do).  Optionally tracks the range of combined-grid cells the emitted centroids fall in (so the
-// merge can sort compact keys).
+// PCL does).  Optionally tracks the range of combined-grid cells the emitted centroids fall in (so the merge can sort
+// compact keys).  FULL adds the min-points filter and, per record, the absolute cell key of the run's first point (z
+// shifted as loaded) and the run's length.
+template <bool FULL>
 struct VgPol {
     static constexpr bool kNeedsKey = false;
     static constexpr bool kPacked = true;
+    static constexpr bool kFilter = FULL;
     using ColT = float;
     const float4* spts;   // the segment's points when they are already in sorted order (null: gather pts[vals[pos]])
     const float4* pts; const uint32_t* vals;
     float4* out; int z_shift; bool verbatim;
     int want_cells; float icx, icz;
     int mn[3], mx[3];
+    // FULL only: the filter's threshold, the key / count outputs (each may be null) and the key's inverse leaf sizes
+    uint32_t min_points;
+    uint64_t* okeys; uint32_t* ocounts;
+    float lx_inv, ly_inv, lz_inv;
     __device__ __forceinline__ void load(uint32_t pos, float4& a, uint4&) const {
         a = spts ? __ldcs(spts + pos) : pts[vals[pos]];
         if (z_shift) a.z = __fadd_rn(a.z, 500.0f);
+    }
+    __device__ __forceinline__ bool emits(const uint32_t* keys, uint32_t pos, uint32_t n) const {
+        return vg_emits(keys, pos, n, min_points);   // k_vg_heads counts the output slots with the same predicate
     }
     __device__ __forceinline__ void start(uint32_t, float&, float&, float&, uint32_t&, float&, float&, float&,
                                           uint32_t&) const {}   // sums start at zero
     __device__ __forceinline__ void emit(uint32_t slot, uint32_t, float sx, float sy, float sz, uint32_t n, float r,
                                          float g, float b, uint32_t, uint32_t first) {
+        if (FULL && slot == kNoSlot) return;   // fewer than min_points points
         float4 o;
-        if (verbatim) {   // PCL: output = *input_
+        if (verbatim) {   // PCL: output = *input_ (the identity keys make every point its own run)
             o = spts ? spts[first] : pts[vals[first]];
         } else {
             const float fn = (float)n;
@@ -428,6 +390,12 @@ struct VgPol {
             o = make_float4(__fdiv_rn(sx, fn), __fdiv_rn(sy, fn), cz, __uint_as_float(rgb));
         }
         out[slot] = o;
+        if (FULL && okeys) {
+            float4 p = spts ? spts[first] : pts[vals[first]];
+            if (z_shift) p.z = __fadd_rn(p.z, 500.0f);
+            okeys[slot] = abs_cell_key(p.x, p.y, p.z, lx_inv, ly_inv, lz_inv);
+        }
+        if (FULL && ocounts) ocounts[slot] = n;
         if (want_cells) {
             const int ci = (int)floorf(__fmul_rn(o.x, icx)), cj = (int)floorf(__fmul_rn(o.y, icx)),
                       ck = (int)floorf(__fmul_rn(__fadd_rn(o.z, 500.0f), icz));
@@ -438,19 +406,23 @@ struct VgPol {
     }
 };
 
-// fast path of engine 1: every run is emitted (min_points <= 1), no key / count outputs.
+// engine 1's run reduction.  FULL = false: every run is emitted (min_points <= 1), no key / count outputs; only this
+// instantiation tracks the cell range and takes a batch-wide output base.  FULL = true: the min-points filter and the
+// optional key / count outputs.
 // Linear grid of tiles_ub * n_seg CTAs; work[0] is the ticket, carries follow.
 #ifndef O3R_VG_MINB
 #define O3R_VG_MINB 5
 #endif
+template <bool FULL>
 __global__ void __launch_bounds__(kThreads, O3R_VG_MINB) k_vg_reduce_w(VgArgs A, const uint32_t* __restrict__ head_off,
                                                           const uint32_t* __restrict__ head_total,
                                                           float4* __restrict__ out, uint32_t* __restrict__ seg_out_off,
                                                           int n_seg, uint32_t* __restrict__ ticket,
                                                           RunCarry* __restrict__ carries, int want_cells, float icx,
                                                           float icz, int* __restrict__ cellbb,
-                                                          const uint32_t* __restrict__ out_base) {
-    __shared__ RunSmem<uint32_t, true> S;
+                                                          const uint32_t* __restrict__ out_base,
+                                                          uint64_t* __restrict__ out_keys, uint32_t* __restrict__ out_counts) {
+    __shared__ std::conditional_t<FULL, RunSmemRanked<uint32_t, true>, RunSmem<uint32_t, true>> S;
     __shared__ int s_bb[6];
     if (threadIdx.x == 0) S.ticket = atomicAdd(ticket, 1u);
     if (threadIdx.x < 6) s_bb[threadIdx.x] = threadIdx.x < 3 ? 0x7fffffff : (int)0x80000000;
@@ -469,11 +441,12 @@ __global__ void __launch_bounds__(kThreads, O3R_VG_MINB) k_vg_reduce_w(VgArgs A,
     const int par = pl.final_parity;
     // a segment that needed no radix pass is already in order: its points are read sequentially, not gathered
     const float4* sp = pl.n_active ? nullptr : A.pts + beg;
-    VgPol pol{sp, A.pts, (par ? A.vals1 : A.vals0) + beg, out + obase, A.z_shift, A.grids && A.grids[s].passthrough,
-              want_cells, icx, icz,
-              {0x7fffffff, 0x7fffffff, 0x7fffffff}, {(int)0x80000000, (int)0x80000000, (int)0x80000000}};
-    run_reduce_tile<uint32_t, VgPol>((par ? A.keys1 : A.keys0) + beg, n, t, head_off[(size_t)s * A.tiles_ub + t], pol, S,
-                                     carries + lin);
+    VgPol<FULL> pol{sp, A.pts, (par ? A.vals1 : A.vals0) + beg, out + obase, A.z_shift, A.grids && A.grids[s].passthrough,
+                    want_cells, icx, icz,
+                    {0x7fffffff, 0x7fffffff, 0x7fffffff}, {(int)0x80000000, (int)0x80000000, (int)0x80000000},
+                    A.min_points, out_keys, out_counts, A.lx_inv, A.ly_inv, A.lz_inv};
+    run_reduce_tile<uint32_t, VgPol<FULL>>((par ? A.keys1 : A.keys0) + beg, n, t, head_off[(size_t)s * A.tiles_ub + t], pol,
+                                           S, carries + lin);
     if (want_cells) {
 #pragma unroll
         for (int a = 0; a < 3; ++a) {
@@ -670,6 +643,7 @@ template <typename KeyT, typename Items>
 struct AccPol {
     static constexpr bool kNeedsKey = true;
     static constexpr bool kPacked = Items::kPacked;
+    static constexpr bool kFilter = false;
     using ColT = uint32_t;
     Items items;
     KeyCodec kc;

@@ -101,7 +101,8 @@ def _heavy_cloud(seed, rgb_max=256, light=3000):
 
 @pytest.mark.parametrize("min_points", [1, 2])
 def test_heavy_runs_retain_downsample(min_points):
-    """RETAIN downsample: min_points 1 runs k_vg_reduce_w (tile hand-off of every heavy run), 2 runs k_vg_reduce."""
+    """RETAIN downsample through the tile hand-off of every heavy run: min_points 1 emits every run, 2 ranks the runs
+    that pass the filter."""
     pts = _heavy_cloud(5)
     got = _retain(pts, V_HEAVY, min_points, pieces=3)
     _eq(got, _oracle_retain(pts, V_HEAVY, min_points))
@@ -137,8 +138,8 @@ def _bright_cloud(seed):
 
 
 def test_bright_cell_retain_colour_matches_pcl():
-    """The RETAIN downsample folds colour channels as floats, as PCL's CentroidPoint does, whichever reduction kernel
-    runs: min_points 1 (k_vg_reduce_w) and 2 (k_vg_reduce) give the oracle's record."""
+    """The RETAIN downsample folds colour channels as floats, as PCL's CentroidPoint does, with and without the
+    min-points filter: min_points 1 and 2 give the oracle's record."""
     pts, r = _bright_cloud(7)
     assert rm.float_fold_channel(r) != rm.uint_sum_channel(r)   # the cell separates the two colour sums
     exp = _oracle_retain(pts, V_HEAVY, 1)
@@ -160,7 +161,7 @@ def _radix_cloud(n, dist, seed):
     rng = np.random.default_rng(seed)
     if dist == "distinct":         # every point its own cell
         cx = rng.permutation(n)
-    elif dist == "one":            # one cell: every pass trivial, k_vg_reduce_w reads the points in place
+    elif dist == "one":            # one cell: every pass trivial, the reduction reads the points in place
         cx = np.full(n, 5)
     elif dist == "two":            # two cells: a 1-bit key
         cx = rng.integers(0, 2, n)
