@@ -25,6 +25,7 @@
 #include <vector>
 
 #include "o3r.h"
+#include "mapfile.hpp"
 #include "ply.hpp"
 #include "png.hpp"
 #include "tmat.hpp"
@@ -56,6 +57,8 @@ struct Pose {
            imageNumbersFile = "images/image_numbers.txt";
     string imagePrefix = "images/", disparityPrefix = "disparities/", segmentlblPrefix = "segmentlabels/";
     string folder = "output/", pose_corrections_file;
+    bool save_map = false;      // --save_map: <run dir>/map.o3rmap after the last cycle
+    string resume_map_file;     // --resume_map FILE: loaded before the first cycle
     int blur_mode = O3R_BLUR_BILATERAL, device = 0;   // the reference's live filter (pose_functions.cpp:1044)
     double Q[16] = {0};
     vector<RawImageData> rawImageDataVec;
@@ -86,6 +89,8 @@ void Pose::printUsage() {
             "      --disparity_prefix P --segmentlbl_prefix P --output DIR --calib FILE\n"
             "  extensions: --blur_mode bilateral|median|box (default bilateral = the reference) --pose_corrections FILE --device N\n"
             "              --no_sor (skip the StatisticalOutlierRemoval the reference applies per frame when jump_pixels > 0)\n"
+            "              --save_map (write the resident map to <run dir>/map.o3rmap after the last cycle)\n"
+            "              --resume_map FILE (continue the map of a map.o3rmap saved with the same --voxel_size and --dont_downsample)\n"
             "  not in this driver (host-side tools of the reference): --visualize --align_point_cloud --smooth_surface\n"
             "      --mesh_surface --segment_cloud --segment_cloud_only --displayUAVPositions\n";
 }
@@ -135,6 +140,8 @@ int Pose::parseCmdArgs(int argc, char** argv) {
         else if (a == "--pose_corrections") pose_corrections_file = need("file");
         else if (a == "--device") device = atoi(need("n"));
         else if (a == "--no_sor") sor = false;
+        else if (a == "--save_map") save_map = true;
+        else if (a == "--resume_map") resume_map_file = need("file");
         else if (a == "--blur_mode") { const string m = need("mode"); blur_mode = (m == "box") ? O3R_BLUR_BOX : (m == "median") ? O3R_BLUR_MEDIAN : O3R_BLUR_BILATERAL; }
         else {
             cout << atoi(argv[i]) << endl;
@@ -349,6 +356,20 @@ int Pose::run() {
     if (do_preview && o3r_cloud_track_changes(ctx, 1) != O3R_OK) {
         cerr << "o3r_cloud_track_changes: " << o3r_last_error(ctx) << endl; o3r_destroy(ctx); return 1;
     }
+    if (!resume_map_file.empty()) {   // after the tracking is on: the first preview.ply already shows the resumed map
+        const uint32_t kind = dont_downsample ? host::MAP_KIND_POINTS : host::MAP_KIND_CELLS;
+        vector<uint8_t> recs;
+        uint64_t n_rec = 0;
+        string err;
+        if (!host::load_map(resume_map_file, kind, voxel_size, recs, &n_rec, &err)) {
+            cerr << "--resume_map: " << err << endl; o3r_destroy(ctx); return 1;
+        }
+        const int rc = kind == host::MAP_KIND_CELLS ? o3r_cloud_import_cells(ctx, (const o3r_cell*)recs.data(), n_rec)
+                                                    : o3r_cloud_append(ctx, (const o3r_point*)recs.data(), n_rec);
+        if (rc) { cerr << "--resume_map: " << resume_map_file << ": " << o3r_last_error(ctx) << endl; o3r_destroy(ctx); return 1; }
+        for (ostream* o : {(ostream*)&cout, (ostream*)&log_file})
+            *o << "Resumed map " << resume_map_file << ": " << n_rec << (kind == host::MAP_KIND_CELLS ? " cells" : " points") << endl;
+    }
     std::map<uint64_t, o3r_point> preview_map;
     vector<o3r_point> chg_pts;
     vector<uint64_t> chg_keys;
@@ -459,6 +480,18 @@ int Pose::run() {
            << "\njump_pixels " << jump_pixels << "\nseq_len " << seq_len << "\nrange_width " << range_width
            << "\nblur_kernel " << blur_kernel << "\nvoxel_size " << voxel_size
            << "\nmin_points_per_voxel " << min_points_per_voxel << "\ndist_nearby " << dist_nearby << endl;
+    if (save_map) {   // the resident state itself (cells with their sums and counts, or cloud_big), before the final downsample
+        const uint32_t kind = dont_downsample ? host::MAP_KIND_POINTS : host::MAP_KIND_CELLS;
+        size_t m = 0;
+        int rc = kind == host::MAP_KIND_CELLS ? o3r_cloud_export_cells(ctx, nullptr, 0, &m) : o3r_cloud_export_points(ctx, nullptr, 0, &m);
+        vector<uint8_t> recs(std::max<size_t>(m, 1) * host::map_record_bytes(kind));
+        if (!rc) rc = kind == host::MAP_KIND_CELLS ? o3r_cloud_export_cells(ctx, (o3r_cell*)recs.data(), m, &m)
+                                                   : o3r_cloud_export_points(ctx, (o3r_point*)recs.data(), m, &m);
+        if (rc) { cerr << "--save_map: " << o3r_last_error(ctx) << endl; o3r_destroy(ctx); return 1; }
+        const string path = folder + "map.o3rmap";
+        if (!host::save_map(path, kind, recs.data(), m, voxel_size)) { cerr << "--save_map: cannot write " << path << endl; o3r_destroy(ctx); return 1; }
+        cerr << "Saved map with " << m << (kind == host::MAP_KIND_CELLS ? " cells" : " points") << " to " << path << endl;
+    }
     size_t n = 0;
     if (!dont_downsample) cout << "downsample before saving..." << endl;
     int rc = o3r_cloud_downsample(ctx, nullptr, 0, &n);       // pose.cpp:527-536

@@ -42,6 +42,16 @@ typedef struct o3r_point {
     uint32_t rgb;
 } o3r_point;
 
+/* Cell record: partial sums on the combined grid.  Exchanged between ranks (o3r_exchange_cycle) and, bit for bit the
+ * resident accumulators, the record of a map checkpoint (o3r_cloud_export_cells / o3r_cloud_import_cells). */
+typedef struct o3r_cell {
+    uint64_t key;            /* (k+2^20)<<42 | (j+2^20)<<21 | (i+2^20) */
+    float    sx, sy, sz;     /* sums of x, y, z+500 (float)            */
+    uint32_t n;              /* points in the partial                   */
+    uint32_t sr, sg, sb;     /* colour sums                             */
+    uint32_t pad;
+} o3r_cell;                  /* 40 bytes */
+
 /* disparity sample formats.  U8 is the reference's native format (pose_functions.cpp:548,1104);
  * F64 is the plane-fitted image of --use_segment_labels (pose_functions.cpp:905,1102);
  * U16 (value / disp_divisor, the commented variant at pose_functions.cpp:1102) and F32 are the
@@ -254,6 +264,34 @@ int o3r_cloud_changes(o3r_ctx* ctx, o3r_point* out, uint64_t* keys, uint32_t* co
 int o3r_cloud_changes_dev(o3r_ctx* ctx, const o3r_point** dev_out, const uint64_t** dev_keys,
                           const uint32_t** dev_counts, size_t* n_out);
 
+/* Checkpoints of the resident map: a map outlives its context (a survey resumed after a restart, two flights merged, a
+ * shard moved to another number of GPUs).  The library does no file I/O; host/mapfile.hpp and mapfile.py define a file.
+ *   - o3r_cloud_export_cells (O3R_MERGE_ACCUMULATE, _TILED, _FUSED without dont_downsample): every resident cell in ascending
+ *     key, cells below min_points_per_voxel included (they are state: a later cycle can lift them over the threshold).  Each
+ *     field is a bit copy of the accumulators; pad is 0.  Query, then fill, as o3r_cloud_downsample: out = NULL with cap = 0
+ *     reports *n_out; a short buffer returns O3R_ERR_CAPACITY with *n_out set.  With a communicator each rank exports the
+ *     shard it owns; a batch still waiting for its o3r_exchange_cycle is not in that shard yet.
+ *   - o3r_cloud_import_cells (same modes): merges the n records as ONE cycle through the ordinary merge.  A resident cell,
+ *     and a key that appears more than once, gets the imported sums added in input order after the resident sums; importing
+ *     an export into an empty context reproduces it bit for bit, and a resumed run ends where the uninterrupted one does: bit
+ *     for bit in O3R_MERGE_ACCUMULATE; in _TILED / _FUSED bit for bit when the batches are merged the same way, but these
+ *     modes pick the engine (and whether to pre-reduce) from the context's own batch history, which a checkpoint does not
+ *     carry, so a resumed map may differ in the centroids within the mode's float-reassociation contract.  Host pointer, copied before the call returns.  The
+ *     records are staged in a buffer of their own: the last batch (o3r_last_batch_points, a pending o3r_exchange_cycle) is
+ *     left intact.  All or nothing: every record is checked on the device first, and if any is refused the call returns
+ *     O3R_ERR_INVALID, merges nothing, and o3r_last_error names the first refused index and its reasons.  A record is
+ *     refused when bit 63 of its key is set, a 21-bit key field is 0 (outside +-(2^20 - 1) cells), n == 0, sx / sy / sz is
+ *     not finite, a colour sum exceeds 255 * n, pad != 0, or (with a communicator) hash64(key) % world != rank.  Whether a
+ *     centroid lies inside its key's cell is not checked: rounding of a genuine sum / n can land it across the boundary.
+ *     With change tracking on, the cells the import grew become pending changes like those of any merge.
+ *   - o3r_cloud_export_points (O3R_MERGE_RETAIN, or any mode with dont_downsample): cloud_big in order, exactly; query then
+ *     fill as above.  o3r_cloud_append is the matching import.
+ *   - O3R_ERR_UNSUPPORTED: the cell calls outside their modes, o3r_cloud_export_points outside its modes or with a
+ *     communicator attached (a sharded point cloud carries frame-order tags a checkpoint cannot carry). */
+int o3r_cloud_export_cells(o3r_ctx* ctx, o3r_cell* out, size_t cap, size_t* n_out);
+int o3r_cloud_import_cells(o3r_ctx* ctx, const o3r_cell* cells, size_t n);
+int o3r_cloud_export_points(o3r_ctx* ctx, o3r_point* out, size_t cap, size_t* n_out);
+
 /* ---- stand-alone stages (parity probes; same kernels as above) ------------------------------- */
 
 /* pcl::VoxelGrid<PointXYZRGB>::filter on a host cloud: leaf (lx,ly,lz) as PCL's setLeafSize floats,
@@ -297,15 +335,6 @@ int o3r_frame_mask(o3r_ctx* ctx, const o3r_frame* frame, int disp_type,
                    uint8_t* mask, size_t cap, size_t* n_scanned);
 
 /* ---- multi-GPU exchange (SURVEY §8e) ---------------------------------------------------------- */
-
-/* Cell record exchanged between ranks: partial sums on the combined grid. */
-typedef struct o3r_cell {
-    uint64_t key;            /* (k+2^20)<<42 | (j+2^20)<<21 | (i+2^20) */
-    float    sx, sy, sz;     /* sums of x, y, z+500 (float)            */
-    uint32_t n;              /* points in the partial                   */
-    uint32_t sr, sg, sb;     /* colour sums                             */
-    uint32_t pad;
-} o3r_cell;                  /* 40 bytes */
 
 /* Parity probe for O3R_MERGE_ACCUMULATE_FUSED: when set, the fused engine also stores every per-frame voxel centroid of
  * the batch, in no particular order, and o3r_last_batch_points returns that multiset. */

@@ -209,6 +209,7 @@ struct o3r_ctx {
         DevBuf* b[] = {&chg_keys[0], &chg_keys[1], &chg_cnt, &chg_off, &chg_part, &chg_pos, &chg_out, &chg_okeys, &chg_ocnt};
         for (DevBuf* x : b) x->release();
     }
+    DevBuf ck_cells, ck_res;          // checkpoints (host_checkpoint.cuh): packed / staged o3r_cell records, the import check's result
     bool keep_frame_voxels = false;   // parity probe: the bucket engine also writes every per-frame voxel centroid (any order)
     size_t last_partials = 0;
     bool last_has_partials = false;

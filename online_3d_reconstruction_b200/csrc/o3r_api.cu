@@ -8,6 +8,7 @@
 #include "host_comm.cuh"
 #include "host_retain.cuh"
 #include "host_changes.cuh"
+#include "host_checkpoint.cuh"
 
 
 // =====================================================================================================================
@@ -139,7 +140,8 @@ void o3r_destroy(o3r_ctx* ctx) {
                       &ctx->crgb, &ctx->partials, &ctx->pr_status, &ctx->bk_frames, &ctx->bk_counts, &ctx->bk_nl, &ctx->bk_pts, &ctx->bk_pos,
                       &ctx->bk_status, &ctx->bk_misc, &ctx->bk_stray, &ctx->tv_tiles, &ctx->tv_misc, &ctx->tv_scratch, &ctx->x_send, &ctx->x_recv, &ctx->x_list, &ctx->sor_hard, &ctx->sor_pts, &ctx->sor_off, &ctx->sor_dist, &ctx->sor_grids,
                       &ctx->sor_pgrids, &ctx->sor_rows, &ctx->sor_thr, &ctx->sor_skeys, &ctx->sor_svals, &ctx->sor_cnt, &ctx->sor_cntoff, &ctx->new_cnt, &ctx->new_off, &ctx->new_keys, &ctx->okeys, &ctx->cloud,
-                      &ctx->rt_agree, &ctx->rt_ftab, &ctx->rt_tags, &ctx->rt_send, &ctx->rt_recv, &ctx->rt_pts, &ctx->rt_out};
+                      &ctx->rt_agree, &ctx->rt_ftab, &ctx->rt_tags, &ctx->rt_send, &ctx->rt_recv, &ctx->rt_pts, &ctx->rt_out,
+                      &ctx->ck_cells, &ctx->ck_res};
     for (DevBuf* b : bufs) b->release();
     ctx->chg_release();
     for (auto& r : ctx->prof) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
@@ -533,6 +535,29 @@ int o3r_cloud_changes_dev(o3r_ctx* ctx, const o3r_point** dev_out, const uint64_
     if (dev_counts) *dev_counts = ctx->chg_ocnt.as<const uint32_t>();
     chg_reset(ctx, false);   // (the records stay in the context's buffers until the next call)
     return O3R_OK;
+}
+
+int o3r_cloud_export_cells(o3r_ctx* ctx, o3r_cell* out, size_t cap, size_t* n_out) {
+    if (!ctx || !n_out) return O3R_ERR_INVALID;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    CU(cudaSetDevice(ctx->p.device));
+    *n_out = 0;
+    return export_cells_impl(ctx, out, cap, n_out);
+}
+
+int o3r_cloud_import_cells(o3r_ctx* ctx, const o3r_cell* cells, size_t n) {
+    if (!ctx || (n && !cells)) return O3R_ERR_INVALID;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    CU(cudaSetDevice(ctx->p.device));
+    return import_cells_impl(ctx, cells, n);
+}
+
+int o3r_cloud_export_points(o3r_ctx* ctx, o3r_point* out, size_t cap, size_t* n_out) {
+    if (!ctx || !n_out) return O3R_ERR_INVALID;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    CU(cudaSetDevice(ctx->p.device));
+    *n_out = 0;
+    return export_points_impl(ctx, out, cap, n_out);
 }
 
 int o3r_voxel_grid(o3r_ctx* ctx, const o3r_point* pts, size_t n, float lx, float ly, float lz, unsigned min_points,

@@ -16,6 +16,7 @@ SYMBOLS = [
     "o3r_frame_cloud", "o3r_frames_cloud", "o3r_frames_cloud_dev", "o3r_frames_prefetch", "o3r_frames_prefetch_cancel", "o3r_last_batch_points",
     "o3r_cloud_transform", "o3r_cloud_append", "o3r_cloud_downsample", "o3r_cloud_downsample_dev", "o3r_cloud_size",
     "o3r_cloud_clear", "o3r_cloud_track_changes", "o3r_cloud_changes", "o3r_cloud_changes_dev",
+    "o3r_cloud_export_cells", "o3r_cloud_import_cells", "o3r_cloud_export_points",
     "o3r_voxel_grid", "o3r_blur_u8", "o3r_frame_mask", "o3r_disp_variance", "o3r_plane_fit", "o3r_sor", "o3r_last_batch_partials",
     "o3r_set_keep_frame_voxels", "o3r_last_batch_engine",
     "o3r_comm_unique_id", "o3r_comm_init", "o3r_comm_attach", "o3r_comm_destroy", "o3r_exchange_cycle",
@@ -67,6 +68,9 @@ def load():
     L.o3r_cloud_track_changes.argtypes = [vp, C.c_int]
     L.o3r_cloud_changes.argtypes = [vp, vp, vp, vp, sz, szp]
     L.o3r_cloud_changes_dev.argtypes = [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), szp]
+    L.o3r_cloud_export_cells.argtypes = [vp, vp, sz, szp]
+    L.o3r_cloud_import_cells.argtypes = [vp, vp, sz]
+    L.o3r_cloud_export_points.argtypes = [vp, vp, sz, szp]
     L.o3r_voxel_grid.argtypes = [vp, vp, sz, C.c_float, C.c_float, C.c_float, C.c_uint, vp, sz, szp, vp, vp,
                                  C.POINTER(C.c_int)]
     L.o3r_blur_u8.argtypes = [vp, vp, sz, C.c_int, C.c_int, C.c_int, C.c_int, vp, sz]

@@ -19,6 +19,8 @@ from . import abi, lib
 class Pose:
     """One reconstruction context (= the read-only `Pose` state after populateData + the global cloud)."""
 
+    world, rank = 1, 0   # the communicator this context is part of (commInit); 1, 0 without one
+
     def __init__(self, params=None, **kw):
         self._L = lib.load()
         self.params = params if params is not None else abi.make_params(**kw)
@@ -205,6 +207,29 @@ class Pose:
         self._check(self._L.o3r_cloud_changes_dev(self._h, C.byref(pts), C.byref(keys), C.byref(counts), C.byref(n)))
         return pts.value, keys.value, counts.value, n.value
 
+    def exportCells(self):
+        """Every resident cell (accumulate modes), ascending key, cells below min_points_per_voxel included: a bit copy of
+        the accumulators as an abi.CELL array.  With a communicator: the shard this rank owns."""
+        n = C.c_size_t(0)
+        self._check(self._L.o3r_cloud_export_cells(self._h, None, 0, C.byref(n)))
+        out = np.empty(max(1, n.value), dtype=abi.CELL)
+        self._check(self._L.o3r_cloud_export_cells(self._h, out.ctypes.data, out.size, C.byref(n)))
+        return out[:n.value]
+
+    def importCells(self, cells):
+        """Merges abi.CELL records into the resident map as one cycle (sums added in input order after the resident ones).
+        All or nothing: a refused record raises O3RError (O3R_ERR_INVALID) naming its index, and nothing is merged."""
+        cells = np.ascontiguousarray(cells, dtype=abi.CELL)
+        self._check(self._L.o3r_cloud_import_cells(self._h, cells.ctypes.data, cells.size))
+
+    def exportPoints(self):
+        """cloud_big in order, exactly (MERGE_RETAIN or dont_downsample, no communicator); appendPoints is the import."""
+        n = C.c_size_t(0)
+        self._check(self._L.o3r_cloud_export_points(self._h, None, 0, C.byref(n)))
+        out = np.empty(max(1, n.value), dtype=abi.POINT)
+        self._check(self._L.o3r_cloud_export_points(self._h, out.ctypes.data, out.size, C.byref(n)))
+        return out[:n.value]
+
     # -- stand-alone stages --------------------------------------------------------------------------------
     def voxelGrid(self, pts, leaf, min_points=0):
         """pcl::VoxelGrid on a host cloud -> (points, keys u64, counts u32, passthrough)."""
@@ -271,9 +296,11 @@ class Pose:
         each rank keeps the points of its frames (f mod world == rank), slot_cells is not used, and downsamplePtCloud
         becomes the collective.  All ranks make the same sequence of createCycleClouds / transformPtCloud / clearCloud calls."""
         self._check(self._L.o3r_comm_init(self._h, world, rank, C.c_char_p(uid), slot_cells))
+        self.world, self.rank = world, rank
 
     def commDestroy(self):
         self._check(self._L.o3r_comm_destroy(self._h))
+        self.world, self.rank = 1, 0
 
     def exchangeCycle(self):
         """Collective, asynchronous: partial cells of the last cycle -> owners (grouped ncclSend/ncclRecv) -> merge.
