@@ -117,6 +117,7 @@ NcclApi* nccl_api() {
 
 #define NC(call)                                                                                      \
     do {                                                                                              \
+        if (ctx->fq.L.n) { int rcf_ = fill_flush(ctx); if (rcf_) return rcf_; }                       \
         ncclResult_t r_ = (call);                                                                     \
         if (r_ != ncclSuccess)                                                                        \
             return ctx->fail(O3R_ERR_CUDA, std::string("NCCL error at " #call ": ") + N->GetErrorString(r_)); \

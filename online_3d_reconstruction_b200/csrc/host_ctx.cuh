@@ -42,6 +42,10 @@ struct Tr {
 struct DevBuf {
     void* p = nullptr;
     size_t cap = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf&) = delete;
+    DevBuf& operator=(const DevBuf&) = delete;
+    ~DevBuf() { release(); }
     template <typename T> T* as() const { return reinterpret_cast<T*>(p); }
     cudaError_t ensure(size_t bytes, cudaStream_t st = nullptr, size_t preserve = 0) {
         if (bytes <= cap) return cudaSuccess;
@@ -64,8 +68,10 @@ struct DevBuf {
 };
 
 // Small device fills (zeroed counters and tables, bbox / cell-range initial values) are not launched one by one: they queue up
-// in the context and leave as ONE kernel in front of the next stream operation (every launch and CUDA call of the library goes
-// through LAUNCH / CU / NC, which flush the queue first), so stream order is what it would have been with separate kernels.
+// in the context and leave as ONE kernel in front of the next stream operation (every launch and CUDA / NCCL call of the
+// library goes through LAUNCH / CU / NC, which flush the queue first), so stream order is what it would have been with
+// separate kernels.  api() selects the context's device before anything is queued or flushed, and flushes what is left
+// before the call returns: no fill outlives the call that queued it.
 struct FillList { uint32_t* p[8]; unsigned long long words[8]; int kind[8]; int n; };
 enum { FILL_ZERO = 0, FILL_BBOX = 1, FILL_CELLBB = 2 };   // bbox: {~0, ~0, ~0, 0, 0, 0} per 6 words; cell range: {INT_MAX x3, INT_MIN x3}
 struct FillQueue {
@@ -241,6 +247,21 @@ struct o3r_ctx {
         err = buf;
         return O3R_ERR_CUDA;
     }
+    // (o3r_destroy makes the device current and drains the streams first; the DevBuf members free themselves after this)
+    ~o3r_ctx() {
+        for (auto& pf : prefetch) if (pf.ev) cudaEventDestroy(pf.ev);
+        for (auto& r : prof) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
+        for (auto e : ev_pool) cudaEventDestroy(e);
+        if (h_counters) cudaFreeHost(h_counters);
+        if (h_nres) cudaFreeHost(h_nres);
+        if (ev_nres) cudaEventDestroy(ev_nres);
+        if (h_offs) cudaFreeHost(h_offs);
+        for (auto e : chunk_ev) cudaEventDestroy(e);
+        if (ev_copy2) cudaEventDestroy(ev_copy2);
+        if (st_copy2) cudaStreamDestroy(st_copy2);
+        if (st_copy) cudaStreamDestroy(st_copy);
+        if (st) cudaStreamDestroy(st);
+    }
 };
 
 int fill_flush(o3r_ctx* ctx);
@@ -321,6 +342,23 @@ int fill_flush(o3r_ctx* ctx) {
     LAUNCH_N("k_fill", k_fill_list, g, kThreads, 0, L);
     return O3R_OK;
 }
+
+// Every C-ABI entry point that takes a context runs its body through api(): under the context's lock, with the context's
+// device current (a raw call: CU would flush queued fills first, while another device may still be current), and with
+// whatever fills the body left queued flushed before it returns.  A failed body's code and message are what the call
+// returns, whatever the flush does.
+template <typename F>
+int api(o3r_ctx* ctx, F&& body) {
+    if (!ctx) return O3R_ERR_INVALID;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    const cudaError_t e = cudaSetDevice(ctx->p.device);
+    if (e != cudaSuccess) return ctx->fail_cuda(e, "cudaSetDevice(ctx->p.device)", __FILE__, __LINE__);
+    const int rc = body();
+    if (!rc) return fill_flush(ctx);
+    if (ctx->fq.L.n) { const std::string err = ctx->err; fill_flush(ctx); ctx->err = err; }
+    return rc;
+}
+
 namespace {
 int fill_queue(o3r_ctx* ctx, void* dst, size_t bytes, int kind) {
     if (bytes == 0) return O3R_OK;

@@ -186,7 +186,6 @@ int retain_downsample_sharded(o3r_ctx* ctx, const float4** res, size_t* m) {
         e[RT_W_ERR] = 1;
         { int rcu = rt_put_words(ctx, w, e, kRtWords); if (rcu) return rcu; }
     }
-    { int rcf = fill_flush(ctx); if (rcf) return rcf; }
     NC(N->AllReduce(w, w, kRtWords, ncclUint32, ncclMax, comm, ctx->st));
     uint32_t hw[kRtWords] = {};
     GridParams G;

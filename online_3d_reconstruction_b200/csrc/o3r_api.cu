@@ -126,36 +126,7 @@ void o3r_destroy(o3r_ctx* ctx) {
     if (ctx->st_copy) cudaStreamSynchronize(ctx->st_copy);
     if (ctx->st) cudaStreamSynchronize(ctx->st);
     if (ctx->comm && ctx->comm_owned && nccl_api()->CommDestroy) nccl_api()->CommDestroy((ncclComm_t)ctx->comm);
-    ctx->comm = nullptr;
-    for (auto& pf : ctx->prefetch) if (pf.ev) cudaEventDestroy(pf.ev);
-    DevBuf* bufs[] = {&ctx->lut_r, &ctx->lut_z, &ctx->d_disp, &ctx->stg[0].disp, &ctx->stg[0].bgr, &ctx->stg[0].labels,
-                      &ctx->stg[0].coef, &ctx->stg[0].kp, &ctx->stg[1].disp, &ctx->stg[1].bgr, &ctx->stg[1].labels,
-                      &ctx->stg[1].coef, &ctx->stg[1].kp,
-                      &ctx->d_frames, &ctx->d_blur, &ctx->d_blurjobs, &ctx->bil_lut, &ctx->pp_labels, &ctx->pp_disp, &ctx->pp_sums,
-                      &ctx->pp_rows, &ctx->pp_coef, &ctx->tile_cnt, &ctx->tile_off, &ctx->bbox,
-                      &ctx->frame_off, &ctx->grids, &ctx->counters, &ctx->pts, &ctx->sortbuf, &ctx->hist,
-                      &ctx->plan_all, &ctx->plan_v2, &ctx->ghist, &ctx->head_cnt, &ctx->head_off, &ctx->vox,
-                      &ctx->vox_off, &ctx->seg2, &ctx->tmat, &ctx->mask, &ctx->runwork, &ctx->spts, &ctx->res_keys[0], &ctx->res_keys[1],
-                      &ctx->res_acc[0], &ctx->res_acc[1], &ctx->res_rgb[0], &ctx->res_rgb[1], &ctx->ckey, &ctx->cacc,
-                      &ctx->crgb, &ctx->partials, &ctx->pr_status, &ctx->bk_frames, &ctx->bk_counts, &ctx->bk_nl, &ctx->bk_pts, &ctx->bk_pos,
-                      &ctx->bk_status, &ctx->bk_misc, &ctx->bk_stray, &ctx->tv_tiles, &ctx->tv_misc, &ctx->tv_scratch, &ctx->x_send, &ctx->x_recv, &ctx->x_list, &ctx->sor_hard, &ctx->sor_pts, &ctx->sor_off, &ctx->sor_dist, &ctx->sor_grids,
-                      &ctx->sor_pgrids, &ctx->sor_rows, &ctx->sor_thr, &ctx->sor_skeys, &ctx->sor_svals, &ctx->sor_cnt, &ctx->sor_cntoff, &ctx->new_cnt, &ctx->new_off, &ctx->new_keys, &ctx->okeys, &ctx->cloud,
-                      &ctx->rt_agree, &ctx->rt_ftab, &ctx->rt_tags, &ctx->rt_send, &ctx->rt_recv, &ctx->rt_pts, &ctx->rt_out,
-                      &ctx->ck_cells, &ctx->ck_res};
-    for (DevBuf* b : bufs) b->release();
-    ctx->chg_release();
-    for (auto& r : ctx->prof) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
-    for (auto e : ctx->ev_pool) cudaEventDestroy(e);
-    if (ctx->h_counters) cudaFreeHost(ctx->h_counters);
-    if (ctx->h_nres) cudaFreeHost(ctx->h_nres);
-    if (ctx->ev_nres) cudaEventDestroy(ctx->ev_nres);
-    if (ctx->h_offs) cudaFreeHost(ctx->h_offs);
-    for (auto e : ctx->chunk_ev) cudaEventDestroy(e);
-    if (ctx->ev_copy2) cudaEventDestroy(ctx->ev_copy2);
-    if (ctx->st_copy2) cudaStreamDestroy(ctx->st_copy2);
-    if (ctx->st_copy) cudaStreamDestroy(ctx->st_copy);
-    if (ctx->st) cudaStreamDestroy(ctx->st);
-    delete ctx;
+    delete ctx;   // (~o3r_ctx: events, pinned memory, streams, then every device buffer)
 }
 
 uint64_t o3r_launch_count(const o3r_ctx* ctx) { return ctx ? ctx->launches : 0; }
@@ -164,51 +135,54 @@ int o3r_last_batch_engine(const o3r_ctx* ctx) { return ctx ? (int)ctx->last_engi
 void* o3r_stream(o3r_ctx* ctx) { return ctx ? (void*)ctx->st : nullptr; }
 
 int o3r_sync(o3r_ctx* ctx) {
-    if (!ctx) return O3R_ERR_INVALID;
-    CU(cudaStreamSynchronize(ctx->st));
-    return O3R_OK;
+    return api(ctx, [&] {
+        CU(cudaStreamSynchronize(ctx->st));
+        return O3R_OK;
+    });
 }
 
 int o3r_profile(o3r_ctx* ctx, int enable) {
-    if (!ctx) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaStreamSynchronize(ctx->st));
-    for (auto& r : ctx->prof) { ctx->ev_pool.push_back(r.a); ctx->ev_pool.push_back(r.b); }
-    ctx->prof.clear();
-    ctx->profiling = enable != 0;
-    return O3R_OK;
+    return api(ctx, [&] {
+        CU(cudaStreamSynchronize(ctx->st));
+        for (auto& r : ctx->prof) { ctx->ev_pool.push_back(r.a); ctx->ev_pool.push_back(r.b); }
+        ctx->prof.clear();
+        ctx->profiling = enable != 0;
+        return O3R_OK;
+    });
 }
 
 int o3r_profile_read(o3r_ctx* ctx, char* buf, size_t cap) {
-    if (!ctx || !buf || cap == 0) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaStreamSynchronize(ctx->st));
-    struct Agg { std::string name; uint64_t n; double ms; };
-    std::vector<Agg> agg;
-    for (auto& r : ctx->prof) {
-        float ms = 0.f;
-        cudaEventElapsedTime(&ms, r.a, r.b);
-        std::string nm = r.name;
-        size_t i = 0;
-        for (; i < agg.size(); ++i) if (agg[i].name == nm) break;
-        if (i == agg.size()) agg.push_back({nm, 0, 0.0});
-        agg[i].n += 1; agg[i].ms += ms;
-    }
-    std::string out;
-    char line[256];
-    for (auto& a : agg) {
-        snprintf(line, sizeof(line), "%s\t%llu\t%.6f\n", a.name.c_str(), (unsigned long long)a.n, a.ms);
-        out += line;
-    }
-    if (out.size() + 1 > cap) return ctx->fail(O3R_ERR_CAPACITY, "profile buffer too small");
-    memcpy(buf, out.c_str(), out.size() + 1);
-    return O3R_OK;
+    if (!buf || cap == 0) return O3R_ERR_INVALID;
+    return api(ctx, [&] {
+        CU(cudaStreamSynchronize(ctx->st));
+        struct Agg { std::string name; uint64_t n; double ms; };
+        std::vector<Agg> agg;
+        for (auto& r : ctx->prof) {
+            float ms = 0.f;
+            cudaEventElapsedTime(&ms, r.a, r.b);
+            std::string nm = r.name;
+            size_t i = 0;
+            for (; i < agg.size(); ++i) if (agg[i].name == nm) break;
+            if (i == agg.size()) agg.push_back({nm, 0, 0.0});
+            agg[i].n += 1; agg[i].ms += ms;
+        }
+        std::string out;
+        char line[256];
+        for (auto& a : agg) {
+            snprintf(line, sizeof(line), "%s\t%llu\t%.6f\n", a.name.c_str(), (unsigned long long)a.n, a.ms);
+            out += line;
+        }
+        if (out.size() + 1 > cap) return ctx->fail(O3R_ERR_CAPACITY, "profile buffer too small");
+        memcpy(buf, out.c_str(), out.size() + 1);
+        return O3R_OK;
+    });
 }
 
 int o3r_set_keep_frame_voxels(o3r_ctx* ctx, int keep) {
-    if (!ctx) return O3R_ERR_INVALID;
-    ctx->keep_frame_voxels = keep != 0;
-    return O3R_OK;
+    return api(ctx, [&] {
+        ctx->keep_frame_voxels = keep != 0;
+        return O3R_OK;
+    });
 }
 
 void* o3r_host_alloc(size_t bytes) {
@@ -219,150 +193,144 @@ void* o3r_host_alloc(size_t bytes) {
 void o3r_host_free(void* p) { if (p) cudaFreeHost(p); }
 
 int o3r_frames_cloud_dev(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_type, uint32_t* frame_counts) {
-    if (!ctx || (n > 0 && !frames)) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    return frames_cloud_impl(ctx, frames, n, disp_type, frame_counts, BatchOpts(), false);
+    if (n > 0 && !frames) return O3R_ERR_INVALID;
+    return api(ctx, [&] { return frames_cloud_impl(ctx, frames, n, disp_type, frame_counts, BatchOpts(), false); });
 }
 
 int o3r_frames_cloud(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_type, uint32_t* frame_counts) {
-    if (!ctx || (n > 0 && !frames)) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    return frames_cloud_impl(ctx, frames, n, disp_type, frame_counts, BatchOpts(), true);
+    if (n > 0 && !frames) return O3R_ERR_INVALID;
+    return api(ctx, [&] { return frames_cloud_impl(ctx, frames, n, disp_type, frame_counts, BatchOpts(), true); });
 }
 
 int o3r_frames_prefetch(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_type) {
-    if (!ctx || n <= 0 || !frames) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    if (disp_type < 0 || disp_type > 3) return ctx->fail(O3R_ERR_INVALID, "bad disp_type");
-    const o3r_params& p = ctx->p;
-    const bool label_mode = p.use_segment_labels && frames[0].labels && frames[0].plane_coef;
-    for (int i = 0; i < n; ++i)
-        if (!frames[i].bgr || (!frames[i].disp && !label_mode) || (label_mode && (!frames[i].labels || !frames[i].plane_coef)))
-            return ctx->fail(O3R_ERR_INVALID, "frame without disparity/colour");
-    int rc = flush_deferred_prefetch(ctx);   // at most one request waits; an older one goes out now
-    if (rc) return rc;
-    ctx->deferred.frames.assign(frames, frames + n);
-    ctx->deferred.disp_type = disp_type;
-    ctx->deferred.pending = true;
-    return O3R_OK;
+    if (n <= 0 || !frames) return O3R_ERR_INVALID;
+    return api(ctx, [&] {
+        if (disp_type < 0 || disp_type > 3) return ctx->fail(O3R_ERR_INVALID, "bad disp_type");
+        const o3r_params& p = ctx->p;
+        const bool label_mode = p.use_segment_labels && frames[0].labels && frames[0].plane_coef;
+        for (int i = 0; i < n; ++i)
+            if (!frames[i].bgr || (!frames[i].disp && !label_mode) || (label_mode && (!frames[i].labels || !frames[i].plane_coef)))
+                return ctx->fail(O3R_ERR_INVALID, "frame without disparity/colour");
+        int rc = flush_deferred_prefetch(ctx);   // at most one request waits; an older one goes out now
+        if (rc) return rc;
+        ctx->deferred.frames.assign(frames, frames + n);
+        ctx->deferred.disp_type = disp_type;
+        ctx->deferred.pending = true;
+        return O3R_OK;
+    });
 }
 
 int o3r_frames_prefetch_cancel(o3r_ctx* ctx) {
-    if (!ctx) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    ctx->deferred.pending = false;           // recorded but not issued: nothing will ever read those buffers
-    ctx->deferred.frames.clear();
-    CU(cudaStreamSynchronize(ctx->st_copy2));   // copies already in flight finish reading the host buffers here
-    CU(cudaStreamSynchronize(ctx->st_copy));
-    for (auto& pf : ctx->prefetch) pf.valid = false;
-    return O3R_OK;
+    return api(ctx, [&] {
+        ctx->deferred.pending = false;           // recorded but not issued: nothing will ever read those buffers
+        ctx->deferred.frames.clear();
+        CU(cudaStreamSynchronize(ctx->st_copy2));   // copies already in flight finish reading the host buffers here
+        CU(cudaStreamSynchronize(ctx->st_copy));
+        for (auto& pf : ctx->prefetch) pf.valid = false;
+        return O3R_OK;
+    });
 }
 
 int o3r_frame_cloud(o3r_ctx* ctx, const o3r_frame* frame, int disp_type, o3r_point* out, size_t cap, size_t* n_out) {
-    if (!ctx || !frame) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    if (n_out) *n_out = 0;
-    BatchOpts opt;
-    opt.merge = false;
-    int rc = frames_cloud_impl(ctx, frame, 1, disp_type, nullptr, opt, true);
-    if (rc) return rc;
-    const float4* src = ctx->last_is_vox ? ctx->vox.as<float4>() : ctx->pts.as<float4>();
-    return copy_out(ctx, src, ctx->last_total, out, cap, n_out);
+    if (!frame) return O3R_ERR_INVALID;
+    return api(ctx, [&] {
+        if (n_out) *n_out = 0;
+        BatchOpts opt;
+        opt.merge = false;
+        int rc = frames_cloud_impl(ctx, frame, 1, disp_type, nullptr, opt, true);
+        if (rc) return rc;
+        const float4* src = ctx->last_is_vox ? ctx->vox.as<float4>() : ctx->pts.as<float4>();
+        return copy_out(ctx, src, ctx->last_total, out, cap, n_out);
+    });
 }
 
 int o3r_frame_mask(o3r_ctx* ctx, const o3r_frame* frame, int disp_type, uint8_t* mask, size_t cap, size_t* n_scanned) {
-    if (!ctx || !frame) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    if (n_scanned) *n_scanned = ctx->npix;
-    if (!mask && cap == 0) return O3R_OK;
-    if (cap < ctx->npix) return ctx->fail(O3R_ERR_CAPACITY, "mask buffer too small");
-    if (ctx->npix == 0) return O3R_OK;
-    CU(ctx->mask.ensure(ctx->npix));
-    BatchOpts opt;
-    opt.merge = false; opt.mask_only = true; opt.mask_dev = ctx->mask.as<uint8_t>();
-    int rc = frames_cloud_impl(ctx, frame, 1, disp_type, nullptr, opt, true);
-    if (rc) return rc;
-    CU(cudaMemcpyAsync(mask, ctx->mask.p, ctx->npix, cudaMemcpyDeviceToHost, ctx->st));
-    CU(cudaStreamSynchronize(ctx->st));
-    return O3R_OK;
+    if (!frame) return O3R_ERR_INVALID;
+    return api(ctx, [&] {
+        if (n_scanned) *n_scanned = ctx->npix;
+        if (!mask && cap == 0) return O3R_OK;
+        if (cap < ctx->npix) return ctx->fail(O3R_ERR_CAPACITY, "mask buffer too small");
+        if (ctx->npix == 0) return O3R_OK;
+        CU(ctx->mask.ensure(ctx->npix));
+        BatchOpts opt;
+        opt.merge = false; opt.mask_only = true; opt.mask_dev = ctx->mask.as<uint8_t>();
+        int rc = frames_cloud_impl(ctx, frame, 1, disp_type, nullptr, opt, true);
+        if (rc) return rc;
+        CU(cudaMemcpyAsync(mask, ctx->mask.p, ctx->npix, cudaMemcpyDeviceToHost, ctx->st));
+        CU(cudaStreamSynchronize(ctx->st));
+        return O3R_OK;
+    });
 }
 
 int o3r_last_batch_points(o3r_ctx* ctx, o3r_point* out, size_t cap, size_t* n_out) {
-    if (!ctx) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    if (ctx->last_engine != Engine::SORT && !ctx->keep_frame_voxels)
-        return ctx->fail(O3R_ERR_UNSUPPORTED, "O3R_MERGE_ACCUMULATE_FUSED does not materialise the per-frame clouds (see o3r_set_keep_frame_voxels)");
-    const float4* src = ctx->last_is_vox ? ctx->vox.as<float4>() : ctx->pts.as<float4>();
-    return copy_out(ctx, src, ctx->last_total, out, cap, n_out);
+    return api(ctx, [&] {
+        if (ctx->last_engine != Engine::SORT && !ctx->keep_frame_voxels)
+            return ctx->fail(O3R_ERR_UNSUPPORTED, "O3R_MERGE_ACCUMULATE_FUSED does not materialise the per-frame clouds (see o3r_set_keep_frame_voxels)");
+        const float4* src = ctx->last_is_vox ? ctx->vox.as<float4>() : ctx->pts.as<float4>();
+        return copy_out(ctx, src, ctx->last_total, out, cap, n_out);
+    });
 }
 
 int o3r_cloud_transform(o3r_ctx* ctx, const float T[16]) {
-    if (!ctx || !T) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    if (!ctx->retain())
-        return ctx->fail(O3R_ERR_UNSUPPORTED,
-                         "o3r_cloud_transform needs O3R_MERGE_RETAIN: accumulated cells cannot be re-binned");
-    ctx->rt_valid = false;   // (on every rank of a sharded cloud, even one without points: the ranks stay in step)
-    if (ctx->n_cloud == 0) return O3R_OK;
-    CU(ctx->tmat.ensure(64));
-    { int rcu = upload_small(ctx, ctx->tmat.p, T, 48); if (rcu) return rcu; }
-    const uint32_t g = std::min<uint32_t>(cdiv(ctx->n_cloud, kThreads), 148 * 16);
-    LAUNCH(k_transform_pts, g, kThreads, 0, ctx->cloud.as<float4>(), ctx->n_cloud, ctx->tmat.as<float>());
-    return O3R_OK;
+    if (!T) return O3R_ERR_INVALID;
+    return api(ctx, [&] {
+        if (!ctx->retain())
+            return ctx->fail(O3R_ERR_UNSUPPORTED,
+                             "o3r_cloud_transform needs O3R_MERGE_RETAIN: accumulated cells cannot be re-binned");
+        ctx->rt_valid = false;   // (on every rank of a sharded cloud, even one without points: the ranks stay in step)
+        if (ctx->n_cloud == 0) return O3R_OK;
+        CU(ctx->tmat.ensure(64));
+        { int rcu = upload_small(ctx, ctx->tmat.p, T, 48); if (rcu) return rcu; }
+        const uint32_t g = std::min<uint32_t>(cdiv(ctx->n_cloud, kThreads), 148 * 16);
+        LAUNCH(k_transform_pts, g, kThreads, 0, ctx->cloud.as<float4>(), ctx->n_cloud, ctx->tmat.as<float>());
+        return O3R_OK;
+    });
 }
 
 int o3r_cloud_append(o3r_ctx* ctx, const o3r_point* pts, size_t n) {
-    if (!ctx || (n && !pts)) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    if (ctx->comm && ctx->retain())
-        return ctx->fail(O3R_ERR_UNSUPPORTED, "o3r_cloud_append on a sharded retained cloud: appended points have no place in the frame order");
-    if (n == 0) return O3R_OK;
-    if (ctx->retain()) {
-        CU(ctx->cloud.ensure((ctx->n_cloud + n) * 16, ctx->st, ctx->n_cloud * 16));
-        CU(cudaMemcpyAsync(ctx->cloud.as<float4>() + ctx->n_cloud, pts, n * 16, cudaMemcpyHostToDevice, ctx->st));
-        CU(cudaStreamSynchronize(ctx->st));   // the caller may reuse or free `pts` as soon as this returns
-        ctx->n_cloud += n;
+    if (n && !pts) return O3R_ERR_INVALID;
+    return api(ctx, [&] {
+        if (ctx->comm && ctx->retain())
+            return ctx->fail(O3R_ERR_UNSUPPORTED, "o3r_cloud_append on a sharded retained cloud: appended points have no place in the frame order");
+        if (n == 0) return O3R_OK;
+        if (ctx->retain()) {
+            CU(ctx->cloud.ensure((ctx->n_cloud + n) * 16, ctx->st, ctx->n_cloud * 16));
+            CU(cudaMemcpyAsync(ctx->cloud.as<float4>() + ctx->n_cloud, pts, n * 16, cudaMemcpyHostToDevice, ctx->st));
+            CU(cudaStreamSynchronize(ctx->st));   // the caller may reuse or free `pts` as soon as this returns
+            ctx->n_cloud += n;
+            return O3R_OK;
+        }
+        CU(ctx->vox.ensure(n * 16));
+        CU(cudaMemcpyAsync(ctx->vox.p, pts, n * 16, cudaMemcpyHostToDevice, ctx->st));
+        ctx->last_n = 0; ctx->last_total = 0; ctx->last_has_cellbb = false;   // the batch buffer was overwritten
+        ctx->last_has_partials = false; ctx->last_partials = 0; ctx->last_engine = Engine::SORT;
+        const int rc = acc_merge_points(ctx, ctx->vox.as<float4>(), n, nullptr);
+        if (rc) return rc;
+        CU(cudaStreamSynchronize(ctx->st));   // (a page-locked `pts` is read asynchronously) the caller may reuse or free it now
         return O3R_OK;
-    }
-    CU(ctx->vox.ensure(n * 16));
-    CU(cudaMemcpyAsync(ctx->vox.p, pts, n * 16, cudaMemcpyHostToDevice, ctx->st));
-    ctx->last_n = 0; ctx->last_total = 0; ctx->last_has_cellbb = false;   // the batch buffer was overwritten
-    ctx->last_has_partials = false; ctx->last_partials = 0; ctx->last_engine = Engine::SORT;
-    const int rc = acc_merge_points(ctx, ctx->vox.as<float4>(), n, nullptr);
-    if (rc) return rc;
-    CU(cudaStreamSynchronize(ctx->st));   // (a page-locked `pts` is read asynchronously) the caller may reuse or free it now
-    return O3R_OK;
+    });
 }
 
 int o3r_cloud_size(o3r_ctx* ctx, size_t* n) {
-    if (!ctx || !n) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    if (ctx->retain()) { *n = ctx->n_cloud; return O3R_OK; }
-    int rc = refresh_nres(ctx, true);
-    if (rc) return rc;
-    *n = ctx->n_res_ub;
-    return O3R_OK;
+    if (!n) return O3R_ERR_INVALID;
+    return api(ctx, [&] {
+        if (ctx->retain()) { *n = ctx->n_cloud; return O3R_OK; }
+        int rc = refresh_nres(ctx, true);
+        if (rc) return rc;
+        *n = ctx->n_res_ub;
+        return O3R_OK;
+    });
 }
 
 int o3r_cloud_clear(o3r_ctx* ctx) {
-    if (!ctx) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    CU(cudaStreamSynchronize(ctx->st));
-    ctx->n_cloud = 0; ctx->n_res_ub = 0; ctx->n_res_exact = true;
-    ctx->rt_reset();
-    ZERO(ctx->counters.as<uint32_t>() + CNT_NRES, 4);
-    if (ctx->chg_on) chg_reset(ctx, false);
-    return O3R_OK;
+    return api(ctx, [&] {
+        CU(cudaStreamSynchronize(ctx->st));
+        ctx->n_cloud = 0; ctx->n_res_ub = 0; ctx->n_res_exact = true;
+        ctx->rt_reset();
+        ZERO(ctx->counters.as<uint32_t>() + CNT_NRES, 4);
+        if (ctx->chg_on) chg_reset(ctx, false);
+        return O3R_OK;
+    });
 }
 
 // engine 1 on an arbitrary device cloud of one segment
@@ -448,181 +416,177 @@ static int downsample_finish(o3r_ctx* ctx, size_t* m) {
 }
 
 int o3r_cloud_downsample(o3r_ctx* ctx, o3r_point* out, size_t cap, size_t* n_out) {
-    if (!ctx) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    if (n_out) *n_out = 0;
-    const float4* res;
-    size_t m;
-    bool pending;
-    int rc = cloud_downsample_dev(ctx, &res, &m, &pending);
-    if (rc) return rc;
-    if (!pending) return copy_out(ctx, res, m, out, cap, n_out);
-    // accumulators: the copy of up to min(cap, bound) records is queued behind the emit kernels, one sync for everything
-    const size_t ncopy = (out && cap) ? std::min(cap, m) : 0;
-    if (ncopy) CU(cudaMemcpyAsync(out, res, ncopy * 16, cudaMemcpyDeviceToHost, ctx->st));
-    rc = downsample_finish(ctx, &m);
-    if (rc) return rc;
-    if (n_out) *n_out = m;
-    if (!out && cap == 0) return O3R_OK;
-    if (cap < m) return ctx->fail(O3R_ERR_CAPACITY, "output buffer too small");
-    return O3R_OK;
+    return api(ctx, [&] {
+        if (n_out) *n_out = 0;
+        const float4* res;
+        size_t m;
+        bool pending;
+        int rc = cloud_downsample_dev(ctx, &res, &m, &pending);
+        if (rc) return rc;
+        if (!pending) return copy_out(ctx, res, m, out, cap, n_out);
+        // accumulators: the copy of up to min(cap, bound) records is queued behind the emit kernels, one sync for everything
+        const size_t ncopy = (out && cap) ? std::min(cap, m) : 0;
+        if (ncopy) CU(cudaMemcpyAsync(out, res, ncopy * 16, cudaMemcpyDeviceToHost, ctx->st));
+        rc = downsample_finish(ctx, &m);
+        if (rc) return rc;
+        if (n_out) *n_out = m;
+        if (!out && cap == 0) return O3R_OK;
+        if (cap < m) return ctx->fail(O3R_ERR_CAPACITY, "output buffer too small");
+        return O3R_OK;
+    });
 }
 
 int o3r_cloud_downsample_dev(o3r_ctx* ctx, const o3r_point** dev_out, size_t* n_out) {
-    if (!ctx || !n_out) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    const float4* res;
-    bool pending;
-    int rc = cloud_downsample_dev(ctx, &res, n_out, &pending);
-    if (rc) return rc;
-    if (pending) { rc = downsample_finish(ctx, n_out); if (rc) return rc; }
-    else CU(cudaStreamSynchronize(ctx->st));
-    if (dev_out) *dev_out = reinterpret_cast<const o3r_point*>(res);
-    return O3R_OK;
+    if (!n_out) return O3R_ERR_INVALID;
+    return api(ctx, [&] {
+        const float4* res;
+        bool pending;
+        int rc = cloud_downsample_dev(ctx, &res, n_out, &pending);
+        if (rc) return rc;
+        if (pending) { rc = downsample_finish(ctx, n_out); if (rc) return rc; }
+        else CU(cudaStreamSynchronize(ctx->st));
+        if (dev_out) *dev_out = reinterpret_cast<const o3r_point*>(res);
+        return O3R_OK;
+    });
 }
 
 int o3r_cloud_track_changes(o3r_ctx* ctx, int enable) {
-    if (!ctx) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    { int rc = chg_check_mode(ctx); if (rc) return rc; }
-    if (!enable) {
-        CU(cudaStreamSynchronize(ctx->st));   // (queued unions may still read or write the buffers)
-        ctx->chg_on = ctx->chg_all = ctx->chg_valid = false;
-        ctx->chg_ub = ctx->chg_m = 0;
-        ctx->chg_release();
+    return api(ctx, [&] {
+        { int rc = chg_check_mode(ctx); if (rc) return rc; }
+        if (!enable) {
+            CU(cudaStreamSynchronize(ctx->st));   // (queued unions may still read or write the buffers)
+            ctx->chg_on = ctx->chg_all = ctx->chg_valid = false;
+            ctx->chg_ub = ctx->chg_m = 0;
+            ctx->chg_release();
+            return O3R_OK;
+        }
+        ctx->chg_on = true;
+        chg_reset(ctx, true);   // the next read returns the full state
         return O3R_OK;
-    }
-    ctx->chg_on = true;
-    chg_reset(ctx, true);   // the next read returns the full state
-    return O3R_OK;
+    });
 }
 
 int o3r_cloud_changes(o3r_ctx* ctx, o3r_point* out, uint64_t* keys, uint32_t* counts, size_t cap, size_t* n_out) {
-    if (!ctx || !n_out) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    *n_out = 0;
-    int rc = chg_compute(ctx);
-    if (rc) return rc;
-    const size_t m = ctx->chg_m;
-    *n_out = m;
-    if (!out && cap == 0) return O3R_OK;   // size query: nothing consumed
-    if (cap < m) return ctx->fail(O3R_ERR_CAPACITY, "output buffer too small");
-    if (m) {
-        if (out) CU(cudaMemcpyAsync(out, ctx->chg_out.p, m * 16, cudaMemcpyDeviceToHost, ctx->st));
-        if (keys) CU(cudaMemcpyAsync(keys, ctx->chg_okeys.p, m * 8, cudaMemcpyDeviceToHost, ctx->st));
-        if (counts) CU(cudaMemcpyAsync(counts, ctx->chg_ocnt.p, m * 4, cudaMemcpyDeviceToHost, ctx->st));
-        CU(cudaStreamSynchronize(ctx->st));
-    }
-    chg_reset(ctx, false);   // delivered: nothing is pending any more
-    return O3R_OK;
+    if (!n_out) return O3R_ERR_INVALID;
+    return api(ctx, [&] {
+        *n_out = 0;
+        int rc = chg_compute(ctx);
+        if (rc) return rc;
+        const size_t m = ctx->chg_m;
+        *n_out = m;
+        if (!out && cap == 0) return O3R_OK;   // size query: nothing consumed
+        if (cap < m) return ctx->fail(O3R_ERR_CAPACITY, "output buffer too small");
+        if (m) {
+            if (out) CU(cudaMemcpyAsync(out, ctx->chg_out.p, m * 16, cudaMemcpyDeviceToHost, ctx->st));
+            if (keys) CU(cudaMemcpyAsync(keys, ctx->chg_okeys.p, m * 8, cudaMemcpyDeviceToHost, ctx->st));
+            if (counts) CU(cudaMemcpyAsync(counts, ctx->chg_ocnt.p, m * 4, cudaMemcpyDeviceToHost, ctx->st));
+            CU(cudaStreamSynchronize(ctx->st));
+        }
+        chg_reset(ctx, false);   // delivered: nothing is pending any more
+        return O3R_OK;
+    });
 }
 
 int o3r_cloud_changes_dev(o3r_ctx* ctx, const o3r_point** dev_out, const uint64_t** dev_keys, const uint32_t** dev_counts,
                           size_t* n_out) {
-    if (!ctx || !n_out) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    *n_out = 0;
-    int rc = chg_compute(ctx);
-    if (rc) return rc;
-    *n_out = ctx->chg_m;
-    if (dev_out) *dev_out = ctx->chg_out.as<const o3r_point>();
-    if (dev_keys) *dev_keys = ctx->chg_okeys.as<const uint64_t>();
-    if (dev_counts) *dev_counts = ctx->chg_ocnt.as<const uint32_t>();
-    chg_reset(ctx, false);   // (the records stay in the context's buffers until the next call)
-    return O3R_OK;
+    if (!n_out) return O3R_ERR_INVALID;
+    return api(ctx, [&] {
+        *n_out = 0;
+        int rc = chg_compute(ctx);
+        if (rc) return rc;
+        *n_out = ctx->chg_m;
+        if (dev_out) *dev_out = ctx->chg_out.as<const o3r_point>();
+        if (dev_keys) *dev_keys = ctx->chg_okeys.as<const uint64_t>();
+        if (dev_counts) *dev_counts = ctx->chg_ocnt.as<const uint32_t>();
+        chg_reset(ctx, false);   // (the records stay in the context's buffers until the next call)
+        return O3R_OK;
+    });
 }
 
 int o3r_cloud_export_cells(o3r_ctx* ctx, o3r_cell* out, size_t cap, size_t* n_out) {
-    if (!ctx || !n_out) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    *n_out = 0;
-    return export_cells_impl(ctx, out, cap, n_out);
+    if (!n_out) return O3R_ERR_INVALID;
+    return api(ctx, [&] {
+        *n_out = 0;
+        return export_cells_impl(ctx, out, cap, n_out);
+    });
 }
 
 int o3r_cloud_import_cells(o3r_ctx* ctx, const o3r_cell* cells, size_t n) {
-    if (!ctx || (n && !cells)) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    return import_cells_impl(ctx, cells, n);
+    if (n && !cells) return O3R_ERR_INVALID;
+    return api(ctx, [&] { return import_cells_impl(ctx, cells, n); });
 }
 
 int o3r_cloud_export_points(o3r_ctx* ctx, o3r_point* out, size_t cap, size_t* n_out) {
-    if (!ctx || !n_out) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    *n_out = 0;
-    return export_points_impl(ctx, out, cap, n_out);
+    if (!n_out) return O3R_ERR_INVALID;
+    return api(ctx, [&] {
+        *n_out = 0;
+        return export_points_impl(ctx, out, cap, n_out);
+    });
 }
 
 int o3r_voxel_grid(o3r_ctx* ctx, const o3r_point* pts, size_t n, float lx, float ly, float lz, unsigned min_points,
                    o3r_point* out, size_t cap, size_t* n_out, uint64_t* keys, uint32_t* counts, int* passthrough) {
-    if (!ctx || !n_out || (n && !pts)) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    *n_out = 0;
-    if (passthrough) *passthrough = 0;
-    if (n == 0) return O3R_OK;
-    if (!(lx > 0) || !(ly > 0) || !(lz > 0)) return ctx->fail(O3R_ERR_INVALID, "leaf size must be positive");
-    CU(ctx->pts.ensure(n * 16));
-    CU(ctx->vox.ensure(n * 16));
-    CU(ctx->ckey.ensure(n * 8));
-    CU(ctx->new_keys.ensure(n * 4));
-    ctx->last_n = 0; ctx->last_total = 0;
-    CU(cudaMemcpyAsync(ctx->pts.p, pts, n * 16, cudaMemcpyHostToDevice, ctx->st));
-    size_t m = 0;
-    int rc = voxel_grid_dev(ctx, ctx->pts.as<float4>(), n, 1.0f / lx, 1.0f / ly, 1.0f / lz, min_points, 0,
-                            ctx->vox.as<float4>(), ctx->ckey.as<uint64_t>(), ctx->new_keys.as<uint32_t>(), &m, passthrough);
-    if (rc) return rc;
-    *n_out = m;
-    if (!out && cap == 0) return O3R_OK;
-    if (cap < m) return ctx->fail(O3R_ERR_CAPACITY, "output buffer too small");
-    if (m) {
-        CU(cudaMemcpyAsync(out, ctx->vox.p, m * 16, cudaMemcpyDeviceToHost, ctx->st));
-        if (keys) CU(cudaMemcpyAsync(keys, ctx->ckey.p, m * 8, cudaMemcpyDeviceToHost, ctx->st));
-        if (counts) CU(cudaMemcpyAsync(counts, ctx->new_keys.p, m * 4, cudaMemcpyDeviceToHost, ctx->st));
-        CU(cudaStreamSynchronize(ctx->st));
-    }
-    return O3R_OK;
+    if (!n_out || (n && !pts)) return O3R_ERR_INVALID;
+    return api(ctx, [&] {
+        *n_out = 0;
+        if (passthrough) *passthrough = 0;
+        if (n == 0) return O3R_OK;
+        if (!(lx > 0) || !(ly > 0) || !(lz > 0)) return ctx->fail(O3R_ERR_INVALID, "leaf size must be positive");
+        CU(ctx->pts.ensure(n * 16));
+        CU(ctx->vox.ensure(n * 16));
+        CU(ctx->ckey.ensure(n * 8));
+        CU(ctx->new_keys.ensure(n * 4));
+        ctx->last_n = 0; ctx->last_total = 0;
+        CU(cudaMemcpyAsync(ctx->pts.p, pts, n * 16, cudaMemcpyHostToDevice, ctx->st));
+        size_t m = 0;
+        int rc = voxel_grid_dev(ctx, ctx->pts.as<float4>(), n, 1.0f / lx, 1.0f / ly, 1.0f / lz, min_points, 0,
+                                ctx->vox.as<float4>(), ctx->ckey.as<uint64_t>(), ctx->new_keys.as<uint32_t>(), &m, passthrough);
+        if (rc) return rc;
+        *n_out = m;
+        if (!out && cap == 0) return O3R_OK;
+        if (cap < m) return ctx->fail(O3R_ERR_CAPACITY, "output buffer too small");
+        if (m) {
+            CU(cudaMemcpyAsync(out, ctx->vox.p, m * 16, cudaMemcpyDeviceToHost, ctx->st));
+            if (keys) CU(cudaMemcpyAsync(keys, ctx->ckey.p, m * 8, cudaMemcpyDeviceToHost, ctx->st));
+            if (counts) CU(cudaMemcpyAsync(counts, ctx->new_keys.p, m * 4, cudaMemcpyDeviceToHost, ctx->st));
+            CU(cudaStreamSynchronize(ctx->st));
+        }
+        return O3R_OK;
+    });
 }
 
 int o3r_blur_u8(o3r_ctx* ctx, const uint8_t* src, size_t src_step, int rows, int cols, int kernel, int mode,
                 uint8_t* dst, size_t dst_step) {
-    if (!ctx || !src || !dst || rows <= 0 || cols <= 0) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    if (kernel < 1 || kernel > kBlurMaxK) return ctx->fail(O3R_ERR_INVALID, "kernel must be in 1..127");
-    if (mode == O3R_BLUR_MEDIAN && (kernel & 1) == 0)
-        return ctx->fail(O3R_ERR_INVALID, "median blur needs an odd kernel (cv::medianBlur asserts)");
-    if (mode != O3R_BLUR_MEDIAN && mode != O3R_BLUR_BOX && mode != O3R_BLUR_BILATERAL)
-        return ctx->fail(O3R_ERR_INVALID, "unknown blur mode");
-    const size_t step = ((size_t)cols + 15) & ~(size_t)15, plane = step * rows;
-    CU(ctx->d_disp.ensure(plane));
-    CU(ctx->d_blur.ensure(plane));
-    CU(ctx->d_blurjobs.ensure(sizeof(BlurJob)));
-    CU(cudaMemcpy2DAsync(ctx->d_disp.p, step, src, src_step, cols, rows, cudaMemcpyHostToDevice, ctx->st));
-    BlurJob job{ctx->d_disp.as<uint8_t>(), step, ctx->d_blur.as<uint8_t>(), step};
-    CU(cudaMemcpyAsync(ctx->d_blurjobs.p, &job, sizeof(job), cudaMemcpyHostToDevice, ctx->st));
-    const dim3 g(cdiv(cols, kBlurStrip), cdiv(rows, blur_rows(mode)), 1);
-    const size_t sm = blur_smem(kernel, mode);
-    if (mode == O3R_BLUR_BILATERAL) {
-        BilateralLut L;
-        int rcl = bilateral_lut(ctx, kernel, &L);
-        if (rcl) return rcl;
-        const dim3 gb(cdiv(cols, kBilW), cdiv(rows, kBilTY), 1);
-        LAUNCH(k_bilateral, gb, dim3(kBilTX, kBilTY), bilateral_smem(L.radius, L.maxk), ctx->d_blurjobs.as<BlurJob>(), L, rows, cols, 0, 0, cols, rows);
-    } else if (mode == O3R_BLUR_MEDIAN)
-        LAUNCH_N("k_blur_median", (k_blur<O3R_BLUR_MEDIAN>), g, kBlurRows, sm, ctx->d_blurjobs.as<BlurJob>(), rows, cols, kernel, 0, 0, cols, rows);
-    else
-        LAUNCH_N("k_blur_box", (k_blur<O3R_BLUR_BOX>), g, kBlurRows, sm, ctx->d_blurjobs.as<BlurJob>(), rows, cols, kernel, 0, 0, cols, rows);
-    CU(cudaMemcpy2DAsync(dst, dst_step, ctx->d_blur.p, step, cols, rows, cudaMemcpyDeviceToHost, ctx->st));
-    CU(cudaStreamSynchronize(ctx->st));
-    return O3R_OK;
+    if (!src || !dst || rows <= 0 || cols <= 0) return O3R_ERR_INVALID;
+    return api(ctx, [&] {
+        if (kernel < 1 || kernel > kBlurMaxK) return ctx->fail(O3R_ERR_INVALID, "kernel must be in 1..127");
+        if (mode == O3R_BLUR_MEDIAN && (kernel & 1) == 0)
+            return ctx->fail(O3R_ERR_INVALID, "median blur needs an odd kernel (cv::medianBlur asserts)");
+        if (mode != O3R_BLUR_MEDIAN && mode != O3R_BLUR_BOX && mode != O3R_BLUR_BILATERAL)
+            return ctx->fail(O3R_ERR_INVALID, "unknown blur mode");
+        const size_t step = ((size_t)cols + 15) & ~(size_t)15, plane = step * rows;
+        CU(ctx->d_disp.ensure(plane));
+        CU(ctx->d_blur.ensure(plane));
+        CU(ctx->d_blurjobs.ensure(sizeof(BlurJob)));
+        CU(cudaMemcpy2DAsync(ctx->d_disp.p, step, src, src_step, cols, rows, cudaMemcpyHostToDevice, ctx->st));
+        BlurJob job{ctx->d_disp.as<uint8_t>(), step, ctx->d_blur.as<uint8_t>(), step};
+        CU(cudaMemcpyAsync(ctx->d_blurjobs.p, &job, sizeof(job), cudaMemcpyHostToDevice, ctx->st));
+        const dim3 g(cdiv(cols, kBlurStrip), cdiv(rows, blur_rows(mode)), 1);
+        const size_t sm = blur_smem(kernel, mode);
+        if (mode == O3R_BLUR_BILATERAL) {
+            BilateralLut L;
+            int rcl = bilateral_lut(ctx, kernel, &L);
+            if (rcl) return rcl;
+            const dim3 gb(cdiv(cols, kBilW), cdiv(rows, kBilTY), 1);
+            LAUNCH(k_bilateral, gb, dim3(kBilTX, kBilTY), bilateral_smem(L.radius, L.maxk), ctx->d_blurjobs.as<BlurJob>(), L, rows, cols, 0, 0, cols, rows);
+        } else if (mode == O3R_BLUR_MEDIAN)
+            LAUNCH_N("k_blur_median", (k_blur<O3R_BLUR_MEDIAN>), g, kBlurRows, sm, ctx->d_blurjobs.as<BlurJob>(), rows, cols, kernel, 0, 0, cols, rows);
+        else
+            LAUNCH_N("k_blur_box", (k_blur<O3R_BLUR_BOX>), g, kBlurRows, sm, ctx->d_blurjobs.as<BlurJob>(), rows, cols, kernel, 0, 0, cols, rows);
+        CU(cudaMemcpy2DAsync(dst, dst_step, ctx->d_blur.p, step, cols, rows, cudaMemcpyDeviceToHost, ctx->st));
+        CU(cudaStreamSynchronize(ctx->st));
+        return O3R_OK;
+    });
 }
 
 // ---- the exchange inside the library: communicator + one call per cycle (SURVEY 8e) --------------------------------------
@@ -637,58 +601,56 @@ int o3r_comm_unique_id(void* id_out) {
 }
 
 int o3r_comm_init(o3r_ctx* ctx, int world, int rank, const void* id, size_t slot_cells) {
-    if (!ctx || !id) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    NcclApi* N = nccl_api();
-    if (!N->err.empty()) return ctx->fail(O3R_ERR_CUDA, N->err);
-    if (ctx->comm) return ctx->fail(O3R_ERR_INVALID, "the context already has a communicator");
-    int rc = comm_setup(ctx, world, rank, slot_cells);
-    if (rc) return rc;
-    ZERO(ctx->counters.as<uint32_t>() + CNT_XFLAG, 8);
-    ncclUniqueId uid;
-    memcpy(&uid, id, sizeof(uid));
-    ncclComm_t c = nullptr;
-    NC(N->CommInitRank(&c, world, uid, rank));
-    ctx->comm = c; ctx->comm_owned = true;
-    return O3R_OK;
+    if (!id) return O3R_ERR_INVALID;
+    return api(ctx, [&] {
+        NcclApi* N = nccl_api();
+        if (!N->err.empty()) return ctx->fail(O3R_ERR_CUDA, N->err);
+        if (ctx->comm) return ctx->fail(O3R_ERR_INVALID, "the context already has a communicator");
+        int rc = comm_setup(ctx, world, rank, slot_cells);
+        if (rc) return rc;
+        ZERO(ctx->counters.as<uint32_t>() + CNT_XFLAG, 8);
+        ncclUniqueId uid;
+        memcpy(&uid, id, sizeof(uid));
+        ncclComm_t c = nullptr;
+        NC(N->CommInitRank(&c, world, uid, rank));
+        ctx->comm = c; ctx->comm_owned = true;
+        return O3R_OK;
+    });
 }
 
 int o3r_comm_attach(o3r_ctx* ctx, void* nccl_comm, int world, int rank, size_t slot_cells) {
-    if (!ctx || !nccl_comm) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    NcclApi* N = nccl_api();
-    if (!N->err.empty()) return ctx->fail(O3R_ERR_CUDA, N->err);
-    if (ctx->comm) return ctx->fail(O3R_ERR_INVALID, "the context already has a communicator");
-    int rc = comm_setup(ctx, world, rank, slot_cells);
-    if (rc) return rc;
-    ZERO(ctx->counters.as<uint32_t>() + CNT_XFLAG, 8);
-    ctx->comm = nccl_comm; ctx->comm_owned = false;
-    return O3R_OK;
+    if (!nccl_comm) return O3R_ERR_INVALID;
+    return api(ctx, [&] {
+        NcclApi* N = nccl_api();
+        if (!N->err.empty()) return ctx->fail(O3R_ERR_CUDA, N->err);
+        if (ctx->comm) return ctx->fail(O3R_ERR_INVALID, "the context already has a communicator");
+        int rc = comm_setup(ctx, world, rank, slot_cells);
+        if (rc) return rc;
+        ZERO(ctx->counters.as<uint32_t>() + CNT_XFLAG, 8);
+        ctx->comm = nccl_comm; ctx->comm_owned = false;
+        return O3R_OK;
+    });
 }
 
 int o3r_comm_destroy(o3r_ctx* ctx) {
-    if (!ctx) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    CU(cudaStreamSynchronize(ctx->st));
-    NcclApi* N = nccl_api();
-    if (ctx->comm && ctx->comm_owned) NC(N->CommDestroy((ncclComm_t)ctx->comm));
-    ctx->comm = nullptr; ctx->comm_owned = false; ctx->world = 1; ctx->rank = 0;
-    ctx->x_send.release(); ctx->x_recv.release(); ctx->x_list.release();
-    ctx->rt_reset();
-    DevBuf* rt_bufs[] = {&ctx->rt_agree, &ctx->rt_ftab, &ctx->rt_tags, &ctx->rt_send, &ctx->rt_recv, &ctx->rt_pts, &ctx->rt_out};
-    for (DevBuf* b : rt_bufs) b->release();
-    return O3R_OK;
+    return api(ctx, [&] {
+        CU(cudaStreamSynchronize(ctx->st));
+        NcclApi* N = nccl_api();
+        if (ctx->comm && ctx->comm_owned) NC(N->CommDestroy((ncclComm_t)ctx->comm));
+        ctx->comm = nullptr; ctx->comm_owned = false; ctx->world = 1; ctx->rank = 0;
+        ctx->x_send.release(); ctx->x_recv.release(); ctx->x_list.release();
+        ctx->rt_reset();
+        DevBuf* rt_bufs[] = {&ctx->rt_agree, &ctx->rt_ftab, &ctx->rt_tags, &ctx->rt_send, &ctx->rt_recv, &ctx->rt_pts, &ctx->rt_out};
+        for (DevBuf* b : rt_bufs) b->release();
+        return O3R_OK;
+    });
 }
 
 int o3r_exchange_cycle(o3r_ctx* ctx) {
-    if (!ctx) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    if (ctx->comm && ctx->retain()) return O3R_OK;   // RETAIN: the points stay where they were made; o3r_cloud_downsample exchanges
-    return exchange_cycle_impl(ctx);
+    return api(ctx, [&] {
+        if (ctx->comm && ctx->retain()) return O3R_OK;   // RETAIN: the points stay where they were made; o3r_cloud_downsample exchanges
+        return exchange_cycle_impl(ctx);
+    });
 }
 
 // ---- pre-pass (SURVEY §8f-3) ---------------------------------------------------------------------------------------------
@@ -762,98 +724,98 @@ int stage_plane_u8(o3r_ctx* ctx, DevBuf& buf, const uint8_t* src, size_t src_ste
 }  // namespace
 
 int o3r_disp_variance(o3r_ctx* ctx, const uint8_t* disp, size_t disp_step, double* variance) {
-    if (!ctx || !disp || !variance) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    size_t step;
-    int rc = stage_plane_u8(ctx, ctx->pp_disp, disp, disp_step, &step);
-    if (rc) return rc;
-    return roi_variance(ctx, ctx->pp_disp.as<uint8_t>(), step, nullptr, 0, nullptr, 0, variance);
+    if (!disp || !variance) return O3R_ERR_INVALID;
+    return api(ctx, [&] {
+        size_t step;
+        int rc = stage_plane_u8(ctx, ctx->pp_disp, disp, disp_step, &step);
+        if (rc) return rc;
+        return roi_variance(ctx, ctx->pp_disp.as<uint8_t>(), step, nullptr, 0, nullptr, 0, variance);
+    });
 }
 
 int o3r_plane_fit(o3r_ctx* ctx, const uint8_t* labels, size_t labels_step, const uint8_t* disp, size_t disp_step,
                   double* coef, int coef_cap, int* n_planes, double* variance) {
-    if (!ctx || !labels || !disp || !coef || !n_planes) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    const o3r_params& p = ctx->p;
-    size_t lstep, dstep;
-    int rc = stage_plane_u8(ctx, ctx->pp_labels, labels, labels_step, &lstep);
-    if (rc) return rc;
-    rc = stage_plane_u8(ctx, ctx->pp_disp, disp, disp_step, &dstep);
-    if (rc) return rc;
-    const size_t sum_bytes = (size_t)256 * kLabSums * 8;
-    CU(ctx->pp_sums.ensure(sum_bytes));
-    ZERO(ctx->pp_sums.p, sum_bytes);
-    LAUNCH(k_label_sums, cdiv(p.rows, 8), kThreads, 0, ctx->pp_labels.as<uint8_t>(), lstep, ctx->pp_disp.as<uint8_t>(), dstep,
-           p.rows, p.cols, p.cols_start_aft_cutout, p.bounding_box, ctx->pp_sums.as<unsigned long long>());
-    std::vector<unsigned long long> S((size_t)256 * kLabSums);
-    CU(cudaMemcpyAsync(S.data(), ctx->pp_sums.p, sum_bytes, cudaMemcpyDeviceToHost, ctx->st));
-    CU(cudaStreamSynchronize(ctx->st));
-    int np = 0;
-    for (int cluster = 1; cluster < 256; ++cluster) {   // :907 (labels are 8-bit); stops at the first absent label (:923)
-        const unsigned long long* s = &S[(size_t)cluster * kLabSums];
-        if (s[0] == 0) break;
-        if (cluster > coef_cap) return ctx->fail(O3R_ERR_CAPACITY, "coef buffer too small");
-        double* c = coef + 3 * (cluster - 1);
-        c[0] = c[1] = c[2] = 0.0;
-        np = cluster;
-        if (s[1] == 0) continue;   // :939-940: no pixel inside the ROI, the label keeps 0.0
-        // :957-965: x = inv_SVD(AtA) * At * b with AtA = [[Sxx Sxy Sx][Sxy Syy Sy][Sx Sy n]], At*b = [Sxd Syd Sd]
-        double A[3][3] = {{(double)s[4], (double)s[5], (double)s[2]}, {(double)s[5], (double)s[6], (double)s[3]},
-                          {(double)s[2], (double)s[3], (double)s[1]}};
-        double V[3][3], w[3];
-        sym3_eigen(A, V, w);
-        const double thr = DBL_EPSILON * 2 * (std::fabs(w[0]) + std::fabs(w[1]) + std::fabs(w[2]));
-        const double rhs[3] = {(double)s[7], (double)s[8], (double)s[9]};
-        for (int i = 0; i < 3; ++i) {
-            double acc = 0;
-            for (int j = 0; j < 3; ++j) {
-                double inv_ij = 0;
-                for (int e = 0; e < 3; ++e)
-                    if (std::fabs(w[e]) > thr) inv_ij += V[i][e] * V[j][e] / w[e];
-                acc += inv_ij * rhs[j];
+    if (!labels || !disp || !coef || !n_planes) return O3R_ERR_INVALID;
+    return api(ctx, [&] {
+        const o3r_params& p = ctx->p;
+        size_t lstep, dstep;
+        int rc = stage_plane_u8(ctx, ctx->pp_labels, labels, labels_step, &lstep);
+        if (rc) return rc;
+        rc = stage_plane_u8(ctx, ctx->pp_disp, disp, disp_step, &dstep);
+        if (rc) return rc;
+        const size_t sum_bytes = (size_t)256 * kLabSums * 8;
+        CU(ctx->pp_sums.ensure(sum_bytes));
+        ZERO(ctx->pp_sums.p, sum_bytes);
+        LAUNCH(k_label_sums, cdiv(p.rows, 8), kThreads, 0, ctx->pp_labels.as<uint8_t>(), lstep, ctx->pp_disp.as<uint8_t>(), dstep,
+               p.rows, p.cols, p.cols_start_aft_cutout, p.bounding_box, ctx->pp_sums.as<unsigned long long>());
+        std::vector<unsigned long long> S((size_t)256 * kLabSums);
+        CU(cudaMemcpyAsync(S.data(), ctx->pp_sums.p, sum_bytes, cudaMemcpyDeviceToHost, ctx->st));
+        CU(cudaStreamSynchronize(ctx->st));
+        int np = 0;
+        for (int cluster = 1; cluster < 256; ++cluster) {   // :907 (labels are 8-bit); stops at the first absent label (:923)
+            const unsigned long long* s = &S[(size_t)cluster * kLabSums];
+            if (s[0] == 0) break;
+            if (cluster > coef_cap) return ctx->fail(O3R_ERR_CAPACITY, "coef buffer too small");
+            double* c = coef + 3 * (cluster - 1);
+            c[0] = c[1] = c[2] = 0.0;
+            np = cluster;
+            if (s[1] == 0) continue;   // :939-940: no pixel inside the ROI, the label keeps 0.0
+            // :957-965: x = inv_SVD(AtA) * At * b with AtA = [[Sxx Sxy Sx][Sxy Syy Sy][Sx Sy n]], At*b = [Sxd Syd Sd]
+            double A[3][3] = {{(double)s[4], (double)s[5], (double)s[2]}, {(double)s[5], (double)s[6], (double)s[3]},
+                              {(double)s[2], (double)s[3], (double)s[1]}};
+            double V[3][3], w[3];
+            sym3_eigen(A, V, w);
+            const double thr = DBL_EPSILON * 2 * (std::fabs(w[0]) + std::fabs(w[1]) + std::fabs(w[2]));
+            const double rhs[3] = {(double)s[7], (double)s[8], (double)s[9]};
+            for (int i = 0; i < 3; ++i) {
+                double acc = 0;
+                for (int j = 0; j < 3; ++j) {
+                    double inv_ij = 0;
+                    for (int e = 0; e < 3; ++e)
+                        if (std::fabs(w[e]) > thr) inv_ij += V[i][e] * V[j][e] / w[e];
+                    acc += inv_ij * rhs[j];
+                }
+                c[i] = acc;
             }
-            c[i] = acc;
         }
-    }
-    *n_planes = np;
-    if (variance) {   // getVariance(new_disp_img, true), :973; the caller applies the > 3 gate (:975-982)
-        CU(ctx->pp_coef.ensure(std::max(np, 1) * 24));
-        if (np) { int rcu = upload_small(ctx, ctx->pp_coef.p, coef, (size_t)np * 24); if (rcu) return rcu; }
-        return roi_variance(ctx, nullptr, 0, ctx->pp_labels.as<uint8_t>(), lstep, ctx->pp_coef.as<double>(), np, variance);
-    }
-    return O3R_OK;
+        *n_planes = np;
+        if (variance) {   // getVariance(new_disp_img, true), :973; the caller applies the > 3 gate (:975-982)
+            CU(ctx->pp_coef.ensure(std::max(np, 1) * 24));
+            if (np) { int rcu = upload_small(ctx, ctx->pp_coef.p, coef, (size_t)np * 24); if (rcu) return rcu; }
+            return roi_variance(ctx, nullptr, 0, ctx->pp_labels.as<uint8_t>(), lstep, ctx->pp_coef.as<double>(), np, variance);
+        }
+        return O3R_OK;
+    });
 }
 
 
 int o3r_sor(o3r_ctx* ctx, const o3r_point* pts, size_t n, int mean_k, double stddev_mul, uint8_t* keep, float* dist,
             double* threshold) {
-    if (!ctx || (n && !pts) || !keep) return O3R_ERR_INVALID;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    CU(cudaSetDevice(ctx->p.device));
-    if (n == 0) return O3R_OK;
-    if (n >= (1ull << 32)) return ctx->fail(O3R_ERR_INVALID, "cloud too large for 32-bit indices");
-    CU(ctx->pts.ensure(n * 16));
-    CU(ctx->seg2.ensure(16));
-    ctx->last_n = 0; ctx->last_total = 0; ctx->last_has_partials = false;
-    CU(cudaMemcpyAsync(ctx->pts.p, pts, n * 16, cudaMemcpyHostToDevice, ctx->st));
-    const uint32_t seg_h[2] = {0u, (uint32_t)n};
-    { int rcu = upload_small(ctx, ctx->seg2.p, seg_h, 8); if (rcu) return rcu; }
-    SortU32 sb;
-    int rc = carve_sort_u32(ctx, n, sb);
-    if (rc) return rc;
-    rc = sor_filter(ctx, sb, ctx->pts.as<float4>(), ctx->seg2.as<uint32_t>(), 1, n, mean_k, stddev_mul);
-    if (rc) return rc;
-    std::vector<float> d(n);
-    double thr = 0;
-    CU(cudaMemcpyAsync(d.data(), ctx->sor_dist.p, n * 4, cudaMemcpyDeviceToHost, ctx->st));
-    CU(cudaMemcpyAsync(&thr, ctx->sor_thr.p, 8, cudaMemcpyDeviceToHost, ctx->st));
-    CU(cudaStreamSynchronize(ctx->st));
-    for (size_t i = 0; i < n; ++i) keep[i] = !((double)d[i] > thr);
-    if (dist) memcpy(dist, d.data(), n * 4);
-    if (threshold) *threshold = thr;
-    return O3R_OK;
+    if ((n && !pts) || !keep) return O3R_ERR_INVALID;
+    return api(ctx, [&] {
+        if (n == 0) return O3R_OK;
+        if (n >= (1ull << 32)) return ctx->fail(O3R_ERR_INVALID, "cloud too large for 32-bit indices");
+        CU(ctx->pts.ensure(n * 16));
+        CU(ctx->seg2.ensure(16));
+        ctx->last_n = 0; ctx->last_total = 0; ctx->last_has_partials = false;
+        CU(cudaMemcpyAsync(ctx->pts.p, pts, n * 16, cudaMemcpyHostToDevice, ctx->st));
+        const uint32_t seg_h[2] = {0u, (uint32_t)n};
+        { int rcu = upload_small(ctx, ctx->seg2.p, seg_h, 8); if (rcu) return rcu; }
+        SortU32 sb;
+        int rc = carve_sort_u32(ctx, n, sb);
+        if (rc) return rc;
+        rc = sor_filter(ctx, sb, ctx->pts.as<float4>(), ctx->seg2.as<uint32_t>(), 1, n, mean_k, stddev_mul);
+        if (rc) return rc;
+        std::vector<float> d(n);
+        double thr = 0;
+        CU(cudaMemcpyAsync(d.data(), ctx->sor_dist.p, n * 4, cudaMemcpyDeviceToHost, ctx->st));
+        CU(cudaMemcpyAsync(&thr, ctx->sor_thr.p, 8, cudaMemcpyDeviceToHost, ctx->st));
+        CU(cudaStreamSynchronize(ctx->st));
+        for (size_t i = 0; i < n; ++i) keep[i] = !((double)d[i] > thr);
+        if (dist) memcpy(dist, d.data(), n * 4);
+        if (threshold) *threshold = thr;
+        return O3R_OK;
+    });
 }
 
 }  // extern "C"
