@@ -205,7 +205,9 @@ int o3r_frames_prefetch_cancel(o3r_ctx* ctx);
 int o3r_frames_cloud_dev(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_type,
                          uint32_t* frame_counts);
 
-/* Copies the last batch's concatenated per-frame clouds (what was appended) to the host. */
+/* Copies the last batch's concatenated per-frame clouds (what was appended) to the host.  The last batch is what the last
+ * o3r_frame_cloud / o3r_frames_cloud[_dev] call produced; no other call changes it (o3r_last_batch_partials /
+ * o3r_last_batch_engine and a pending o3r_exchange_cycle read the same batch). */
 int o3r_last_batch_points(o3r_ctx* ctx, o3r_point* out, size_t cap, size_t* n_out);
 
 /* ---- global cloud ----------------------------------------------------------------------------- */
@@ -277,8 +279,8 @@ int o3r_cloud_changes_dev(o3r_ctx* ctx, const o3r_point** dev_out, const uint64_
  *     for bit in O3R_MERGE_ACCUMULATE; in _TILED / _FUSED bit for bit when the batches are merged the same way, but these
  *     modes pick the engine (and whether to pre-reduce) from the context's own batch history, which a checkpoint does not
  *     carry, so a resumed map may differ in the centroids within the mode's float-reassociation contract.  Host pointer, copied before the call returns.  The
- *     records are staged in a buffer of their own: the last batch (o3r_last_batch_points, a pending o3r_exchange_cycle) is
- *     left intact.  All or nothing: every record is checked on the device first, and if any is refused the call returns
+ *     records are staged in a buffer of their own; like every call outside the frame path, the import leaves the last
+ *     batch (o3r_last_batch_points, a pending o3r_exchange_cycle) intact.  All or nothing: every record is checked on the device first, and if any is refused the call returns
  *     O3R_ERR_INVALID, merges nothing, and o3r_last_error names the first refused index and its reasons.  A record is
  *     refused when bit 63 of its key is set, a 21-bit key field is 0 (outside +-(2^20 - 1) cells), n == 0, sx / sy / sz is
  *     not finite, a colour sum exceeds 255 * n, pad != 0, or (with a communicator) hash64(key) % world != rank.  Whether a

@@ -13,10 +13,10 @@ enum class Verdict { ACCEPT, RERUN, NEXT_ENGINE };
 
 // the batch's fills and sizing common to both fused engines (after the engine's own buffers are sized)
 int fused_prepare(o3r_ctx* ctx, size_t cap_batch) {
-    if (ctx->keep_frame_voxels) CU(ctx->vox.ensure(cap_batch * 16));
+    if (ctx->keep_frame_voxels) CU(ctx->last.vox.ensure(cap_batch * 16));
     FILL(ctx->counters.as<uint32_t>() + CNT_CELLBB, 24, FILL_CELLBB);
     ZERO(ctx->counters.as<uint32_t>() + CNT_PART, 8);
-    ctx->tiled_now = false;
+    ctx->pre.now = false;
     return O3R_OK;
 }
 
@@ -111,25 +111,25 @@ struct BkMisc {
     uint8_t* pass;
 };
 BkMisc bk_misc(o3r_ctx* ctx, int n) {
-    uint32_t* m = ctx->bk_misc.as<uint32_t>();
+    uint32_t* m = ctx->bk.misc.as<uint32_t>();
     return BkMisc{m, m + 2, m + 4, m + 5, m + 7, m + 6, m + 64, reinterpret_cast<uint8_t*>(m + 64 + n)};
 }
 
 // sizes the engine's buffers for a batch and queues its fills
 int bk_prepare(o3r_ctx* ctx, const BkPlan& pl, int n, size_t cap_batch, size_t cap_chunk) {
-    CU(ctx->bk_frames.ensure((size_t)n * sizeof(BkFrame)));
-    { int rcu = upload_small(ctx, ctx->bk_frames.p, pl.fr.data(), (size_t)n * sizeof(BkFrame)); if (rcu) return rcu; }
-    CU(ctx->bk_counts.ensure(pl.max_chunk_nb * 4 + 64));
+    CU(ctx->bk.frames.ensure((size_t)n * sizeof(BkFrame)));
+    { int rcu = upload_small(ctx, ctx->bk.frames.p, pl.fr.data(), (size_t)n * sizeof(BkFrame)); if (rcu) return rcu; }
+    CU(ctx->bk.counts.ensure(pl.max_chunk_nb * 4 + 64));
     const size_t nl_ub = std::min(pl.max_chunk_nb, cap_chunk);
-    CU(ctx->bk_nl.ensure(nl_ub * 16 + 64));
-    CU(ctx->bk_pts.ensure(cap_chunk * 16));
-    CU(ctx->bk_pos.ensure(cap_chunk * 8));   // ordering keys (leaf key | scan position)
-    CU(ctx->bk_status.ensure(((size_t)cdiv(pl.max_chunk_nb, kBkScanTile) + 1) * 8 + 64));
-    CU(ctx->bk_stray.ensure((size_t)kBkStrayCap * sizeof(o3r_cell)));
-    CU(ctx->bk_misc.ensure(256 + (size_t)n * 4 + (size_t)n));
+    CU(ctx->bk.nl.ensure(nl_ub * 16 + 64));
+    CU(ctx->bk.pts.ensure(cap_chunk * 16));
+    CU(ctx->bk.pos.ensure(cap_chunk * 8));   // ordering keys (leaf key | scan position)
+    CU(ctx->bk.status.ensure(((size_t)cdiv(pl.max_chunk_nb, kBkScanTile) + 1) * 8 + 64));
+    CU(ctx->bk.stray.ensure((size_t)kBkStrayCap * sizeof(o3r_cell)));
+    CU(ctx->bk.misc.ensure(256 + (size_t)n * 4 + (size_t)n));
     // every partial cell holds at least one point, and a bucket emits at most kBkMaxPart of them
     const size_t part_ub = std::min(cap_batch, pl.total_nb) + (size_t)kBkStrayCap * pl.chunk_nb.size();
-    CU(ctx->partials.ensure(std::max<size_t>(part_ub, 1) * sizeof(o3r_cell)));
+    CU(ctx->last.partials.ensure(std::max<size_t>(part_ub, 1) * sizeof(o3r_cell)));
     CU(ctx->bbox.ensure((size_t)n * 6 * 4));
     const int rc = fused_prepare(ctx, cap_batch);
     if (rc) return rc;
@@ -139,39 +139,39 @@ int bk_prepare(o3r_ctx* ctx, const BkPlan& pl, int n, size_t cap_batch, size_t c
     return O3R_OK;
 }
 
-// one chunk of frames [f0, f0 + nc) through hist -> scan -> scatter -> reduce; partial cells are appended to ctx->partials at
+// one chunk of frames [f0, f0 + nc) through hist -> scan -> scatter -> reduce; partial cells are appended to ctx->last.partials at
 // the device-side base cnt[CNT_PART] (advanced here)
 template <int DT>
 int bk_run_chunk(o3r_ctx* ctx, const AParams& P, const BkPlan& pl, int ci, int f0, int nc, int n, size_t cap_chunk) {
     uint32_t* cnt = ctx->counters.as<uint32_t>();
     const BkMisc M = bk_misc(ctx, n);
     const size_t nb = pl.chunk_nb[ci];
-    const FrameDev* fr = ctx->d_frames.as<FrameDev>() + f0;
-    const BkFrame* bk = ctx->bk_frames.as<BkFrame>() + f0;
+    const FrameDev* fr = ctx->in.frames.as<FrameDev>() + f0;
+    const BkFrame* bk = ctx->bk.frames.as<BkFrame>() + f0;
     const uint32_t scan_tiles = cdiv(nb, kBkScanTile);
     const size_t nl_ub = std::min(nb, cap_chunk);
-    unsigned long long* st_scan = ctx->bk_status.as<unsigned long long>();
-    ZERO(ctx->bk_counts.p, nb * 4);
-    ZERO(ctx->bk_status.p, ((size_t)scan_tiles + 1) * 8);
+    unsigned long long* st_scan = ctx->bk.status.as<unsigned long long>();
+    ZERO(ctx->bk.counts.p, nb * 4);
+    ZERO(ctx->bk.status.p, ((size_t)scan_tiles + 1) * 8);
     ZERO(M.totals, 20);   // totals, both tickets, stray count
     ZERO(cnt + CNT_PARTCHUNK, 4);
     const dim3 grid(P.tiles_per_frame, nc);
     uint32_t* bbox = ctx->bbox.as<uint32_t>() + (size_t)f0 * 6;
     FILL(bbox, (size_t)(nc) * 24, FILL_BBOX);
-    LAUNCH_N("k_bk_hist", (k_bk_hist<DT>), grid, kThreads, 0, P, fr, bk, ctx->inv_f, ctx->bk_counts.as<uint32_t>(), bbox, M.flags);
+    LAUNCH_N("k_bk_hist", (k_bk_hist<DT>), grid, kThreads, 0, P, fr, bk, ctx->inv_f, ctx->bk.counts.as<uint32_t>(), bbox, M.flags);
     LAUNCH(k_bk_frames, cdiv(nc, 64), 64, 0, nc, bbox, ctx->inv_f, M.pass + f0, M.fvox + f0);
-    LAUNCH(k_bk_scan, scan_tiles, kThreads, 0, ctx->bk_counts.as<uint32_t>(), (uint32_t)nb, bk, M.pass + f0, nc,
-           ctx->bk_nl.as<uint4>(), st_scan, M.t_scan, M.totals, M.flags);
+    LAUNCH(k_bk_scan, scan_tiles, kThreads, 0, ctx->bk.counts.as<uint32_t>(), (uint32_t)nb, bk, M.pass + f0, nc,
+           ctx->bk.nl.as<uint4>(), st_scan, M.t_scan, M.totals, M.flags);
     LAUNCH_N("k_bk_scatter", (k_bk_scatter<DT>), grid, kThreads, 0, P, fr, bk, M.pass + f0, ctx->inv_f,
-             ctx->bk_counts.as<uint32_t>(), ctx->bk_pts.as<float4>(), ctx->bk_pos.as<unsigned long long>(), M.flags);
+             ctx->bk.counts.as<uint32_t>(), ctx->bk.pts.as<float4>(), ctx->bk.pos.as<unsigned long long>(), M.flags);
     const uint32_t rgrid = std::max(1u, std::min<uint32_t>(cdiv(nl_ub, kRdG), 148 * 4));
-    float4* dbg = ctx->keep_frame_voxels ? ctx->vox.as<float4>() : nullptr;
-    LAUNCH(k_bk_reduce, rgrid, kThreads, bk_reduce_smem(), ctx->bk_pts.as<float4>(), ctx->bk_pos.as<unsigned long long>(),
-           ctx->bk_nl.as<uint4>(), M.totals, ctx->inv_c, ctx->inv_cz, ctx->partials.as<o3r_cell>(),
+    float4* dbg = ctx->keep_frame_voxels ? ctx->last.vox.as<float4>() : nullptr;
+    LAUNCH(k_bk_reduce, rgrid, kThreads, bk_reduce_smem(), ctx->bk.pts.as<float4>(), ctx->bk.pos.as<unsigned long long>(),
+           ctx->bk.nl.as<uint4>(), M.totals, ctx->inv_c, ctx->inv_cz, ctx->last.partials.as<o3r_cell>(),
            cnt + CNT_PART, M.stray_cnt, (uint32_t)kBkStrayCap, M.t_reduce, M.fvox + f0, reinterpret_cast<int*>(cnt + CNT_CELLBB),
            M.flags, dbg, M.dbg_cnt);
-    LAUNCH(k_bk_strays, 1, 1024, 0, ctx->partials.as<o3r_cell>(), cnt + CNT_PART, M.totals, M.stray_cnt, (uint32_t)kBkStrayCap,
-           ctx->bk_stray.as<o3r_cell>(), cnt + CNT_PARTCHUNK, M.flags);
+    LAUNCH(k_bk_strays, 1, 1024, 0, ctx->last.partials.as<o3r_cell>(), cnt + CNT_PART, M.totals, M.stray_cnt, (uint32_t)kBkStrayCap,
+           ctx->bk.stray.as<o3r_cell>(), cnt + CNT_PARTCHUNK, M.flags);
     LAUNCH(k_add_u32, 1, 32, 0, cnt + CNT_PART, cnt + CNT_PARTCHUNK);
     return O3R_OK;
 }
@@ -179,18 +179,18 @@ int bk_run_chunk(o3r_ctx* ctx, const AParams& P, const BkPlan& pl, int ci, int f
 // queues the copies of the per-frame voxel COUNTS (h_offs[1..n]) and the two overflow flag words (h_offs[n+1..n+2])
 int bk_read_back(o3r_ctx* ctx, int n) {
     const BkMisc M = bk_misc(ctx, n);
-    CU(cudaMemcpyAsync(ctx->h_offs + 1, M.fvox, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->st));
-    CU(cudaMemcpyAsync(ctx->h_offs + n + 1, M.flags, 8, cudaMemcpyDeviceToHost, ctx->st));
+    CU(cudaMemcpyAsync(ctx->last.h_offs + 1, M.fvox, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->st));
+    CU(cudaMemcpyAsync(ctx->last.h_offs + n + 1, M.flags, 8, cudaMemcpyDeviceToHost, ctx->st));
     return O3R_OK;
 }
 
 // on the landed read-back: a bucket too full / a point outside the grid bound sends this batch and the context's later ones
 // to the sort engine
 Verdict bk_verdict(o3r_ctx* ctx, int n) {
-    const uint32_t* h = ctx->h_offs;
+    const uint32_t* h = ctx->last.h_offs;
     if (!(h[n + 1] | h[n + 2])) return Verdict::ACCEPT;
     if (trace_on()) fprintf(stderr, "[o3r trace] bucket engine overflow flags %u %u: falling back to the sort engine\n", h[n + 1], h[n + 2]);
-    ctx->bucket_off = true;
+    ctx->bk.off = true;
     return Verdict::NEXT_ENGINE;
 }
 

@@ -1,13 +1,12 @@
 // host_checkpoint.cuh — checkpoints of the resident map (o3r_cloud_export_cells / o3r_cloud_import_cells /
 // o3r_cloud_export_points).  An export packs the accumulators into o3r_cell records (k_cells_pack) and copies them out; an
-// import stages the caller's records in a buffer of its own (ck_cells: the last batch's buffers, which a pending
-// o3r_exchange_cycle still reads, stay untouched), validates every record on the device (k_cells_check) and only then merges
-// them as one cycle through the ordinary engine-2 merge.  Kernels: checkpoint.cuh.
+// import stages the caller's records in a buffer of its own (ck_cells), validates every record on the device (k_cells_check)
+// and only then merges them as one cycle through the ordinary engine-2 merge.  Kernels: checkpoint.cuh.
 // (host side of libo3r.so; included by o3r_api.cu, one translation unit)
 #pragma once
 
 #include "checkpoint.cuh"
-#include "host_merge.cuh"
+#include "host_comm.cuh"
 
 namespace {
 
@@ -22,22 +21,19 @@ int export_cells_impl(o3r_ctx* ctx, o3r_cell* out, size_t cap, size_t* n_out) {
     { int rc = ck_check_cells_mode(ctx); if (rc) return rc; }
     { int rc = refresh_nres(ctx, false); if (rc) return rc; }
     uint32_t* cnt = ctx->counters.as<uint32_t>();
-    const size_t n_ub = ctx->n_res_ub;
+    const size_t n_ub = ctx->res.n_ub;
     // pack and queue the copy behind it unless the buffer is known to be short; one sync for the copy and the exact count
-    const bool fill = out && cap && n_ub && !(ctx->n_res_exact && cap < n_ub);
+    const bool fill = out && cap && n_ub && !res_exceeds(ctx, cap);
     if (fill) {
         CU(ctx->ck_cells.ensure(n_ub * sizeof(o3r_cell)));
-        LAUNCH(k_cells_pack, std::min<uint32_t>(cdiv(n_ub, kThreads), 148 * 16), kThreads, 0, cnt + CNT_NRES,
-               ctx->res_keys[ctx->res_cur].as<uint64_t>(), ctx->res_acc[ctx->res_cur].as<float4>(),
-               ctx->res_rgb[ctx->res_cur].as<uint4>(), ctx->ck_cells.as<o3r_cell>());
+        const ResCells R = res_cells(ctx);
+        LAUNCH(k_cells_pack, std::min<uint32_t>(cdiv(n_ub, kThreads), 148 * 16), kThreads, 0, cnt + CNT_NRES, R.keys, R.acc,
+               R.rgb, ctx->ck_cells.as<o3r_cell>());
         CU(cudaMemcpyAsync(out, ctx->ck_cells.p, std::min(cap, n_ub) * sizeof(o3r_cell), cudaMemcpyDeviceToHost, ctx->st));
     }
-    { int rc = read_counters(ctx); if (rc) return rc; }
-    const size_t m = ctx->h_counters[CNT_NRES];
-    ctx->n_res_ub = m;
-    ctx->n_res_exact = true;
-    if (ctx->comm && ctx->h_counters[CNT_XFLAG])   // (not cleared: the next o3r_cloud_downsample reports it too)
-        return ctx->fail(O3R_ERR_CAPACITY, "exchange slot overflow: cells were dropped; create the communicator with more slot_cells");
+    { int rc = res_read_back(ctx); if (rc) return rc; }
+    const size_t m = ctx->res.n_ub;
+    if (ctx->comm && ctx->h_counters[CNT_XFLAG]) return x_overflow(ctx);   // (not cleared: the next o3r_cloud_downsample reports it too)
     *n_out = m;
     if (!out && cap == 0) return O3R_OK;
     if (cap < m) return ctx->fail(O3R_ERR_CAPACITY, "output buffer too small");
@@ -90,7 +86,7 @@ int export_points_impl(o3r_ctx* ctx, o3r_point* out, size_t cap, size_t* n_out) 
         return ctx->fail(O3R_ERR_UNSUPPORTED, "o3r_cloud_export_points needs O3R_MERGE_RETAIN or dont_downsample: use o3r_cloud_export_cells");
     if (ctx->comm)
         return ctx->fail(O3R_ERR_UNSUPPORTED, "o3r_cloud_export_points on a sharded point cloud: its frame-order tags cannot be exported");
-    return copy_out(ctx, ctx->cloud.as<float4>(), ctx->n_cloud, out, cap, n_out);
+    return copy_out(ctx, ctx->res.cloud.as<float4>(), ctx->res.n_cloud, out, cap, n_out);
 }
 
 }  // namespace

@@ -123,24 +123,28 @@ NcclApi* nccl_api() {
             return ctx->fail(O3R_ERR_CUDA, std::string("NCCL error at " #call ": ") + N->GetErrorString(r_)); \
     } while (0)
 
+int x_overflow(o3r_ctx* ctx) {
+    return ctx->fail(O3R_ERR_CAPACITY, "exchange slot overflow: cells were dropped; create the communicator with more slot_cells");
+}
+
 int comm_setup(o3r_ctx* ctx, int world, int rank, size_t slot_cells) {
     if (world < 1 || world > 256 || rank < 0 || rank >= world || slot_cells == 0 || slot_cells >= (1ull << 31))
         return ctx->fail(O3R_ERR_INVALID, "bad communicator arguments");
     if (ctx->retain()) {   // RETAIN / dont_downsample: the points stay where they are made (host_retain.cuh); no slots
-        if (ctx->n_cloud) return ctx->fail(O3R_ERR_INVALID, "a sharded retained cloud starts empty: attach the communicator before the first cycle");
-        CU(ctx->rt_agree.ensure(((size_t)16 + 4 * (size_t)world + 4) * 4));
+        if (ctx->res.n_cloud) return ctx->fail(O3R_ERR_INVALID, "a sharded retained cloud starts empty: attach the communicator before the first cycle");
+        CU(ctx->rt.agree.ensure(((size_t)16 + 4 * (size_t)world + 4) * 4));
         CU(ctx->seg2.ensure(16));   // (these four are what the downsample's agreement steps touch: they never fail later)
         CU(ctx->bbox.ensure(6 * 4));
         CU(ctx->grids.ensure(sizeof(GridParams)));
-        ctx->world = world; ctx->rank = rank; ctx->slot_cap = (uint32_t)slot_cells;
-        ctx->rt_reset();
+        ctx->world = world; ctx->rank = rank; ctx->x.slot_cap = (uint32_t)slot_cells;
+        ctx->rt.reset();
         return O3R_OK;
     }
-    ctx->world = world; ctx->rank = rank; ctx->slot_cap = (uint32_t)slot_cells;
+    ctx->world = world; ctx->rank = rank; ctx->x.slot_cap = (uint32_t)slot_cells;
     const size_t bytes = (size_t)world * (slot_cells + 1) * sizeof(o3r_cell);
-    CU(ctx->x_send.ensure(bytes));
-    CU(ctx->x_recv.ensure(bytes));
-    CU(ctx->x_list.ensure((size_t)world * slot_cells * sizeof(o3r_cell)));
+    CU(ctx->x.send.ensure(bytes));
+    CU(ctx->x.recv.ensure(bytes));
+    CU(ctx->x.list.ensure((size_t)world * slot_cells * sizeof(o3r_cell)));
     return O3R_OK;
 }
 
@@ -149,20 +153,20 @@ int comm_setup(o3r_ctx* ctx, int world, int rank, size_t slot_cells) {
 int exchange_cycle_impl(o3r_ctx* ctx) {
     NcclApi* N = nccl_api();
     if (!ctx->comm) return ctx->fail(O3R_ERR_INVALID, "no communicator: call o3r_comm_init / o3r_comm_attach first");
-    const uint32_t world = (uint32_t)ctx->world, cap = ctx->slot_cap;
+    const uint32_t world = (uint32_t)ctx->world, cap = ctx->x.slot_cap;
     uint32_t* cnt = ctx->counters.as<uint32_t>();
     // ---- this rank's cycle, pre-reduced on the combined grid (sort by compact cell key + in-order partial sums against an empty
     //      resident: voxel.cuh engine 2): the cycle's frames overlap, so ~8x fewer records cross NVLink and reach the owners' merge
     size_t nub = 0;
-    if (ctx->last_is_vox && ctx->last_total) {
-        const int* bbp = ctx->last_has_cellbb ? ctx->last_cellbb : nullptr;
+    if (ctx->last.is_vox && ctx->last.total) {
+        const int* bbp = ctx->last.has_cellbb ? ctx->last.cellbb : nullptr;
         int rc;
-        if (ctx->last_has_partials) {
-            AccItemsCells items{ctx->partials.as<o3r_cell>(), nullptr, nullptr};
-            rc = acc_build_cycle(ctx, items, ctx->last_partials, false, bbp);
+        if (ctx->last.has_partials) {
+            AccItemsCells items{ctx->last.partials.as<o3r_cell>(), nullptr, nullptr};
+            rc = acc_build_cycle(ctx, items, ctx->last.n_part, false, bbp);
         } else {   // exact-order modes keep the batch as voxel points
-            AccItemsPts items{ctx->vox.as<float4>(), nullptr, nullptr};
-            rc = acc_build_cycle(ctx, items, ctx->last_total, false, bbp);
+            AccItemsPts items{ctx->last.vox.as<float4>(), nullptr, nullptr};
+            rc = acc_build_cycle(ctx, items, ctx->last.total, false, bbp);
         }
         if (rc) return rc;
         nub = ctx->n_cyc_ub;
@@ -189,11 +193,11 @@ int exchange_cycle_impl(o3r_ctx* ctx) {
         if (rc) return rc;
     }
     LAUNCH(k_pack_slots_cyc, g, kThreads, 0, cnt + CNT_CYC, sb.v1, ctx->ckey.as<uint64_t>(), ctx->cacc.as<float4>(), ctx->crgb.as<uint4>(),
-           ocnt, world, cap, ctx->x_send.as<o3r_cell>(), cnt + CNT_XFLAG);
+           ocnt, world, cap, ctx->x.send.as<o3r_cell>(), cnt + CNT_XFLAG);
     // ---- all-to-all of the slots
     const size_t slot_bytes = (size_t)(cap + 1) * sizeof(o3r_cell);
-    char* snd = ctx->x_send.as<char>();
-    char* rcv = ctx->x_recv.as<char>();
+    char* snd = ctx->x.send.as<char>();
+    char* rcv = ctx->x.recv.as<char>();
     CU(cudaMemcpyAsync(rcv + (size_t)ctx->rank * slot_bytes, snd + (size_t)ctx->rank * slot_bytes, slot_bytes, cudaMemcpyDeviceToDevice, ctx->st));
     if (world > 1) {
         NC(N->GroupStart());
@@ -206,14 +210,14 @@ int exchange_cycle_impl(o3r_ctx* ctx) {
     }
     // ---- merge what this rank owns (item count stays on the device; absolute keys: no cell range has to be agreed on)
     const size_t n_ub = (size_t)world * cap;
-    LAUNCH(k_unpack_slots, std::min<uint32_t>(cdiv(n_ub, kThreads), 148 * 8), kThreads, 0, ctx->x_recv.as<o3r_cell>(), world, cap,
-           ctx->x_list.as<o3r_cell>(), cnt + CNT_XRECV);
-    AccItemsCells items{ctx->x_list.as<o3r_cell>(), nullptr, nullptr};
+    LAUNCH(k_unpack_slots, std::min<uint32_t>(cdiv(n_ub, kThreads), 148 * 8), kThreads, 0, ctx->x.recv.as<o3r_cell>(), world, cap,
+           ctx->x.list.as<o3r_cell>(), cnt + CNT_XRECV);
+    AccItemsCells items{ctx->x.list.as<o3r_cell>(), nullptr, nullptr};
     int rc = acc_build_cycle_abs(ctx, items, n_ub, true, cnt + CNT_XRECV);
     if (rc) return rc;
     rc = acc_apply_cycle(ctx);
     if (rc) return rc;
-    ctx->x_pending_check = true;   // the overflow flag is read with the next o3r_cloud_downsample, which waits for the GPU anyway
+    ctx->x.pending_check = true;   // the overflow flag is read with the next o3r_cloud_downsample, which waits for the GPU anyway
     return O3R_OK;
 }
 

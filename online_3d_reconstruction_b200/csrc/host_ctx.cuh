@@ -9,6 +9,7 @@
 #include <cmath>
 #include <cstdio>
 #include <cstring>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <type_traits>
@@ -45,6 +46,11 @@ struct DevBuf {
     DevBuf() = default;
     DevBuf(const DevBuf&) = delete;
     DevBuf& operator=(const DevBuf&) = delete;
+    DevBuf(DevBuf&& o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+    DevBuf& operator=(DevBuf&& o) noexcept {   // (frees what this held: a record is reset by assigning a fresh one)
+        if (this != &o) { release(); p = o.p; cap = o.cap; o.p = nullptr; o.cap = 0; }
+        return *this;
+    }
     ~DevBuf() { release(); }
     template <typename T> T* as() const { return reinterpret_cast<T*>(p); }
     cudaError_t ensure(size_t bytes, cudaStream_t st = nullptr, size_t preserve = 0) {
@@ -93,34 +99,106 @@ enum { CNT_PTS = 0, CNT_VOX = 1, CNT_CYC = 2, CNT_NEW = 3, CNT_EMIT = 4, CNT_NEW
 // engine of the merged path that served a batch; the values are what o3r_last_batch_engine returns
 enum class Engine { SORT = 0, BUCKET = 1, TILE = 2 };
 
-}  // namespace
+// ---- the context's records --------------------------------------------------------------------------------------------
+// Between calls, only these records carry state; each frees what it holds.  Declared here (o3r_ctx holds them by value and
+// every host_*.cuh needs it complete); each comment names the code that owns and writes the record.
 
-struct o3r_ctx {
-    o3r_params p;
-    std::mutex mu;
-    std::string err;
-    uint64_t launches = 0;
-    FillQueue fq;   // pending device fills (see FillList)
-    cudaStream_t st = nullptr, st_copy = nullptr, st_copy2 = nullptr;   // two copy streams: the per-copy set-up gaps of one hide behind the other
-    cudaEvent_t ev_copy2 = nullptr;
-    std::vector<cudaEvent_t> chunk_ev;
-    int chunk_frames = 10, chunk_frames_dev = 1 << 30;
-    cudaEvent_t chunk_event(size_t i) {
-        while (chunk_ev.size() <= i) {
-            cudaEvent_t e;
-            cudaEventCreateWithFlags(&e, cudaEventDisableTiming);
-            chunk_ev.push_back(e);
-        }
-        return chunk_ev[i];
+// The last batch (host_frames.cuh): what the last o3r_frame_cloud / o3r_frames_cloud[_dev] call produced, read by
+// o3r_last_batch_* and by a pending o3r_exchange_cycle.  No other call writes it or its payload buffers.
+struct LastBatch {
+    int n = 0;                        // frames
+    size_t total = 0;                 // points (or per-frame voxels) of all frames, off[n]
+    std::vector<uint32_t> off;        // per-frame offsets into pts / vox
+    bool is_vox = false;              // the payload is per-frame voxels (vox), not points (pts)
+    bool has_cellbb = false;          // cellbb = {imin, jmin, kmin, imax, jmax, kmax} of the payload's combined-grid cells
+    int cellbb[6] = {0, 0, 0, 0, 0, 0};
+    bool has_partials = false;        // TILED / FUSED: the batch also stands as n_part partial cells in `partials`
+    size_t n_part = 0;
+    Engine engine = Engine::SORT;     // not SORT: the batch materialised no per-frame clouds
+    // payload; the sort engine also uses pts as its chunk scratch, the fused engines size partials / vox in their *_prepare
+    DevBuf pts, vox, partials;
+    uint32_t* h_offs = nullptr;       // pinned read-back of the offsets and the engines' flag words
+    size_t h_offs_cap = 0;
+    void clear() {
+        n = 0; total = 0; off.clear(); is_vox = false; has_cellbb = false; has_partials = false; n_part = 0;
+        engine = Engine::SORT;
     }
-    int nx = 0, ny = 0;
-    uint32_t npix = 0;
-    int canon = 0;
-    float leaf_f = 0, inv_f = 0, leaf_c = 0, inv_c = 0, inv_cz = 0;
-    DevBuf lut_r, lut_z;
-    // input staging (host-pointer entry points)
-    // double-buffered: a prefetch of the next cycle's inputs fills one set while the kernels read the other
-    struct Staging { DevBuf disp, bgr, labels, coef, kp; } stg[2];
+    ~LastBatch() { if (h_offs) cudaFreeHost(h_offs); }
+};
+
+// The resident map (host_merge.cuh): accumulators (ACCUMULATE) or points (RETAIN / dont_downsample).
+struct Resident {
+    DevBuf keys[2], acc[2], rgb[2];   // double-buffered: a merge writes the other set
+    int cur = 0;
+    // The exact cell count lives on the device (counters[CNT_NRES]); the host keeps an upper bound that is enough to size
+    // buffers and launches, and tightens it from an asynchronous read-back of the previous merge.
+    size_t n_ub = 0;
+    bool n_exact = true;
+    uint32_t* h_n = nullptr;          // pinned
+    cudaEvent_t ev_n = nullptr;
+    DevBuf cloud;                     // RETAIN / dont_downsample: the points
+    size_t n_cloud = 0;
+    ~Resident() { if (h_n) cudaFreeHost(h_n); if (ev_n) cudaEventDestroy(ev_n); }
+};
+
+// Change tracking of the resident map (host_changes.cuh); the context holds one exactly while tracking is on.  The pending
+// set D (sorted unique absolute cell keys, double-buffered, count in counters[CNT_CHG0 + cur], host upper bound ub) or
+// "everything" after an enable; the last emitted result (m records in out / okeys / ocnt), valid until the tracked state
+// changes.
+struct ChangeTracking {
+    bool all = false, valid = false;
+    int cur = 0;
+    size_t ub = 0, m = 0;
+    DevBuf keys[2], cnt, off, part, pos, out, okeys, ocnt;
+};
+
+// The accumulate exchange of a communicator (host_comm.cuh); o3r_comm_destroy replaces it with a fresh one.
+struct Exchange {
+    uint32_t slot_cap = 0;            // cells per (source, destination) slot
+    DevBuf send, recv, list;
+    bool pending_check = false;       // exchanges ran since the overflow flag was last reported
+};
+
+// The sharded RETAIN form of the exchange (host_retain.cuh): the points stay on the rank that made them; per appended frame
+// its first point in the local cloud, its cycle and its global frame index (the order tag of cloud_big order); the last
+// collective result.  o3r_comm_destroy replaces it with a fresh one; reset() forgets the cloud's history, not the buffers.
+struct RetainShard {
+    struct Frame { size_t first; uint32_t cycle, frame; };
+    std::vector<Frame> frames;
+    uint32_t cycles = 0;              // o3r_frames_cloud* calls since the communicator came (or the last clear)
+    bool valid = false;               // out holds the result for the current local cloud
+    size_t m = 0;
+    size_t ftab_n = 0;                // frame records already in ftab
+    DevBuf agree, ftab, tags, send, recv, pts, out;
+    void reset() { frames.clear(); cycles = 0; valid = false; m = 0; ftab_n = 0; }
+};
+
+// The fused tile engine (host_tile.cuh): look-back words; flags / ticket / per-frame counts / pass-through guesses, and the
+// engine policy the context's batches have taught it.
+struct TileState {
+    DevBuf tiles, misc, scratch;      // per-tile {count, scratch position, offset}; flags / counters; records in arrival order
+    size_t scratch_cap = 0, part_cap = 0;   // records the scratch list / the batch's partial list hold (grown on overflow)
+    bool off = false;                 // a batch exceeded the engine's limits: the bucket / sort engine serve this context from then on
+    int R = -1;                       // window radius in use (-1: not chosen yet)
+    int guess = -1;                   // PCL's overflow guard on the last frame seen (-1: none yet) = the guess for the next batch
+    uint32_t attr = 0;                // k_tv instantiations whose shared-memory attribute is set
+};
+
+// The fused bucket engine (host_bucket.cuh): per-frame bucket grids, bucket counters / cursors, non-empty bucket list, binned
+// points + scan positions, look-back words, flags / totals / tickets / per-frame counts, stray records.
+struct BucketState {
+    DevBuf frames, counts, nl, pts, pos, status, misc, stray;
+    bool off = false;                 // a batch overflowed the engine's limits: the sort engine serves this context from then on
+};
+
+// The sort engine's tile pre-reduction in TILED mode (host_frames.cuh): skipped while it does not reduce (probed again every
+// 16th batch); `now`: the running batch pre-reduces; status: its look-back words.
+struct PreReduce { unsigned poor = 0, batches = 0; bool now = false; DevBuf status; };
+
+// Input staging of the host-pointer frame path (host_frames.cuh), double-buffered: a prefetch of the next cycle's inputs
+// fills one set while the kernels read the other.
+struct InputStaging {
+    struct Set { DevBuf disp, bgr, labels, coef, kp; } stg[2];
     struct Prefetch {                   // one record per staging set
         bool valid = false;
         int n = 0, disp_type = 0;
@@ -144,99 +222,97 @@ struct o3r_ctx {
         prefetch[s].valid = false;
         return s;
     }
-    DevBuf d_disp;   // scratch plane of o3r_blur_u8
-    DevBuf d_frames, d_blur, d_blurjobs;
-    DevBuf pp_labels, pp_disp, pp_sums, pp_rows, pp_coef;   // pre-pass scratch (plane fit / variance gate)
-    DevBuf bil_lut;            // bilateral LUTs (colour weights, space weights, per-row tap extents) of bil_kernel
-    int bil_kernel = -1, bil_radius = 0, bil_maxk = 0;
-    // per-batch work buffers
-    DevBuf tile_cnt, tile_off, bbox, frame_off, grids, counters, pts, sortbuf, hist, plan_all, plan_v2, ghist;
-    DevBuf head_cnt, head_off, vox, vox_off, seg2, tmat, mask, runwork, spts;
-    uint32_t* h_counters = nullptr;   // pinned
-    uint32_t* h_offs = nullptr;       // pinned, frame offsets readback
-    size_t h_offs_cap = 0;
-    // last batch
-    int last_n = 0;
-    size_t last_total = 0;
-    bool last_is_vox = false;
-    bool last_has_cellbb = false;
-    int last_cellbb[6] = {0, 0, 0, 0, 0, 0};
-    std::vector<uint32_t> last_off;
-    // resident cloud: accumulators (ACCUMULATE) ...
-    DevBuf res_keys[2], res_acc[2], res_rgb[2];
-    int res_cur = 0;
-    // The exact resident cell count lives on the device (counters[CNT_NRES]); the host keeps an upper bound that is
-    // enough to size buffers and launches, and tightens it from an asynchronous read-back of the previous merge.
-    size_t n_res_ub = 0;
-    bool n_res_exact = true;
-    uint32_t* h_nres = nullptr;       // pinned
-    cudaEvent_t ev_nres = nullptr;
-    size_t n_cyc_ub = 0;
-    DevBuf ckey, cacc, crgb, new_cnt, new_off, new_keys, okeys;
-    DevBuf sor_hard, sor_pts, sor_off, sor_dist, sor_grids, sor_pgrids, sor_rows, sor_thr, sor_skeys, sor_svals, sor_cnt, sor_cntoff;   // SOR scratch
-    DevBuf partials, pr_status;   // TILED mode: the batch's tile partials (o3r_cell) and the look-back words
-    // FUSED mode (bucket.cuh): per-frame bucket grids, bucket counters / cursors, non-empty bucket list, binned points + scan
-    // positions, look-back words, flags / totals / tickets / per-frame counts
-    DevBuf bk_frames, bk_counts, bk_nl, bk_pts, bk_pos, bk_status, bk_misc, bk_stray;
-    bool bucket_off = false;          // a batch overflowed the engine's limits: the sort engine serves this context from then on
-    Engine last_engine = Engine::SORT;   // not SORT: the last batch materialised no per-frame clouds
-    // FUSED mode, tile engine (tile.cuh): look-back words; flags / ticket / per-frame counts / pass-through guesses
-    DevBuf tv_tiles, tv_misc, tv_scratch;   // per-tile {count, scratch position, offset}; flags / counters; records in arrival order
-    size_t tv_scratch_cap = 0, tv_part_cap = 0;   // records the scratch list / the batch's partial list hold (grown on overflow)
-    bool tv_off = false;              // a batch exceeded the engine's limits: the bucket / sort engine serve this context from then on
-    int tv_R = -1;                    // window radius in use (-1: not chosen yet)
-    int tv_guess = -1;                // PCL's overflow guard on the last frame seen (-1: none yet) = the guess for the next batch
-    uint32_t tv_attr = 0;             // k_tv instantiations whose shared-memory attribute is set
-    // multi-GPU exchange inside the library (host_comm.cuh)
-    void* comm = nullptr;             // ncclComm_t
-    bool comm_owned = false;
-    int world = 1, rank = 0;
-    uint32_t slot_cap = 0;            // cells per (source, destination) slot
-    DevBuf x_send, x_recv, x_list;
-    bool x_pending_check = false;
-    // ... and its RETAIN form (host_retain.cuh): the points stay on the rank that made them; per appended frame its first point
-    // in the local cloud, its cycle and its global frame index (the order tag of cloud_big order); the last collective result
-    struct RtFrame { size_t first; uint32_t cycle, frame; };
-    std::vector<RtFrame> rt_frames;
-    uint32_t rt_cycles = 0;           // o3r_frames_cloud* calls since the communicator came (or the last clear)
-    bool rt_valid = false;            // rt_out holds the result for the current local cloud
-    size_t rt_m = 0;
-    size_t rt_ftab_n = 0;             // frame records already in rt_ftab
-    DevBuf rt_agree, rt_ftab, rt_tags, rt_send, rt_recv, rt_pts, rt_out;
-    void rt_reset() { rt_frames.clear(); rt_cycles = 0; rt_valid = false; rt_m = 0; rt_ftab_n = 0; }
-    // change tracking of the resident cloud (host_changes.cuh): the pending set D (sorted unique absolute cell keys,
-    // double-buffered, count in counters[CNT_CHG0 + chg_cur], host upper bound chg_ub) or "everything" after an enable;
-    // the last emitted result (chg_m records in chg_out / chg_okeys / chg_ocnt), valid until the tracked state changes
-    bool chg_on = false, chg_all = false, chg_valid = false;
-    int chg_cur = 0;
-    size_t chg_ub = 0, chg_m = 0;
-    DevBuf chg_keys[2], chg_cnt, chg_off, chg_part, chg_pos, chg_out, chg_okeys, chg_ocnt;
-    void chg_release() {
-        DevBuf* b[] = {&chg_keys[0], &chg_keys[1], &chg_cnt, &chg_off, &chg_part, &chg_pos, &chg_out, &chg_okeys, &chg_ocnt};
-        for (DevBuf* x : b) x->release();
+    int chunk_frames = 10, chunk_frames_dev = 1 << 30;   // frames per launch sequence (host / device inputs)
+    std::vector<cudaEvent_t> chunk_ev;
+    cudaEvent_t chunk_event(size_t i) {
+        while (chunk_ev.size() <= i) {
+            cudaEvent_t e;
+            cudaEventCreateWithFlags(&e, cudaEventDisableTiming);
+            chunk_ev.push_back(e);
+        }
+        return chunk_ev[i];
     }
-    DevBuf ck_cells, ck_res;          // checkpoints (host_checkpoint.cuh): packed / staged o3r_cell records, the import check's result
-    bool keep_frame_voxels = false;   // parity probe: the bucket engine also writes every per-frame voxel centroid (any order)
-    size_t last_partials = 0;
-    bool last_has_partials = false;
-    // ... or points (RETAIN / dont_downsample)
-    DevBuf cloud;
-    size_t n_cloud = 0;
+    DevBuf frames;                      // the batch's FrameDev descriptors
+    ~InputStaging() {
+        for (auto& pf : prefetch) if (pf.ev) cudaEventDestroy(pf.ev);
+        for (auto e : chunk_ev) cudaEventDestroy(e);
+    }
+};
 
-    // optional per-kernel event timing (bench.py's roofline leg)
-    struct ProfRec { const char* name; cudaEvent_t a, b; };
-    bool profiling = false;
-    std::vector<ProfRec> prof;
-    std::vector<cudaEvent_t> ev_pool;
-    cudaEvent_t ev_get() {
-        if (!ev_pool.empty()) { cudaEvent_t e = ev_pool.back(); ev_pool.pop_back(); return e; }
+// StatisticalOutlierRemoval (host_sor.cuh): the kept points and their offsets (pts / off), the distances and thresholds, and
+// the grid / sort scratch of sor_filter
+struct SorScratch { DevBuf hard, pts, off, dist, grids, pgrids, rows, thr, skeys, svals, cnt, cntoff, spts; };
+
+// Blurs (o3r_blur_u8 and the frame path's blur_kernel): o3r_blur_u8's source plane, the blurred planes and jobs, and the
+// bilateral LUTs (colour weights, space weights, per-row tap extents) of `kernel`, cached by bilateral_lut
+struct Blur { DevBuf disp, out, jobs, lut; int kernel = -1, radius = 0, maxk = 0; };
+
+// The pre-pass (o3r_disp_variance / o3r_plane_fit in o3r_api.cu): plane fit / variance gate scratch
+struct PrePass { DevBuf labels, disp, sums, rows, coef; };
+
+// Optional per-kernel event timing (o3r_profile; bench.py's roofline leg)
+struct Profiling {
+    struct Rec { const char* name; cudaEvent_t a, b; };
+    bool on = false;
+    std::vector<Rec> recs;
+    std::vector<cudaEvent_t> pool;
+    cudaEvent_t get() {
+        if (!pool.empty()) { cudaEvent_t e = pool.back(); pool.pop_back(); return e; }
         cudaEvent_t e; cudaEventCreate(&e); return e;
     }
+    ~Profiling() {
+        for (auto& r : recs) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
+        for (auto e : pool) cudaEventDestroy(e);
+    }
+};
+
+}  // namespace
+
+struct o3r_ctx {
+    o3r_params p;
+    std::mutex mu;
+    std::string err;
+    uint64_t launches = 0;
+    FillQueue fq;   // pending device fills (see FillList)
+    cudaStream_t st = nullptr, st_copy = nullptr, st_copy2 = nullptr;   // two copy streams: the per-copy set-up gaps of one hide behind the other
+    cudaEvent_t ev_copy2 = nullptr;
+    DevBuf counters;
+    uint32_t* h_counters = nullptr;   // pinned
+    // set by o3r_create / o3r_set_keep_frame_voxels / o3r_comm_*
+    int nx = 0, ny = 0;
+    uint32_t npix = 0;
+    int canon = 0;
+    float leaf_f = 0, inv_f = 0, leaf_c = 0, inv_c = 0, inv_cz = 0;
+    DevBuf lut_r, lut_z;
+    bool keep_frame_voxels = false;   // parity probe: the fused engines also write every per-frame voxel centroid (any order)
+    void* comm = nullptr;             // ncclComm_t (host_comm.cuh)
+    bool comm_owned = false;
+    int world = 1, rank = 0;
+
+    LastBatch last;
+    Resident res;
+    std::unique_ptr<ChangeTracking> chg;
+    Exchange x;
+    RetainShard rt;
+    TileState tv;
+    BucketState bk;
+    PreReduce pre;
+    InputStaging in;
+    SorScratch sor;
+    Blur blur;
+    PrePass pp;
+    Profiling prof;
+
+    // Shared per-call scratch: sized on demand and used by several paths within one call.  It holds nothing a later call
+    // reads; the one exception is the result o3r_cloud_downsample_dev points at (in ckey or cacc), valid until the next call.
+    DevBuf tile_cnt, tile_off, bbox, frame_off, grids, sortbuf, hist, plan_all, plan_v2, ghist;
+    DevBuf head_cnt, head_off, vox_off, seg2, tmat, mask, runwork;
+    DevBuf ckey, cacc, crgb, new_cnt, new_off, new_keys, okeys;   // a cycle's cell list and the merge's work buffers
+    size_t n_cyc_ub = 0;              // cells of the cycle list built by the running call
+    DevBuf in_pts, out_pts;           // caller points staged by o3r_voxel_grid / o3r_sor / o3r_cloud_append; o3r_voxel_grid's result
+    DevBuf ck_cells, ck_res;          // checkpoints (host_checkpoint.cuh): packed / staged o3r_cell records, the import check's result
 
     bool retain() const { return p.dont_downsample || p.merge_mode == O3R_MERGE_RETAIN; }
-    // tile pre-reduction is skipped while it does not reduce (probed again every 16th batch)
-    unsigned tiled_poor = 0, tiled_batches = 0;
-    bool tiled_now = false;
     bool tiled() const { return !p.dont_downsample && (p.merge_mode == O3R_MERGE_ACCUMULATE_TILED || p.merge_mode == O3R_MERGE_ACCUMULATE_FUSED); }
     bool fused() const { return !p.dont_downsample && p.merge_mode == O3R_MERGE_ACCUMULATE_FUSED; }
     int fail(int code, const std::string& m) { err = m; return code; }
@@ -247,16 +323,9 @@ struct o3r_ctx {
         err = buf;
         return O3R_ERR_CUDA;
     }
-    // (o3r_destroy makes the device current and drains the streams first; the DevBuf members free themselves after this)
+    // (o3r_destroy makes the device current and drains the streams first; the records and buffers free themselves after this)
     ~o3r_ctx() {
-        for (auto& pf : prefetch) if (pf.ev) cudaEventDestroy(pf.ev);
-        for (auto& r : prof) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
-        for (auto e : ev_pool) cudaEventDestroy(e);
         if (h_counters) cudaFreeHost(h_counters);
-        if (h_nres) cudaFreeHost(h_nres);
-        if (ev_nres) cudaEventDestroy(ev_nres);
-        if (h_offs) cudaFreeHost(h_offs);
-        for (auto e : chunk_ev) cudaEventDestroy(e);
         if (ev_copy2) cudaEventDestroy(ev_copy2);
         if (st_copy2) cudaStreamDestroy(st_copy2);
         if (st_copy) cudaStreamDestroy(st_copy);
@@ -277,8 +346,8 @@ int fill_flush(o3r_ctx* ctx);
     do {                                                                      \
         if (ctx->fq.L.n) { int rcf_ = fill_flush(ctx); if (rcf_) return rcf_; } \
         cudaEvent_t pa_ = nullptr, pb_ = nullptr;                             \
-        if (ctx->profiling) {                                                 \
-            pa_ = ctx->ev_get(); pb_ = ctx->ev_get();                         \
+        if (ctx->prof.on) {                                                   \
+            pa_ = ctx->prof.get(); pb_ = ctx->prof.get();                     \
             cudaEventRecord(pa_, ctx->st);                                    \
         }                                                                     \
         kernel<<<grid, block, smem, ctx->st>>>(__VA_ARGS__);                  \
@@ -287,7 +356,7 @@ int fill_flush(o3r_ctx* ctx);
         if (e_ != cudaSuccess) return ctx->fail_cuda(e_, #kernel, __FILE__, __LINE__);  \
         if (pa_) {                                                            \
             cudaEventRecord(pb_, ctx->st);                                    \
-            ctx->prof.push_back({name, pa_, pb_});                            \
+            ctx->prof.recs.push_back({name, pa_, pb_});                       \
         }                                                                     \
     } while (0)
 #define LAUNCH(kernel, grid, block, smem, ...) LAUNCH_N(#kernel, kernel, grid, block, smem, __VA_ARGS__)
@@ -389,7 +458,8 @@ int read_counters(o3r_ctx* ctx) {
 // LUTs of cv::bilateralFilter(src, dst, d = k, sigmaColor = 2k, sigmaSpace = k/2) (pose_functions.cpp:1044), computed on the
 // host with std::exp exactly as OpenCV 3.1 bilateralFilter_8u (and the oracle) do, cached per kernel size.
 int bilateral_lut(o3r_ctx* ctx, int k, BilateralLut* out) {
-    if (ctx->bil_kernel != k) {
+    Blur& B = ctx->blur;
+    if (B.kernel != k) {
         double sigma_color = (double)(k * 2), sigma_space = (double)(k / 2);
         if (sigma_color <= 0) sigma_color = 1;
         if (sigma_space <= 0) sigma_space = 1;
@@ -410,15 +480,15 @@ int bilateral_lut(o3r_ctx* ctx, int k, BilateralLut* out) {
         std::vector<unsigned char> blob(bytes);
         memcpy(blob.data(), buf.data(), buf.size() * 4);
         memcpy(blob.data() + buf.size() * 4, jm.data(), jm.size() * 4);
-        CU(ctx->bil_lut.ensure(bytes));
-        { int rcu = upload_small(ctx, ctx->bil_lut.p, blob.data(), bytes); if (rcu) return rcu; }
-        ctx->bil_kernel = k; ctx->bil_radius = radius; ctx->bil_maxk = maxk;
+        CU(B.lut.ensure(bytes));
+        { int rcu = upload_small(ctx, B.lut.p, blob.data(), bytes); if (rcu) return rcu; }
+        B.kernel = k; B.radius = radius; B.maxk = maxk;
         CU(cudaFuncSetAttribute(k_bilateral, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bilateral_smem(radius, maxk)));
     }
-    out->color_w = ctx->bil_lut.as<float>();
+    out->color_w = B.lut.as<float>();
     out->space_w = out->color_w + 256;
-    out->jmax = reinterpret_cast<const int*>(out->space_w + ctx->bil_maxk);
-    out->radius = ctx->bil_radius; out->maxk = ctx->bil_maxk;
+    out->jmax = reinterpret_cast<const int*>(out->space_w + B.maxk);
+    out->radius = B.radius; out->maxk = B.maxk;
     return O3R_OK;
 }
 

@@ -61,7 +61,7 @@ void frames_signature(const o3r_frame* frames, int n, std::vector<const void*>& 
 // sizes staging set `set` for the frames and fills their device-side descriptors (everything but T)
 int stage_layout(o3r_ctx* ctx, const o3r_frame* frames, int n, bool label_mode, int J, const StageGeom& G, int set,
                  std::vector<FrameDev>& fd) {
-    o3r_ctx::Staging& S = ctx->stg[set];
+    InputStaging::Set& S = ctx->in.stg[set];
     size_t kp_total = 0, coef_total = 0;
     for (int i = 0; i < n; ++i) {
         const o3r_frame& f = frames[i];
@@ -167,15 +167,15 @@ int stage_copy(o3r_ctx* ctx, const o3r_frame* frames, const std::vector<FrameDev
 
 // issues the copies of a recorded prefetch request into a free staging set
 int flush_deferred_prefetch(o3r_ctx* ctx) {
-    if (!ctx->deferred.pending) return O3R_OK;
-    ctx->deferred.pending = false;
+    if (!ctx->in.deferred.pending) return O3R_OK;
+    ctx->in.deferred.pending = false;
     const o3r_params& p = ctx->p;
-    const o3r_frame* frames = ctx->deferred.frames.data();
-    const int n = (int)ctx->deferred.frames.size(), disp_type = ctx->deferred.disp_type;
+    const o3r_frame* frames = ctx->in.deferred.frames.data();
+    const int n = (int)ctx->in.deferred.frames.size(), disp_type = ctx->in.deferred.disp_type;
     const bool label_mode = p.use_segment_labels && frames[0].labels && frames[0].plane_coef;
     const StageGeom G = stage_geom(p, disp_type);
-    const int set = ctx->free_stage_set();
-    o3r_ctx::Prefetch& pf = ctx->prefetch[set];
+    const int set = ctx->in.free_stage_set();
+    InputStaging::Prefetch& pf = ctx->in.prefetch[set];
     pf.valid = false;
     std::vector<FrameDev> fd(n);
     int rc = stage_layout(ctx, frames, n, label_mode, p.jump_pixels, G, set, fd);
@@ -185,15 +185,15 @@ int flush_deferred_prefetch(o3r_ctx* ctx) {
     if (!pf.ev) CU(cudaEventCreateWithFlags(&pf.ev, cudaEventDisableTiming));
     CU(cudaEventRecord(pf.ev, ctx->st_copy));
     frames_signature(frames, n, pf.sig);
-    pf.n = n; pf.disp_type = disp_type; pf.seq = ++ctx->prefetch_seq; pf.valid = true;
+    pf.n = n; pf.disp_type = disp_type; pf.seq = ++ctx->in.prefetch_seq; pf.valid = true;
     return O3R_OK;
 }
 
 // the O3R_TRACE line of a FUSED batch: the engine it starts with and the context state that chose it
 void trace_fused_engine(const o3r_ctx* ctx, Engine e, const AParams& P, const BatchOpts& opt) {
     fprintf(stderr, "[o3r trace] fused: engine %s (want_keys %d merge %d tile_off %d bucket_off %d canon %d vec %d R %d)\n",
-            e == Engine::TILE ? "tile" : e == Engine::BUCKET ? "bucket" : "sort", P.want_keys, (int)opt.merge, (int)ctx->tv_off,
-            (int)ctx->bucket_off, ctx->canon, P.vec, ctx->tv_R);
+            e == Engine::TILE ? "tile" : e == Engine::BUCKET ? "bucket" : "sort", P.want_keys, (int)opt.merge, (int)ctx->tv.off,
+            (int)ctx->bk.off, ctx->canon, P.vec, ctx->tv.R);
 }
 
 // The batched per-frame path.  `frames` hold host pointers (host_inputs: every frame is copied to device staging
@@ -202,13 +202,13 @@ int frames_cloud_impl(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_typ
                       const BatchOpts& opt, bool host_inputs) {
     const o3r_params& p = ctx->p;
     const bool trace = trace_on();
-    ctx->busy_set = -1;
+    ctx->in.busy_set = -1;
     const double tr0 = now_ms();
     // sharded RETAIN: every call is one cycle of the order tag, whatever it holds (n = 0: this rank has no frame in it)
     const bool rt_shard = opt.merge && ctx->comm && ctx->retain();
-    const uint32_t rt_cycle = ctx->rt_cycles;
-    if (rt_shard) { ++ctx->rt_cycles; ctx->rt_valid = false; }
-    if (n <= 0) { ctx->last_n = 0; ctx->last_total = 0; return O3R_OK; }
+    const uint32_t rt_cycle = ctx->rt.cycles;
+    if (rt_shard) { ++ctx->rt.cycles; ctx->rt.valid = false; }
+    if (n <= 0) { ctx->last.clear(); return O3R_OK; }
     if (n > 65535) return ctx->fail(O3R_ERR_INVALID, "too many frames in one batch");
     if (disp_type < 0 || disp_type > 3) return ctx->fail(O3R_ERR_INVALID, "bad disp_type");
     const bool label_mode = p.use_segment_labels && frames[0].labels && frames[0].plane_coef;
@@ -253,7 +253,8 @@ int frames_cloud_impl(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_typ
     P.want_keys = !p.dont_downsample && !opt.mask_only;
     P.want_bbox = P.want_keys;
     if (P.tiles_per_frame == 0) {  // nothing to scan (J == 0 and no keypoints)
-        ctx->last_n = n; ctx->last_total = 0; ctx->last_off.assign(n + 1, 0);
+        ctx->last.clear();
+        ctx->last.n = n; ctx->last.off.assign(n + 1, 0);
         if (frame_counts) std::fill(frame_counts, frame_counts + n, 0u);
         return O3R_OK;
     }
@@ -271,28 +272,28 @@ int frames_cloud_impl(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_typ
         // the OLDEST matching prefetch: a caller that recycles its host buffers issues the next cycle's prefetch
         // (same pointers) before this call, and that copy is still in flight
         for (int s = 0; s < 2; ++s) {
-            const o3r_ctx::Prefetch& pf = ctx->prefetch[s];
+            const InputStaging::Prefetch& pf = ctx->in.prefetch[s];
             if (pf.valid && pf.n == n && pf.disp_type == disp_type && pf.sig == sig &&
-                (!prefetched || pf.seq < ctx->prefetch[set].seq)) {
+                (!prefetched || pf.seq < ctx->in.prefetch[set].seq)) {
                 prefetched = true; set = s;
             }
         }
-        if (!prefetched && ctx->deferred.pending && (int)ctx->deferred.frames.size() == n &&
-            ctx->deferred.disp_type == disp_type) {   // recorded but not issued yet (nothing ran in between): issue it now
+        if (!prefetched && ctx->in.deferred.pending && (int)ctx->in.deferred.frames.size() == n &&
+            ctx->in.deferred.disp_type == disp_type) {   // recorded but not issued yet (nothing ran in between): issue it now
             std::vector<const void*> dsig;
-            frames_signature(ctx->deferred.frames.data(), n, dsig);
+            frames_signature(ctx->in.deferred.frames.data(), n, dsig);
             if (dsig == sig) {
                 int rcf = flush_deferred_prefetch(ctx);
                 if (rcf) return rcf;
                 for (int s = 0; s < 2; ++s)
-                    if (ctx->prefetch[s].valid && ctx->prefetch[s].seq == ctx->prefetch_seq) { prefetched = true; set = s; }
+                    if (ctx->in.prefetch[s].valid && ctx->in.prefetch[s].seq == ctx->in.prefetch_seq) { prefetched = true; set = s; }
             }
         }
-        if (prefetched) ctx->prefetch[set].valid = false;
-        if (!prefetched) set = ctx->free_stage_set();
-        ctx->busy_set = set;
+        if (prefetched) ctx->in.prefetch[set].valid = false;
+        if (!prefetched) set = ctx->in.free_stage_set();
+        ctx->in.busy_set = set;
     }
-    if (blur) CU(ctx->d_blur.ensure((size_t)n * p.rows * blur_step));
+    if (blur) CU(ctx->blur.out.ensure((size_t)n * p.rows * blur_step));
     std::vector<FrameDev> fd(n);
     std::vector<BlurJob> jobs(blur ? n : 0);
     bool vec = (J == 1) && (ctx->nx % 4 == 0) && (P.x0 % 4 == 0) && !label_mode;
@@ -318,29 +319,29 @@ int frames_cloud_impl(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_typ
         for (int k = 0; k < 12; ++k) d.T[k] = f.T[k];
         if (blur) {
             jobs[i].src = d.disp; jobs[i].sstep = d.disp_step;
-            jobs[i].dst = ctx->d_blur.as<uint8_t>() + (size_t)i * p.rows * blur_step; jobs[i].dstep = blur_step;
+            jobs[i].dst = ctx->blur.out.as<uint8_t>() + (size_t)i * p.rows * blur_step; jobs[i].dstep = blur_step;
             d.disp = jobs[i].dst; d.disp_step = blur_step;
         }
         if (!label_mode) vec = vec && ((uintptr_t)d.disp % 16 == 0) && (d.disp_step % (4 * es) == 0);
         vec = vec && ((uintptr_t)d.bgr % 4 == 0) && (d.bgr_step % 4 == 0);
     }
     P.vec = vec;
-    CU(ctx->d_frames.ensure((size_t)n * sizeof(FrameDev)));
-    { int rcu = upload_small(ctx, ctx->d_frames.p, fd.data(), (size_t)n * sizeof(FrameDev)); if (rcu) return rcu; }
+    CU(ctx->in.frames.ensure((size_t)n * sizeof(FrameDev)));
+    { int rcu = upload_small(ctx, ctx->in.frames.p, fd.data(), (size_t)n * sizeof(FrameDev)); if (rcu) return rcu; }
     if (blur) {
-        CU(ctx->d_blurjobs.ensure((size_t)n * sizeof(BlurJob)));
-        { int rcu = upload_small(ctx, ctx->d_blurjobs.p, jobs.data(), (size_t)n * sizeof(BlurJob)); if (rcu) return rcu; }
+        CU(ctx->blur.jobs.ensure((size_t)n * sizeof(BlurJob)));
+        { int rcu = upload_small(ctx, ctx->blur.jobs.p, jobs.data(), (size_t)n * sizeof(BlurJob)); if (rcu) return rcu; }
     }
 
     // ---- buffers: batch-wide outputs, chunk-sized scratch
     // host inputs: chunks let the copies overlap the kernels; device inputs: one launch sequence for the whole batch
-    const int chunk = std::max(1, std::min(n, (host_inputs && !prefetched) ? ctx->chunk_frames : ctx->chunk_frames_dev));
+    const int chunk = std::max(1, std::min(n, (host_inputs && !prefetched) ? ctx->in.chunk_frames : ctx->in.chunk_frames_dev));
     if (prefetched && trace) {
-        const bool done = cudaEventQuery(ctx->prefetch[set].ev) == cudaSuccess;
+        const bool done = cudaEventQuery(ctx->in.prefetch[set].ev) == cudaSuccess;
         cudaGetLastError();
         fprintf(stderr, "[o3r trace] prefetched inputs %s at entry\n", done ? "ready" : "still in flight");
     }
-    if (prefetched) CU(cudaStreamWaitEvent(ctx->st, ctx->prefetch[set].ev, 0));
+    if (prefetched) CU(cudaStreamWaitEvent(ctx->st, ctx->in.prefetch[set].ev, 0));
     const size_t per_frame_cap = (size_t)P.npix + (size_t)max_kp;
     const size_t cap_batch = per_frame_cap * n, cap_chunk = per_frame_cap * chunk;
     if (cap_batch >= (1ull << 32)) return ctx->fail(O3R_ERR_INVALID, "batch exceeds 2^32 samples; use fewer frames");
@@ -354,7 +355,7 @@ int frames_cloud_impl(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_typ
     BkPlan bkp;
     TvPlan tvp;
     const bool fused_ok = ctx->fused() && P.want_keys && opt.merge && !opt.mask_only && !(p.sor_mean_k > 0 && J > 0);
-    auto bucket_ok = [&] { return fused_ok && !ctx->bucket_off && bk_plan(ctx, frames, n, chunk, disp_type, label_mode, bkp); };
+    auto bucket_ok = [&] { return fused_ok && !ctx->bk.off && bk_plan(ctx, frames, n, chunk, disp_type, label_mode, bkp); };
     Engine engine = fused_ok && tv_begin(ctx, P, frames, n, tvp) ? Engine::TILE : bucket_ok() ? Engine::BUCKET : Engine::SORT;
     if (trace && ctx->fused()) trace_fused_engine(ctx, engine, P, opt);
     bool inputs_resident = false;   // second attempt: the staging buffers already hold every frame
@@ -373,26 +374,26 @@ int frames_cloud_impl(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_typ
                                                       : bk_prepare(ctx, bkp, n, cap_batch, cap_chunk);
                 if (rc) return rc;
             } else if (P.want_keys) {
-                CU(ctx->pts.ensure(cap_chunk * 16));
-                CU(ctx->vox.ensure(cap_batch * 16));
+                CU(ctx->last.pts.ensure(cap_chunk * 16));
+                CU(ctx->last.vox.ensure(cap_batch * 16));
                 int rc = carve_sort_u32(ctx, cap_chunk, sb);
                 if (rc) return rc;
                 if (!ctx->retain()) FILL(cnt + CNT_CELLBB, 24, FILL_CELLBB);
                 // (a chunk that could hold 2^30 per-frame voxels goes around it: k_cell_prereduce's look-back word counts 30 bits)
-                ctx->tiled_now = ctx->tiled() && !(ctx->tiled_poor && (ctx->tiled_batches % 16) != 0) && cap_chunk < kRsWideSeg;
-                ++ctx->tiled_batches;
-                if (ctx->tiled_now) {   // worst case one partial per item; never reached in practice (~1/8)
-                    CU(ctx->partials.ensure(cap_batch * sizeof(o3r_cell)));
-                    CU(ctx->pr_status.ensure(((size_t)cdiv(cap_chunk, kPrTile) + 16) * 4));
+                ctx->pre.now = ctx->tiled() && !(ctx->pre.poor && (ctx->pre.batches % 16) != 0) && cap_chunk < kRsWideSeg;
+                ++ctx->pre.batches;
+                if (ctx->pre.now) {   // worst case one partial per item; never reached in practice (~1/8)
+                    CU(ctx->last.partials.ensure(cap_batch * sizeof(o3r_cell)));
+                    CU(ctx->pre.status.ensure(((size_t)cdiv(cap_chunk, kPrTile) + 16) * 4));
                     ZERO(cnt + CNT_PART, 8);
                 }
             } else {
-                CU(ctx->pts.ensure(cap_batch * 16));
+                CU(ctx->last.pts.ensure(cap_batch * 16));
             }
             ZERO(cnt + CNT_BASE, 4);
             ZERO(ctx->vox_off.p, 4);
         }
-        if (!opt.mask_only) ctx->last_is_vox = P.want_keys;
+        if (!opt.mask_only) ctx->last.is_vox = P.want_keys;
         uint32_t* goff = ctx->vox_off.as<uint32_t>();
 
         for (int f0 = 0; f0 < n; f0 += chunk) {
@@ -400,17 +401,17 @@ int frames_cloud_impl(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_typ
             if (host_inputs && !prefetched && !inputs_resident) {  // H2D of this chunk on the copy stream; the compute stream waits for its event only
                 int rc = stage_copy(ctx, frames, fd_stage, f0, nc, label_mode, G);
                 if (rc) return rc;
-                cudaEvent_t ev = ctx->chunk_event(f0 / chunk);
+                cudaEvent_t ev = ctx->in.chunk_event(f0 / chunk);
                 CU(cudaEventRecord(ev, ctx->st_copy));
                 CU(cudaStreamWaitEvent(ctx->st, ev, 0));
             }
-            const FrameDev* fr = ctx->d_frames.as<FrameDev>() + f0;
+            const FrameDev* fr = ctx->in.frames.as<FrameDev>() + f0;
             if (blur) {
                 const int rx0 = P.x0, rx1 = p.cols - p.bounding_box, ry0 = p.bounding_box, ry1 = p.rows - p.bounding_box;
                 if (rx1 > rx0 && ry1 > ry0) {
                     const dim3 g(cdiv(rx1 - rx0, kBlurStrip), cdiv(ry1 - ry0, blur_rows(p.blur_mode)), nc);
                     const size_t sm = blur_smem(p.blur_kernel, p.blur_mode);
-                    const BlurJob* bj = ctx->d_blurjobs.as<BlurJob>() + f0;
+                    const BlurJob* bj = ctx->blur.jobs.as<BlurJob>() + f0;
                     if (p.blur_mode == O3R_BLUR_BILATERAL) {
                         BilateralLut L;
                         int rcl = bilateral_lut(ctx, p.blur_kernel, &L);
@@ -426,7 +427,7 @@ int frames_cloud_impl(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_typ
             // tile engine: planes -> partial cells of the chunk, per-frame voxel counts, exact bboxes; bucket engine: the same through
             // hist -> scan -> scatter -> reduce; sort engine: stage A, whose V1 mode writes the chunk scratch and whose
             // dont_downsample mode writes the batch buffer at the running base
-            float4* pts_out = ctx->pts.as<float4>();
+            float4* pts_out = ctx->last.pts.as<float4>();
             const uint32_t* base_a = P.want_keys ? nullptr : cnt + CNT_BASE;
             uint32_t* goff_a = P.want_keys ? nullptr : goff + f0;
             int rc = with_disp_type(disp_type, [&](auto dt) {
@@ -437,16 +438,16 @@ int frames_cloud_impl(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_typ
             });
             if (rc) return rc;
             if (engine != Engine::SORT) continue;
-            if (opt.mask_only) { ctx->busy_set = -1; return O3R_OK; }   // (single frame; the last batch's state is untouched)
-            const float4* vg_pts = ctx->pts.as<float4>();
+            if (opt.mask_only) { ctx->in.busy_set = -1; return O3R_OK; }   // (single frame; the last batch's state is untouched)
+            const float4* vg_pts = ctx->last.pts.as<float4>();
             const uint32_t* vg_off = ctx->frame_off.as<uint32_t>();
             if (P.want_keys && p.sor_mean_k > 0 && J > 0) {
                 // StatisticalOutlierRemoval first (pose_functions.cpp:1673-1686); the VoxelGrid then sees the filtered cloud, so
                 // its bbox, grid and leaf indices are recomputed from the kept points
                 rc = sor_filter(ctx, sb, vg_pts, vg_off, nc, per_frame_cap, p.sor_mean_k, p.sor_stddev_mul);
                 if (rc) return rc;
-                vg_pts = ctx->sor_pts.as<float4>();
-                vg_off = ctx->sor_off.as<uint32_t>();
+                vg_pts = ctx->sor.pts.as<float4>();
+                vg_off = ctx->sor.off.as<uint32_t>();
                 const uint32_t tl = std::max(1u, cdiv(per_frame_cap, kTileV));
                 FILL(ctx->bbox.as<uint32_t>(), (size_t)(nc) * 24, FILL_BBOX);
                 LAUNCH(k_bbox_pts, dim3(tl, nc), kThreads, 0, vg_pts, vg_off, 0, ctx->bbox.as<uint32_t>());
@@ -458,15 +459,15 @@ int frames_cloud_impl(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_typ
             if (P.want_keys) {  // per-frame VoxelGrid, leaf voxel_size / 5 (pose_functions.cpp:1698), appended at the base
                 rc = vg_sorted_reduce(ctx, sb, vg_pts, vg_off, nc, per_frame_cap,
                                       ctx->grids.as<GridParams>(), ctx->inv_f, ctx->inv_f, ctx->inv_f, 0, 0,
-                                      ctx->vox.as<float4>(), goff + f0, nullptr, nullptr, !ctx->retain(), cnt + CNT_BASE);
+                                      ctx->last.vox.as<float4>(), goff + f0, nullptr, nullptr, !ctx->retain(), cnt + CNT_BASE);
                 if (rc) return rc;
-                if (ctx->tiled_now) {   // group the chunk's voxel centroids by combined-grid cell, tile by tile
+                if (ctx->pre.now) {   // group the chunk's voxel centroids by combined-grid cell, tile by tile
                     const uint32_t pt = cdiv(cap_chunk, kPrTile);
-                    uint32_t* stw = ctx->pr_status.as<uint32_t>();
+                    uint32_t* stw = ctx->pre.status.as<uint32_t>();
                     ZERO(stw, ((size_t)pt + 16) * 4);
                     ZERO(cnt + CNT_PARTCHUNK, 4);
-                    LAUNCH(k_cell_prereduce, pt, kThreads, 0, ctx->vox.as<float4>(), cnt + CNT_BASE, cnt + CNT_VOX, ctx->inv_c,
-                           ctx->inv_cz, ctx->partials.as<o3r_cell>(), cnt + CNT_PART, cnt + CNT_PARTCHUNK, stw, stw + pt);
+                    LAUNCH(k_cell_prereduce, pt, kThreads, 0, ctx->last.vox.as<float4>(), cnt + CNT_BASE, cnt + CNT_VOX, ctx->inv_c,
+                           ctx->inv_cz, ctx->last.partials.as<o3r_cell>(), cnt + CNT_PART, cnt + CNT_PARTCHUNK, stw, stw + pt);
                     LAUNCH(k_add_u32, 1, 32, 0, cnt + CNT_PART, cnt + CNT_PARTCHUNK);
                 }
                 LAUNCH(k_add_base, 1, 32, 0, cnt + CNT_BASE, cnt + CNT_VOX, goff + f0 + nc);
@@ -477,28 +478,28 @@ int frames_cloud_impl(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_typ
 
         // ---- per-frame output offsets (+ the combined-grid cell range) back to the host: the one sync of the frame path
         const size_t offs_words = (size_t)n + 3 + ((size_t)n + 3) / 4 + 1;   // offsets / counts, two flag words, n flag bytes
-        if (ctx->h_offs_cap < offs_words) {
-            if (ctx->h_offs) cudaFreeHost(ctx->h_offs);
-            ctx->h_offs_cap = std::max<size_t>(offs_words, 256);
-            CU(cudaMallocHost((void**)&ctx->h_offs, ctx->h_offs_cap * 4));
+        if (ctx->last.h_offs_cap < offs_words) {
+            if (ctx->last.h_offs) cudaFreeHost(ctx->last.h_offs);
+            ctx->last.h_offs_cap = std::max<size_t>(offs_words, 256);
+            CU(cudaMallocHost((void**)&ctx->last.h_offs, ctx->last.h_offs_cap * 4));
         }
         if (engine != Engine::SORT) {   // per-frame counts and the engine's flags
             const int rc = engine == Engine::TILE ? tv_read_back(ctx, n) : bk_read_back(ctx, n);
             if (rc) return rc;
         } else {
-            CU(cudaMemcpyAsync(ctx->h_offs, goff, (size_t)(n + 1) * 4, cudaMemcpyDeviceToHost, ctx->st));
+            CU(cudaMemcpyAsync(ctx->last.h_offs, goff, (size_t)(n + 1) * 4, cudaMemcpyDeviceToHost, ctx->st));
         }
-        ctx->last_has_cellbb = ctx->last_is_vox && !ctx->retain();
-        if (ctx->last_has_cellbb)
+        ctx->last.has_cellbb = ctx->last.is_vox && !ctx->retain();
+        if (ctx->last.has_cellbb)
             CU(cudaMemcpyAsync(ctx->h_counters + CNT_CELLBB, cnt + CNT_CELLBB, 24, cudaMemcpyDeviceToHost, ctx->st));
         // the kernels of this call are queued: now issue the copies of a recorded prefetch (next cycle's inputs).  The
         // staging set they go to is not the one these kernels read.
-        if (ctx->deferred.pending && !opt.mask_only) {
+        if (ctx->in.deferred.pending && !opt.mask_only) {
             int rcf = flush_deferred_prefetch(ctx);
             if (rcf) return rcf;
         }
-        ctx->last_has_partials = ctx->last_is_vox && ((ctx->tiled() && ctx->tiled_now) || engine != Engine::SORT);
-        if (ctx->last_has_partials)
+        ctx->last.has_partials = ctx->last.is_vox && ((ctx->tiled() && ctx->pre.now) || engine != Engine::SORT);
+        if (ctx->last.has_partials)
             CU(cudaMemcpyAsync(ctx->h_counters + CNT_PART, cnt + CNT_PART, 4, cudaMemcpyDeviceToHost, ctx->st));
         tr1 = now_ms();
         CU(cudaStreamSynchronize(ctx->st));
@@ -510,42 +511,43 @@ int frames_cloud_impl(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_typ
                 if (v == Verdict::NEXT_ENGINE) engine = engine == Engine::TILE && bucket_ok() ? Engine::BUCKET : Engine::SORT;
                 continue;
             }
-            ctx->h_offs[0] = 0;   // per-frame counts -> offsets
-            for (int i = 0; i < n; ++i) ctx->h_offs[i + 1] += ctx->h_offs[i];
+            ctx->last.h_offs[0] = 0;   // per-frame counts -> offsets
+            for (int i = 0; i < n; ++i) ctx->last.h_offs[i + 1] += ctx->last.h_offs[i];
         }
         break;
     }
-    ctx->last_engine = engine;
-    ctx->busy_set = -1;
-    ctx->last_partials = ctx->last_has_partials ? ctx->h_counters[CNT_PART] : 0;
+    ctx->last.engine = engine;
+    ctx->in.busy_set = -1;
+    const size_t n_part = ctx->last.has_partials ? ctx->h_counters[CNT_PART] : 0;
     // The tile pre-reduction pays only when it reduces: a 40-byte partial replaces a 16-byte voxel in the merge.  On grids
     // finer than the point spacing (e.g. 4K at voxel_size 0.01) nearly every voxel is its own cell: merge the voxels then.
-    if (ctx->last_has_partials && engine == Engine::SORT) {
-        ctx->tiled_poor = ctx->last_partials * 2 > ctx->h_offs[n];
-        if (ctx->tiled_poor) { ctx->last_has_partials = false; ctx->last_partials = 0; }
+    if (ctx->last.has_partials && engine == Engine::SORT) {
+        ctx->pre.poor = n_part * 2 > ctx->last.h_offs[n];
+        ctx->last.has_partials = !ctx->pre.poor;
     }
-    if (ctx->last_has_cellbb) memcpy(ctx->last_cellbb, ctx->h_counters + CNT_CELLBB, 24);
-    ctx->last_off.assign(ctx->h_offs, ctx->h_offs + n + 1);
-    ctx->last_n = n;
-    ctx->last_total = ctx->last_off[n];
+    ctx->last.n_part = ctx->last.has_partials ? n_part : 0;
+    if (ctx->last.has_cellbb) memcpy(ctx->last.cellbb, ctx->h_counters + CNT_CELLBB, 24);
+    ctx->last.off.assign(ctx->last.h_offs, ctx->last.h_offs + n + 1);
+    ctx->last.n = n;
+    ctx->last.total = ctx->last.off[n];
     if (frame_counts)
-        for (int i = 0; i < n; ++i) frame_counts[i] = ctx->last_off[i + 1] - ctx->last_off[i];
+        for (int i = 0; i < n; ++i) frame_counts[i] = ctx->last.off[i + 1] - ctx->last.off[i];
     if (!opt.merge || (ctx->comm && !ctx->retain())) return O3R_OK;   // with a communicator, o3r_exchange_cycle merges the cycle
-    const float4* outp = ctx->last_is_vox ? ctx->vox.as<float4>() : ctx->pts.as<float4>();
+    const float4* outp = ctx->last.is_vox ? ctx->last.vox.as<float4>() : ctx->last.pts.as<float4>();
     if (ctx->retain()) {
-        const size_t base = ctx->n_cloud;
-        const int rca = cloud_append_dev(ctx, outp, ctx->last_total);
+        const size_t base = ctx->res.n_cloud;
+        const int rca = cloud_append_dev(ctx, outp, ctx->last.total);
         if (rca) return rca;
         if (rt_shard)   // rank r's frame i is the cycle's frame i * world + r
             for (int i = 0; i < n; ++i)
-                if (ctx->last_off[i + 1] > ctx->last_off[i])
-                    ctx->rt_frames.push_back({base + ctx->last_off[i], rt_cycle, (uint32_t)i * (uint32_t)ctx->world + (uint32_t)ctx->rank});
+                if (ctx->last.off[i + 1] > ctx->last.off[i])
+                    ctx->rt.frames.push_back({base + ctx->last.off[i], rt_cycle, (uint32_t)i * (uint32_t)ctx->world + (uint32_t)ctx->rank});
         return O3R_OK;
     }
-    const int* bbp = ctx->last_has_cellbb ? ctx->last_cellbb : nullptr;
-    if (engine != Engine::SORT && ctx->last_partials == 0) return O3R_OK;   // nothing valid in the whole batch
-    const int rcm = ctx->last_has_partials ? acc_merge_cells(ctx, ctx->partials.as<o3r_cell>(), ctx->last_partials, bbp)
-                                           : acc_merge_points(ctx, outp, ctx->last_total, bbp);
+    const int* bbp = ctx->last.has_cellbb ? ctx->last.cellbb : nullptr;
+    if (engine != Engine::SORT && ctx->last.n_part == 0) return O3R_OK;   // nothing valid in the whole batch
+    const int rcm = ctx->last.has_partials ? acc_merge_cells(ctx, ctx->last.partials.as<o3r_cell>(), ctx->last.n_part, bbp)
+                                           : acc_merge_points(ctx, outp, ctx->last.total, bbp);
     if (trace) fprintf(stderr, "[o3r trace] frames_cloud: enqueue %.3f ms, sync wait %.3f ms, merge enqueue %.3f ms\n", tr1 - tr0, tr2 - tr1, now_ms() - tr2);
     return rcm;
 }

@@ -51,10 +51,10 @@ int acc_build_cycle_t(o3r_ctx* ctx, Items items, size_t n, bool use_resident, co
     A.seg_off = seg; A.plan = plan;
     A.tiles_ub = cdiv(n, kTileV);
     A.kc = kc;
-    const int cur = ctx->res_cur;
-    A.res_keys = ctx->res_keys[cur].as<uint64_t>();
-    A.res_acc = ctx->res_acc[cur].as<float4>();
-    A.res_rgb = ctx->res_rgb[cur].as<uint4>();
+    const int cur = ctx->res.cur;
+    A.res_keys = ctx->res.keys[cur].as<uint64_t>();
+    A.res_acc = ctx->res.acc[cur].as<float4>();
+    A.res_rgb = ctx->res.rgb[cur].as<uint4>();
     A.n_res_ptr = cnt + (use_resident ? CNT_NRES : CNT_ZERO);
     CU(ctx->head_cnt.ensure((size_t)A.tiles_ub * 4));
     CU(ctx->head_off.ensure((size_t)A.tiles_ub * 4));
@@ -78,14 +78,40 @@ int acc_build_cycle_t(o3r_ctx* ctx, Items items, size_t n, bool use_resident, co
     return O3R_OK;
 }
 
+// ---- the resident map (Resident, host_ctx.cuh) --------------------------------------------------------------------
 // Tightens the host's upper bound of the resident cell count from the read-back of the last merge.
 int refresh_nres(o3r_ctx* ctx, bool block) {
-    if (ctx->n_res_exact) return O3R_OK;
-    if (block) CU(cudaEventSynchronize(ctx->ev_nres));
-    else if (cudaEventQuery(ctx->ev_nres) != cudaSuccess) { cudaGetLastError(); return O3R_OK; }
-    ctx->n_res_ub = *ctx->h_nres;
-    ctx->n_res_exact = true;
+    if (ctx->res.n_exact) return O3R_OK;
+    if (block) CU(cudaEventSynchronize(ctx->res.ev_n));
+    else if (cudaEventQuery(ctx->res.ev_n) != cudaSuccess) { cudaGetLastError(); return O3R_OK; }
+    ctx->res.n_ub = *ctx->res.h_n;
+    ctx->res.n_exact = true;
     return O3R_OK;
+}
+
+// Reads every counter back (one sync): h_counters is valid afterwards, and the resident count exact.
+int res_read_back(o3r_ctx* ctx) {
+    { int rc = read_counters(ctx); if (rc) return rc; }
+    ctx->res.n_ub = ctx->h_counters[CNT_NRES];
+    ctx->res.n_exact = true;
+    return O3R_OK;
+}
+
+// Empties the resident map (o3r_cloud_clear); the caller has synchronised the stream.
+int res_clear(o3r_ctx* ctx) {
+    ctx->res.n_cloud = 0; ctx->res.n_ub = 0; ctx->res.n_exact = true;
+    ZERO(ctx->counters.as<uint32_t>() + CNT_NRES, 4);
+    return O3R_OK;
+}
+
+// true when the host knows the resident count exactly and it exceeds `cap`
+bool res_exceeds(const o3r_ctx* ctx, size_t cap) { return ctx->res.n_exact && cap < ctx->res.n_ub; }
+
+// the resident accumulators' current set: what every reader of the shard sees (the count is counters[CNT_NRES])
+struct ResCells { const uint64_t* keys; const float4* acc; const uint4* rgb; };
+ResCells res_cells(const o3r_ctx* ctx) {
+    const int c = ctx->res.cur;
+    return {ctx->res.keys[c].as<uint64_t>(), ctx->res.acc[c].as<float4>(), ctx->res.rgb[c].as<uint4>()};
 }
 
 // Builds the cycle's cell list (ckey/cacc/crgb, count in counters[CNT_CYC]) from items, continuing from the resident sums when
@@ -148,45 +174,45 @@ int acc_apply_cycle(o3r_ctx* ctx) {
     const size_t n_cyc_ub = ctx->n_cyc_ub;
     if (n_cyc_ub == 0) return O3R_OK;
     uint32_t* cnt = ctx->counters.as<uint32_t>();
-    const int cur = ctx->res_cur, nxt = cur ^ 1;
+    const int cur = ctx->res.cur, nxt = cur ^ 1;
     const uint32_t tiles = cdiv(n_cyc_ub, kTileV);
-    const size_t tot_ub = ctx->n_res_ub + n_cyc_ub;
+    const size_t tot_ub = ctx->res.n_ub + n_cyc_ub;
     Tr tr("acc_apply");
     if (tot_ub >= (1ull << 32)) return ctx->fail(O3R_ERR_NOMEM, "resident shard could exceed 2^32 cells");
     CU(ctx->new_cnt.ensure((size_t)tiles * 4));
     CU(ctx->new_off.ensure((size_t)tiles * 4));
     // the shard grows a little every cycle: reserve in big steps (>= 4 M cells, doubling), a reallocation is a
     // cudaMalloc + cudaFree = a device-wide sync of several ms in the middle of the cycle
-    if (ctx->res_keys[nxt].cap < tot_ub * 8 || ctx->res_acc[nxt].cap < tot_ub * 16 || ctx->res_rgb[nxt].cap < tot_ub * 16) {
+    if (ctx->res.keys[nxt].cap < tot_ub * 8 || ctx->res.acc[nxt].cap < tot_ub * 16 || ctx->res.rgb[nxt].cap < tot_ub * 16) {
         const size_t cells = std::max<size_t>(2 * tot_ub, (size_t)1 << 22);
-        CU(ctx->res_keys[nxt].ensure(cells * 8));
-        CU(ctx->res_acc[nxt].ensure(cells * 16));
-        CU(ctx->res_rgb[nxt].ensure(cells * 16));
+        CU(ctx->res.keys[nxt].ensure(cells * 8));
+        CU(ctx->res.acc[nxt].ensure(cells * 16));
+        CU(ctx->res.rgb[nxt].ensure(cells * 16));
     }
     CU(ctx->new_keys.ensure(n_cyc_ub * 8));
     { int rc = chg_reserve(ctx, n_cyc_ub); if (rc) return rc; }
-    if (tr.on) fprintf(stderr, "[o3r trace] n_res_ub %zu n_cyc_ub %zu\n", ctx->n_res_ub, n_cyc_ub);
+    if (tr.on) fprintf(stderr, "[o3r trace] n_res_ub %zu n_cyc_ub %zu\n", ctx->res.n_ub, n_cyc_ub);
     tr.mark("ensures");
     LAUNCH(k_acc_update, tiles, kThreads, 0, cnt + CNT_CYC, ctx->cacc.as<float4>(), ctx->crgb.as<uint4>(),
-           ctx->res_acc[cur].as<float4>(), ctx->res_rgb[cur].as<uint4>(), ctx->new_cnt.as<uint32_t>());
+           ctx->res.acc[cur].as<float4>(), ctx->res.rgb[cur].as<uint4>(), ctx->new_cnt.as<uint32_t>());
     LAUNCH(k_scan_u32, 1, kScanThreads, 0, ctx->new_cnt.as<uint32_t>(), ctx->new_off.as<uint32_t>(), tiles,
            cnt + CNT_NEWSCAN);
     LAUNCH(k_acc_place_new, tiles, kThreads, 0, cnt + CNT_CYC, ctx->ckey.as<uint64_t>(), ctx->cacc.as<float4>(),
-           ctx->crgb.as<uint4>(), ctx->new_off.as<uint32_t>(), ctx->res_keys[cur].as<uint64_t>(), cnt + CNT_NRES,
-           ctx->res_keys[nxt].as<uint64_t>(), ctx->res_acc[nxt].as<float4>(), ctx->res_rgb[nxt].as<uint4>(),
+           ctx->crgb.as<uint4>(), ctx->new_off.as<uint32_t>(), ctx->res.keys[cur].as<uint64_t>(), cnt + CNT_NRES,
+           ctx->res.keys[nxt].as<uint64_t>(), ctx->res.acc[nxt].as<float4>(), ctx->res.rgb[nxt].as<uint4>(),
            ctx->new_keys.as<uint64_t>());
-    if (ctx->n_res_ub) {
-        const uint32_t g = std::min<uint32_t>(cdiv(ctx->n_res_ub, kThreads), 148 * 16);
-        LAUNCH(k_acc_place_old, g, kThreads, 0, cnt + CNT_NRES, ctx->res_keys[cur].as<uint64_t>(),
-               ctx->res_acc[cur].as<float4>(), ctx->res_rgb[cur].as<uint4>(), ctx->new_keys.as<uint64_t>(), cnt + CNT_NEW,
-               ctx->res_keys[nxt].as<uint64_t>(), ctx->res_acc[nxt].as<float4>(), ctx->res_rgb[nxt].as<uint4>());
+    if (ctx->res.n_ub) {
+        const uint32_t g = std::min<uint32_t>(cdiv(ctx->res.n_ub, kThreads), 148 * 16);
+        LAUNCH(k_acc_place_old, g, kThreads, 0, cnt + CNT_NRES, ctx->res.keys[cur].as<uint64_t>(),
+               ctx->res.acc[cur].as<float4>(), ctx->res.rgb[cur].as<uint4>(), ctx->new_keys.as<uint64_t>(), cnt + CNT_NEW,
+               ctx->res.keys[nxt].as<uint64_t>(), ctx->res.acc[nxt].as<float4>(), ctx->res.rgb[nxt].as<uint4>());
     }
     LAUNCH(k_acc_finish, 1, 32, 0, cnt + CNT_NRES, cnt + CNT_NEW);
-    ctx->res_cur = nxt;
-    ctx->n_res_ub = tot_ub;
-    ctx->n_res_exact = false;
-    CU(cudaMemcpyAsync(ctx->h_nres, cnt + CNT_NRES, 4, cudaMemcpyDeviceToHost, ctx->st));
-    CU(cudaEventRecord(ctx->ev_nres, ctx->st));
+    ctx->res.cur = nxt;
+    ctx->res.n_ub = tot_ub;
+    ctx->res.n_exact = false;
+    CU(cudaMemcpyAsync(ctx->res.h_n, cnt + CNT_NRES, 4, cudaMemcpyDeviceToHost, ctx->st));
+    CU(cudaEventRecord(ctx->res.ev_n, ctx->st));
     tr.mark("launches");
     return chg_cycle(ctx, n_cyc_ub);
 }
@@ -207,9 +233,9 @@ int acc_merge_cells(o3r_ctx* ctx, const o3r_cell* cells, size_t n, const int* bb
 
 int cloud_append_dev(o3r_ctx* ctx, const float4* pts, size_t n) {
     if (n == 0) return O3R_OK;
-    CU(ctx->cloud.ensure((ctx->n_cloud + n) * 16, ctx->st, ctx->n_cloud * 16));
-    CU(cudaMemcpyAsync(ctx->cloud.as<float4>() + ctx->n_cloud, pts, n * 16, cudaMemcpyDeviceToDevice, ctx->st));
-    ctx->n_cloud += n;
+    CU(ctx->res.cloud.ensure((ctx->res.n_cloud + n) * 16, ctx->st, ctx->res.n_cloud * 16));
+    CU(cudaMemcpyAsync(ctx->res.cloud.as<float4>() + ctx->res.n_cloud, pts, n * 16, cudaMemcpyDeviceToDevice, ctx->st));
+    ctx->res.n_cloud += n;
     return O3R_OK;
 }
 

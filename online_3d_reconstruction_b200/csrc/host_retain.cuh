@@ -20,70 +20,70 @@ namespace {
 
 // (named phases for o3r_profile_read: the split of the collective into local prep, exchange and owner reduction)
 cudaEvent_t rt_phase_begin(o3r_ctx* ctx) {
-    if (!ctx->profiling) return nullptr;
-    cudaEvent_t e = ctx->ev_get();
+    if (!ctx->prof.on) return nullptr;
+    cudaEvent_t e = ctx->prof.get();
     cudaEventRecord(e, ctx->st);
     return e;
 }
 void rt_phase_end(o3r_ctx* ctx, const char* name, cudaEvent_t a) {
     if (!a) return;
-    cudaEvent_t b = ctx->ev_get();
+    cudaEvent_t b = ctx->prof.get();
     cudaEventRecord(b, ctx->st);
-    ctx->prof.push_back({name, a, b});
+    ctx->prof.recs.push_back({name, a, b});
 }
 
 inline uint32_t rt_bits(uint32_t v) { uint32_t b = 0; while (v) { ++b; v >>= 1; } return b; }
 
-// engine 1 over `n` points with the global grid already in ctx->grids (z shifted by 500, the combined grid) -> ctx->rt_out
+// engine 1 over `n` points with the global grid already in ctx->grids (z shifted by 500, the combined grid) -> ctx->rt.out
 int rt_engine1(o3r_ctx* ctx, const float4* pts, size_t n, size_t* m) {
     *m = 0;
     if (n == 0) return O3R_OK;
-    CU(ctx->rt_out.ensure(n * 16));
+    CU(ctx->rt.out.ensure(n * 16));
     const uint32_t seg_h[2] = {0u, (uint32_t)n};
     { int rcu = upload_small(ctx, ctx->seg2.p, seg_h, 8); if (rcu) return rcu; }
     return vg_one_segment(ctx, pts, ctx->seg2.as<uint32_t>(), n, ctx->inv_c, ctx->inv_c, ctx->inv_cz,
-                          ctx->p.min_points_per_voxel, 1, ctx->rt_out.as<float4>(), nullptr, nullptr, m);
+                          ctx->p.min_points_per_voxel, 1, ctx->rt.out.as<float4>(), nullptr, nullptr, m);
 }
 
 // step 1, local part: the z-shifted bbox of the local cloud and the words of the first agreement
 int rt_local_bbox(o3r_ctx* ctx, uint32_t n_frames, uint32_t* w) {
-    const size_t n = ctx->n_cloud;
+    const size_t n = ctx->res.n_cloud;
     if (n > kRtMaxPoints) return ctx->fail(O3R_ERR_INVALID, "local cloud too large for 32-bit indices");
-    if (n && ctx->rt_frames.empty()) return ctx->fail(O3R_ERR_INVALID, "retained points without a frame record");
+    if (n && ctx->rt.frames.empty()) return ctx->fail(O3R_ERR_INVALID, "retained points without a frame record");
     FILL(ctx->bbox.as<uint32_t>(), 24, FILL_BBOX);
     if (n) {
         const uint32_t seg_h[2] = {0u, (uint32_t)n};
         { int rcu = upload_small(ctx, ctx->seg2.p, seg_h, 8); if (rcu) return rcu; }
-        LAUNCH(k_bbox_pts, dim3(cdiv(n, kTileV), 1), kThreads, 0, ctx->cloud.as<float4>(), ctx->seg2.as<uint32_t>(), 1,
+        LAUNCH(k_bbox_pts, dim3(cdiv(n, kTileV), 1), kThreads, 0, ctx->res.cloud.as<float4>(), ctx->seg2.as<uint32_t>(), 1,
                ctx->bbox.as<uint32_t>());
     }
-    LAUNCH(k_rt_agree_pack, 1, 32, 0, ctx->bbox.as<uint32_t>(), n_frames, ctx->rt_cycles, 0u, w);
+    LAUNCH(k_rt_agree_pack, 1, 32, 0, ctx->bbox.as<uint32_t>(), n_frames, ctx->rt.cycles, 0u, w);
     return O3R_OK;
 }
 
-// step 2, local part: owner + tag per point, stable bucketing by owner into ctx->rt_send; counts land in `ocnt`
+// step 2, local part: owner + tag per point, stable bucketing by owner into ctx->rt.send; counts land in `ocnt`
 int rt_route(o3r_ctx* ctx, uint32_t fbits, uint32_t** ocnt_out) {
     const uint32_t world = (uint32_t)ctx->world;
-    const size_t n = ctx->n_cloud;
+    const size_t n = ctx->res.n_cloud;
     CU(ctx->okeys.ensure((size_t)kMaxPasses * kRsBins * 4 + sizeof(SortPlan)));
     uint32_t* ocnt = ctx->okeys.as<uint32_t>();
     *ocnt_out = ocnt;
     ZERO(ocnt, (size_t)kMaxPasses * kRsBins * 4);
     if (n == 0) return O3R_OK;
     // the device copy of the frame table grows with the cloud: only the records added since the last downsample are copied
-    const size_t nf = ctx->rt_frames.size(), done = std::min(ctx->rt_ftab_n, nf);
+    const size_t nf = ctx->rt.frames.size(), done = std::min(ctx->rt.ftab_n, nf);
     if (nf > done) {
         std::vector<RtFrameDev> tail(nf - done);
         for (size_t i = done; i < nf; ++i) {
-            const o3r_ctx::RtFrame& f = ctx->rt_frames[i];
+            const RetainShard::Frame& f = ctx->rt.frames[i];
             tail[i - done] = {(uint32_t)f.first, f.cycle, f.frame};
         }
-        CU(ctx->rt_ftab.ensure(nf * sizeof(RtFrameDev), ctx->st, done * sizeof(RtFrameDev)));
-        CU(cudaMemcpyAsync(ctx->rt_ftab.as<RtFrameDev>() + done, tail.data(), tail.size() * sizeof(RtFrameDev), cudaMemcpyHostToDevice, ctx->st));
-        ctx->rt_ftab_n = nf;
+        CU(ctx->rt.ftab.ensure(nf * sizeof(RtFrameDev), ctx->st, done * sizeof(RtFrameDev)));
+        CU(cudaMemcpyAsync(ctx->rt.ftab.as<RtFrameDev>() + done, tail.data(), tail.size() * sizeof(RtFrameDev), cudaMemcpyHostToDevice, ctx->st));
+        ctx->rt.ftab_n = nf;
     }
-    CU(ctx->rt_tags.ensure(n * 4));
-    CU(ctx->rt_send.ensure(n * sizeof(RtRec)));
+    CU(ctx->rt.tags.ensure(n * 4));
+    CU(ctx->rt.send.ensure(n * sizeof(RtRec)));
     SortU32 sb;
     int rc = carve_sort_u32(ctx, n, sb);
     if (rc) return rc;
@@ -95,12 +95,12 @@ int rt_route(o3r_ctx* ctx, uint32_t fbits, uint32_t** ocnt_out) {
     pl.active_mask = 1; pl.final_parity = 1; pl.n_active = 1; pl.n_passes = 1; pl.bits[0] = 8;
     { int rcu = upload_small(ctx, plan, &pl, sizeof(pl)); if (rcu) return rcu; }
     const uint32_t g = std::min<uint32_t>(cdiv(n, kThreads), 148 * 8);
-    LAUNCH(k_rt_route, g, kThreads, 0, ctx->cloud.as<float4>(), (uint32_t)n, ctx->rt_ftab.as<RtFrameDev>(), (uint32_t)nf, fbits,
-           ctx->inv_c, ctx->inv_c, ctx->inv_cz, world, sb.k0, ctx->rt_tags.as<uint32_t>(), ocnt);
+    LAUNCH(k_rt_route, g, kThreads, 0, ctx->res.cloud.as<float4>(), (uint32_t)n, ctx->rt.ftab.as<RtFrameDev>(), (uint32_t)nf, fbits,
+           ctx->inv_c, ctx->inv_c, ctx->inv_cz, world, sb.k0, ctx->rt.tags.as<uint32_t>(), ocnt);
     rc = sort_pairs<uint32_t>(ctx, sb.k0, sb.k1, sb.v0, sb.v1, ctx->seg2.as<uint32_t>(), 1, n, plan, 1, 1, ocnt, 0);
     if (rc) return rc;
-    LAUNCH(k_rt_pack, g, kThreads, 0, ctx->cloud.as<float4>(), ctx->rt_tags.as<uint32_t>(), sb.v1, (uint32_t)n,
-           ctx->rt_send.as<RtRec>());
+    LAUNCH(k_rt_pack, g, kThreads, 0, ctx->res.cloud.as<float4>(), ctx->rt.tags.as<uint32_t>(), sb.v1, (uint32_t)n,
+           ctx->rt.send.as<RtRec>());
     return O3R_OK;
 }
 
@@ -108,8 +108,8 @@ int rt_route(o3r_ctx* ctx, uint32_t fbits, uint32_t** ocnt_out) {
 int rt_owner_reduce(o3r_ctx* ctx, size_t n_own, uint32_t tag_bits, size_t* m) {
     *m = 0;
     if (n_own == 0) return O3R_OK;
-    const RtRec* rec = ctx->rt_recv.as<RtRec>();
-    CU(ctx->rt_pts.ensure(n_own * 16));
+    const RtRec* rec = ctx->rt.recv.as<RtRec>();
+    CU(ctx->rt.pts.ensure(n_own * 16));
     const uint32_t seg_h[2] = {0u, (uint32_t)n_own};
     { int rcu = upload_small(ctx, ctx->seg2.p, seg_h, 8); if (rcu) return rcu; }
     const uint32_t* seg = ctx->seg2.as<uint32_t>();
@@ -130,8 +130,8 @@ int rt_owner_reduce(o3r_ctx* ctx, size_t n_own, uint32_t tag_bits, size_t* m) {
     LAUNCH(k_rs_plan, 1, kThreads, 0, ctx->ghist.as<uint32_t>(), seg, plan, nullptr);
     rc = sort_pairs<uint32_t>(ctx, sb.k0, sb.k1, sb.v0, sb.v1, seg, 1, n_own, plan, 4, 1, ctx->ghist.as<uint32_t>());
     if (rc) return rc;
-    LAUNCH(k_rt_gather, g, kThreads, 0, rec, (uint32_t)n_own, plan, sb.v0, sb.v1, ctx->rt_pts.as<float4>());
-    return rt_engine1(ctx, ctx->rt_pts.as<float4>(), n_own, m);
+    LAUNCH(k_rt_gather, g, kThreads, 0, rec, (uint32_t)n_own, plan, sb.v0, sb.v1, ctx->rt.pts.as<float4>());
+    return rt_engine1(ctx, ctx->rt.pts.as<float4>(), n_own, m);
 }
 
 // every rank leaves the collective with an error: the failing rank with its own, the others naming the peer
@@ -163,12 +163,12 @@ int rt_read_verdict(o3r_ctx* ctx, uint32_t* w, uint32_t* hw, GridParams* G) {
 // alike.  What ends a rank's part early is an NCCL call that fails or a stream that no longer runs (a read-back of an agreement
 // fails): the communicator is then unusable for every rank and the caller's recourse is NCCL's own (ncclCommAbort).
 int retain_downsample_sharded(o3r_ctx* ctx, const float4** res, size_t* m) {
-    *res = ctx->rt_out.as<float4>(); *m = 0;
-    if (ctx->rt_valid) { *m = ctx->rt_m; return O3R_OK; }   // the local cloud has not changed since: no communication
+    *res = ctx->rt.out.as<float4>(); *m = 0;
+    if (ctx->rt.valid) { *m = ctx->rt.m; return O3R_OK; }   // the local cloud has not changed since: no communication
     NcclApi* N = nccl_api();
     const uint32_t world = (uint32_t)ctx->world, rank = (uint32_t)ctx->rank;
     ncclComm_t comm = (ncclComm_t)ctx->comm;
-    uint32_t* w = ctx->rt_agree.as<uint32_t>();
+    uint32_t* w = ctx->rt.agree.as<uint32_t>();
     uint32_t* csend = w + kRtWords;
     uint32_t* crecv = csend + 2 * world;
     uint32_t* bstat = crecv + 2 * world;
@@ -179,7 +179,7 @@ int retain_downsample_sharded(o3r_ctx* ctx, const float4** res, size_t* m) {
     // ---- 1. global bbox, frame / cycle ranges and status: one all-reduce (max)
     cudaEvent_t ph = rt_phase_begin(ctx);
     uint32_t n_frames = 0;
-    for (const o3r_ctx::RtFrame& f : ctx->rt_frames) n_frames = std::max(n_frames, f.frame + 1);
+    for (const RetainShard::Frame& f : ctx->rt.frames) n_frames = std::max(n_frames, f.frame + 1);
     if (local(rt_local_bbox(ctx, n_frames, w))) {
         ctx->fq.clear();   // (fills of the failed step: nothing reads them)
         uint32_t e[kRtWords] = {};
@@ -253,12 +253,12 @@ int retain_downsample_sharded(o3r_ctx* ctx, const float4** res, size_t* m) {
     if (verdict == V_WRAP) return ctx->fail(O3R_ERR_UNSUPPORTED, "sharded downsample: the combined grid has more than 2^32 cells");
     if (verdict == V_TAG)
         return ctx->fail(O3R_ERR_UNSUPPORTED, "sharded downsample: cycles x frames per cycle exceed the 32-bit order tag; clear the cloud");
-    if (verdict == V_EMPTY) { ctx->rt_valid = true; ctx->rt_m = 0; rt_phase_end(ctx, "retain_exchange", ph); return O3R_OK; }
+    if (verdict == V_EMPTY) { ctx->rt.valid = true; ctx->rt.m = 0; rt_phase_end(ctx, "retain_exchange", ph); return O3R_OK; }
     if (verdict == V_PASS) {   // no further communication
-        int rc = rt_engine1(ctx, ctx->cloud.as<float4>(), ctx->n_cloud, m);
+        int rc = rt_engine1(ctx, ctx->res.cloud.as<float4>(), ctx->res.n_cloud, m);
         if (rc) return rc;
-        ctx->rt_valid = true; ctx->rt_m = *m;
-        *res = ctx->rt_out.as<float4>();
+        ctx->rt.valid = true; ctx->rt.m = *m;
+        *res = ctx->rt.out.as<float4>();
         rt_phase_end(ctx, "retain_exchange", ph);
         return O3R_OK;
     }
@@ -267,7 +267,7 @@ int retain_downsample_sharded(o3r_ctx* ctx, const float4** res, size_t* m) {
     uint32_t bufs_bad = 0;
     if (n_own > kRtMaxPoints) { bufs_bad = 1; local(ctx->fail(O3R_ERR_INVALID, "owned points exceed the 32-bit index range")); }
     else {
-        cudaError_t e = ctx->rt_recv.ensure(std::max<size_t>(n_own, 1) * sizeof(RtRec));
+        cudaError_t e = ctx->rt.recv.ensure(std::max<size_t>(n_own, 1) * sizeof(RtRec));
         if (e != cudaSuccess) { bufs_bad = 1; local(ctx->fail_cuda(e, "rt_recv.ensure", __FILE__, __LINE__)); }
     }
     { int rcu = rt_put_words(ctx, bstat, &bufs_bad, 1); if (rcu) return rcu; }
@@ -276,8 +276,8 @@ int retain_downsample_sharded(o3r_ctx* ctx, const float4** res, size_t* m) {
     CU(cudaMemcpyAsync(&any_bad, bstat, 4, cudaMemcpyDeviceToHost, ctx->st));
     CU(cudaStreamSynchronize(ctx->st));
     if (any_bad) return rt_collective_fail(ctx, local_rc, local_err);
-    const char* snd = ctx->rt_send.as<char>();
-    char* rcv = ctx->rt_recv.as<char>();
+    const char* snd = ctx->rt.send.as<char>();
+    char* rcv = ctx->rt.recv.as<char>();
     constexpr size_t R = sizeof(RtRec);
     if (scnt[rank]) CU(cudaMemcpyAsync(rcv + roff[rank] * R, snd + soff[rank] * R, scnt[rank] * R, cudaMemcpyDeviceToDevice, ctx->st));
     if (world > 1) {   // both sides of a pair know its size: empty buckets are skipped on both
@@ -299,8 +299,8 @@ int retain_downsample_sharded(o3r_ctx* ctx, const float4** res, size_t* m) {
     int rc = rt_owner_reduce(ctx, n_own, fbits + sbits, m);
     if (rc) return rc;
     rt_phase_end(ctx, "retain_reduce", ph);
-    ctx->rt_valid = true; ctx->rt_m = *m;
-    *res = ctx->rt_out.as<float4>();
+    ctx->rt.valid = true; ctx->rt.m = *m;
+    *res = ctx->rt.out.as<float4>();
     return O3R_OK;
 }
 

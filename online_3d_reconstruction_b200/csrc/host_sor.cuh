@@ -7,30 +7,30 @@
 namespace {
 
 // ---- pcl::StatisticalOutlierRemoval on the frames of a chunk (pose_functions.cpp:1673-1686) -----------------------------
-// in: pts with segment offsets seg_off[n_seg + 1] (device).  out: ctx->sor_pts / ctx->sor_off (same layout, kept points
-// in their original order).  Uses the sort buffers (free again afterwards) and ctx->bbox / ctx->spts as scratch.
+// in: pts with segment offsets seg_off[n_seg + 1] (device).  out: ctx->sor.pts / ctx->sor.off (same layout, kept points
+// in their original order).  Uses the sort buffers (free again afterwards) and ctx->bbox / ctx->sor.spts as scratch.
 int sor_filter(o3r_ctx* ctx, const SortU32& sb, const float4* pts, const uint32_t* seg_off, int n_seg, size_t per_seg_cap,
                int mean_k, double stddev_mul) {
     if (mean_k < 1) return ctx->fail(O3R_ERR_INVALID, "sor_mean_k must be positive");
     if (mean_k + 1 > kSorMaxK) return ctx->fail(O3R_ERR_INVALID, "sor_mean_k too large (max 127)");
     const size_t cap = per_seg_cap * n_seg;
     const uint32_t tiles = std::max(1u, cdiv(per_seg_cap, kTileV));
-    CU(ctx->sor_pts.ensure(cap * 16));
-    CU(ctx->sor_off.ensure((size_t)(n_seg + 1) * 4));
-    CU(ctx->sor_dist.ensure(cap * 4));
-    CU(ctx->sor_skeys.ensure(cap * 4));
-    CU(ctx->sor_svals.ensure(cap * 4));
-    CU(ctx->spts.ensure(cap * 16));
-    CU(ctx->sor_grids.ensure((size_t)n_seg * sizeof(SorGrid)));
-    CU(ctx->sor_pgrids.ensure((size_t)n_seg * sizeof(GridParams)));
-    CU(ctx->sor_rows.ensure((size_t)n_seg * (kSorCellsCap + 1) * 4));
-    CU(ctx->sor_thr.ensure((size_t)n_seg * 8));
-    CU(ctx->sor_cnt.ensure((size_t)tiles * n_seg * 4));
-    CU(ctx->sor_cntoff.ensure((size_t)tiles * n_seg * 4));
+    CU(ctx->sor.pts.ensure(cap * 16));
+    CU(ctx->sor.off.ensure((size_t)(n_seg + 1) * 4));
+    CU(ctx->sor.dist.ensure(cap * 4));
+    CU(ctx->sor.skeys.ensure(cap * 4));
+    CU(ctx->sor.svals.ensure(cap * 4));
+    CU(ctx->sor.spts.ensure(cap * 16));
+    CU(ctx->sor.grids.ensure((size_t)n_seg * sizeof(SorGrid)));
+    CU(ctx->sor.pgrids.ensure((size_t)n_seg * sizeof(GridParams)));
+    CU(ctx->sor.rows.ensure((size_t)n_seg * (kSorCellsCap + 1) * 4));
+    CU(ctx->sor.thr.ensure((size_t)n_seg * 8));
+    CU(ctx->sor.cnt.ensure((size_t)tiles * n_seg * 4));
+    CU(ctx->sor.cntoff.ensure((size_t)tiles * n_seg * 4));
     CU(ctx->bbox.ensure((size_t)n_seg * 6 * 4));
-    SorGrid* grids = ctx->sor_grids.as<SorGrid>();
-    GridParams* pgrids = ctx->sor_pgrids.as<GridParams>();
-    uint32_t* cell_start = ctx->sor_rows.as<uint32_t>();   // [n_seg][kSorCellsCap + 1]
+    SorGrid* grids = ctx->sor.grids.as<SorGrid>();
+    GridParams* pgrids = ctx->sor.pgrids.as<GridParams>();
+    uint32_t* cell_start = ctx->sor.rows.as<uint32_t>();   // [n_seg][kSorCellsCap + 1]
     uint32_t* cnt = ctx->counters.as<uint32_t>();
     const uint32_t gl = std::min<uint32_t>(std::max(1u, cdiv(per_seg_cap, kThreads)), 148 * 4);
     FILL(ctx->bbox.as<uint32_t>(), (size_t)(n_seg) * 24, FILL_BBOX);
@@ -49,28 +49,28 @@ int sor_filter(o3r_ctx* ctx, const SortU32& sb, const float4* pts, const uint32_
         rc = sort_pairs<uint32_t>(ctx, sb.k0, sb.k1, sb.v0, sb.v1, seg_off, n_seg, per_seg_cap, plan, 4, 1, ctx->ghist.as<uint32_t>());
         if (rc) return rc;
         LAUNCH(k_sor_cells, dim3(gl, n_seg), kThreads, 0, sb.k0, sb.k1, sb.v0, sb.v1, plan, pts, seg_off, grids, cell_start,
-               ctx->sor_skeys.as<uint32_t>(), ctx->sor_svals.as<uint32_t>(), ctx->spts.as<float4>());
+               ctx->sor.skeys.as<uint32_t>(), ctx->sor.svals.as<uint32_t>(), ctx->sor.spts.as<float4>());
         if (round == 0)
-            LAUNCH(k_sor_calib, n_seg, kSorThreads, heap_bytes, ctx->spts.as<float4>(), ctx->sor_skeys.as<uint32_t>(), seg_off, grids,
+            LAUNCH(k_sor_calib, n_seg, kSorThreads, heap_bytes, ctx->sor.spts.as<float4>(), ctx->sor.skeys.as<uint32_t>(), seg_off, grids,
                    pgrids, ctx->bbox.as<uint32_t>(), cell_start, mean_k);
     }
-    CU(ctx->sor_hard.ensure(cap * 8 + 64));
-    uint32_t* n_hard = reinterpret_cast<uint32_t*>(ctx->sor_hard.as<char>() + cap * 8);
+    CU(ctx->sor.hard.ensure(cap * 8 + 64));
+    uint32_t* n_hard = reinterpret_cast<uint32_t*>(ctx->sor.hard.as<char>() + cap * 8);
     ZERO(n_hard, 4);
     CU(cudaFuncSetAttribute(k_sor_knn_hard, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)heap_bytes));
-    LAUNCH(k_sor_knn, dim3(std::max(1u, cdiv(per_seg_cap, kSorThreads)), n_seg), kSorThreads, heap_bytes, ctx->spts.as<float4>(),
-           ctx->sor_skeys.as<uint32_t>(), ctx->sor_svals.as<uint32_t>(), seg_off, grids, cell_start, mean_k,
-           ctx->sor_dist.as<float>(), ctx->sor_hard.as<uint2>(), n_hard);
-    LAUNCH(k_sor_knn_hard, std::max(1u, cdiv(cap, kSorThreads)), kSorThreads, heap_bytes, ctx->spts.as<float4>(),
-           ctx->sor_skeys.as<uint32_t>(), ctx->sor_svals.as<uint32_t>(), seg_off, grids, cell_start, mean_k,
-           ctx->sor_dist.as<float>(), ctx->sor_hard.as<uint2>(), n_hard);
-    LAUNCH(k_sor_stats, n_seg, kThreads, 0, ctx->sor_dist.as<float>(), seg_off, stddev_mul, ctx->sor_thr.as<double>());
-    LAUNCH(k_sor_count, dim3(tiles, n_seg), kThreads, 0, ctx->sor_dist.as<float>(), seg_off, ctx->sor_thr.as<double>(), tiles,
-           ctx->sor_cnt.as<uint32_t>());
-    LAUNCH(k_scan_u32, 1, kScanThreads, 0, ctx->sor_cnt.as<uint32_t>(), ctx->sor_cntoff.as<uint32_t>(), (uint32_t)((size_t)tiles * n_seg),
+    LAUNCH(k_sor_knn, dim3(std::max(1u, cdiv(per_seg_cap, kSorThreads)), n_seg), kSorThreads, heap_bytes, ctx->sor.spts.as<float4>(),
+           ctx->sor.skeys.as<uint32_t>(), ctx->sor.svals.as<uint32_t>(), seg_off, grids, cell_start, mean_k,
+           ctx->sor.dist.as<float>(), ctx->sor.hard.as<uint2>(), n_hard);
+    LAUNCH(k_sor_knn_hard, std::max(1u, cdiv(cap, kSorThreads)), kSorThreads, heap_bytes, ctx->sor.spts.as<float4>(),
+           ctx->sor.skeys.as<uint32_t>(), ctx->sor.svals.as<uint32_t>(), seg_off, grids, cell_start, mean_k,
+           ctx->sor.dist.as<float>(), ctx->sor.hard.as<uint2>(), n_hard);
+    LAUNCH(k_sor_stats, n_seg, kThreads, 0, ctx->sor.dist.as<float>(), seg_off, stddev_mul, ctx->sor.thr.as<double>());
+    LAUNCH(k_sor_count, dim3(tiles, n_seg), kThreads, 0, ctx->sor.dist.as<float>(), seg_off, ctx->sor.thr.as<double>(), tiles,
+           ctx->sor.cnt.as<uint32_t>());
+    LAUNCH(k_scan_u32, 1, kScanThreads, 0, ctx->sor.cnt.as<uint32_t>(), ctx->sor.cntoff.as<uint32_t>(), (uint32_t)((size_t)tiles * n_seg),
            cnt + CNT_PTS);
-    LAUNCH(k_sor_compact, dim3(tiles, n_seg), kThreads, 0, pts, ctx->sor_dist.as<float>(), seg_off, ctx->sor_thr.as<double>(), tiles,
-           ctx->sor_cntoff.as<uint32_t>(), cnt + CNT_PTS, n_seg, ctx->sor_pts.as<float4>(), ctx->sor_off.as<uint32_t>());
+    LAUNCH(k_sor_compact, dim3(tiles, n_seg), kThreads, 0, pts, ctx->sor.dist.as<float>(), seg_off, ctx->sor.thr.as<double>(), tiles,
+           ctx->sor.cntoff.as<uint32_t>(), cnt + CNT_PTS, n_seg, ctx->sor.pts.as<float4>(), ctx->sor.off.as<uint32_t>());
     return O3R_OK;
 }
 

@@ -88,13 +88,13 @@ bool tv_plan(const o3r_ctx* ctx, const AParams& P, const o3r_frame* frames, int 
 
 // false = the engine does not serve this batch; otherwise the first guesses and (once per context) the window radius
 bool tv_begin(o3r_ctx* ctx, const AParams& P, const o3r_frame* frames, int n, TvPlan& pl) {
-    if (ctx->tv_off || !tv_plan(ctx, P, frames, n, pl)) return false;
-    pl.guess.assign(n, (uint8_t)(ctx->tv_guess >= 0 ? ctx->tv_guess : (pl.guess_pass ? 1 : 0)));
-    if (ctx->tv_R < 0) {   // smallest window that covers the nominal depth range (disparities up to 2 min_disparity)
+    if (ctx->tv.off || !tv_plan(ctx, P, frames, n, pl)) return false;
+    pl.guess.assign(n, (uint8_t)(ctx->tv.guess >= 0 ? ctx->tv.guess : (pl.guess_pass ? 1 : 0)));
+    if (ctx->tv.R < 0) {   // smallest window that covers the nominal depth range (disparities up to 2 min_disparity)
         const double w_need = std::fabs(ctx->p.Q[14] * 2.0 * ctx->p.min_disparity + ctx->p.Q[15]);
-        ctx->tv_R = kTvMaxR;
+        ctx->tv.R = kTvMaxR;
         for (int r = 1; r <= kTvMaxR; ++r)
-            if (pl.wlim(r) >= w_need) { ctx->tv_R = r; break; }
+            if (pl.wlim(r) >= w_need) { ctx->tv.R = r; break; }
     }
     return true;
 }
@@ -106,7 +106,7 @@ struct TvMisc {
     uint8_t *guess, *actual;
 };
 TvMisc tv_misc(o3r_ctx* ctx, int n) {
-    uint32_t* m = ctx->tv_misc.as<uint32_t>();
+    uint32_t* m = ctx->tv.misc.as<uint32_t>();
     uint8_t* b = reinterpret_cast<uint8_t*>(m + 16 + n);
     return TvMisc{m, m + 1, m + 2, m + 3, m + 4, m + 16, b, b + n};
 }
@@ -114,18 +114,18 @@ TvMisc tv_misc(o3r_ctx* ctx, int n) {
 // The record lists are sized from what the previous batches needed (the device reports overflow, the host grows and reruns):
 // a tile can emit up to kTvItems records, a typical one a few dozen.
 int tv_prepare(o3r_ctx* ctx, TvPlan& pl, int n, int chunk, size_t cap_batch) {
-    pl.R = std::all_of(pl.guess.begin(), pl.guess.end(), [](uint8_t g) { return g != 0; }) ? 0 : ctx->tv_R;
+    pl.R = std::all_of(pl.guess.begin(), pl.guess.end(), [](uint8_t g) { return g != 0; }) ? 0 : ctx->tv.R;
     const size_t tiles_chunk = pl.tiles_per_frame * (size_t)chunk, tiles_batch = pl.tiles_per_frame * (size_t)n;
-    CU(ctx->tv_tiles.ensure(3 * (tiles_chunk + 4) * 4));
-    CU(ctx->tv_misc.ensure((16 + (size_t)n) * 4 + 2 * (size_t)n + 16));
+    CU(ctx->tv.tiles.ensure(3 * (tiles_chunk + 4) * 4));
+    CU(ctx->tv.misc.ensure((16 + (size_t)n) * 4 + 2 * (size_t)n + 16));
     CU(ctx->bbox.ensure((size_t)n * 6 * 4));
     const size_t hard_chunk = std::min(tiles_chunk * (size_t)kTvItems, pl.tiles_per_frame ? cap_batch / n * chunk : 0);
     const size_t hard_batch = std::min(tiles_batch * (size_t)kTvItems, cap_batch);
-    ctx->tv_scratch_cap = std::min(std::max(ctx->tv_scratch_cap, tiles_chunk * 256), std::max<size_t>(hard_chunk, 1));
-    ctx->tv_part_cap = std::min(std::max(ctx->tv_part_cap, tiles_batch * 256), std::max<size_t>(hard_batch, 1));
-    if (ctx->tv_scratch_cap >= (1ull << 32) || ctx->tv_part_cap >= (1ull << 32)) return ctx->fail(O3R_ERR_INVALID, "batch too large for the tile engine");
-    CU(ctx->tv_scratch.ensure(ctx->tv_scratch_cap * sizeof(o3r_cell)));
-    CU(ctx->partials.ensure(ctx->tv_part_cap * sizeof(o3r_cell)));
+    ctx->tv.scratch_cap = std::min(std::max(ctx->tv.scratch_cap, tiles_chunk * 256), std::max<size_t>(hard_chunk, 1));
+    ctx->tv.part_cap = std::min(std::max(ctx->tv.part_cap, tiles_batch * 256), std::max<size_t>(hard_batch, 1));
+    if (ctx->tv.scratch_cap >= (1ull << 32) || ctx->tv.part_cap >= (1ull << 32)) return ctx->fail(O3R_ERR_INVALID, "batch too large for the tile engine");
+    CU(ctx->tv.scratch.ensure(ctx->tv.scratch_cap * sizeof(o3r_cell)));
+    CU(ctx->last.partials.ensure(ctx->tv.part_cap * sizeof(o3r_cell)));
     const TvMisc M = tv_misc(ctx, n);
     ZERO(M.flags, (16 + (size_t)n) * 4);
     const int rc = upload_small(ctx, M.guess, pl.guess.data(), (size_t)n);
@@ -136,23 +136,23 @@ int tv_prepare(o3r_ctx* ctx, TvPlan& pl, int n, int chunk, size_t cap_batch) {
 template <int DT, int R>
 int tv_launch(o3r_ctx* ctx, const AParams& P, const TvArgs& A, uint32_t n_tiles) {
     const uint32_t bit = 1u << (DT * (kTvMaxR + 1) + R);
-    if (!(ctx->tv_attr & bit)) {   // (the attribute is per function and device)
+    if (!(ctx->tv.attr & bit)) {   // (the attribute is per function and device)
         CU(cudaFuncSetAttribute(k_tv<DT, R>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tv_smem<R>()));
         cudaFuncSetAttribute(k_tv<DT, R>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-        ctx->tv_attr |= bit;
+        ctx->tv.attr |= bit;
     }
     LAUNCH_N("k_tv", (k_tv<DT, R>), n_tiles, kTvThreads, tv_smem<R>(), P, A);
     return O3R_OK;
 }
 
-// one chunk of frames [f0, f0 + nc): the fused kernel + the guard check; partial cells are appended to ctx->partials at the
+// one chunk of frames [f0, f0 + nc): the fused kernel + the guard check; partial cells are appended to ctx->last.partials at the
 // device-side base cnt[CNT_PART] (advanced here)
 template <int DT>
 int tv_run_chunk(o3r_ctx* ctx, const AParams& P, const TvPlan& pl, int f0, int nc, int n) {
     uint32_t* cnt = ctx->counters.as<uint32_t>();
     const TvMisc M = tv_misc(ctx, n);
     const uint32_t n_tiles = (uint32_t)(pl.tiles_per_frame * (size_t)nc);
-    uint32_t* tile_cnt = ctx->tv_tiles.as<uint32_t>();
+    uint32_t* tile_cnt = ctx->tv.tiles.as<uint32_t>();
     uint32_t* tile_at = tile_cnt + (pl.tiles_per_frame * (size_t)nc + 4);
     uint32_t* tile_off = tile_at + (pl.tiles_per_frame * (size_t)nc + 4);
     ZERO(M.ticket, 4);
@@ -161,7 +161,7 @@ int tv_run_chunk(o3r_ctx* ctx, const AParams& P, const TvPlan& pl, int f0, int n
     uint32_t* bbox = ctx->bbox.as<uint32_t>() + (size_t)f0 * 6;
     FILL(bbox, (size_t)(nc) * 24, FILL_BBOX);
     TvArgs A;
-    A.frames = ctx->d_frames.as<FrameDev>() + f0;
+    A.frames = ctx->in.frames.as<FrameDev>() + f0;
     A.frame_pass = M.guess + f0;
     A.ntx = pl.ntx; A.nty = pl.nty; A.n_frames = nc;
     A.inv_f = ctx->inv_f; A.icx = ctx->inv_c; A.icz = ctx->inv_cz;
@@ -172,8 +172,8 @@ int tv_run_chunk(o3r_ctx* ctx, const AParams& P, const TvPlan& pl, int f0, int n
             if (std::fabs(ctx->p.Q[14] * d + ctx->p.Q[15]) < A.wlim) dl = d; else if (dl >= 0) break;
         A.dlim_i = dl;
     }
-    A.scratch = ctx->tv_scratch.as<o3r_cell>();
-    A.scratch_cap = (uint32_t)ctx->tv_scratch_cap;
+    A.scratch = ctx->tv.scratch.as<o3r_cell>();
+    A.scratch_cap = (uint32_t)ctx->tv.scratch_cap;
     A.cursor = M.cursor;
     A.tile_cnt = tile_cnt;
     A.tile_at = tile_at;
@@ -182,7 +182,7 @@ int tv_run_chunk(o3r_ctx* ctx, const AParams& P, const TvPlan& pl, int f0, int n
     A.bbox = bbox;
     A.cellbb = reinterpret_cast<int*>(cnt + CNT_CELLBB);
     A.flags = M.flags;
-    A.dbg_vox = ctx->keep_frame_voxels ? ctx->vox.as<float4>() : nullptr;
+    A.dbg_vox = ctx->keep_frame_voxels ? ctx->last.vox.as<float4>() : nullptr;
     A.dbg_cnt = M.dbg_cnt;
     int rc;
     switch (pl.R) {
@@ -195,8 +195,8 @@ int tv_run_chunk(o3r_ctx* ctx, const AParams& P, const TvPlan& pl, int f0, int n
     if (rc) return rc;
     // tile order: offsets = scan of the per-tile counts, then one warp per tile copies its records behind the batch's list
     LAUNCH(k_scan_u32, 1, kScanThreads, 0, tile_cnt, tile_off, n_tiles, cnt + CNT_PARTCHUNK);
-    LAUNCH(k_tv_compact, cdiv(n_tiles, kWarps), kThreads, 0, ctx->tv_scratch.as<o3r_cell>(), tile_cnt, tile_at, tile_off, n_tiles,
-           ctx->partials.as<o3r_cell>(), cnt + CNT_PART, cnt + CNT_PARTCHUNK, (uint32_t)ctx->tv_part_cap, M.cursor, M.max_cursor,
+    LAUNCH(k_tv_compact, cdiv(n_tiles, kWarps), kThreads, 0, ctx->tv.scratch.as<o3r_cell>(), tile_cnt, tile_at, tile_off, n_tiles,
+           ctx->last.partials.as<o3r_cell>(), cnt + CNT_PART, cnt + CNT_PARTCHUNK, (uint32_t)ctx->tv.part_cap, M.cursor, M.max_cursor,
            M.flags, nc, bbox, ctx->inv_f, M.guess + f0, M.actual + f0);
     LAUNCH(k_add_u32, 1, 32, 0, cnt + CNT_PART, cnt + CNT_PARTCHUNK);
     return O3R_OK;
@@ -206,38 +206,38 @@ int tv_run_chunk(o3r_ctx* ctx, const AParams& P, const TvPlan& pl, int f0, int n
 // (h_offs[n+2]) and the guard's actual verdicts (n bytes from h_offs[n+3])
 int tv_read_back(o3r_ctx* ctx, int n) {
     const TvMisc M = tv_misc(ctx, n);
-    CU(cudaMemcpyAsync(ctx->h_offs + 1, M.fvox, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->st));
-    CU(cudaMemcpyAsync(ctx->h_offs + n + 1, M.flags, 4, cudaMemcpyDeviceToHost, ctx->st));
-    CU(cudaMemcpyAsync(ctx->h_offs + n + 2, M.max_cursor, 4, cudaMemcpyDeviceToHost, ctx->st));
-    CU(cudaMemcpyAsync(ctx->h_offs + n + 3, M.actual, (size_t)n, cudaMemcpyDeviceToHost, ctx->st));
+    CU(cudaMemcpyAsync(ctx->last.h_offs + 1, M.fvox, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->st));
+    CU(cudaMemcpyAsync(ctx->last.h_offs + n + 1, M.flags, 4, cudaMemcpyDeviceToHost, ctx->st));
+    CU(cudaMemcpyAsync(ctx->last.h_offs + n + 2, M.max_cursor, 4, cudaMemcpyDeviceToHost, ctx->st));
+    CU(cudaMemcpyAsync(ctx->last.h_offs + n + 3, M.actual, (size_t)n, cudaMemcpyDeviceToHost, ctx->st));
     return O3R_OK;
 }
 
 // on the landed read-back (and the partial count in h_counters[CNT_PART]).  A raised flag reruns the batch with what the device
 // found out; when no window is wide enough, this batch and the context's later ones go to the next engine.
 Verdict tv_verdict(o3r_ctx* ctx, TvPlan& pl, int n) {
-    const uint32_t* h = ctx->h_offs;
+    const uint32_t* h = ctx->last.h_offs;
     const uint32_t fl = h[n + 1];
     const uint8_t* actual = reinterpret_cast<const uint8_t*>(h + n + 3);
     if (fl) {
         if (trace_on()) fprintf(stderr, "[o3r trace] tile engine flags %u (R %d)\n", fl, pl.R);
         if (fl & TV_FLAG_SPACE) {   // a record list was too short: what the batch needs is known now (+ 25 %)
-            ctx->tv_scratch_cap = std::max(ctx->tv_scratch_cap, (size_t)h[n + 2] + h[n + 2] / 4 + 1024);
-            ctx->tv_part_cap = std::max(ctx->tv_part_cap, (size_t)ctx->h_counters[CNT_PART] + ctx->h_counters[CNT_PART] / 4 + 1024);
+            ctx->tv.scratch_cap = std::max(ctx->tv.scratch_cap, (size_t)h[n + 2] + h[n + 2] / 4 + 1024);
+            ctx->tv.part_cap = std::max(ctx->tv.part_cap, (size_t)ctx->h_counters[CNT_PART] + ctx->h_counters[CNT_PART] / 4 + 1024);
         }
         if (fl & TV_FLAG_PASS) pl.guess.assign(actual, actual + n);   // the bboxes are exact: so is this
         else if (fl & TV_FLAG_RANGE) {   // a disparity beyond the window's reach: widen it
-            if (pl.R >= kTvMaxR) { ctx->tv_off = true; return Verdict::NEXT_ENGINE; }
-            ctx->tv_R = pl.R + 1;
+            if (pl.R >= kTvMaxR) { ctx->tv.off = true; return Verdict::NEXT_ENGINE; }
+            ctx->tv.R = pl.R + 1;
         }
         return Verdict::RERUN;
     }
-    ctx->tv_guess = actual[n - 1];
+    ctx->tv.guess = actual[n - 1];
     // A combined grid fine against the sideways scatter of the points leaves one record per 1-3 points: a 40-byte record per
     // 16-byte point is then a loss, and the sort engine's direct merge of the points serves the context from here on.
     size_t total_vox = 0;
     for (int i = 0; i < n; ++i) total_vox += h[i + 1];
-    if ((size_t)ctx->h_counters[CNT_PART] * 4 > total_vox && total_vox > 0) ctx->tv_off = ctx->bucket_off = true;
+    if ((size_t)ctx->h_counters[CNT_PART] * 4 > total_vox && total_vox > 0) ctx->tv.off = ctx->bk.off = true;
     return Verdict::ACCEPT;
 }
 

@@ -60,11 +60,11 @@ int o3r_create(const o3r_params* params, o3r_ctx** out_ctx) {
     if ((e = cudaStreamCreateWithFlags(&ctx->st_copy, cudaStreamNonBlocking)) != cudaSuccess) return bail(e, "stream");
     if ((e = cudaStreamCreateWithFlags(&ctx->st_copy2, cudaStreamNonBlocking)) != cudaSuccess) return bail(e, "stream");
     if ((e = cudaEventCreateWithFlags(&ctx->ev_copy2, cudaEventDisableTiming)) != cudaSuccess) return bail(e, "event");
-    if (const char* cf = getenv("O3R_CHUNK_FRAMES")) ctx->chunk_frames = std::max(1, atoi(cf));
-    if (const char* cf = getenv("O3R_CHUNK_FRAMES_DEV")) ctx->chunk_frames_dev = std::max(1, atoi(cf));
+    if (const char* cf = getenv("O3R_CHUNK_FRAMES")) ctx->in.chunk_frames = std::max(1, atoi(cf));
+    if (const char* cf = getenv("O3R_CHUNK_FRAMES_DEV")) ctx->in.chunk_frames_dev = std::max(1, atoi(cf));
     if ((e = cudaMallocHost((void**)&ctx->h_counters, CNT_N * 4)) != cudaSuccess) return bail(e, "pinned");
-    if ((e = cudaMallocHost((void**)&ctx->h_nres, 4)) != cudaSuccess) return bail(e, "pinned");
-    if ((e = cudaEventCreateWithFlags(&ctx->ev_nres, cudaEventDisableTiming)) != cudaSuccess) return bail(e, "event");
+    if ((e = cudaMallocHost((void**)&ctx->res.h_n, 4)) != cudaSuccess) return bail(e, "pinned");
+    if ((e = cudaEventCreateWithFlags(&ctx->res.ev_n, cudaEventDisableTiming)) != cudaSuccess) return bail(e, "event");
     if ((e = ctx->counters.ensure(CNT_N * 4)) != cudaSuccess) return bail(e, "counters");
     if ((e = cudaMemsetAsync(ctx->counters.p, 0, CNT_N * 4, ctx->st)) != cudaSuccess) return bail(e, "memset");
     // 1/(q14*d+q15) and (float)(q11 * that) for u8 disparities
@@ -130,8 +130,8 @@ void o3r_destroy(o3r_ctx* ctx) {
 }
 
 uint64_t o3r_launch_count(const o3r_ctx* ctx) { return ctx ? ctx->launches : 0; }
-size_t o3r_last_batch_partials(const o3r_ctx* ctx) { return (ctx && ctx->last_has_partials) ? ctx->last_partials : 0; }
-int o3r_last_batch_engine(const o3r_ctx* ctx) { return ctx ? (int)ctx->last_engine : 0; }
+size_t o3r_last_batch_partials(const o3r_ctx* ctx) { return (ctx && ctx->last.has_partials) ? ctx->last.n_part : 0; }
+int o3r_last_batch_engine(const o3r_ctx* ctx) { return ctx ? (int)ctx->last.engine : 0; }
 void* o3r_stream(o3r_ctx* ctx) { return ctx ? (void*)ctx->st : nullptr; }
 
 int o3r_sync(o3r_ctx* ctx) {
@@ -144,9 +144,9 @@ int o3r_sync(o3r_ctx* ctx) {
 int o3r_profile(o3r_ctx* ctx, int enable) {
     return api(ctx, [&] {
         CU(cudaStreamSynchronize(ctx->st));
-        for (auto& r : ctx->prof) { ctx->ev_pool.push_back(r.a); ctx->ev_pool.push_back(r.b); }
-        ctx->prof.clear();
-        ctx->profiling = enable != 0;
+        for (auto& r : ctx->prof.recs) { ctx->prof.pool.push_back(r.a); ctx->prof.pool.push_back(r.b); }
+        ctx->prof.recs.clear();
+        ctx->prof.on = enable != 0;
         return O3R_OK;
     });
 }
@@ -157,7 +157,7 @@ int o3r_profile_read(o3r_ctx* ctx, char* buf, size_t cap) {
         CU(cudaStreamSynchronize(ctx->st));
         struct Agg { std::string name; uint64_t n; double ms; };
         std::vector<Agg> agg;
-        for (auto& r : ctx->prof) {
+        for (auto& r : ctx->prof.recs) {
             float ms = 0.f;
             cudaEventElapsedTime(&ms, r.a, r.b);
             std::string nm = r.name;
@@ -213,20 +213,20 @@ int o3r_frames_prefetch(o3r_ctx* ctx, const o3r_frame* frames, int n, int disp_t
                 return ctx->fail(O3R_ERR_INVALID, "frame without disparity/colour");
         int rc = flush_deferred_prefetch(ctx);   // at most one request waits; an older one goes out now
         if (rc) return rc;
-        ctx->deferred.frames.assign(frames, frames + n);
-        ctx->deferred.disp_type = disp_type;
-        ctx->deferred.pending = true;
+        ctx->in.deferred.frames.assign(frames, frames + n);
+        ctx->in.deferred.disp_type = disp_type;
+        ctx->in.deferred.pending = true;
         return O3R_OK;
     });
 }
 
 int o3r_frames_prefetch_cancel(o3r_ctx* ctx) {
     return api(ctx, [&] {
-        ctx->deferred.pending = false;           // recorded but not issued: nothing will ever read those buffers
-        ctx->deferred.frames.clear();
+        ctx->in.deferred.pending = false;           // recorded but not issued: nothing will ever read those buffers
+        ctx->in.deferred.frames.clear();
         CU(cudaStreamSynchronize(ctx->st_copy2));   // copies already in flight finish reading the host buffers here
         CU(cudaStreamSynchronize(ctx->st_copy));
-        for (auto& pf : ctx->prefetch) pf.valid = false;
+        for (auto& pf : ctx->in.prefetch) pf.valid = false;
         return O3R_OK;
     });
 }
@@ -239,8 +239,8 @@ int o3r_frame_cloud(o3r_ctx* ctx, const o3r_frame* frame, int disp_type, o3r_poi
         opt.merge = false;
         int rc = frames_cloud_impl(ctx, frame, 1, disp_type, nullptr, opt, true);
         if (rc) return rc;
-        const float4* src = ctx->last_is_vox ? ctx->vox.as<float4>() : ctx->pts.as<float4>();
-        return copy_out(ctx, src, ctx->last_total, out, cap, n_out);
+        const float4* src = ctx->last.is_vox ? ctx->last.vox.as<float4>() : ctx->last.pts.as<float4>();
+        return copy_out(ctx, src, ctx->last.total, out, cap, n_out);
     });
 }
 
@@ -264,10 +264,10 @@ int o3r_frame_mask(o3r_ctx* ctx, const o3r_frame* frame, int disp_type, uint8_t*
 
 int o3r_last_batch_points(o3r_ctx* ctx, o3r_point* out, size_t cap, size_t* n_out) {
     return api(ctx, [&] {
-        if (ctx->last_engine != Engine::SORT && !ctx->keep_frame_voxels)
+        if (ctx->last.engine != Engine::SORT && !ctx->keep_frame_voxels)
             return ctx->fail(O3R_ERR_UNSUPPORTED, "O3R_MERGE_ACCUMULATE_FUSED does not materialise the per-frame clouds (see o3r_set_keep_frame_voxels)");
-        const float4* src = ctx->last_is_vox ? ctx->vox.as<float4>() : ctx->pts.as<float4>();
-        return copy_out(ctx, src, ctx->last_total, out, cap, n_out);
+        const float4* src = ctx->last.is_vox ? ctx->last.vox.as<float4>() : ctx->last.pts.as<float4>();
+        return copy_out(ctx, src, ctx->last.total, out, cap, n_out);
     });
 }
 
@@ -277,12 +277,12 @@ int o3r_cloud_transform(o3r_ctx* ctx, const float T[16]) {
         if (!ctx->retain())
             return ctx->fail(O3R_ERR_UNSUPPORTED,
                              "o3r_cloud_transform needs O3R_MERGE_RETAIN: accumulated cells cannot be re-binned");
-        ctx->rt_valid = false;   // (on every rank of a sharded cloud, even one without points: the ranks stay in step)
-        if (ctx->n_cloud == 0) return O3R_OK;
+        ctx->rt.valid = false;   // (on every rank of a sharded cloud, even one without points: the ranks stay in step)
+        if (ctx->res.n_cloud == 0) return O3R_OK;
         CU(ctx->tmat.ensure(64));
         { int rcu = upload_small(ctx, ctx->tmat.p, T, 48); if (rcu) return rcu; }
-        const uint32_t g = std::min<uint32_t>(cdiv(ctx->n_cloud, kThreads), 148 * 16);
-        LAUNCH(k_transform_pts, g, kThreads, 0, ctx->cloud.as<float4>(), ctx->n_cloud, ctx->tmat.as<float>());
+        const uint32_t g = std::min<uint32_t>(cdiv(ctx->res.n_cloud, kThreads), 148 * 16);
+        LAUNCH(k_transform_pts, g, kThreads, 0, ctx->res.cloud.as<float4>(), ctx->res.n_cloud, ctx->tmat.as<float>());
         return O3R_OK;
     });
 }
@@ -294,17 +294,15 @@ int o3r_cloud_append(o3r_ctx* ctx, const o3r_point* pts, size_t n) {
             return ctx->fail(O3R_ERR_UNSUPPORTED, "o3r_cloud_append on a sharded retained cloud: appended points have no place in the frame order");
         if (n == 0) return O3R_OK;
         if (ctx->retain()) {
-            CU(ctx->cloud.ensure((ctx->n_cloud + n) * 16, ctx->st, ctx->n_cloud * 16));
-            CU(cudaMemcpyAsync(ctx->cloud.as<float4>() + ctx->n_cloud, pts, n * 16, cudaMemcpyHostToDevice, ctx->st));
+            CU(ctx->res.cloud.ensure((ctx->res.n_cloud + n) * 16, ctx->st, ctx->res.n_cloud * 16));
+            CU(cudaMemcpyAsync(ctx->res.cloud.as<float4>() + ctx->res.n_cloud, pts, n * 16, cudaMemcpyHostToDevice, ctx->st));
             CU(cudaStreamSynchronize(ctx->st));   // the caller may reuse or free `pts` as soon as this returns
-            ctx->n_cloud += n;
+            ctx->res.n_cloud += n;
             return O3R_OK;
         }
-        CU(ctx->vox.ensure(n * 16));
-        CU(cudaMemcpyAsync(ctx->vox.p, pts, n * 16, cudaMemcpyHostToDevice, ctx->st));
-        ctx->last_n = 0; ctx->last_total = 0; ctx->last_has_cellbb = false;   // the batch buffer was overwritten
-        ctx->last_has_partials = false; ctx->last_partials = 0; ctx->last_engine = Engine::SORT;
-        const int rc = acc_merge_points(ctx, ctx->vox.as<float4>(), n, nullptr);
+        CU(ctx->in_pts.ensure(n * 16));
+        CU(cudaMemcpyAsync(ctx->in_pts.p, pts, n * 16, cudaMemcpyHostToDevice, ctx->st));
+        const int rc = acc_merge_points(ctx, ctx->in_pts.as<float4>(), n, nullptr);
         if (rc) return rc;
         CU(cudaStreamSynchronize(ctx->st));   // (a page-locked `pts` is read asynchronously) the caller may reuse or free it now
         return O3R_OK;
@@ -314,10 +312,10 @@ int o3r_cloud_append(o3r_ctx* ctx, const o3r_point* pts, size_t n) {
 int o3r_cloud_size(o3r_ctx* ctx, size_t* n) {
     if (!n) return O3R_ERR_INVALID;
     return api(ctx, [&] {
-        if (ctx->retain()) { *n = ctx->n_cloud; return O3R_OK; }
+        if (ctx->retain()) { *n = ctx->res.n_cloud; return O3R_OK; }
         int rc = refresh_nres(ctx, true);
         if (rc) return rc;
-        *n = ctx->n_res_ub;
+        *n = ctx->res.n_ub;
         return O3R_OK;
     });
 }
@@ -325,10 +323,9 @@ int o3r_cloud_size(o3r_ctx* ctx, size_t* n) {
 int o3r_cloud_clear(o3r_ctx* ctx) {
     return api(ctx, [&] {
         CU(cudaStreamSynchronize(ctx->st));
-        ctx->n_cloud = 0; ctx->n_res_ub = 0; ctx->n_res_exact = true;
-        ctx->rt_reset();
-        ZERO(ctx->counters.as<uint32_t>() + CNT_NRES, 4);
-        if (ctx->chg_on) chg_reset(ctx, false);
+        ctx->rt.reset();
+        { int rc = res_clear(ctx); if (rc) return rc; }
+        if (ctx->chg) chg_reset(ctx, false);
         return O3R_OK;
     });
 }
@@ -365,15 +362,15 @@ static int cloud_downsample_dev(o3r_ctx* ctx, const float4** res, size_t* m, boo
     *res = nullptr; *m = 0;
     if (exact_pending) *exact_pending = false;
     if (ctx->p.dont_downsample) {  // pose.cpp:533-536: cloud_small = cloud_big
-        *res = ctx->cloud.as<float4>(); *m = ctx->n_cloud;
+        *res = ctx->res.cloud.as<float4>(); *m = ctx->res.n_cloud;
         return O3R_OK;
     }
     uint32_t* cnt = ctx->counters.as<uint32_t>();
     if (ctx->retain() && ctx->comm) return retain_downsample_sharded(ctx, res, m);   // collective (host_retain.cuh)
     if (ctx->retain()) {  // one-shot pcl::VoxelGrid over cloud_big, exactly pose_functions.cpp:1654-1709
-        if (ctx->n_cloud == 0) return O3R_OK;
-        CU(ctx->ckey.ensure(ctx->n_cloud * 16));   // result points (<= n_cloud)
-        int rc = voxel_grid_dev(ctx, ctx->cloud.as<float4>(), ctx->n_cloud, ctx->inv_c, ctx->inv_c, ctx->inv_cz,
+        if (ctx->res.n_cloud == 0) return O3R_OK;
+        CU(ctx->ckey.ensure(ctx->res.n_cloud * 16));   // result points (<= n_cloud)
+        int rc = voxel_grid_dev(ctx, ctx->res.cloud.as<float4>(), ctx->res.n_cloud, ctx->inv_c, ctx->inv_c, ctx->inv_cz,
                                 ctx->p.min_points_per_voxel, 1, ctx->ckey.as<float4>(), nullptr, nullptr, m, nullptr);
         if (rc) return rc;
         *res = ctx->ckey.as<float4>();
@@ -381,18 +378,17 @@ static int cloud_downsample_dev(o3r_ctx* ctx, const float4** res, size_t* m, boo
     }
     // device-driven: launches are sized by the host's upper bound of the resident count, the kernels read the exact one
     { int rc0 = refresh_nres(ctx, false); if (rc0) return rc0; }
-    const size_t n_ub = ctx->n_res_ub;
+    const size_t n_ub = ctx->res.n_ub;
     if (n_ub == 0) return O3R_OK;
-    const int cur = ctx->res_cur;
+    const ResCells R = res_cells(ctx);
     const uint32_t tiles = cdiv(n_ub, kTileV);
     CU(ctx->new_cnt.ensure((size_t)tiles * 4));
     CU(ctx->new_off.ensure((size_t)tiles * 4));
     CU(ctx->cacc.ensure(n_ub * 16));
-    LAUNCH(k_acc_emit_cnt, tiles, kThreads, 0, cnt + CNT_NRES, ctx->res_acc[cur].as<float4>(), ctx->p.min_points_per_voxel,
+    LAUNCH(k_acc_emit_cnt, tiles, kThreads, 0, cnt + CNT_NRES, R.acc, ctx->p.min_points_per_voxel,
            ctx->new_cnt.as<uint32_t>());
     LAUNCH(k_scan_u32, 1, kScanThreads, 0, ctx->new_cnt.as<uint32_t>(), ctx->new_off.as<uint32_t>(), tiles, cnt + CNT_EMIT);
-    LAUNCH(k_acc_emit, tiles, kThreads, 0, cnt + CNT_NRES, ctx->res_acc[cur].as<float4>(), ctx->res_rgb[cur].as<uint4>(),
-           ctx->p.min_points_per_voxel, ctx->new_off.as<uint32_t>(), ctx->cacc.as<float4>());
+    LAUNCH(k_acc_emit, tiles, kThreads, 0, cnt + CNT_NRES, R.acc, R.rgb, ctx->p.min_points_per_voxel, ctx->new_off.as<uint32_t>(), ctx->cacc.as<float4>());
     *res = ctx->cacc.as<float4>();
     *m = n_ub;   // upper bound; the exact count is cnt[CNT_EMIT] once the stream has run (callers read it back)
     if (exact_pending) *exact_pending = true;
@@ -401,16 +397,11 @@ static int cloud_downsample_dev(o3r_ctx* ctx, const float4** res, size_t* m, boo
 
 // one read-back of the exact output count (and of the resident count, which tightens the host's bound)
 static int downsample_finish(o3r_ctx* ctx, size_t* m) {
-    uint32_t* cnt = ctx->counters.as<uint32_t>();
-    CU(cudaMemcpyAsync(ctx->h_counters, cnt, CNT_N * 4, cudaMemcpyDeviceToHost, ctx->st));
-    CU(cudaStreamSynchronize(ctx->st));
+    { int rc = res_read_back(ctx); if (rc) return rc; }
     *m = ctx->h_counters[CNT_EMIT];
-    ctx->n_res_ub = ctx->h_counters[CNT_NRES];
-    ctx->n_res_exact = true;
-    if (ctx->x_pending_check) {   // the exchanges since the last read-back: did a slot overflow?
-        ctx->x_pending_check = false;
-        if (ctx->h_counters[CNT_XFLAG])
-            return ctx->fail(O3R_ERR_CAPACITY, "exchange slot overflow: cells were dropped; create the communicator with more slot_cells");
+    if (ctx->x.pending_check) {   // the exchanges since the last read-back: did a slot overflow?
+        ctx->x.pending_check = false;
+        if (ctx->h_counters[CNT_XFLAG]) return x_overflow(ctx);
     }
     return O3R_OK;
 }
@@ -455,12 +446,10 @@ int o3r_cloud_track_changes(o3r_ctx* ctx, int enable) {
         { int rc = chg_check_mode(ctx); if (rc) return rc; }
         if (!enable) {
             CU(cudaStreamSynchronize(ctx->st));   // (queued unions may still read or write the buffers)
-            ctx->chg_on = ctx->chg_all = ctx->chg_valid = false;
-            ctx->chg_ub = ctx->chg_m = 0;
-            ctx->chg_release();
+            ctx->chg.reset();
             return O3R_OK;
         }
-        ctx->chg_on = true;
+        if (!ctx->chg) ctx->chg.reset(new ChangeTracking());
         chg_reset(ctx, true);   // the next read returns the full state
         return O3R_OK;
     });
@@ -472,14 +461,14 @@ int o3r_cloud_changes(o3r_ctx* ctx, o3r_point* out, uint64_t* keys, uint32_t* co
         *n_out = 0;
         int rc = chg_compute(ctx);
         if (rc) return rc;
-        const size_t m = ctx->chg_m;
+        const size_t m = ctx->chg->m;
         *n_out = m;
         if (!out && cap == 0) return O3R_OK;   // size query: nothing consumed
         if (cap < m) return ctx->fail(O3R_ERR_CAPACITY, "output buffer too small");
         if (m) {
-            if (out) CU(cudaMemcpyAsync(out, ctx->chg_out.p, m * 16, cudaMemcpyDeviceToHost, ctx->st));
-            if (keys) CU(cudaMemcpyAsync(keys, ctx->chg_okeys.p, m * 8, cudaMemcpyDeviceToHost, ctx->st));
-            if (counts) CU(cudaMemcpyAsync(counts, ctx->chg_ocnt.p, m * 4, cudaMemcpyDeviceToHost, ctx->st));
+            if (out) CU(cudaMemcpyAsync(out, ctx->chg->out.p, m * 16, cudaMemcpyDeviceToHost, ctx->st));
+            if (keys) CU(cudaMemcpyAsync(keys, ctx->chg->okeys.p, m * 8, cudaMemcpyDeviceToHost, ctx->st));
+            if (counts) CU(cudaMemcpyAsync(counts, ctx->chg->ocnt.p, m * 4, cudaMemcpyDeviceToHost, ctx->st));
             CU(cudaStreamSynchronize(ctx->st));
         }
         chg_reset(ctx, false);   // delivered: nothing is pending any more
@@ -494,10 +483,10 @@ int o3r_cloud_changes_dev(o3r_ctx* ctx, const o3r_point** dev_out, const uint64_
         *n_out = 0;
         int rc = chg_compute(ctx);
         if (rc) return rc;
-        *n_out = ctx->chg_m;
-        if (dev_out) *dev_out = ctx->chg_out.as<const o3r_point>();
-        if (dev_keys) *dev_keys = ctx->chg_okeys.as<const uint64_t>();
-        if (dev_counts) *dev_counts = ctx->chg_ocnt.as<const uint32_t>();
+        *n_out = ctx->chg->m;
+        if (dev_out) *dev_out = ctx->chg->out.as<const o3r_point>();
+        if (dev_keys) *dev_keys = ctx->chg->okeys.as<const uint64_t>();
+        if (dev_counts) *dev_counts = ctx->chg->ocnt.as<const uint32_t>();
         chg_reset(ctx, false);   // (the records stay in the context's buffers until the next call)
         return O3R_OK;
     });
@@ -532,21 +521,20 @@ int o3r_voxel_grid(o3r_ctx* ctx, const o3r_point* pts, size_t n, float lx, float
         if (passthrough) *passthrough = 0;
         if (n == 0) return O3R_OK;
         if (!(lx > 0) || !(ly > 0) || !(lz > 0)) return ctx->fail(O3R_ERR_INVALID, "leaf size must be positive");
-        CU(ctx->pts.ensure(n * 16));
-        CU(ctx->vox.ensure(n * 16));
+        CU(ctx->in_pts.ensure(n * 16));
+        CU(ctx->out_pts.ensure(n * 16));
         CU(ctx->ckey.ensure(n * 8));
         CU(ctx->new_keys.ensure(n * 4));
-        ctx->last_n = 0; ctx->last_total = 0;
-        CU(cudaMemcpyAsync(ctx->pts.p, pts, n * 16, cudaMemcpyHostToDevice, ctx->st));
+        CU(cudaMemcpyAsync(ctx->in_pts.p, pts, n * 16, cudaMemcpyHostToDevice, ctx->st));
         size_t m = 0;
-        int rc = voxel_grid_dev(ctx, ctx->pts.as<float4>(), n, 1.0f / lx, 1.0f / ly, 1.0f / lz, min_points, 0,
-                                ctx->vox.as<float4>(), ctx->ckey.as<uint64_t>(), ctx->new_keys.as<uint32_t>(), &m, passthrough);
+        int rc = voxel_grid_dev(ctx, ctx->in_pts.as<float4>(), n, 1.0f / lx, 1.0f / ly, 1.0f / lz, min_points, 0,
+                                ctx->out_pts.as<float4>(), ctx->ckey.as<uint64_t>(), ctx->new_keys.as<uint32_t>(), &m, passthrough);
         if (rc) return rc;
         *n_out = m;
         if (!out && cap == 0) return O3R_OK;
         if (cap < m) return ctx->fail(O3R_ERR_CAPACITY, "output buffer too small");
         if (m) {
-            CU(cudaMemcpyAsync(out, ctx->vox.p, m * 16, cudaMemcpyDeviceToHost, ctx->st));
+            CU(cudaMemcpyAsync(out, ctx->out_pts.p, m * 16, cudaMemcpyDeviceToHost, ctx->st));
             if (keys) CU(cudaMemcpyAsync(keys, ctx->ckey.p, m * 8, cudaMemcpyDeviceToHost, ctx->st));
             if (counts) CU(cudaMemcpyAsync(counts, ctx->new_keys.p, m * 4, cudaMemcpyDeviceToHost, ctx->st));
             CU(cudaStreamSynchronize(ctx->st));
@@ -565,12 +553,12 @@ int o3r_blur_u8(o3r_ctx* ctx, const uint8_t* src, size_t src_step, int rows, int
         if (mode != O3R_BLUR_MEDIAN && mode != O3R_BLUR_BOX && mode != O3R_BLUR_BILATERAL)
             return ctx->fail(O3R_ERR_INVALID, "unknown blur mode");
         const size_t step = ((size_t)cols + 15) & ~(size_t)15, plane = step * rows;
-        CU(ctx->d_disp.ensure(plane));
-        CU(ctx->d_blur.ensure(plane));
-        CU(ctx->d_blurjobs.ensure(sizeof(BlurJob)));
-        CU(cudaMemcpy2DAsync(ctx->d_disp.p, step, src, src_step, cols, rows, cudaMemcpyHostToDevice, ctx->st));
-        BlurJob job{ctx->d_disp.as<uint8_t>(), step, ctx->d_blur.as<uint8_t>(), step};
-        CU(cudaMemcpyAsync(ctx->d_blurjobs.p, &job, sizeof(job), cudaMemcpyHostToDevice, ctx->st));
+        CU(ctx->blur.disp.ensure(plane));
+        CU(ctx->blur.out.ensure(plane));
+        CU(ctx->blur.jobs.ensure(sizeof(BlurJob)));
+        CU(cudaMemcpy2DAsync(ctx->blur.disp.p, step, src, src_step, cols, rows, cudaMemcpyHostToDevice, ctx->st));
+        BlurJob job{ctx->blur.disp.as<uint8_t>(), step, ctx->blur.out.as<uint8_t>(), step};
+        CU(cudaMemcpyAsync(ctx->blur.jobs.p, &job, sizeof(job), cudaMemcpyHostToDevice, ctx->st));
         const dim3 g(cdiv(cols, kBlurStrip), cdiv(rows, blur_rows(mode)), 1);
         const size_t sm = blur_smem(kernel, mode);
         if (mode == O3R_BLUR_BILATERAL) {
@@ -578,12 +566,12 @@ int o3r_blur_u8(o3r_ctx* ctx, const uint8_t* src, size_t src_step, int rows, int
             int rcl = bilateral_lut(ctx, kernel, &L);
             if (rcl) return rcl;
             const dim3 gb(cdiv(cols, kBilW), cdiv(rows, kBilTY), 1);
-            LAUNCH(k_bilateral, gb, dim3(kBilTX, kBilTY), bilateral_smem(L.radius, L.maxk), ctx->d_blurjobs.as<BlurJob>(), L, rows, cols, 0, 0, cols, rows);
+            LAUNCH(k_bilateral, gb, dim3(kBilTX, kBilTY), bilateral_smem(L.radius, L.maxk), ctx->blur.jobs.as<BlurJob>(), L, rows, cols, 0, 0, cols, rows);
         } else if (mode == O3R_BLUR_MEDIAN)
-            LAUNCH_N("k_blur_median", (k_blur<O3R_BLUR_MEDIAN>), g, kBlurRows, sm, ctx->d_blurjobs.as<BlurJob>(), rows, cols, kernel, 0, 0, cols, rows);
+            LAUNCH_N("k_blur_median", (k_blur<O3R_BLUR_MEDIAN>), g, kBlurRows, sm, ctx->blur.jobs.as<BlurJob>(), rows, cols, kernel, 0, 0, cols, rows);
         else
-            LAUNCH_N("k_blur_box", (k_blur<O3R_BLUR_BOX>), g, kBlurRows, sm, ctx->d_blurjobs.as<BlurJob>(), rows, cols, kernel, 0, 0, cols, rows);
-        CU(cudaMemcpy2DAsync(dst, dst_step, ctx->d_blur.p, step, cols, rows, cudaMemcpyDeviceToHost, ctx->st));
+            LAUNCH_N("k_blur_box", (k_blur<O3R_BLUR_BOX>), g, kBlurRows, sm, ctx->blur.jobs.as<BlurJob>(), rows, cols, kernel, 0, 0, cols, rows);
+        CU(cudaMemcpy2DAsync(dst, dst_step, ctx->blur.out.p, step, cols, rows, cudaMemcpyDeviceToHost, ctx->st));
         CU(cudaStreamSynchronize(ctx->st));
         return O3R_OK;
     });
@@ -638,10 +626,8 @@ int o3r_comm_destroy(o3r_ctx* ctx) {
         NcclApi* N = nccl_api();
         if (ctx->comm && ctx->comm_owned) NC(N->CommDestroy((ncclComm_t)ctx->comm));
         ctx->comm = nullptr; ctx->comm_owned = false; ctx->world = 1; ctx->rank = 0;
-        ctx->x_send.release(); ctx->x_recv.release(); ctx->x_list.release();
-        ctx->rt_reset();
-        DevBuf* rt_bufs[] = {&ctx->rt_agree, &ctx->rt_ftab, &ctx->rt_tags, &ctx->rt_send, &ctx->rt_recv, &ctx->rt_pts, &ctx->rt_out};
-        for (DevBuf* b : rt_bufs) b->release();
+        ctx->x = Exchange();
+        ctx->rt = RetainShard();
         return O3R_OK;
     });
 }
@@ -696,13 +682,13 @@ int roi_variance(o3r_ctx* ctx, const uint8_t* d_disp, size_t dstep, const uint8_
     const o3r_params& p = ctx->p;
     const int nrow = p.rows - 2 * p.bounding_box, ncol = p.cols - p.bounding_box - p.cols_start_aft_cutout;
     if (nrow <= 0 || ncol <= 0) return ctx->fail(O3R_ERR_INVALID, "empty ROI");
-    CU(ctx->pp_rows.ensure((size_t)nrow * 8));
+    CU(ctx->pp.rows.ensure((size_t)nrow * 8));
     std::vector<double> rows_h(nrow);
     double mean = 0.0;
     for (int pass = 0; pass < 2; ++pass) {
         LAUNCH(k_row_moment, nrow, kThreads, 0, d_disp, dstep, d_labels, lstep, d_coef, n_planes, p.cols,
-               p.cols_start_aft_cutout, p.bounding_box, p.min_disparity, pass, mean, ctx->pp_rows.as<double>());
-        CU(cudaMemcpyAsync(rows_h.data(), ctx->pp_rows.p, (size_t)nrow * 8, cudaMemcpyDeviceToHost, ctx->st));
+               p.cols_start_aft_cutout, p.bounding_box, p.min_disparity, pass, mean, ctx->pp.rows.as<double>());
+        CU(cudaMemcpyAsync(rows_h.data(), ctx->pp.rows.p, (size_t)nrow * 8, cudaMemcpyDeviceToHost, ctx->st));
         CU(cudaStreamSynchronize(ctx->st));
         double s = 0.0;
         for (int r = 0; r < nrow; ++r) s += rows_h[r];
@@ -727,9 +713,9 @@ int o3r_disp_variance(o3r_ctx* ctx, const uint8_t* disp, size_t disp_step, doubl
     if (!disp || !variance) return O3R_ERR_INVALID;
     return api(ctx, [&] {
         size_t step;
-        int rc = stage_plane_u8(ctx, ctx->pp_disp, disp, disp_step, &step);
+        int rc = stage_plane_u8(ctx, ctx->pp.disp, disp, disp_step, &step);
         if (rc) return rc;
-        return roi_variance(ctx, ctx->pp_disp.as<uint8_t>(), step, nullptr, 0, nullptr, 0, variance);
+        return roi_variance(ctx, ctx->pp.disp.as<uint8_t>(), step, nullptr, 0, nullptr, 0, variance);
     });
 }
 
@@ -739,17 +725,17 @@ int o3r_plane_fit(o3r_ctx* ctx, const uint8_t* labels, size_t labels_step, const
     return api(ctx, [&] {
         const o3r_params& p = ctx->p;
         size_t lstep, dstep;
-        int rc = stage_plane_u8(ctx, ctx->pp_labels, labels, labels_step, &lstep);
+        int rc = stage_plane_u8(ctx, ctx->pp.labels, labels, labels_step, &lstep);
         if (rc) return rc;
-        rc = stage_plane_u8(ctx, ctx->pp_disp, disp, disp_step, &dstep);
+        rc = stage_plane_u8(ctx, ctx->pp.disp, disp, disp_step, &dstep);
         if (rc) return rc;
         const size_t sum_bytes = (size_t)256 * kLabSums * 8;
-        CU(ctx->pp_sums.ensure(sum_bytes));
-        ZERO(ctx->pp_sums.p, sum_bytes);
-        LAUNCH(k_label_sums, cdiv(p.rows, 8), kThreads, 0, ctx->pp_labels.as<uint8_t>(), lstep, ctx->pp_disp.as<uint8_t>(), dstep,
-               p.rows, p.cols, p.cols_start_aft_cutout, p.bounding_box, ctx->pp_sums.as<unsigned long long>());
+        CU(ctx->pp.sums.ensure(sum_bytes));
+        ZERO(ctx->pp.sums.p, sum_bytes);
+        LAUNCH(k_label_sums, cdiv(p.rows, 8), kThreads, 0, ctx->pp.labels.as<uint8_t>(), lstep, ctx->pp.disp.as<uint8_t>(), dstep,
+               p.rows, p.cols, p.cols_start_aft_cutout, p.bounding_box, ctx->pp.sums.as<unsigned long long>());
         std::vector<unsigned long long> S((size_t)256 * kLabSums);
-        CU(cudaMemcpyAsync(S.data(), ctx->pp_sums.p, sum_bytes, cudaMemcpyDeviceToHost, ctx->st));
+        CU(cudaMemcpyAsync(S.data(), ctx->pp.sums.p, sum_bytes, cudaMemcpyDeviceToHost, ctx->st));
         CU(cudaStreamSynchronize(ctx->st));
         int np = 0;
         for (int cluster = 1; cluster < 256; ++cluster) {   // :907 (labels are 8-bit); stops at the first absent label (:923)
@@ -780,9 +766,9 @@ int o3r_plane_fit(o3r_ctx* ctx, const uint8_t* labels, size_t labels_step, const
         }
         *n_planes = np;
         if (variance) {   // getVariance(new_disp_img, true), :973; the caller applies the > 3 gate (:975-982)
-            CU(ctx->pp_coef.ensure(std::max(np, 1) * 24));
-            if (np) { int rcu = upload_small(ctx, ctx->pp_coef.p, coef, (size_t)np * 24); if (rcu) return rcu; }
-            return roi_variance(ctx, nullptr, 0, ctx->pp_labels.as<uint8_t>(), lstep, ctx->pp_coef.as<double>(), np, variance);
+            CU(ctx->pp.coef.ensure(std::max(np, 1) * 24));
+            if (np) { int rcu = upload_small(ctx, ctx->pp.coef.p, coef, (size_t)np * 24); if (rcu) return rcu; }
+            return roi_variance(ctx, nullptr, 0, ctx->pp.labels.as<uint8_t>(), lstep, ctx->pp.coef.as<double>(), np, variance);
         }
         return O3R_OK;
     });
@@ -795,21 +781,20 @@ int o3r_sor(o3r_ctx* ctx, const o3r_point* pts, size_t n, int mean_k, double std
     return api(ctx, [&] {
         if (n == 0) return O3R_OK;
         if (n >= (1ull << 32)) return ctx->fail(O3R_ERR_INVALID, "cloud too large for 32-bit indices");
-        CU(ctx->pts.ensure(n * 16));
+        CU(ctx->in_pts.ensure(n * 16));
         CU(ctx->seg2.ensure(16));
-        ctx->last_n = 0; ctx->last_total = 0; ctx->last_has_partials = false;
-        CU(cudaMemcpyAsync(ctx->pts.p, pts, n * 16, cudaMemcpyHostToDevice, ctx->st));
+        CU(cudaMemcpyAsync(ctx->in_pts.p, pts, n * 16, cudaMemcpyHostToDevice, ctx->st));
         const uint32_t seg_h[2] = {0u, (uint32_t)n};
         { int rcu = upload_small(ctx, ctx->seg2.p, seg_h, 8); if (rcu) return rcu; }
         SortU32 sb;
         int rc = carve_sort_u32(ctx, n, sb);
         if (rc) return rc;
-        rc = sor_filter(ctx, sb, ctx->pts.as<float4>(), ctx->seg2.as<uint32_t>(), 1, n, mean_k, stddev_mul);
+        rc = sor_filter(ctx, sb, ctx->in_pts.as<float4>(), ctx->seg2.as<uint32_t>(), 1, n, mean_k, stddev_mul);
         if (rc) return rc;
         std::vector<float> d(n);
         double thr = 0;
-        CU(cudaMemcpyAsync(d.data(), ctx->sor_dist.p, n * 4, cudaMemcpyDeviceToHost, ctx->st));
-        CU(cudaMemcpyAsync(&thr, ctx->sor_thr.p, 8, cudaMemcpyDeviceToHost, ctx->st));
+        CU(cudaMemcpyAsync(d.data(), ctx->sor.dist.p, n * 4, cudaMemcpyDeviceToHost, ctx->st));
+        CU(cudaMemcpyAsync(&thr, ctx->sor.thr.p, 8, cudaMemcpyDeviceToHost, ctx->st));
         CU(cudaStreamSynchronize(ctx->st));
         for (size_t i = 0; i < n; ++i) keep[i] = !((double)d[i] > thr);
         if (dist) memcpy(dist, d.data(), n * 4);
