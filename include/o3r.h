@@ -96,6 +96,12 @@ enum {
                                  0 sort   — everything else (StatisticalOutlierRemoval on, a Q without the rectified-stereo
                                             sparsity, device-side limits of the other two exceeded, a combined grid so fine
                                             that nothing reduces): runs as ACCUMULATE_TILED.
+                                 A chunk of up to 65535 frames (a device-pointer or prefetched batch is one chunk) keeps
+                                 every frame's count on engines 1 / 2; engine 1 keeps at most 8192 stray records (voxels on
+                                 the border of their bucket's cell, a couple per frame) a chunk, and a chunk with more
+                                 moves this batch and the context's later ones to engine 0.  u8 disparities whose
+                                 |q14 d + q15| is not monotone over (min_disparity, 255] raise engine 2's range check.
+                                 Whichever engine serves a batch, the results are the same.
                                  o3r_last_batch_points is unsupported while engines 1 / 2 serve the batch (frame_counts are
                                  still reported).  Same result contract as ACCUMULATE_TILED: keys, counts, colour sums exact,
                                  centroids within float reassociation (<= 1e-5 relative), reproducible bit for bit           */

@@ -28,9 +28,11 @@
 // O3R_MERGE_ACCUMULATE_TILED: keys, counts, colour sums exact, centroids equal to the oracle's left fold within float
 // reassociation (<= 1e-5 relative), reproducible bit for bit from run to run.
 //
-// Limits (checked on the device; the host then reruns the batch through the sort engine and stays there):
-// a bucket with more than kBkCapSlow points, more than kBkMaxPart distinct combined cells in one bucket, a point outside
-// the host's conservative per-frame bucket grid.
+// Limits (checked on the device; the host then reruns the batch through the sort engine and stays there): a bucket with
+// more than kBkCapSlow points (histogram), or more than one reduce CTA holds (kRdCap), more than kRdStray strays in one
+// bucket or more than the host's stray cap in one chunk (reduce), a point outside the host's conservative per-frame bucket
+// grid.  A frame whose grid the host cannot bound (w changing sign, a cell index past 8e6 leaf edges, more than 2^24
+// buckets) keeps the batch off this engine from the start.
 #pragma once
 #include "common.cuh"
 #include "sort.cuh"
@@ -40,11 +42,7 @@ namespace o3r {
 
 constexpr int kBkB = 5;                            // bucket edge in leaf cells (= voxel_size / leaf)
 constexpr int kBkSub = kBkB * kBkB;                // leaf columns per bucket (<= 32: one lane per column in the scan)
-constexpr int kBkCap = 128;                        // points the reduce ranks in shared memory at once (a bucket, or one leaf column of a big one)
-constexpr int kBkCapSlow = 65535;                  // larger buckets (parallax overlaps) are ranked one leaf column at a time; a column holds <= kBkCap
-constexpr int kBkRounds = kBkCap / 32;
-constexpr int kBkPerWarp = 4;                      // buckets a warp takes per ticket
-constexpr int kBkMaxPart = 8;                      // partial cells per bucket
+constexpr int kBkCapSlow = 65535;                  // points of one bucket: its count shares a 32-bit word with the frame index
 constexpr int kBkScanItems = 8;
 constexpr int kBkScanTile = kThreads * kBkScanItems;
 #ifndef O3R_BK_MINB
@@ -159,12 +157,11 @@ __device__ __forceinline__ void st_relaxed_u64(unsigned long long* p, unsigned l
 }
 constexpr unsigned long long kBk64Local = 1ull << 62, kBk64Global = 2ull << 62, kBk64Mask = (1ull << 62) - 1ull;
 
-// counts[g] becomes the bucket's first slot (the scatter's cursor); nl[r] = {first slot, points | frame << 16 | pass-through
-// << 31, I, J} of the r-th non-empty bucket ((I, J) = the bucket's position in units of kBkB leaf cells = its nominal cell on
-// the combined grid); totals = {points, non-empty buckets}
+// counts[g] becomes the bucket's first slot (the scatter's cursor); nl[r] = {first slot, points | frame << 16, I, J} of the
+// r-th non-empty bucket ((I, J) = the bucket's position in units of kBkB leaf cells = its nominal cell on the combined grid;
+// the frame is chunk-local and takes all 16 bits: a chunk holds up to 65535 frames); totals = {points, non-empty buckets}
 __global__ void __launch_bounds__(kThreads) k_bk_scan(uint32_t* __restrict__ counts, uint32_t nb_total,
-                                                      const BkFrame* __restrict__ bk, const uint8_t* __restrict__ frame_pass,
-                                                      int n_frames, uint4* __restrict__ nl,
+                                                      const BkFrame* __restrict__ bk, int n_frames, uint4* __restrict__ nl,
                                                       unsigned long long* __restrict__ status, uint32_t* __restrict__ ticket,
                                                       uint32_t* __restrict__ totals, uint32_t* __restrict__ flags) {
     __shared__ unsigned long long s_w[kWarps + 2];
@@ -261,8 +258,7 @@ __global__ void __launch_bounds__(kThreads) k_bk_scan(uint32_t* __restrict__ cou
             const BkFrame Bf = bk[f];
             const uint32_t lg = g - Bf.base;
             const int nI = Bf.i0c / kBkB + (int)(lg % (uint32_t)Bf.ni), nJ = Bf.j0c / kBkB + (int)(lg / (uint32_t)Bf.ni);
-            nl[rank++] = make_uint4(start, min(c[q], 0xffffu) | ((uint32_t)f << 16) | (frame_pass[f] ? 0x80000000u : 0u),
-                                    (uint32_t)nI, (uint32_t)nJ);
+            nl[rank++] = make_uint4(start, min(c[q], 0xffffu) | ((uint32_t)f << 16), (uint32_t)nI, (uint32_t)nJ);
             start += c[q];
         }
     }
@@ -455,6 +451,7 @@ struct RdSmem {
     uint32_t bin[kRdBins + 4];             // per bin: count, then first position ([n_bins] = total)
     uint32_t startbits[kRdCap / 32 + 1];   // bit p: position p starts a bin
     uint4 ent[kRdG];
+    uint8_t pass[kRdG];                    // per bucket: its frame passes through PCL's guard (looked up by frame index)
     uint32_t bstart[kRdG + 1];             // first point of each bucket, relative to the sub-batch
     uint8_t cb[kRdCap / 32 + 4];           // bucket that holds position 32 c (the lookup walks on from there)
     uint32_t sub_b1, sub_n;                // the sub-batch: buckets [b0, sub_b1), sub_n points
@@ -512,7 +509,7 @@ __device__ __forceinline__ bool bk_cell_less(const o3r_cell& a, const o3r_cell& 
 // out[*out_base + totals[1] + ...]  strays, appended through *stray_cnt (at most stray_cap)
 __global__ void __launch_bounds__(kThreads, O3R_BK_MINB) k_bk_reduce(
     const float4* __restrict__ pts, const unsigned long long* __restrict__ keys, const uint4* __restrict__ nl,
-    const uint32_t* __restrict__ totals, float icx, float icz, o3r_cell* __restrict__ out,
+    const uint8_t* __restrict__ frame_pass, const uint32_t* __restrict__ totals, float icx, float icz, o3r_cell* __restrict__ out,
     const uint32_t* __restrict__ out_base, uint32_t* __restrict__ stray_cnt, uint32_t stray_cap, uint32_t* __restrict__ ticket,
     uint32_t* __restrict__ frame_vox, int* __restrict__ cellbb, uint32_t* __restrict__ flags, float4* __restrict__ dbg_vox,
     uint32_t* __restrict__ dbg_cnt) {
@@ -533,7 +530,11 @@ __global__ void __launch_bounds__(kThreads, O3R_BK_MINB) k_bk_reduce(
         const uint32_t r0 = S.ticket;
         if (r0 >= NR) break;
         const int nb = (int)min((uint32_t)kRdG, NR - r0);
-        if (tid < nb) S.ent[tid] = nl[r0 + tid];
+        if (tid < nb) {
+            const uint4 e = nl[r0 + tid];
+            S.ent[tid] = e;
+            S.pass[tid] = frame_pass[e.y >> 16];
+        }
         __syncthreads();
         for (int b0 = 0; b0 < nb;) {
             // ---- sub-batch: as many of the ticket's buckets as fit (normally all of them)
@@ -583,7 +584,7 @@ __global__ void __launch_bounds__(kThreads, O3R_BK_MINB) k_bk_reduce(
                     S.pts[i] = __ldcs(pts + base + i);
                     int bl = S.cb[i >> 5];
                     while (bl + 1 < nbb && S.bstart[bl + 1] <= i) ++bl;
-                    const bool pass = (S.ent[b0 + bl].y >> 31) != 0u;
+                    const bool pass = S.pass[b0 + bl] != 0;
                     const uint32_t bin = (uint32_t)bl * kBkSub + bk_key_col(key[k], pass);
                     bs[k] = bin | (atomicAdd(&S.bin[bin], 1u) << 16);
                 }
@@ -638,7 +639,7 @@ __global__ void __launch_bounds__(kThreads, O3R_BK_MINB) k_bk_reduce(
                 int bl = S.cb[pos >> 5];
                 while (bl + 1 < nbb && S.bstart[bl + 1] <= pos) ++bl;
                 const uint4 ent = S.ent[b0 + bl];
-                const bool pass = (ent.y >> 31) != 0u;
+                const bool pass = S.pass[b0 + bl] != 0;
                 const uint32_t k32 = S.fkey[pos];
                 const bool head = pass || ((S.startbits[pos >> 5] >> (pos & 31u)) & 1u) || S.fkey[pos - 1] != k32;
                 if (!head) continue;
@@ -732,7 +733,7 @@ __global__ void __launch_bounds__(kThreads, O3R_BK_MINB) k_bk_reduce(
                         cmn[2] = min(cmn[2], kz); cmx[2] = max(cmx[2], kz);
                     }
                     out0[r0 + b0 + bl] = mainc;
-                    atomicAdd(&frame_vox[(ent.y >> 16) & 0x7fffu], nh);
+                    atomicAdd(&frame_vox[ent.y >> 16], nh);
                     if (ns) {
                         const uint32_t at = atomicAdd(stray_cnt, ns);
                         if (at + ns > stray_cap) atomicOr(flags + 1, BK_FLAG_PART);

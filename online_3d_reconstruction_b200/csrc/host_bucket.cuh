@@ -127,7 +127,7 @@ int bk_prepare(o3r_ctx* ctx, const BkPlan& pl, int n, size_t cap_batch, size_t c
     CU(ctx->bk.status.ensure(((size_t)cdiv(pl.max_chunk_nb, kBkScanTile) + 1) * 8 + 64));
     CU(ctx->bk.stray.ensure((size_t)kBkStrayCap * sizeof(o3r_cell)));
     CU(ctx->bk.misc.ensure(256 + (size_t)n * 4 + (size_t)n));
-    // every partial cell holds at least one point, and a bucket emits at most kBkMaxPart of them
+    // one main partial per non-empty bucket (it holds at least one point), plus the strays of every chunk
     const size_t part_ub = std::min(cap_batch, pl.total_nb) + (size_t)kBkStrayCap * pl.chunk_nb.size();
     CU(ctx->last.partials.ensure(std::max<size_t>(part_ub, 1) * sizeof(o3r_cell)));
     CU(ctx->bbox.ensure((size_t)n * 6 * 4));
@@ -160,14 +160,14 @@ int bk_run_chunk(o3r_ctx* ctx, const AParams& P, const BkPlan& pl, int ci, int f
     FILL(bbox, (size_t)(nc) * 24, FILL_BBOX);
     LAUNCH_N("k_bk_hist", (k_bk_hist<DT>), grid, kThreads, 0, P, fr, bk, ctx->inv_f, ctx->bk.counts.as<uint32_t>(), bbox, M.flags);
     LAUNCH(k_bk_frames, cdiv(nc, 64), 64, 0, nc, bbox, ctx->inv_f, M.pass + f0, M.fvox + f0);
-    LAUNCH(k_bk_scan, scan_tiles, kThreads, 0, ctx->bk.counts.as<uint32_t>(), (uint32_t)nb, bk, M.pass + f0, nc,
+    LAUNCH(k_bk_scan, scan_tiles, kThreads, 0, ctx->bk.counts.as<uint32_t>(), (uint32_t)nb, bk, nc,
            ctx->bk.nl.as<uint4>(), st_scan, M.t_scan, M.totals, M.flags);
     LAUNCH_N("k_bk_scatter", (k_bk_scatter<DT>), grid, kThreads, 0, P, fr, bk, M.pass + f0, ctx->inv_f,
              ctx->bk.counts.as<uint32_t>(), ctx->bk.pts.as<float4>(), ctx->bk.pos.as<unsigned long long>(), M.flags);
     const uint32_t rgrid = std::max(1u, std::min<uint32_t>(cdiv(nl_ub, kRdG), 148 * 4));
     float4* dbg = ctx->keep_frame_voxels ? ctx->last.vox.as<float4>() : nullptr;
     LAUNCH(k_bk_reduce, rgrid, kThreads, bk_reduce_smem(), ctx->bk.pts.as<float4>(), ctx->bk.pos.as<unsigned long long>(),
-           ctx->bk.nl.as<uint4>(), M.totals, ctx->inv_c, ctx->inv_cz, ctx->last.partials.as<o3r_cell>(),
+           ctx->bk.nl.as<uint4>(), M.pass + f0, M.totals, ctx->inv_c, ctx->inv_cz, ctx->last.partials.as<o3r_cell>(),
            cnt + CNT_PART, M.stray_cnt, (uint32_t)kBkStrayCap, M.t_reduce, M.fvox + f0, reinterpret_cast<int*>(cnt + CNT_CELLBB),
            M.flags, dbg, M.dbg_cnt);
     LAUNCH(k_bk_strays, 1, 1024, 0, ctx->last.partials.as<o3r_cell>(), cnt + CNT_PART, M.totals, M.stray_cnt, (uint32_t)kBkStrayCap,

@@ -166,10 +166,11 @@ int tv_run_chunk(o3r_ctx* ctx, const AParams& P, const TvPlan& pl, int f0, int n
     A.ntx = pl.ntx; A.nty = pl.nty; A.n_frames = nc;
     A.inv_f = ctx->inv_f; A.icx = ctx->inv_c; A.icz = ctx->inv_cz;
     A.wlim = pl.R > 0 ? pl.wlim(pl.R) : INFINITY;
-    {   // the largest u8 disparity that keeps |q14 d + q15| below the bound
-        int dl = -1;
-        for (int d = 0; d < 256; ++d)
-            if (std::fabs(ctx->p.Q[14] * d + ctx->p.Q[15]) < A.wlim) dl = d; else if (dl >= 0) break;
+    {   // the kernel's LUT path flags d > dlim_i: every live u8 disparity (thr_i, dlim_i] must keep |q14 d + q15| below the
+        // bound.  Scan up from the first live one and stop at the first that breaks it: when |w| is not monotone over the live
+        // range (q15 of the opposite sign to q14), disparities past that point are flagged even where |w| drops back below.
+        int dl = std::max(P.thr_i, -1);
+        for (int d = dl + 1; d < 256 && std::fabs(ctx->p.Q[14] * d + ctx->p.Q[15]) < A.wlim; ++d) dl = d;
         A.dlim_i = dl;
     }
     A.scratch = ctx->tv.scratch.as<o3r_cell>();

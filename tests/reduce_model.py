@@ -72,6 +72,31 @@ def accumulate_downsample(pts, v, min_points=1):
     return out, key[starts][keep], lens[keep].astype(np.uint32)
 
 
+SUMS = np.dtype([("key", "<u8"), ("sx", "<f8"), ("sy", "<f8"), ("sz", "<f8"), ("ax", "<f8"), ("ay", "<f8"), ("az", "<f8"),
+                 ("n", "<u4"), ("sr", "<u8"), ("sg", "<u8"), ("sb", "<u8")])
+
+
+def cell_sums(pts, v):
+    """-> the exact per-cell sums of the combined grid (what exportCells() holds), ascending key, as a SUMS array: point count
+    and colour channel sums exact; x, y and z + 500 (the shift in float32, as on the device) summed in float64, with the
+    sums of their absolute values (ax, ay, az) as the scale a reassociated float32 sum is compared on."""
+    pts = np.ascontiguousarray(pts, dtype=abi.POINT)
+    i, j, k = cells(pts, v)
+    key = cell_keys(i, j, k)
+    uk, inv = np.unique(key, return_inverse=True)
+    out = np.zeros(len(uk), dtype=SUMS)
+    out["key"] = uk
+    out["n"] = np.bincount(inv, minlength=len(uk))
+    vals = (pts["x"].astype(np.float64), pts["y"].astype(np.float64), (pts["z"].astype(F32) + F32(500.0)).astype(np.float64))
+    for f, a, x in zip(("sx", "sy", "sz"), ("ax", "ay", "az"), vals):
+        out[f] = np.bincount(inv, weights=x, minlength=len(uk))
+        out[a] = np.bincount(inv, weights=np.abs(x), minlength=len(uk))
+    c = pts["rgb"].astype(np.uint64)
+    for f, sh in (("sr", 16), ("sg", 8), ("sb", 0)):
+        out[f] = np.bincount(inv, weights=((c >> np.uint64(sh)) & np.uint64(255)).astype(np.float64), minlength=len(uk))
+    return out
+
+
 def float_fold_channel(vals):
     """CentroidPoint's colour: a float32 left fold of the channel values, uint32(sum / n)."""
     s = np.add.accumulate(np.asarray(vals, dtype=F32), dtype=F32)[-1]

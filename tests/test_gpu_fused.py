@@ -190,8 +190,8 @@ def test_fused_tile_engine_widens_its_window_when_a_disparity_is_out_of_reach():
 def test_fused_big_buckets_are_ranked_column_by_column(voxel):
     """voxel_size 0.12: a leaf spans more pixels than the tile engine's widest window (the device raises the range flag
     on the first batch and the context moves to the bucket engine), and several hundred points fall into one 5x5-leaf bucket:
-    above 128 the warp ranks one leaf column at a time (PCL's order is column-major inside a bucket), same bit-exact per-frame
-    centroids."""
+    the reduce ranks every point inside its (bucket, leaf column) bin — PCL's order is column-major inside a bucket — same
+    bit-exact per-frame centroids."""
     keep = []
     geom = SMALL4
     p = abi.make_params(jump_pixels=1, voxel_size=voxel, merge_mode=FUSED, **geom)

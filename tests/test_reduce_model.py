@@ -42,3 +42,23 @@ def test_bright_cell_channel_cycle_separates_the_two_colour_sums():
     vals = np.tile(np.array([255, 253, 254], dtype=np.uint32), 50000)
     assert rm.float_fold_channel(vals) == 253
     assert rm.uint_sum_channel(vals) == 254
+
+
+@pytest.mark.parametrize("seed,v", [(5, 0.05), (6, 0.25)])
+def test_cell_sums_match_oracle(seed, v):
+    """cell_sums (the exact per-cell sums the GPU tests compare exportCells() with) against the oracle's combined VoxelGrid:
+    same cells in key order, and sums / n equal to its centroids (colours exact, coordinates within float rounding)."""
+    pts = _cloud(seed, 20000, 3.0, 3000)
+    p = abi.make_params(voxel_size=v, min_points_per_voxel=1)
+    exp = ob.downsample_pt_cloud(p, pts, True)
+    s = rm.cell_sums(pts, v)
+    _, keys, counts = rm.accumulate_downsample(pts, v)
+    assert np.array_equal(s["key"], keys) and np.array_equal(s["n"], counts) and s["n"].sum() == len(pts)
+    assert len(s) == len(exp) and s["n"].max() >= 3000
+    n = s["n"].astype(np.float32)
+    rgb = [(s[f].astype(np.float32) / n).astype(np.uint32) for f in ("sr", "sg", "sb")]
+    assert np.array_equal((rgb[0] << np.uint32(16)) | (rgb[1] << np.uint32(8)) | rgb[2], exp["rgb"])
+    for f, a, sh in (("sx", "ax", 0.0), ("sy", "ay", 0.0), ("sz", "az", 500.0)):
+        c = s[f] / s["n"]
+        e = exp[f[1]].astype(np.float64) + sh
+        assert np.all(np.abs(c - e) <= 1e-5 * s[a] / s["n"])   # the oracle folds in float32
