@@ -47,6 +47,7 @@ __device__ __forceinline__ int dev_reflect101(int i, int n) {
 template <int MODE>
 __global__ void __launch_bounds__(kBlurRows) k_blur(const BlurJob* __restrict__ jobs, int rows, int cols, int k,
                                                     int rx0, int ry0, int rx1, int ry1) {
+    wait_prior();
     extern __shared__ __align__(16) unsigned char bsm[];
     constexpr int ROWS = MODE == O3R_BLUR_MEDIAN ? kMedRows : kBlurRows;
     const BlurJob job = jobs[blockIdx.z];
@@ -183,6 +184,7 @@ inline size_t bilateral_smem(int radius, int maxk) {
 
 __global__ void __launch_bounds__(kBilTX * kBilTY) k_bilateral(const BlurJob* __restrict__ jobs, BilateralLut L, int rows,
                                                                int cols, int rx0, int ry0, int rx1, int ry1) {
+    wait_prior();
     extern __shared__ __align__(16) unsigned char bsm[];
     const BlurJob job = jobs[blockIdx.z];
     const int r = L.radius, tw = kBilW + 2 * r, th = kBilTY + 2 * r;

@@ -84,6 +84,7 @@ __global__ void __launch_bounds__(kThreads) k_bk_hist(AParams P, const FrameDev*
                                                       const BkFrame* __restrict__ bk, float inv_f,
                                                       uint32_t* __restrict__ counts, uint32_t* __restrict__ bbox,
                                                       uint32_t* __restrict__ flags) {
+    wait_prior();
     __shared__ double rl[256];
     __shared__ float zl[256];
     __shared__ uint32_t s_red[8];
@@ -138,6 +139,7 @@ __global__ void __launch_bounds__(kThreads) k_bk_hist(AParams P, const FrameDev*
 // per frame: PCL's int32 overflow guard on the exact bbox (pass-through frames keep their points verbatim)
 __global__ void k_bk_frames(int n_frames, const uint32_t* __restrict__ bbox, float inv_f, uint8_t* __restrict__ frame_pass,
                             uint32_t* __restrict__ frame_vox) {
+    wait_prior();
     const int f = blockIdx.x * blockDim.x + threadIdx.x;
     if (f >= n_frames) return;
     const GridParams G = make_grid(bbox + 6 * f, inv_f, inv_f, inv_f);
@@ -164,6 +166,7 @@ __global__ void __launch_bounds__(kThreads) k_bk_scan(uint32_t* __restrict__ cou
                                                       const BkFrame* __restrict__ bk, int n_frames, uint4* __restrict__ nl,
                                                       unsigned long long* __restrict__ status, uint32_t* __restrict__ ticket,
                                                       uint32_t* __restrict__ totals, uint32_t* __restrict__ flags) {
+    wait_prior();
     __shared__ unsigned long long s_w[kWarps + 2];
     __shared__ uint32_t s_ticket;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -312,6 +315,7 @@ __global__ void __launch_bounds__(kThreads, 5) k_bk_scatter(AParams P, const Fra
                                                          float inv_f, uint32_t* __restrict__ cursor, float4* __restrict__ pts,
                                                          unsigned long long* __restrict__ keys_out,
                                                          const uint32_t* __restrict__ flags) {
+    wait_prior();
     __shared__ double rl[256];
     __shared__ float zl[256];
     __shared__ __align__(16) BkScatterWarp s_w[kWarps];
@@ -513,6 +517,7 @@ __global__ void __launch_bounds__(kThreads, O3R_BK_MINB) k_bk_reduce(
     const uint32_t* __restrict__ out_base, uint32_t* __restrict__ stray_cnt, uint32_t stray_cap, uint32_t* __restrict__ ticket,
     uint32_t* __restrict__ frame_vox, int* __restrict__ cellbb, uint32_t* __restrict__ flags, float4* __restrict__ dbg_vox,
     uint32_t* __restrict__ dbg_cnt) {
+    wait_prior();
     extern __shared__ __align__(16) unsigned char bk_smem_raw[];
     RdSmem& S = *reinterpret_cast<RdSmem*>(bk_smem_raw);
     if (flags[0]) return;   // raised by the histogram / scan (complete before this kernel starts): uniform exit
@@ -766,6 +771,7 @@ __global__ void __launch_bounds__(1024) k_bk_strays(o3r_cell* __restrict__ out, 
                                                     const uint32_t* __restrict__ totals, const uint32_t* __restrict__ stray_cnt,
                                                     uint32_t stray_cap, o3r_cell* __restrict__ tmp, uint32_t* __restrict__ chunk_total,
                                                     const uint32_t* __restrict__ flags) {
+    wait_prior();
     if (flags[0]) { if (threadIdx.x == 0) *chunk_total = 0u; return; }
     const uint32_t NR = totals[1], n = min(*stray_cnt, stray_cap);
     if (threadIdx.x == 0) *chunk_total = NR + n;

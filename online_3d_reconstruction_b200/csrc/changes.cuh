@@ -28,6 +28,7 @@ __device__ __forceinline__ uint32_t merge_path(const uint64_t* a, uint32_t na, c
 __global__ void __launch_bounds__(kThreads) k_chg_part(const uint64_t* __restrict__ a, const uint32_t* __restrict__ na_ptr,
                                                        const uint64_t* __restrict__ b, const uint32_t* __restrict__ nb_ptr,
                                                        uint32_t tiles, uint32_t* __restrict__ part) {
+    wait_prior();
     const uint32_t t = blockIdx.x * kThreads + threadIdx.x;
     if (t > tiles) return;
     const uint32_t na = *na_ptr, nb = *nb_ptr;
@@ -42,6 +43,7 @@ __global__ void __launch_bounds__(kThreads) k_chg_union(const uint64_t* __restri
                                                         const uint64_t* __restrict__ b, const uint32_t* __restrict__ nb_ptr,
                                                         const uint32_t* __restrict__ part, uint32_t* __restrict__ cnt,
                                                         const uint32_t* __restrict__ off, uint64_t* __restrict__ out) {
+    wait_prior();
     __shared__ uint64_t s_a[kTileV], s_b[kTileV];
     __shared__ uint32_t s_scan[34];
     const uint32_t na = *na_ptr, nb = *nb_ptr, n = na + nb;
@@ -108,6 +110,7 @@ __global__ void __launch_bounds__(kThreads) k_chg_emit_cnt(const uint64_t* __res
                                                            const float4* __restrict__ res_acc, uint32_t min_points,
                                                            uint32_t* __restrict__ pos, uint32_t* __restrict__ cnt,
                                                            uint32_t* __restrict__ err) {
+    wait_prior();
     const uint32_t n = *n_ptr, n_res = *n_res_ptr;
     const uint32_t t = blockIdx.x;
     uint32_t c = 0;
@@ -145,6 +148,7 @@ __global__ void __launch_bounds__(kThreads) k_chg_emit(const uint32_t* __restric
                                                        const uint4* __restrict__ res_rgb, const uint32_t* __restrict__ off,
                                                        float4* __restrict__ out, uint64_t* __restrict__ out_keys,
                                                        uint32_t* __restrict__ out_counts) {
+    wait_prior();
     __shared__ uint32_t s_scan[34];
     const uint32_t n = *n_ptr;
     const uint32_t t = blockIdx.x;

@@ -16,6 +16,7 @@ enum : uint32_t {
 __global__ void __launch_bounds__(kThreads) k_cells_pack(const uint32_t* __restrict__ n_res_ptr, const uint64_t* __restrict__ res_keys,
                                                          const float4* __restrict__ res_acc, const uint4* __restrict__ res_rgb,
                                                          o3r_cell* __restrict__ out) {
+    wait_prior();
     const uint32_t n_res = *n_res_ptr;
     for (uint32_t i = blockIdx.x * kThreads + threadIdx.x; i < n_res; i += gridDim.x * kThreads) {
         const float4 a = res_acc[i];
@@ -33,6 +34,7 @@ __global__ void __launch_bounds__(kThreads) k_cells_pack(const uint32_t* __restr
 // start at ~0, res[1] at 0.  world = 0: no ownership check.
 __global__ void __launch_bounds__(kThreads) k_cells_check(const o3r_cell* __restrict__ cells, uint32_t n, uint32_t world,
                                                           uint32_t rank, unsigned long long* __restrict__ res) {
+    wait_prior();
     uint32_t all = 0u;
     for (uint32_t i = blockIdx.x * kThreads + threadIdx.x; i < n; i += gridDim.x * kThreads) {
         const o3r_cell c = cells[i];

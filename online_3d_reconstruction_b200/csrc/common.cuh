@@ -12,6 +12,14 @@ constexpr int kThreads = 256;          // every kernel in this library runs 256-
 constexpr int kWarps = kThreads / 32;
 constexpr unsigned kFull = 0xffffffffu;
 
+// Every __global__ of the library calls this first, before any global read, write or atomic.  The library launches its
+// kernels with programmatic stream serialisation (LAUNCH_N, host_ctx.cuh): a kernel may be launched and its CTAs placed
+// while the previous kernel on the stream is still draining, and this waits until that kernel has completed and its writes
+// are visible.  Since every kernel waits here before it touches memory, stream order holds transitively.  No kernel
+// triggers its dependents early, so what overlaps is the launch and the CTA rasterisation only.  (A no-op in a kernel
+// launched without the attribute.)
+__device__ __forceinline__ void wait_prior() { cudaGridDependencySynchronize(); }
+
 // One frame's inputs as the kernels see them (device pointers).
 struct FrameDev {
     const uint8_t* disp;

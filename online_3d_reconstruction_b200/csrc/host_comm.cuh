@@ -23,6 +23,7 @@ __global__ void __launch_bounds__(kThreads) k_pack_slots_cyc(const uint32_t* __r
                                                              const uint4* __restrict__ crgb, const uint32_t* __restrict__ counts,
                                                              uint32_t world, uint32_t slot_cap, o3r_cell* __restrict__ slots,
                                                              uint32_t* __restrict__ xflag) {
+    wait_prior();
     __shared__ uint32_t s_start[257];
     const uint32_t n = *n_cyc_ptr;
     if (threadIdx.x == 0) {
@@ -58,6 +59,7 @@ __global__ void __launch_bounds__(kThreads) k_pack_slots_cyc(const uint32_t* __r
 // received slots (one per source rank, in rank order) -> contiguous list + count, all on the device
 __global__ void __launch_bounds__(kThreads) k_unpack_slots(const o3r_cell* __restrict__ slots, uint32_t world, uint32_t slot_cap,
                                                            o3r_cell* __restrict__ out, uint32_t* __restrict__ n_out) {
+    wait_prior();
     __shared__ uint32_t s_start[257];
     if (threadIdx.x == 0) {
         uint32_t a = 0;
@@ -119,6 +121,7 @@ NcclApi* nccl_api() {
     do {                                                                                              \
         if (ctx->fq.L.n) { int rcf_ = fill_flush(ctx); if (rcf_) return rcf_; }                       \
         ncclResult_t r_ = (call);                                                                     \
+        ctx->pdl_off = true;                                                                          \
         if (r_ != ncclSuccess)                                                                        \
             return ctx->fail(O3R_ERR_CUDA, std::string("NCCL error at " #call ": ") + N->GetErrorString(r_)); \
     } while (0)

@@ -78,7 +78,8 @@ struct DevBuf {
 // library goes through LAUNCH / CU / NC, which flush the queue first), so stream order is what it would have been with
 // separate kernels.  api() selects the context's device before anything is queued or flushed, and flushes what is left
 // before the call returns: no fill outlives the call that queued it.
-struct FillList { uint32_t* p[8]; unsigned long long words[8]; int kind[8]; int n; };
+constexpr int kFillMax = 16;   // fills per flush: enough for every fill a fused cycle queues in front of its first kernel
+struct FillList { uint32_t* p[kFillMax]; unsigned long long words[kFillMax]; int kind[kFillMax]; int n; };
 enum { FILL_ZERO = 0, FILL_BBOX = 1, FILL_CELLBB = 2 };   // bbox: {~0, ~0, ~0, 0, 0, 0} per 6 words; cell range: {INT_MAX x3, INT_MIN x3}
 struct FillQueue {
     FillList L{};
@@ -181,6 +182,8 @@ struct TileState {
     bool off = false;                 // a batch exceeded the engine's limits: the bucket / sort engine serve this context from then on
     int R = -1;                       // window radius in use (-1: not chosen yet)
     int guess = -1;                   // PCL's overflow guard on the last frame seen (-1: none yet) = the guess for the next batch
+    const uint8_t* guess_at = nullptr;   // where in `misc` the last uploaded per-frame guesses lie, and what they are
+    std::vector<uint8_t> guess_dev;
     uint32_t attr = 0;                // k_tv instantiations whose shared-memory attribute is set
 };
 
@@ -273,6 +276,7 @@ struct o3r_ctx {
     std::mutex mu;
     std::string err;
     uint64_t launches = 0;
+    bool pdl_off = false;   // the next launch waits for the stream in full (set after NCCL calls, see LAUNCH_N)
     FillQueue fq;   // pending device fills (see FillList)
     cudaStream_t st = nullptr, st_copy = nullptr, st_copy2 = nullptr;   // two copy streams: the per-copy set-up gaps of one hide behind the other
     cudaEvent_t ev_copy2 = nullptr;
@@ -342,6 +346,10 @@ int fill_flush(o3r_ctx* ctx);
         if (e_ != cudaSuccess) return ctx->fail_cuda(e_, #call, __FILE__, __LINE__);    \
     } while (0)
 
+// Kernels go out with programmatic stream serialisation: the next kernel's launch overlaps the tail of the previous one,
+// and its wait_prior() (common.cuh) restores the full dependency before it touches memory.  Copies and event records keep
+// plain stream order.  The first launch of an API call and the first after an NCCL call go without it (ctx->pdl_off):
+// kernels the library does not own (the caller's, NCCL's) do not promise to leave their trigger to their completion.
 #define LAUNCH_N(name, kernel, grid, block, smem, ...)                        \
     do {                                                                      \
         if (ctx->fq.L.n) { int rcf_ = fill_flush(ctx); if (rcf_) return rcf_; } \
@@ -350,9 +358,17 @@ int fill_flush(o3r_ctx* ctx);
             pa_ = ctx->prof.get(); pb_ = ctx->prof.get();                     \
             cudaEventRecord(pa_, ctx->st);                                    \
         }                                                                     \
-        kernel<<<grid, block, smem, ctx->st>>>(__VA_ARGS__);                  \
+        cudaLaunchAttribute at_[1];                                           \
+        at_[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;       \
+        at_[0].val.programmaticStreamSerializationAllowed = ctx->pdl_off ? 0 : 1; \
+        ctx->pdl_off = false;                                                 \
+        cudaLaunchConfig_t cfg_ = {};                                         \
+        cfg_.gridDim = dim3(grid); cfg_.blockDim = dim3(block);               \
+        cfg_.dynamicSmemBytes = (smem); cfg_.stream = ctx->st;                \
+        cfg_.attrs = at_; cfg_.numAttrs = 1;                                  \
+        cudaError_t e_ = cudaLaunchKernelEx(&cfg_, kernel, __VA_ARGS__);      \
         ++ctx->launches;                                                      \
-        cudaError_t e_ = cudaGetLastError();                                  \
+        if (e_ == cudaSuccess) e_ = cudaGetLastError();                       \
         if (e_ != cudaSuccess) return ctx->fail_cuda(e_, #kernel, __FILE__, __LINE__);  \
         if (pa_) {                                                            \
             cudaEventRecord(pb_, ctx->st);                                    \
@@ -370,6 +386,7 @@ inline uint32_t cdiv(size_t a, size_t b) { return (uint32_t)((a + b - 1) / b); }
 // occupies the H2D engine, and the whole cycle would wait for it.
 struct SmallBlob { uint32_t w[960]; };   // 3840 bytes (kernel parameters are limited to 4 KB)
 __global__ void k_put_blob(uint32_t* __restrict__ dst, SmallBlob b, int n_words) {
+    wait_prior();
     for (int i = threadIdx.x; i < n_words; i += blockDim.x) dst[i] = b.w[i];
 }
 int upload_small(o3r_ctx* ctx, void* dst, const void* src, size_t bytes) {
@@ -386,6 +403,7 @@ int upload_small(o3r_ctx* ctx, void* dst, const void* src, size_t bytes) {
 // Fills run as kernels on the compute stream for the same reason: cudaMemsetAsync may be served by a copy engine and then
 // queues behind an input prefetch.  `bytes` and `dst` are multiples of 4 (all callers fill u32 tables).
 __global__ void __launch_bounds__(kThreads) k_fill_list(FillList L) {
+    wait_prior();
     for (int r = 0; r < L.n; ++r) {
         uint32_t* dst = L.p[r];
         const size_t n_words = L.words[r], stride = (size_t)gridDim.x * kThreads;
@@ -422,6 +440,7 @@ int api(o3r_ctx* ctx, F&& body) {
     std::lock_guard<std::mutex> lk(ctx->mu);
     const cudaError_t e = cudaSetDevice(ctx->p.device);
     if (e != cudaSuccess) return ctx->fail_cuda(e, "cudaSetDevice(ctx->p.device)", __FILE__, __LINE__);
+    ctx->pdl_off = true;   // the caller may have queued its own kernels on the stream since the last call (see LAUNCH_N)
     const int rc = body();
     if (!rc) return fill_flush(ctx);
     if (ctx->fq.L.n) { const std::string err = ctx->err; fill_flush(ctx); ctx->err = err; }
@@ -431,7 +450,7 @@ int api(o3r_ctx* ctx, F&& body) {
 namespace {
 int fill_queue(o3r_ctx* ctx, void* dst, size_t bytes, int kind) {
     if (bytes == 0) return O3R_OK;
-    if (ctx->fq.L.n == 8) { int rc = fill_flush(ctx); if (rc) return rc; }
+    if (ctx->fq.L.n == kFillMax) { int rc = fill_flush(ctx); if (rc) return rc; }
     ctx->fq.add(dst, bytes, kind);
     return O3R_OK;
 }

@@ -28,14 +28,22 @@ int acc_build_cycle_t(o3r_ctx* ctx, Items items, size_t n, bool use_resident, co
     CU(ctx->seg2.ensure(16));
     CU(ctx->ghist.ensure(kMaxPasses * kRsBins * 4));
     CU(ctx->plan_v2.ensure(sizeof(SortPlan)));
-    if (!n_dev) {
-        const uint32_t seg_h[2] = {0u, (uint32_t)n};
-        int rcu = upload_small(ctx, ctx->seg2.p, seg_h, 8);
-        if (rcu) return rcu;
-    }   // (else k_acc_key writes the segment from the device-side count)
+    const uint32_t tiles_ub = cdiv(n, kTileV);
+    CU(ctx->head_cnt.ensure((size_t)tiles_ub * 4));
+    CU(ctx->head_off.ensure((size_t)tiles_ub * 4));
+    // one record per cell of the cycle (<= n_cyc_ub <= n), reserved in big steps so steady-state cycles never reallocate
+    const size_t cyc_cap = std::max<size_t>(std::min<size_t>(n, ctx->n_cyc_ub ? ctx->n_cyc_ub : n), (size_t)1 << 20);
+    CU(ctx->ckey.ensure(cyc_cap * 8));
+    CU(ctx->cacc.ensure(cyc_cap * 16));
+    CU(ctx->crgb.ensure(cyc_cap * 16));
+    const size_t wbytes = 64 + ((size_t)tiles_ub + 1) * sizeof(RunCarry);
+    CU(ctx->runwork.ensure(wbytes));
+    tr.mark("ensures");
+    // (every buffer is sized before the fills are queued: a CU() between two fills would flush them as separate kernels)
     ZERO(ctx->ghist.p, kMaxPasses * kRsBins * 4);
     ZERO(cnt + CNT_NEW, 4);
-    const uint32_t* seg = ctx->seg2.as<uint32_t>();
+    ZERO(ctx->runwork.p, wbytes);
+    const uint32_t* seg = ctx->seg2.as<uint32_t>();   // {0, item count}: written by k_acc_key
     const uint32_t gk = std::min<uint32_t>(cdiv(n, kThreads), 148 * 8);
     SortPlan* plan = ctx->plan_v2.as<SortPlan>();
     LAUNCH(k_rs_layout, 1, 32, 0, 1, (const GridParams*)nullptr, total_bits, plan);
@@ -49,24 +57,13 @@ int acc_build_cycle_t(o3r_ctx* ctx, Items items, size_t n, bool use_resident, co
     AccArgs<KeyT> A;
     A.keys0 = k0; A.keys1 = k1; A.vals0 = v0; A.vals1 = v1;
     A.seg_off = seg; A.plan = plan;
-    A.tiles_ub = cdiv(n, kTileV);
+    A.tiles_ub = tiles_ub;
     A.kc = kc;
     const int cur = ctx->res.cur;
     A.res_keys = ctx->res.keys[cur].as<uint64_t>();
     A.res_acc = ctx->res.acc[cur].as<float4>();
     A.res_rgb = ctx->res.rgb[cur].as<uint4>();
     A.n_res_ptr = cnt + (use_resident ? CNT_NRES : CNT_ZERO);
-    CU(ctx->head_cnt.ensure((size_t)A.tiles_ub * 4));
-    CU(ctx->head_off.ensure((size_t)A.tiles_ub * 4));
-    // one record per cell of the cycle (<= n_cyc_ub <= n), reserved in big steps so steady-state cycles never reallocate
-    const size_t cyc_cap = std::max<size_t>(std::min<size_t>(n, ctx->n_cyc_ub ? ctx->n_cyc_ub : n), (size_t)1 << 20);
-    CU(ctx->ckey.ensure(cyc_cap * 8));
-    CU(ctx->cacc.ensure(cyc_cap * 16));
-    CU(ctx->crgb.ensure(cyc_cap * 16));
-    const size_t wbytes = 64 + ((size_t)A.tiles_ub + 1) * sizeof(RunCarry);
-    CU(ctx->runwork.ensure(wbytes));
-    ZERO(ctx->runwork.p, wbytes);
-    tr.mark("ensures");
     LAUNCH_N("k_acc_heads", (k_acc_heads<KeyT>), A.tiles_ub, kThreads, 0, A, v0, v1, ctx->head_cnt.as<uint32_t>(),
              cnt + CNT_NEW);
     LAUNCH(k_scan_u32, 1, kScanThreads, 0, ctx->head_cnt.as<uint32_t>(), ctx->head_off.as<uint32_t>(), A.tiles_ub,

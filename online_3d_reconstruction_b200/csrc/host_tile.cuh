@@ -127,9 +127,13 @@ int tv_prepare(o3r_ctx* ctx, TvPlan& pl, int n, int chunk, size_t cap_batch) {
     CU(ctx->tv.scratch.ensure(ctx->tv.scratch_cap * sizeof(o3r_cell)));
     CU(ctx->last.partials.ensure(ctx->tv.part_cap * sizeof(o3r_cell)));
     const TvMisc M = tv_misc(ctx, n);
-    ZERO(M.flags, (16 + (size_t)n) * 4);
-    const int rc = upload_small(ctx, M.guess, pl.guess.data(), (size_t)n);
-    if (rc) return rc;
+    ZERO(M.flags, (16 + (size_t)n) * 4);   // (the guess bytes follow these words: the fill leaves them alone)
+    if (ctx->tv.guess_at != M.guess || ctx->tv.guess_dev != pl.guess) {   // steady state: the device holds these guesses already
+        const int rc = upload_small(ctx, M.guess, pl.guess.data(), (size_t)n);
+        if (rc) return rc;
+        ctx->tv.guess_at = M.guess;
+        ctx->tv.guess_dev = pl.guess;
+    }
     return fused_prepare(ctx, cap_batch);
 }
 

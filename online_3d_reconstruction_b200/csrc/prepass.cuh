@@ -17,6 +17,7 @@ constexpr int kLabSums = 10;   // total, n, Sx, Sy, Sxx, Sxy, Syy, Sxd, Syd, Sd
 __global__ void __launch_bounds__(kThreads) k_label_sums(const uint8_t* __restrict__ labels, size_t lstep,
                                                          const uint8_t* __restrict__ disp, size_t dstep, int rows, int cols,
                                                          int x0, int bb, unsigned long long* __restrict__ out) {
+    wait_prior();
     __shared__ unsigned long long acc[256 * kLabSums];
     for (int i = threadIdx.x; i < 256 * kLabSums; i += kThreads) acc[i] = 0ull;
     __syncthreads();
@@ -76,6 +77,7 @@ __global__ void __launch_bounds__(kThreads) k_row_moment(const uint8_t* __restri
                                                          const double* __restrict__ coef, int n_planes, int cols, int x0,
                                                          int bb, double min_disp, int pass, double mean,
                                                          double* __restrict__ row_out) {
+    wait_prior();
     __shared__ double sm[kThreads];
     const int y = bb + blockIdx.x;
     double s = 0.0;

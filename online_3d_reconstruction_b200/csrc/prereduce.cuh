@@ -47,6 +47,7 @@ __global__ void __launch_bounds__(kThreads, 5) k_cell_prereduce(const float4* __
                                                                 const uint32_t* __restrict__ out_base,
                                                                 uint32_t* __restrict__ chunk_total,
                                                                 uint32_t* __restrict__ status, uint32_t* __restrict__ ticket) {
+    wait_prior();
     __shared__ PrSmem S;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const unsigned lt = (1u << lane) - 1u;
@@ -194,6 +195,7 @@ __global__ void __launch_bounds__(kThreads, 5) k_cell_prereduce(const float4* __
 }
 
 __global__ void k_add_u32(uint32_t* dst, const uint32_t* src) {
+    wait_prior();
     if (threadIdx.x == 0) *dst += *src;
 }
 

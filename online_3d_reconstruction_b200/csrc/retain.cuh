@@ -25,6 +25,7 @@ enum { RT_W_BBOX = 0, RT_W_FRAMES = 6, RT_W_CYCLES = 7, RT_W_ERR = 8, RT_W_WRAP 
 // minimum corner travels complemented, so one max-reduction yields min and max of the order-preserving encoding
 __global__ void k_rt_agree_pack(const uint32_t* __restrict__ bbox, uint32_t n_frames, uint32_t n_cycles, uint32_t err,
                                 uint32_t* __restrict__ w) {
+    wait_prior();
     const int t = threadIdx.x;
     if (t < 3) w[RT_W_BBOX + t] = ~bbox[t];
     else if (t < 6) w[RT_W_BBOX + t] = bbox[t];
@@ -39,6 +40,7 @@ __global__ void k_rt_agree_pack(const uint32_t* __restrict__ bbox, uint32_t n_fr
 // cells, which the owner hash would keep apart.
 __global__ void k_rt_grid(uint32_t* __restrict__ w, float ix, float iy, float iz, uint32_t* __restrict__ bbox,
                           GridParams* __restrict__ grid) {
+    wait_prior();
     if (threadIdx.x != 0) return;
     uint32_t bb[6];
     for (int a = 0; a < 3; ++a) { bb[a] = ~w[RT_W_BBOX + a]; bb[3 + a] = w[RT_W_BBOX + 3 + a]; }
@@ -62,6 +64,7 @@ __global__ void __launch_bounds__(kThreads) k_rt_route(const float4* __restrict_
                                                        uint32_t n_frames, uint32_t fbits, float ix, float iy, float iz, uint32_t world,
                                                        uint32_t* __restrict__ okeys, uint32_t* __restrict__ tags,
                                                        uint32_t* __restrict__ counts) {
+    wait_prior();
     __shared__ uint32_t s_cnt[256];   // (world <= 256)
     for (uint32_t r = threadIdx.x; r < world; r += kThreads) s_cnt[r] = 0u;
     __syncthreads();
@@ -90,6 +93,7 @@ __global__ void __launch_bounds__(kThreads) k_rt_route(const float4* __restrict_
 // points in owner order (perm = the stable owner sort's values) -> the send buffer, one contiguous bucket per owner
 __global__ void __launch_bounds__(kThreads) k_rt_pack(const float4* __restrict__ pts, const uint32_t* __restrict__ tags,
                                                       const uint32_t* __restrict__ perm, uint32_t n, RtRec* __restrict__ out) {
+    wait_prior();
     for (uint32_t j = blockIdx.x * kThreads + threadIdx.x; j < n; j += gridDim.x * kThreads) {
         const uint32_t i = perm[j];
         const float4 p = pts[i];
@@ -102,6 +106,7 @@ __global__ void __launch_bounds__(kThreads) k_rt_pack(const float4* __restrict__
 // per-destination counts + a clear status word: the counts agreement of a rank whose routing succeeded (a failed rank
 // writes zero counts and a set status from the host instead)
 __global__ void k_rt_counts(const uint32_t* __restrict__ counts, uint32_t world, uint32_t* __restrict__ out) {
+    wait_prior();
     for (uint32_t d = threadIdx.x; d < world; d += blockDim.x) {
         out[2 * d] = counts[d];
         out[2 * d + 1] = 0u;
@@ -109,6 +114,7 @@ __global__ void k_rt_counts(const uint32_t* __restrict__ counts, uint32_t world,
 }
 
 __global__ void __launch_bounds__(kThreads) k_rt_tags(const RtRec* __restrict__ rec, uint32_t n, uint32_t* __restrict__ keys) {
+    wait_prior();
     for (uint32_t i = blockIdx.x * kThreads + threadIdx.x; i < n; i += gridDim.x * kThreads) keys[i] = rec[i].tag;
 }
 
@@ -116,6 +122,7 @@ __global__ void __launch_bounds__(kThreads) k_rt_tags(const RtRec* __restrict__ 
 __global__ void __launch_bounds__(kThreads) k_rt_gather(const RtRec* __restrict__ rec, uint32_t n, const SortPlan* __restrict__ plan,
                                                         const uint32_t* __restrict__ v0, const uint32_t* __restrict__ v1,
                                                         float4* __restrict__ out) {
+    wait_prior();
     const bool ident = plan->n_active == 0;
     const uint32_t* perm = plan->final_parity ? v1 : v0;
     for (uint32_t i = blockIdx.x * kThreads + threadIdx.x; i < n; i += gridDim.x * kThreads) {

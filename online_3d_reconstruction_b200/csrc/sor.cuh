@@ -41,6 +41,7 @@ struct SorGrid {
 // Also fills the GridParams fields the radix-sort planner reads (key_bits, passthrough, empty).
 __global__ void k_sor_grid(int n_seg, const uint32_t* __restrict__ bbox, const uint32_t* __restrict__ seg_off, int mean_k,
                            SorGrid* __restrict__ grids, GridParams* __restrict__ plan_grids) {
+    wait_prior();
     const int s = blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= n_seg) return;
     const uint32_t n = seg_off[s + 1] - seg_off[s];
@@ -91,6 +92,7 @@ __device__ __forceinline__ uint32_t sor_cell(const SorGrid& G, float x, float y,
 
 __global__ void __launch_bounds__(kThreads) k_sor_key(const float4* __restrict__ pts, const uint32_t* __restrict__ seg_off,
                                                       const SorGrid* __restrict__ grids, uint32_t* __restrict__ keys) {
+    wait_prior();
     const int s = blockIdx.y;
     const uint32_t beg = seg_off[s], n = seg_off[s + 1] - beg;
     const SorGrid G = grids[s];
@@ -111,6 +113,7 @@ __global__ void __launch_bounds__(kThreads) k_sor_cells(const uint32_t* __restri
                                                         const uint32_t* __restrict__ seg_off, const SorGrid* __restrict__ grids,
                                                         uint32_t* __restrict__ cell_start, uint32_t* __restrict__ skeys,
                                                         uint32_t* __restrict__ svals, float4* __restrict__ spts) {
+    wait_prior();
     const int s = blockIdx.y;
     const uint32_t beg = seg_off[s], n = seg_off[s + 1] - beg;
     const uint32_t cells = (uint32_t)grids[s].nc[0] * (uint32_t)grids[s].nc[1] * (uint32_t)grids[s].nc[2];
@@ -273,6 +276,7 @@ __global__ void __launch_bounds__(kSorThreads) k_sor_calib(const float4* __restr
                                                            const uint32_t* __restrict__ seg_off, SorGrid* __restrict__ grids,
                                                            GridParams* __restrict__ plan_grids, const uint32_t* __restrict__ bbox,
                                                            const uint32_t* __restrict__ cell_start, int mean_k) {
+    wait_prior();
     extern __shared__ float sor_heap[];
     __shared__ float s_r[kSorThreads];
     __shared__ float s_r90;
@@ -332,6 +336,7 @@ __global__ void __launch_bounds__(kSorThreads) k_sor_knn(const float4* __restric
                                                          const SorGrid* __restrict__ grids, const uint32_t* __restrict__ cell_start, int mean_k,
                                                          float* __restrict__ dist, uint2* __restrict__ hard,
                                                          uint32_t* __restrict__ n_hard) {
+    wait_prior();
     extern __shared__ float sor_heap[];
     const int s = blockIdx.y;
     const uint32_t beg = seg_off[s], n = seg_off[s + 1] - beg;
@@ -360,6 +365,7 @@ __global__ void __launch_bounds__(kSorThreads) k_sor_knn_hard(const float4* __re
                                                               const uint32_t* __restrict__ cell_start, int mean_k,
                                                               float* __restrict__ dist, const uint2* __restrict__ hard,
                                                               const uint32_t* __restrict__ n_hard) {
+    wait_prior();
     extern __shared__ float sor_heap[];
     const uint32_t i = blockIdx.x * kSorThreads + threadIdx.x;
     if (i >= *n_hard) return;
@@ -381,6 +387,7 @@ __global__ void __launch_bounds__(kSorThreads) k_sor_knn_hard(const float4* __re
 // per frame: mean / stddev of the distances -> removal threshold (double).  One CTA per frame, fixed-order tree.
 __global__ void __launch_bounds__(kThreads) k_sor_stats(const float* __restrict__ dist, const uint32_t* __restrict__ seg_off,
                                                         double stddev_mul, double* __restrict__ threshold) {
+    wait_prior();
     __shared__ double s_sum[kThreads], s_sq[kThreads];
     const int s = blockIdx.x;
     const uint32_t beg = seg_off[s], n = seg_off[s + 1] - beg;
@@ -411,6 +418,7 @@ __global__ void __launch_bounds__(kThreads) k_sor_stats(const float* __restrict_
 __global__ void __launch_bounds__(kThreads) k_sor_count(const float* __restrict__ dist, const uint32_t* __restrict__ seg_off,
                                                         const double* __restrict__ threshold, uint32_t tiles_ub,
                                                         uint32_t* __restrict__ tile_cnt) {
+    wait_prior();
     __shared__ uint32_t s_c;
     const int s = blockIdx.y;
     const uint32_t beg = seg_off[s], n = seg_off[s + 1] - beg;
@@ -434,6 +442,7 @@ __global__ void __launch_bounds__(kThreads) k_sor_compact(const float4* __restri
                                                           uint32_t tiles_ub, const uint32_t* __restrict__ tile_off,
                                                           const uint32_t* __restrict__ total, int n_seg,
                                                           float4* __restrict__ out, uint32_t* __restrict__ out_off) {
+    wait_prior();
     __shared__ uint32_t s_scan[34];
     const int s = blockIdx.y;
     const uint32_t beg = seg_off[s], n = seg_off[s + 1] - beg;

@@ -55,6 +55,7 @@ struct SortPlan {
 constexpr int kScanThreads = 1024;
 __global__ void __launch_bounds__(kScanThreads) k_scan_u32(const uint32_t* __restrict__ in, uint32_t* __restrict__ out,
                                                            uint32_t n, uint32_t* __restrict__ total_out) {
+    wait_prior();
     __shared__ uint32_t s_w[32];
     __shared__ uint32_t s_tot;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -106,6 +107,7 @@ __global__ void __launch_bounds__(kScanThreads) k_scan_u32(const uint32_t* __res
 // ---- digit layout: split `key_bits` live bits into the fewest passes of <= 10 bits -------------------------------
 // key_bits comes from the segment's VoxelGrid (grids[s].key_bits) or is the same for all segments (fixed_bits).
 __global__ void k_rs_layout(int n_seg, const GridParams* __restrict__ grids, int fixed_bits, SortPlan* __restrict__ plan) {
+    wait_prior();
     const int s = blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= n_seg) return;
     int kb = grids ? grids[s].key_bits : fixed_bits;
@@ -131,6 +133,7 @@ __global__ void k_rs_layout(int n_seg, const GridParams* __restrict__ grids, int
 // is what the radix pass needs: computed once here instead of once per tile.
 __global__ void __launch_bounds__(kThreads) k_rs_plan(uint32_t* __restrict__ ghist, const uint32_t* __restrict__ seg_off,
                                                       SortPlan* __restrict__ plan, const GridParams* __restrict__ grids) {
+    wait_prior();
     __shared__ int s_trivial[kMaxPasses];
     __shared__ uint32_t s_scan[34];
     const int s = blockIdx.x;
@@ -187,6 +190,7 @@ __device__ __forceinline__ void hist_add(uint32_t* sh, uint32_t d, unsigned vm, 
 template <typename KeyT, int MAXP>
 __global__ void __launch_bounds__(kThreads) k_rs_ghist(const KeyT* __restrict__ keys, const uint32_t* __restrict__ seg_off,
                                                        const SortPlan* __restrict__ plan, uint32_t* __restrict__ ghist) {
+    wait_prior();
     __shared__ uint32_t sh[MAXP * kRsBins];
     const int s = blockIdx.y;
     const uint32_t t = blockIdx.x;
@@ -265,6 +269,7 @@ __global__ void __launch_bounds__(kThreads, sizeof(KeyT) == 4 ? O3R_RS_MINB : (O
     const uint32_t* __restrict__ seg_off, const SortPlan* __restrict__ plan, int pass, uint32_t tiles_ub,
     const uint32_t* __restrict__ ghist, StT* __restrict__ status, uint32_t* __restrict__ ticket, int iota_first,
     int ghist_is_prefix) {
+    wait_prior();
     constexpr int kFlagShift = (int)sizeof(StT) * 8 - 2;
     constexpr StT kLocal = (StT)1 << kFlagShift, kGlobal = (StT)2 << kFlagShift, kCountMask = kLocal - 1;
     extern __shared__ __align__(16) unsigned char rs_smem[];

@@ -209,6 +209,7 @@ template <int DT>
 __global__ void __launch_bounds__(kThreads) k_pre(AParams P, const FrameDev* __restrict__ frames,
                                                   uint32_t* __restrict__ tile_cnt, uint32_t* __restrict__ bbox,
                                                   uint8_t* __restrict__ mask_out) {
+    wait_prior();
     __shared__ double rl[256];
     __shared__ float zl[256];
     __shared__ uint32_t s_red[8];
@@ -266,6 +267,7 @@ __global__ void k_a_post(int n_frames, int tiles_per_frame, const uint32_t* __re
                          const uint32_t* __restrict__ total, const uint32_t* __restrict__ bbox, float ix, float iy,
                          float iz, int want_grid, uint32_t* __restrict__ frame_off, GridParams* __restrict__ grids,
                          const uint32_t* __restrict__ out_base, uint32_t* __restrict__ goff) {
+    wait_prior();
     const int f = blockIdx.x * blockDim.x + threadIdx.x;
     if (f > n_frames) return;
     const uint32_t o = (f == n_frames) ? *total : tile_off[(size_t)f * tiles_per_frame];
@@ -282,6 +284,7 @@ __global__ void __launch_bounds__(kThreads) k_emit(AParams P, const FrameDev* __
                                                    const GridParams* __restrict__ grids,
                                                    float4* __restrict__ pts, uint32_t* __restrict__ keys,
                                                    const uint32_t* __restrict__ out_base) {
+    wait_prior();
     __shared__ double rl[256];
     __shared__ float zl[256];
     __shared__ uint32_t s_scan[34];

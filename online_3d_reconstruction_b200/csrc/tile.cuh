@@ -292,6 +292,7 @@ __device__ __forceinline__ uint32_t tv_block_excl_scan(uint32_t v, uint32_t* sm,
 
 template <int DT, int R>
 __global__ void __launch_bounds__(kTvThreads, tv_ctas_per_sm<R>()) k_tv(AParams P, TvArgs A) {
+    wait_prior();
     typedef TvGeom<R> G;
     typedef typename TvMask<R>::type M;
     extern __shared__ __align__(16) unsigned char tv_smem_raw[];
@@ -779,6 +780,7 @@ __global__ void __launch_bounds__(kThreads) k_tv_compact(const o3r_cell* __restr
                                                          uint32_t* __restrict__ max_cursor, uint32_t* __restrict__ flags, int n_frames,
                                                          const uint32_t* __restrict__ bbox, float inv_f,
                                                          const uint8_t* __restrict__ guess, uint8_t* __restrict__ actual) {
+    wait_prior();
     if (blockIdx.x == 0 && threadIdx.x == 0) atomicMax(max_cursor, *cursor);
     // per frame: PCL's int32 overflow guard on the exact bbox against the guess the tile kernel ran on
     if (blockIdx.x == gridDim.x - 1)

@@ -23,6 +23,7 @@ constexpr int kTileV = kThreads * 4;  // 1024 sorted elements per CTA in the run
 // (bbox arrays start as {~0, ~0, ~0, 0, 0, 0} per segment: FILL_BBOX of the host's fill queue)
 __global__ void __launch_bounds__(kThreads) k_bbox_pts(const float4* __restrict__ pts, const uint32_t* __restrict__ seg_off,
                                                        int z_shift, uint32_t* __restrict__ bbox) {
+    wait_prior();
     __shared__ uint32_t s_red[6];
     const int s = blockIdx.y;
     const uint32_t beg = seg_off[s], n = seg_off[s + 1] - beg;
@@ -58,6 +59,7 @@ __global__ void __launch_bounds__(kThreads) k_bbox_pts(const float4* __restrict_
 
 __global__ void k_grid_params(int n_seg, const uint32_t* __restrict__ bbox, float ix, float iy, float iz,
                               GridParams* __restrict__ grids) {
+    wait_prior();
     const int s = blockIdx.x * blockDim.x + threadIdx.x;
     if (s < n_seg) grids[s] = make_grid(bbox + 6 * s, ix, iy, iz);
 }
@@ -66,6 +68,7 @@ __global__ void k_grid_params(int n_seg, const uint32_t* __restrict__ bbox, floa
 __global__ void __launch_bounds__(kThreads) k_vg_key(const float4* __restrict__ pts, const uint32_t* __restrict__ seg_off,
                                                      const GridParams* __restrict__ grids, int z_shift,
                                                      uint32_t* __restrict__ keys) {
+    wait_prior();
     const int s = blockIdx.y;
     const uint32_t beg = seg_off[s], n = seg_off[s + 1] - beg;
     const GridParams G = grids[s];
@@ -100,6 +103,7 @@ __device__ __forceinline__ bool vg_emits(const uint32_t* keys, uint32_t pos, uin
 }
 
 __global__ void __launch_bounds__(kThreads) k_vg_heads(VgArgs A, uint32_t* __restrict__ head_cnt) {
+    wait_prior();
     const int s = blockIdx.y;
     const uint32_t t = blockIdx.x;
     const uint32_t beg = A.seg_off[s], n = A.seg_off[s + 1] - beg;
@@ -422,6 +426,7 @@ __global__ void __launch_bounds__(kThreads, O3R_VG_MINB) k_vg_reduce_w(VgArgs A,
                                                           float icz, int* __restrict__ cellbb,
                                                           const uint32_t* __restrict__ out_base,
                                                           uint64_t* __restrict__ out_keys, uint32_t* __restrict__ out_counts) {
+    wait_prior();
     __shared__ std::conditional_t<FULL, RunSmemRanked<uint32_t, true>, RunSmem<uint32_t, true>> S;
     __shared__ int s_bb[6];
     if (threadIdx.x == 0) S.ticket = atomicAdd(ticket, 1u);
@@ -523,6 +528,7 @@ struct AccItemsCells {  // items are partial cells received from other ranks
 // cell 0, so a non-finite item widens the range to INT_MIN instead, which the host refuses like any cell beyond +-2^20.
 template <typename Items>
 __global__ void __launch_bounds__(kThreads) k_acc_cellbb(Items items, uint32_t n, float ix, float iz, int* __restrict__ cellbb) {
+    wait_prior();
     int mn[3] = {0x7fffffff, 0x7fffffff, 0x7fffffff}, mx[3] = {(int)0x80000000, (int)0x80000000, (int)0x80000000};
     for (uint32_t v = blockIdx.x * kThreads + threadIdx.x; v < n; v += gridDim.x * kThreads) {
         int c[3];
@@ -540,6 +546,7 @@ __global__ void __launch_bounds__(kThreads) k_acc_cellbb(Items items, uint32_t n
 
 // after a chunk: advance the batch-wide output position and record it as the next frame's offset
 __global__ void k_add_base(uint32_t* base, const uint32_t* total, uint32_t* goff_end) {
+    wait_prior();
     if (threadIdx.x == 0) { *base += *total; *goff_end = *base; }
 }
 
@@ -549,11 +556,10 @@ __global__ void __launch_bounds__(kThreads) k_acc_key(Items items, uint32_t n, f
                                                       const SortPlan* __restrict__ plan, KeyT* __restrict__ keys,
                                                       uint32_t* __restrict__ vals, uint32_t* __restrict__ ghist,
                                                       const uint32_t* __restrict__ n_dev, uint32_t* __restrict__ seg_out) {
+    wait_prior();
     __shared__ uint32_t sh[kMaxPasses * kRsBins];
-    if (n_dev) {   // the item count lives on the device (n is the host's bound); publish the segment for the sort
-        n = min(n, *n_dev);
-        if (blockIdx.x == 0 && threadIdx.x == 0) { seg_out[0] = 0u; seg_out[1] = n; }
-    }
+    if (n_dev) n = min(n, *n_dev);   // the item count lives on the device (n is the host's bound)
+    if (blockIdx.x == 0 && threadIdx.x == 0) { seg_out[0] = 0u; seg_out[1] = n; }   // the segment of the sort
     const int np = plan[0].n_passes;
     for (int i = threadIdx.x; i < np * kRsBins; i += kThreads) sh[i] = 0;
     __syncthreads();
@@ -598,6 +604,7 @@ struct AccArgs {
 template <typename KeyT>
 __global__ void __launch_bounds__(kThreads) k_acc_heads(AccArgs<KeyT> A, uint32_t* __restrict__ vals0, uint32_t* __restrict__ vals1,
                                                         uint32_t* __restrict__ head_cnt, uint32_t* __restrict__ n_new) {
+    wait_prior();
     const uint32_t t = blockIdx.x;
     const uint32_t n = A.seg_off[1];
     uint32_t c = 0, fresh = 0;
@@ -673,6 +680,7 @@ __global__ void __launch_bounds__(kThreads, 5) k_acc_reduce(AccArgs<KeyT> A, Ite
                                                          uint64_t* __restrict__ ckey, float4* __restrict__ cacc,
                                                          uint4* __restrict__ crgb, uint32_t* __restrict__ ticket,
                                                          RunCarry* __restrict__ carries) {
+    wait_prior();
     __shared__ RunSmem<KeyT, Items::kPacked> S;
     if (threadIdx.x == 0) S.ticket = atomicAdd(ticket, 1u);
     __syncthreads();
@@ -692,6 +700,7 @@ __global__ void __launch_bounds__(kThreads, 5) k_acc_reduce(AccArgs<KeyT> A, Ite
 __global__ void __launch_bounds__(kThreads) k_acc_update(const uint32_t* __restrict__ n_cyc_ptr, const float4* __restrict__ cacc,
                                                          const uint4* __restrict__ crgb, float4* __restrict__ res_acc,
                                                          uint4* __restrict__ res_rgb, uint32_t* __restrict__ new_cnt) {
+    wait_prior();
     const uint32_t n_cyc = *n_cyc_ptr;
     const uint32_t t = blockIdx.x;
     uint32_t c = 0;
@@ -725,6 +734,7 @@ __global__ void __launch_bounds__(kThreads) k_acc_place_new(const uint32_t* __re
                                                             const uint32_t* __restrict__ n_res_ptr,
                                                             uint64_t* __restrict__ dst_keys, float4* __restrict__ dst_acc,
                                                             uint4* __restrict__ dst_rgb, uint64_t* __restrict__ new_keys) {
+    wait_prior();
     __shared__ uint32_t s_scan[34];
     const uint32_t n_cyc = *n_cyc_ptr, n_res = *n_res_ptr;
     const uint32_t t = blockIdx.x;
@@ -765,6 +775,7 @@ __global__ void __launch_bounds__(kThreads) k_acc_place_old(const uint32_t* __re
                                                             const uint32_t* __restrict__ n_new_ptr,
                                                             uint64_t* __restrict__ dst_keys, float4* __restrict__ dst_acc,
                                                             uint4* __restrict__ dst_rgb) {
+    wait_prior();
     const uint32_t n_res = *n_res_ptr, n_new = *n_new_ptr;
     for (uint32_t i = blockIdx.x * kThreads + threadIdx.x; i < n_res; i += gridDim.x * kThreads) {
         const uint64_t k = res_keys[i];
@@ -782,6 +793,7 @@ __global__ void __launch_bounds__(kThreads) k_acc_place_old(const uint32_t* __re
 
 // the merged shard now holds n_res + n_new cells
 __global__ void k_acc_finish(uint32_t* n_res, const uint32_t* n_new) {
+    wait_prior();
     if (threadIdx.x == 0) *n_res += *n_new;
 }
 
@@ -789,6 +801,7 @@ __global__ void k_acc_finish(uint32_t* n_res, const uint32_t* n_new) {
 // (launched over an upper bound of the resident cell count; the exact count is read from the device)
 __global__ void __launch_bounds__(kThreads) k_acc_emit_cnt(const uint32_t* __restrict__ n_res_ptr, const float4* __restrict__ res_acc,
                                                            uint32_t min_points, uint32_t* __restrict__ cnt) {
+    wait_prior();
     const uint32_t n_res = *n_res_ptr;
     const uint32_t t = blockIdx.x;
     uint32_t c = 0;
@@ -818,6 +831,7 @@ __device__ __forceinline__ float4 acc_centroid(const float4 a, const uint4 c) {
 __global__ void __launch_bounds__(kThreads) k_acc_emit(const uint32_t* __restrict__ n_res_ptr, const float4* __restrict__ res_acc,
                                                        const uint4* __restrict__ res_rgb, uint32_t min_points,
                                                        const uint32_t* __restrict__ off, float4* __restrict__ out) {
+    wait_prior();
     __shared__ uint32_t s_scan[34];
     const uint32_t n_res = *n_res_ptr;
     const uint32_t t = blockIdx.x;
@@ -850,6 +864,7 @@ __host__ __device__ __forceinline__ uint64_t hash64(uint64_t x) {  // splitmix64
 __global__ void __launch_bounds__(kThreads) k_owner(const uint32_t* __restrict__ n_cyc_ptr, const uint64_t* __restrict__ ckey,
                                                     uint32_t world, uint32_t* __restrict__ okeys, uint32_t* __restrict__ ovals,
                                                     uint32_t* __restrict__ counts, uint32_t* __restrict__ seg) {
+    wait_prior();
     __shared__ uint32_t s_cnt[256];   // (world <= 256) the CTA's histogram: one global atomic per owner and CTA, not per cell
     const uint32_t n_cyc = *n_cyc_ptr;
     if (blockIdx.x == 0 && threadIdx.x == 0) { seg[0] = 0u; seg[1] = n_cyc; }
@@ -873,6 +888,7 @@ __global__ void __launch_bounds__(kThreads) k_owner(const uint32_t* __restrict__
 
 // rigid transform of a resident point cloud in place (pose.cpp:353)
 __global__ void __launch_bounds__(kThreads) k_transform_pts(float4* __restrict__ pts, size_t n, const float* __restrict__ Tm) {
+    wait_prior();
     __shared__ float T[12];
     if (threadIdx.x < 12) T[threadIdx.x] = Tm[threadIdx.x];
     __syncthreads();
