@@ -58,6 +58,7 @@ struct Pose {
     string imagePrefix = "images/", disparityPrefix = "disparities/", segmentlblPrefix = "segmentlabels/";
     string folder = "output/", pose_corrections_file;
     bool save_map = false;      // --save_map: <run dir>/map.o3rmap after the last cycle
+    bool register_map = false;  // --register_map: from the second cycle on, correct the drift against the map
     string resume_map_file;     // --resume_map FILE: loaded before the first cycle
     int blur_mode = O3R_BLUR_BILATERAL, device = 0;   // the reference's live filter (pose_functions.cpp:1044)
     double Q[16] = {0};
@@ -90,6 +91,9 @@ void Pose::printUsage() {
             "  extensions: --blur_mode bilateral|median|box (default bilateral = the reference) --pose_corrections FILE --device N\n"
             "              --no_sor (skip the StatisticalOutlierRemoval the reference applies per frame when jump_pixels > 0)\n"
             "              --save_map (write the resident map to <run dir>/map.o3rmap after the last cycle)\n"
+            "              --register_map (from the second cycle on, register the cycle's first, middle and last frame clouds\n"
+            "                against the map, gate max(3 voxel_size, 1 m), and premultiply the running correction into every\n"
+            "                later frame's matrix)\n"
             "              --resume_map FILE (continue the map of a map.o3rmap saved with the same --voxel_size and --dont_downsample)\n"
             "  not in this driver (host-side tools of the reference): --visualize --align_point_cloud --smooth_surface\n"
             "      --mesh_surface --segment_cloud --segment_cloud_only --displayUAVPositions\n";
@@ -127,6 +131,7 @@ int Pose::parseCmdArgs(int argc, char** argv) {
         else if (a == "--range_width") { range_width = atoi(need("n")); cout << "range_width " << range_width << endl; }
         else if (a == "--log") { log_stuff = atoi(need("0/1")) != 0; cout << "log " << log_stuff << endl; }
         else if (a == "--preview") preview = true;
+        else if (a == "--register_map") register_map = true;
         else if (a == "--use_segment_labels") { cout << "use_segment_labels" << endl; use_segment_labels = true; }
         else if (a == "--only_MAVLink") { only_MAVLink = true; cout << "only_MAVLink " << endl; }
         else if (a == "--dont_downsample") { dont_downsample = true; cout << "dont_downsample " << endl; }
@@ -375,6 +380,12 @@ int Pose::run() {
     vector<uint64_t> chg_keys;
     vector<o3r_point> hexPos_MAVLink, hexPos_FM;
     vector<int> accepted_nums;
+    // --register_map: the running drift correction (what the reference's ICP block multiplies into the later frames,
+    // pose.cpp:318-319), and the staging of the clouds it registers
+    Mat4 drift = host::mat4_identity();
+    vector<o3r_point> reg_pts, frame_pts((size_t)rows * cols);
+    if (register_map && dont_downsample)
+        cout << "--register_map needs the combined grid, which --dont_downsample skips: no registration" << endl;
     int current_idx = 0, cycle = 0;
     const int last_idx = (int)rawImageDataVec.size() - 1;
     size_t accepted = 0;
@@ -399,6 +410,7 @@ int Pose::run() {
             Mat4 t = host::generate_tmat(r.tx, r.ty, r.tz, r.qx, r.qy, r.qz, r.qw);   // :198
             auto c = corrections.find(r.img_num);
             if (c != corrections.end()) t = host::mat4_mul(c->second, t);               // :232
+            if (register_map) t = host::mat4_mul(drift, t);                             // :318-319
             o3r_frame f{};
             if (use_segment_labels) {   // createPlaneFittedDisparityImages (pose_functions.cpp:900-985) on the GPU
                 if (r.segment_label.empty()) { cout << r.img_num << " could not read segment labels. \tRejected!" << endl; log_file << r.img_num << " could not read segment labels. \tRejected!" << endl; current_idx++; continue; }
@@ -434,6 +446,40 @@ int Pose::run() {
             accepted_nums.push_back(r.img_num);
             cout << "\tAccepted!" << endl;
             current_idx++; images_in_cycle++;
+        }
+        if (register_map && !dont_downsample && cycle > 0 && !batch.empty()) {
+            // the cycle's first, middle and last frames as the library makes their clouds, registered against the map
+            const int disp_type = use_segment_labels ? O3R_DISP_F64 : O3R_DISP_U8;
+            const size_t nb = batch.size();
+            reg_pts.clear();
+            vector<size_t> pick{0};
+            if (nb / 2 != pick.back()) pick.push_back(nb / 2);
+            if (nb - 1 != pick.back()) pick.push_back(nb - 1);
+            for (size_t i : pick) {
+                size_t m = 0;
+                if (o3r_frame_cloud(ctx, &batch[i], disp_type, frame_pts.data(), frame_pts.size(), &m) != O3R_OK) {
+                    cerr << "o3r_frame_cloud: " << o3r_last_error(ctx) << endl; o3r_destroy(ctx); return 1;
+                }
+                reg_pts.insert(reg_pts.end(), frame_pts.begin(), frame_pts.begin() + m);
+            }
+            const Mat4 I = host::mat4_identity();
+            Mat4 T;
+            o3r_register_stats st{};
+            o3r_register_params rp{20, std::max(3.0 * voxel_size, 1.0), 1e-5, 1e-4, 1e-3};   // a cycle may drift more than 3 voxels
+            if (o3r_cloud_register(ctx, reg_pts.data(), reg_pts.size(), I.m, &rp, T.m, &st) != O3R_OK) {
+                cerr << "o3r_cloud_register: " << o3r_last_error(ctx) << endl; o3r_destroy(ctx); return 1;
+            }
+            drift = host::mat4_mul(T, drift);
+            for (auto& f : batch) {
+                Mat4 ft;
+                memcpy(ft.m, f.T, sizeof(ft.m));
+                ft = host::mat4_mul(T, ft);
+                memcpy(f.T, ft.m, sizeof(f.T));
+            }
+            char line[256];
+            snprintf(line, sizeof(line), "Map registration: %u/%zu, rms %.4f -> %.4f, rank %u, t = (%.4f, %.4f, %.4f)", st.n_inliers,
+                     reg_pts.size(), st.rms_initial, st.rms_final, st.rank, T.m[3], T.m[7], T.m[11]);
+            for (ostream* o : {(ostream*)&cout, (ostream*)&log_file}) *o << line << endl;
         }
         const double t2 = now_s();
         cout << "\nMatching features and finding transformations time: " << (t2 - t0) << " sec" << endl;

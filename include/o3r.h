@@ -300,6 +300,55 @@ int o3r_cloud_export_cells(o3r_ctx* ctx, o3r_cell* out, size_t cap, size_t* n_ou
 int o3r_cloud_import_cells(o3r_ctx* ctx, const o3r_cell* cells, size_t n);
 int o3r_cloud_export_points(o3r_ctx* ctx, o3r_point* out, size_t cap, size_t* n_out);
 
+/* Registration of a cloud against the resident map (O3R_MERGE_ACCUMULATE, _TILED, _FUSED; one GPU): the drift correction
+ * that stands in for the reference's per-cycle ICP block (pose.cpp:267-320).  Deterministic point-to-plane Gauss-Newton.
+ *   - Result.  T_out is the rigid transform T, starting from T_init, such that T * p lies on the map.  T_init is row-major
+ *     with last row 0 0 0 1.  To correct a frame, premultiply the frame's T by T_out.
+ *   - The map.  The cells o3r_cloud_downsample would emit (count >= min_points_per_voxel), each at its output centroid c.
+ *   - Correspondence.  A transformed source point p' falls into the combined-grid cell the merge would bin it in (so a point
+ *     equal to a map point lands in that point's cell).  It has a correspondence when that cell is in the map, a normal
+ *     exists for it and |r| <= max_distance.
+ *   - Normal.  The least-squares plane z - z0 = a (x - x0) + b (y - y0) + d, in double, over the centroids of the hit cell
+ *     (x0, y0, z0) and of its 8 horizontal neighbours at the same k that are in the map; it needs at least 3 cells and a
+ *     well-conditioned 3 x 3 system (det > 1e-3 * Suu * Sww * S1), otherwise there is no normal.  n = (-a, -b, 1) / |.|,
+ *     r = n . (p' - c) with c the hit cell's centroid.
+ *   - Solve.  The rotation is linearised about a pivot: the centroid of the source points under T_init, fixed for the call
+ *     (stats->pivot).  The 6 x 6 normal equations (order wx, wy, wz, tx, ty, tz) are solved by a symmetric eigen-decomposition;
+ *     directions whose eigenvalue is below degenerate_ratio * the largest are not updated (on flat ground x, y and yaw cannot
+ *     be observed: rank 3).  The rotation update is an axis-angle (Rodrigues), composed in double.
+ *   - Stop after max_iterations, or when one update rotates less than min_rotation AND translates less than min_translation
+ *     (converged = 1; that update is applied).  An iteration with fewer than 6 correspondences ends the call with O3R_OK,
+ *     T_out = T_init and rank 0.
+ *   - stats (may be NULL): iterations = updates applied; n_inliers, rms_final and info (J^T J) are those of the last
+ *     linearisation, rms_initial that of the first (RMS of the inliers' r; 0 without inliers).
+ *   - Reproducible: the same inputs (map included) give the same T_out and stats bit for bit; every sum is taken in a fixed
+ *     order.  All iterations are queued at once; the call synchronises once, at the end.
+ *   - No side effects: the resident map, the change-tracking pending set, the last batch and the prefetch state are left as
+ *     they were.  Host points are staged in a buffer of the call's own; _dev takes device points on ctx's device.
+ *   - O3R_ERR_INVALID: a non-finite point, a T_init that is not rigid, or parameters out of range (max_iterations >= 1,
+ *     max_distance > 0, min_rotation / min_translation >= 0, 0 <= degenerate_ratio <= 1); checked before any result is
+ *     formed, nothing else happens.  O3R_ERR_UNSUPPORTED: O3R_MERGE_RETAIN, dont_downsample, or a communicator attached. */
+typedef struct o3r_register_params {
+    int    max_iterations;     /* Gauss-Newton iterations, >= 1                              (default 20)               */
+    double max_distance;       /* correspondence gate |r| in metres, > 0                      (default 3 * voxel_size)   */
+    double min_rotation;       /* stop when an update rotates less than this, radians         (default 1e-5)             */
+    double min_translation;    /* ... and translates less than this, metres                   (default 1e-4)             */
+    double degenerate_ratio;   /* directions with eigenvalue < ratio * max are not updated    (default 1e-3)             */
+} o3r_register_params;         /* NULL = defaults */
+
+typedef struct o3r_register_stats {
+    uint32_t iterations, converged, rank;   /* rank = directions that were updated (0..6)                               */
+    uint32_t n_inliers;                     /* correspondences of the last iteration                                    */
+    double   rms_initial, rms_final;        /* RMS point-to-plane residual of the inliers, first / last                 */
+    double   pivot[3];                      /* the point the rotation is linearised about                               */
+    double   info[36];                      /* J^T J of the last iteration, order (wx, wy, wz, tx, ty, tz)              */
+} o3r_register_stats;
+
+int o3r_cloud_register(o3r_ctx* ctx, const o3r_point* pts, size_t n, const float T_init[16],
+                       const o3r_register_params* params, float T_out[16], o3r_register_stats* stats);
+int o3r_cloud_register_dev(o3r_ctx* ctx, const o3r_point* dev_pts, size_t n, const float T_init[16],
+                           const o3r_register_params* params, float T_out[16], o3r_register_stats* stats);
+
 /* ---- stand-alone stages (parity probes; same kernels as above) ------------------------------- */
 
 /* pcl::VoxelGrid<PointXYZRGB>::filter on a host cloud: leaf (lx,ly,lz) as PCL's setLeafSize floats,

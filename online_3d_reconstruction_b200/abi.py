@@ -71,6 +71,38 @@ Q_CAM13 = (1.0, 0.0, 0.0, -5.2425751876831055e+02,
            0.0, 0.0, 1.6853548938735339e+00, 0.0)
 
 
+class RegisterParams(C.Structure):
+    """o3r_register_params: Gauss-Newton limits of o3r_cloud_register."""
+    _fields_ = [
+        ("max_iterations", C.c_int),
+        ("max_distance", C.c_double),
+        ("min_rotation", C.c_double),
+        ("min_translation", C.c_double),
+        ("degenerate_ratio", C.c_double),
+    ]
+
+
+class RegisterStats(C.Structure):
+    """o3r_register_stats: what o3r_cloud_register reports besides T_out."""
+    _fields_ = [
+        ("iterations", C.c_uint32), ("converged", C.c_uint32), ("rank", C.c_uint32),
+        ("n_inliers", C.c_uint32),
+        ("rms_initial", C.c_double), ("rms_final", C.c_double),
+        ("pivot", C.c_double * 3),
+        ("info", C.c_double * 36),
+    ]
+
+
+def make_register_params(voxel_size, *, max_iterations=20, max_distance=None, min_rotation=1e-5, min_translation=1e-4,
+                         degenerate_ratio=1e-3):
+    """The library's defaults (max_distance = 3 * voxel_size)."""
+    r = RegisterParams()
+    r.max_iterations = max_iterations
+    r.max_distance = 3.0 * voxel_size if max_distance is None else max_distance
+    r.min_rotation, r.min_translation, r.degenerate_ratio = min_rotation, min_translation, degenerate_ratio
+    return r
+
+
 def make_params(rows=720, cols=1280, *, jump_pixels=10, voxel_size=0.1, min_points_per_voxel=1,
                 blur_kernel=1, blur_mode=BLUR_MEDIAN, dont_downsample=False, use_segment_labels=False,
                 Q=Q_CAM13, min_disparity=64.0, bounding_box=20, cutout_ratio=8, disp_divisor=200.0,

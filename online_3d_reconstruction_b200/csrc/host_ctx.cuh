@@ -250,6 +250,14 @@ struct SorScratch { DevBuf hard, pts, off, dist, grids, pgrids, rows, thr, skeys
 // bilateral LUTs (colour weights, space weights, per-row tap extents) of `kernel`, cached by bilateral_lut
 struct Blur { DevBuf disp, out, jobs, lut; int kernel = -1, radius = 0, maxk = 0; };
 
+// Registration against the resident map (host_register.cuh): the staged host points, the CTA partial sums, the iteration
+// state on the device and its pinned read-back
+struct Registration {
+    DevBuf pts, part, state;
+    void* h_state = nullptr;
+    ~Registration() { if (h_state) cudaFreeHost(h_state); }
+};
+
 // The pre-pass (o3r_disp_variance / o3r_plane_fit in o3r_api.cu): plane fit / variance gate scratch
 struct PrePass { DevBuf labels, disp, sums, rows, coef; };
 
@@ -305,6 +313,7 @@ struct o3r_ctx {
     SorScratch sor;
     Blur blur;
     PrePass pp;
+    Registration reg;
     Profiling prof;
 
     // Shared per-call scratch: sized on demand and used by several paths within one call.  It holds nothing a later call

@@ -9,6 +9,7 @@
 #include "host_retain.cuh"
 #include "host_changes.cuh"
 #include "host_checkpoint.cuh"
+#include "host_register.cuh"
 
 
 // =====================================================================================================================
@@ -511,6 +512,18 @@ int o3r_cloud_export_points(o3r_ctx* ctx, o3r_point* out, size_t cap, size_t* n_
         *n_out = 0;
         return export_points_impl(ctx, out, cap, n_out);
     });
+}
+
+int o3r_cloud_register(o3r_ctx* ctx, const o3r_point* pts, size_t n, const float T_init[16], const o3r_register_params* params,
+                       float T_out[16], o3r_register_stats* stats) {
+    if ((n && !pts) || !T_init || !T_out) return O3R_ERR_INVALID;
+    return api(ctx, [&] { return register_impl(ctx, pts, true, n, T_init, params, T_out, stats); });
+}
+
+int o3r_cloud_register_dev(o3r_ctx* ctx, const o3r_point* dev_pts, size_t n, const float T_init[16],
+                           const o3r_register_params* params, float T_out[16], o3r_register_stats* stats) {
+    if ((n && !dev_pts) || !T_init || !T_out) return O3R_ERR_INVALID;
+    return api(ctx, [&] { return register_impl(ctx, dev_pts, false, n, T_init, params, T_out, stats); });
 }
 
 int o3r_voxel_grid(o3r_ctx* ctx, const o3r_point* pts, size_t n, float lx, float ly, float lz, unsigned min_points,

@@ -485,6 +485,13 @@ struct KeyCodec {
     }
 };
 
+// the combined-grid cell of a point: leaf (v, v, 1000) over z + 500 (ix = 1 / v, iz = 1 / 1000 as floats).  The merge bins
+// points with it and o3r_cloud_register looks them up with it, so a point equal to a map point lands in that point's cell.
+__device__ __forceinline__ void combined_cell(float x, float y, float z, float ix, float iz, int& i, int& j, int& k) {
+    i = (int)floorf(__fmul_rn(x, ix)); j = (int)floorf(__fmul_rn(y, ix));
+    k = (int)floorf(__fmul_rn(__fadd_rn(z, 500.0f), iz));
+}
+
 struct AccItemsPts {   // items are points of weight 1 (z gets +500)
     const float4* pts;
     const float4* spts;    // the points themselves when nothing had to be sorted (already in order), else null
@@ -497,8 +504,7 @@ struct AccItemsPts {   // items are points of weight 1 (z gets +500)
     }
     __device__ __forceinline__ void cell(uint32_t v, float ix, float iz, int& i, int& j, int& k) const {
         const float4 p = pts[v];
-        i = (int)floorf(__fmul_rn(p.x, ix)); j = (int)floorf(__fmul_rn(p.y, ix));
-        k = (int)floorf(__fmul_rn(__fadd_rn(p.z, 500.0f), iz));
+        combined_cell(p.x, p.y, p.z, ix, iz, i, j, k);
     }
     __device__ __forceinline__ bool finite(uint32_t v) const {
         const float4 p = pts[v];

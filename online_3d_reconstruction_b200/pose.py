@@ -230,6 +230,27 @@ class Pose:
         self._check(self._L.o3r_cloud_export_points(self._h, out.ctypes.data, out.size, C.byref(n)))
         return out[:n.value]
 
+    def registerCloud(self, pts, T_init=None, device_pointer=None, **params):
+        """o3r_cloud_register: the rigid T (starting from T_init, identity by default) such that T * p lies on the resident
+        map (accumulate modes) -> (T_out float32 4x4, stats dict).  params: max_iterations, max_distance, min_rotation,
+        min_translation, degenerate_ratio (abi.make_register_params defaults).  device_pointer=(ptr, n) registers device
+        points through o3r_cloud_register_dev instead of the host array `pts`."""
+        rp = abi.make_register_params(self.params.voxel_size, **params)
+        T0 = np.eye(4, dtype=np.float32) if T_init is None else np.asarray(T_init, dtype=np.float32).reshape(4, 4)
+        Tin = (C.c_float * 16)(*T0.reshape(16))
+        Tout = (C.c_float * 16)()
+        st = abi.RegisterStats()
+        if device_pointer is not None:
+            ptr, n = device_pointer
+            self._check(self._L.o3r_cloud_register_dev(self._h, ptr, n, Tin, C.byref(rp), Tout, C.byref(st)))
+        else:
+            pts = np.ascontiguousarray(pts, dtype=abi.POINT)
+            self._check(self._L.o3r_cloud_register(self._h, pts.ctypes.data, pts.size, Tin, C.byref(rp), Tout, C.byref(st)))
+        stats = dict(iterations=st.iterations, converged=st.converged, rank=st.rank, n_inliers=st.n_inliers,
+                     rms_initial=st.rms_initial, rms_final=st.rms_final, pivot=np.array(st.pivot[:]),
+                     info=np.array(st.info[:]).reshape(6, 6))
+        return np.array(Tout[:], dtype=np.float32).reshape(4, 4), stats
+
     # -- stand-alone stages --------------------------------------------------------------------------------
     def voxelGrid(self, pts, leaf, min_points=0):
         """pcl::VoxelGrid on a host cloud -> (points, keys u64, counts u32, passthrough)."""
