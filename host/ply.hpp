@@ -46,6 +46,37 @@ inline bool save_ply_binary(const std::string& path, const o3r_point* pts, size_
     return ok;
 }
 
+// a triangle mesh (o3r_cloud_mesh): binary little endian, vertex = x y z nx ny nz (floats) + red green blue (uchars),
+// 27 bytes; face = a uchar count (3) and three int vertex indices, 13 bytes
+inline bool save_mesh_ply(const std::string& path, const o3r_point* pts, const float* normals, size_t n, const uint32_t* tris,
+                          size_t m) {
+    FILE* f = fopen(path.c_str(), "wb");
+    if (!f) return false;
+    fprintf(f,
+            "ply\nformat binary_little_endian 1.0\nelement vertex %zu\n"
+            "property float x\nproperty float y\nproperty float z\n"
+            "property float nx\nproperty float ny\nproperty float nz\n"
+            "property uchar red\nproperty uchar green\nproperty uchar blue\n"
+            "element face %zu\nproperty list uchar int vertex_indices\nend_header\n",
+            n, m);
+    std::vector<uint8_t> rec(n * 27);
+    for (size_t i = 0; i < n; ++i) {
+        uint8_t* r = &rec[i * 27];
+        memcpy(r, &pts[i].x, 12);
+        memcpy(r + 12, normals + i * 3, 12);
+        r[24] = (pts[i].rgb >> 16) & 255; r[25] = (pts[i].rgb >> 8) & 255; r[26] = pts[i].rgb & 255;
+    }
+    bool ok = rec.empty() || fwrite(rec.data(), 1, rec.size(), f) == rec.size();
+    std::vector<uint8_t> face(m * 13);
+    for (size_t t = 0; t < m; ++t) {
+        uint8_t* r = &face[t * 13];
+        r[0] = 3;
+        memcpy(r + 1, tris + t * 3, 12);   // indices < 2^31: the int and uint32 bits agree
+    }
+    ok = ok && (face.empty() || fwrite(face.data(), 1, face.size(), f) == face.size());
+    return fclose(f) == 0 && ok;
+}
+
 // reads the vertex element of a PLY written by PCL (binary_little_endian, x y z [+ red green blue])
 inline bool read_ply(const std::string& path, std::vector<o3r_point>& out) {
     out.clear();

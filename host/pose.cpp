@@ -59,6 +59,8 @@ struct Pose {
     string folder = "output/", pose_corrections_file;
     bool save_map = false;      // --save_map: <run dir>/map.o3rmap after the last cycle
     bool register_map = false;  // --register_map: from the second cycle on, correct the drift against the map
+    bool save_mesh = false;     // --save_mesh: <run dir>/mesh.ply after the last cycle
+    double mesh_max_step = HUGE_VAL;   // --mesh_max_step M: drop mesh triangles whose |dz| exceeds M (default: keep all)
     string resume_map_file;     // --resume_map FILE: loaded before the first cycle
     int blur_mode = O3R_BLUR_BILATERAL, device = 0;   // the reference's live filter (pose_functions.cpp:1044)
     double Q[16] = {0};
@@ -95,6 +97,8 @@ void Pose::printUsage() {
             "                against the map, gate max(3 voxel_size, 1 m), and premultiply the running correction into every\n"
             "                later frame's matrix)\n"
             "              --resume_map FILE (continue the map of a map.o3rmap saved with the same --voxel_size and --dont_downsample)\n"
+            "              --save_mesh (write the map's height field as a triangle mesh to <run dir>/mesh.ply after the last cycle)\n"
+            "              --mesh_max_step M (with --save_mesh: drop triangles whose largest |dz| exceeds M metres; default none)\n"
             "  not in this driver (host-side tools of the reference): --visualize --align_point_cloud --smooth_surface\n"
             "      --mesh_surface --segment_cloud --segment_cloud_only --displayUAVPositions\n";
 }
@@ -146,6 +150,11 @@ int Pose::parseCmdArgs(int argc, char** argv) {
         else if (a == "--device") device = atoi(need("n"));
         else if (a == "--no_sor") sor = false;
         else if (a == "--save_map") save_map = true;
+        else if (a == "--save_mesh") save_mesh = true;
+        else if (a == "--mesh_max_step") {
+            mesh_max_step = atof(need("m"));
+            if (!(mesh_max_step >= 0)) throw "Exception: --mesh_max_step must be >= 0!";
+        }
         else if (a == "--resume_map") resume_map_file = need("file");
         else if (a == "--blur_mode") { const string m = need("mode"); blur_mode = (m == "box") ? O3R_BLUR_BOX : (m == "median") ? O3R_BLUR_MEDIAN : O3R_BLUR_BILATERAL; }
         else {
@@ -386,6 +395,8 @@ int Pose::run() {
     vector<o3r_point> reg_pts, frame_pts((size_t)rows * cols);
     if (register_map && dont_downsample)
         cout << "--register_map needs the combined grid, which --dont_downsample skips: no registration" << endl;
+    if (save_mesh && dont_downsample)
+        cout << "--save_mesh needs the combined grid, which --dont_downsample skips: no mesh.ply is written" << endl;
     int current_idx = 0, cycle = 0;
     const int last_idx = (int)rawImageDataVec.size() - 1;
     size_t accepted = 0;
@@ -549,6 +560,20 @@ int Pose::run() {
     string path = folder + "cloud.ply";
     host::save_ply_binary(path, cloud_small.data(), n);
     cerr << "Saved Point Cloud with " << n << " data points to " << path << endl;
+    if (save_mesh && !dont_downsample) {   // the map's height field; its vertices are cloud.ply's points, in the same order
+        size_t nv = 0, nt = 0;
+        rc = o3r_cloud_mesh(ctx, mesh_max_step, nullptr, nullptr, 0, &nv, nullptr, 0, &nt);
+        vector<o3r_point> verts(nv);
+        vector<float> normals(nv * 3);
+        vector<uint32_t> tris(nt * 3);
+        if (!rc) rc = o3r_cloud_mesh(ctx, mesh_max_step, verts.data(), normals.data(), nv, &nv, tris.data(), nt, &nt);
+        if (rc) { cerr << "--save_mesh: " << o3r_last_error(ctx) << endl; o3r_destroy(ctx); return 1; }
+        path = folder + "mesh.ply";
+        if (!host::save_mesh_ply(path, verts.data(), normals.data(), nv, tris.data(), nt)) {
+            cerr << "--save_mesh: cannot write " << path << endl; o3r_destroy(ctx); return 1;
+        }
+        cerr << "Saved mesh with " << nv << " vertices and " << nt << " triangles to " << path << endl;
+    }
     hexPos_FM.insert(hexPos_FM.end(), hexPos_MAVLink.begin(), hexPos_MAVLink.end());   // pose.cpp:553
     path = folder + "cloud_uavpos.ply";
     host::save_ply_binary(path, hexPos_FM.data(), hexPos_FM.size());

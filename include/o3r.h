@@ -349,6 +349,43 @@ int o3r_cloud_register(o3r_ctx* ctx, const o3r_point* pts, size_t n, const float
 int o3r_cloud_register_dev(o3r_ctx* ctx, const o3r_point* dev_pts, size_t n, const float T_init[16],
                            const o3r_register_params* params, float T_out[16], o3r_register_stats* stats);
 
+/* Triangle mesh of the resident map (O3R_MERGE_ACCUMULATE, _TILED, _FUSED; one GPU).  The combined grid's leaf is
+ * (v, v, 1000) over z + 500, so the map is a height field: one centroid per (i, j) column and k, and every cell is connected
+ * to its grid neighbours.  This stands in for the reference's --mesh_surface (meshSurface, pose_functions.cpp:1747: PCL's
+ * greedy projection triangulation of an arbitrary cloud); it is not a port of it.
+ *   - Vertices.  Exactly o3r_cloud_downsample's output, the same records in the same order, bit for bit, so cloud.ply and
+ *     the mesh share one vertex list.  Cells below min_points_per_voxel are not vertices.  A vertex no triangle uses is still
+ *     listed.
+ *   - Quads.  Cells A = (i, j), B = (i+1, j), C = (i, j+1), D = (i+1, j+1) at the same k; only vertices count, and
+ *     neighbours beyond +-(2^20 - 1) do not exist.  With all four, the quad is split along the diagonal with the smaller
+ *     float32 |dz|: A-D when |zA - zD| <= |zB - zC|, giving (A, B, D), (A, D, C); else B-C, giving (A, B, C), (B, D, C).
+ *     With exactly three, one triangle: A missing (B, D, C); B missing (A, D, C); C missing (A, B, D); D missing (A, B, C).
+ *     Every triangle winds counter-clockwise in (i, j): its normal points up.
+ *   - Gate.  A triangle is kept iff the largest float32 |dz| over its three vertex pairs, as a double, is <= max_step
+ *     (INFINITY: no gate).  It cuts the walls that would otherwise hang from roofs and tree crowns.
+ *   - Order.  Ascending key of the quad's A corner, then the order above.  tris holds 3 vertex indices per triangle.
+ *   - Normals (optional, 3 floats per vertex).  n = (-a, -b, 1) / |.| of o3r_cloud_register's plane fit at that cell (the
+ *     cell and its 8 same-k neighbours that are vertices, the same arithmetic); (0, 0, 0) without a fit: fewer than 3
+ *     cells, a singular system, or |i| or |j| = 2^20 - 1.
+ *   - Query, then fill, as o3r_cloud_downsample: all three outputs NULL with vcap = tcap = 0 reports *n_verts and *n_tris;
+ *     a vcap or tcap short of them returns O3R_ERR_CAPACITY with both counts set.  Any output may be NULL in a fill; it is
+ *     then not written.  Every call recomputes the mesh and synchronises once.
+ *   - o3r_cloud_mesh_dev: the result stays in device buffers owned by the context, valid until the next call on it; any of
+ *     the three pointers may be NULL.
+ *   - No side effects: the resident map, the change-tracking pending set, the last batch and the prefetch state are left as
+ *     they were.
+ *   - O3R_ERR_INVALID: max_step negative or NaN.  O3R_ERR_UNSUPPORTED: O3R_MERGE_RETAIN, dont_downsample, a communicator
+ *     attached (a cell's neighbours may live on other ranks), or a map of 2^31 or more vertices (32-bit indices).
+ *   - A sharded map is meshed on one context: export every rank's shard (o3r_cloud_export_cells, e.g. mapfile.save), then
+ *     load all the shard files into one context without a communicator (mapfile.load, which as a rank of world 1 keeps
+ *     every cell and imports them with o3r_cloud_import_cells) and mesh there. */
+int o3r_cloud_mesh(o3r_ctx* ctx, double max_step,
+                   o3r_point* verts, float* normals, size_t vcap, size_t* n_verts,
+                   uint32_t* tris, size_t tcap, size_t* n_tris);
+int o3r_cloud_mesh_dev(o3r_ctx* ctx, double max_step,
+                       const o3r_point** verts, const float** normals, size_t* n_verts,
+                       const uint32_t** tris, size_t* n_tris);
+
 /* ---- stand-alone stages (parity probes; same kernels as above) ------------------------------- */
 
 /* pcl::VoxelGrid<PointXYZRGB>::filter on a host cloud: leaf (lx,ly,lz) as PCL's setLeafSize floats,

@@ -258,6 +258,14 @@ struct Registration {
     ~Registration() { if (h_state) cudaFreeHost(h_state); }
 };
 
+// Meshing of the resident map (host_mesh.cuh): per-tile vertex / triangle counts and offsets, the two totals and their pinned
+// read-back, the resident position -> vertex map, and the result (vertices, normals, triangles) o3r_cloud_mesh_dev points at
+struct Meshing {
+    DevBuf vcnt, voff, tcnt, toff, tot, vmap, verts, normals, tris;
+    uint32_t* h_tot = nullptr;
+    ~Meshing() { if (h_tot) cudaFreeHost(h_tot); }
+};
+
 // The pre-pass (o3r_disp_variance / o3r_plane_fit in o3r_api.cu): plane fit / variance gate scratch
 struct PrePass { DevBuf labels, disp, sums, rows, coef; };
 
@@ -314,6 +322,7 @@ struct o3r_ctx {
     Blur blur;
     PrePass pp;
     Registration reg;
+    Meshing mesh;
     Profiling prof;
 
     // Shared per-call scratch: sized on demand and used by several paths within one call.  It holds nothing a later call

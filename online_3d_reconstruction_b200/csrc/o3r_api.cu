@@ -10,6 +10,7 @@
 #include "host_changes.cuh"
 #include "host_checkpoint.cuh"
 #include "host_register.cuh"
+#include "host_mesh.cuh"
 
 
 // =====================================================================================================================
@@ -524,6 +525,31 @@ int o3r_cloud_register_dev(o3r_ctx* ctx, const o3r_point* dev_pts, size_t n, con
                            const o3r_register_params* params, float T_out[16], o3r_register_stats* stats) {
     if ((n && !dev_pts) || !T_init || !T_out) return O3R_ERR_INVALID;
     return api(ctx, [&] { return register_impl(ctx, dev_pts, false, n, T_init, params, T_out, stats); });
+}
+
+int o3r_cloud_mesh(o3r_ctx* ctx, double max_step, o3r_point* verts, float* normals, size_t vcap, size_t* n_verts,
+                   uint32_t* tris, size_t tcap, size_t* n_tris) {
+    if (!n_verts || !n_tris) return O3R_ERR_INVALID;
+    return api(ctx, [&] {
+        const MeshOut out{verts, normals, vcap, tris, tcap};
+        return mesh_impl(ctx, max_step, &out, n_verts, n_tris);
+    });
+}
+
+int o3r_cloud_mesh_dev(o3r_ctx* ctx, double max_step, const o3r_point** verts, const float** normals, size_t* n_verts,
+                       const uint32_t** tris, size_t* n_tris) {
+    if (!n_verts || !n_tris) return O3R_ERR_INVALID;
+    return api(ctx, [&] {
+        if (verts) *verts = nullptr;
+        if (normals) *normals = nullptr;
+        if (tris) *tris = nullptr;
+        const int rc = mesh_impl(ctx, max_step, nullptr, n_verts, n_tris);
+        if (rc) return rc;
+        if (verts) *verts = ctx->mesh.verts.as<const o3r_point>();
+        if (normals) *normals = ctx->mesh.normals.as<const float>();
+        if (tris) *tris = ctx->mesh.tris.as<const uint32_t>();
+        return O3R_OK;
+    });
 }
 
 int o3r_voxel_grid(o3r_ctx* ctx, const o3r_point* pts, size_t n, float lx, float ly, float lz, unsigned min_points,

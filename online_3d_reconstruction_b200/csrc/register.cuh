@@ -104,6 +104,70 @@ __global__ void k_reg_init(const double* __restrict__ part, uint32_t blocks, siz
     S->done = S->bad_input || n == 0;
 }
 
+// The local plane of the map at combined-grid cell (ci, cj, ck): z - z0 = a (x - x0) + b (y - y0) + d, in double, over the
+// centroids of the cell (x0, y0, z0) and of its 8 horizontal neighbours at the same k that are in the map (count >=
+// min_points), summed in the order row j, j-1, j+1, each i-1, i, i+1.  True with the plane's unit normal
+// n = (-a, -b, 1) / |.|; false when the cell is outside +-(2^20 - 2) in i or j (its neighbours would leave the key range) or
+// +-(2^20 - 1) in k, is not in the map, has fewer than 3 such cells, or the 3 x 3 system is singular (det <= kRegFitCond *
+// Suu * Sww * S1).  k_reg_step and the mesh's normals (mesh.cuh) both call it, so the two cannot drift apart.
+__device__ __forceinline__ bool reg_fit(const uint64_t* __restrict__ res_keys, const float4* __restrict__ res_acc, uint32_t n_res,
+                                        uint32_t min_points, int ci, int cj, int ck, double& x0, double& y0, double& z0,
+                                        double& nx, double& ny, double& nz) {
+    const int lim = (1 << 20) - 1;
+    if (ci < -lim + 1 || ci > lim - 1 || cj < -lim + 1 || cj > lim - 1 || ck < -lim || ck > lim) return false;
+    // One lower bound per row (a row's cells are consecutive keys); the cell's own row goes first, and without the cell
+    // in the map there is no plane.
+    uint64_t k0 = reg_key(ci - 1, cj, ck);
+    uint32_t at = reg_lower_bound(res_keys, n_res, k0);
+    float hx[3], hy[3], hz[3];
+    uint32_t hit = 0;
+#pragma unroll
+    for (int di = 0; di < 3; ++di)
+        if (at < n_res && res_keys[at] == k0 + (uint64_t)di) {
+            const float4 a = res_acc[at++];
+            if (__float_as_uint(a.w) >= min_points) {
+                const float4 c = acc_centroid(a, make_uint4(0u, 0u, 0u, 0u));
+                hx[di] = c.x; hy[di] = c.y; hz[di] = c.z;
+                hit |= 1u << di;
+            }
+        }
+    if (!(hit & 2u)) return false;
+    x0 = hx[1]; y0 = hy[1]; z0 = hz[1];
+    double Suu = 0, Suw = 0, Su = 0, Sww = 0, Sw = 0, S1 = 0, Suh = 0, Swh = 0, Sh = 0;
+    auto add = [&](float fx, float fy, float fz) {
+        const double u = (double)fx - x0, w = (double)fy - y0, h = (double)fz - z0;
+        Suu += u * u; Suw += u * w; Su += u; Sww += w * w; Sw += w; S1 += 1.0;
+        Suh += u * h; Swh += w * h; Sh += h;
+    };
+#pragma unroll
+    for (int di = 0; di < 3; ++di)
+        if (hit & (1u << di)) add(hx[di], hy[di], hz[di]);
+#pragma unroll
+    for (int dj = -1; dj <= 1; dj += 2) {
+        k0 = reg_key(ci - 1, cj + dj, ck);
+        at = reg_lower_bound(res_keys, n_res, k0);
+#pragma unroll
+        for (int di = 0; di < 3; ++di)
+            if (at < n_res && res_keys[at] == k0 + (uint64_t)di) {
+                const float4 a = res_acc[at++];
+                if (__float_as_uint(a.w) >= min_points) {
+                    const float4 c = acc_centroid(a, make_uint4(0u, 0u, 0u, 0u));
+                    add(c.x, c.y, c.z);
+                }
+            }
+    }
+    if (S1 < 3.0) return false;
+    const double c00 = Sww * S1 - Sw * Sw, c01 = Sw * Su - Suw * S1, c02 = Suw * Sw - Sww * Su;
+    const double c11 = Suu * S1 - Su * Su, c12 = Su * Suw - Suu * Sw;
+    const double det = Suu * c00 + Suw * c01 + Su * c02;
+    if (!(det > kRegFitCond * Suu * Sww * S1)) return false;
+    const double a = (c00 * Suh + c01 * Swh + c02 * Sh) / det;
+    const double b = (c01 * Suh + c11 * Swh + c12 * Sh) / det;
+    const double nn = sqrt(a * a + b * b + 1.0);
+    nx = -a / nn; ny = -b / nn; nz = 1.0 / nn;
+    return true;
+}
+
 // One Gauss-Newton linearisation: per CTA the sums of the normal equations over the point's correspondences.
 __global__ void __launch_bounds__(kThreads) k_reg_step(const float4* __restrict__ pts, size_t n, const RegState* __restrict__ S,
                                                        RegParams P, const uint64_t* __restrict__ res_keys,
@@ -117,7 +181,6 @@ __global__ void __launch_bounds__(kThreads) k_reg_step(const float4* __restrict_
     if (threadIdx.x < 3) piv[threadIdx.x] = S->pivot[threadIdx.x];
     __syncthreads();
     const uint32_t n_res = *n_res_ptr;
-    const int lim = (1 << 20) - 1;
     double H[21], g[6], cnt = 0.0, ss = 0.0;
 #pragma unroll
     for (int q = 0; q < 21; ++q) H[q] = 0.0;
@@ -129,59 +192,9 @@ __global__ void __launch_bounds__(kThreads) k_reg_step(const float4* __restrict_
         reg_apply(T, p.x, p.y, p.z, x, y, z);
         int ci, cj, ck;
         combined_cell((float)x, (float)y, (float)z, P.inv_c, P.inv_cz, ci, cj, ck);
-        if (ci < -lim + 1 || ci > lim - 1 || cj < -lim + 1 || cj > lim - 1 || ck < -lim || ck > lim) continue;
-        // The fit's cells: the hit cell and its horizontal neighbours at the same k that are in the map, summed in the order
-        // row j, j-1, j+1, each i-1, i, i+1.  One lower bound per row (a row's cells are consecutive keys); the hit row goes
-        // first, and without the hit cell in the map the point has no correspondence.
-        uint64_t k0 = reg_key(ci - 1, cj, ck);
-        uint32_t at = reg_lower_bound(res_keys, n_res, k0);
-        float hx[3], hy[3], hz[3];
-        uint32_t hit = 0;
-#pragma unroll
-        for (int di = 0; di < 3; ++di)
-            if (at < n_res && res_keys[at] == k0 + (uint64_t)di) {
-                const float4 a = res_acc[at++];
-                if (__float_as_uint(a.w) >= P.min_points) {
-                    const float4 c = acc_centroid(a, make_uint4(0u, 0u, 0u, 0u));
-                    hx[di] = c.x; hy[di] = c.y; hz[di] = c.z;
-                    hit |= 1u << di;
-                }
-            }
-        if (!(hit & 2u)) continue;
-        // z - z0 = a (x - x0) + b (y - y0) + d over those cells' centroids, in double
-        const double x0 = hx[1], y0 = hy[1], z0 = hz[1];
-        double Suu = 0, Suw = 0, Su = 0, Sww = 0, Sw = 0, S1 = 0, Suh = 0, Swh = 0, Sh = 0;
-        auto add = [&](float fx, float fy, float fz) {
-            const double u = (double)fx - x0, w = (double)fy - y0, h = (double)fz - z0;
-            Suu += u * u; Suw += u * w; Su += u; Sww += w * w; Sw += w; S1 += 1.0;
-            Suh += u * h; Swh += w * h; Sh += h;
-        };
-#pragma unroll
-        for (int di = 0; di < 3; ++di)
-            if (hit & (1u << di)) add(hx[di], hy[di], hz[di]);
-#pragma unroll
-        for (int dj = -1; dj <= 1; dj += 2) {
-            k0 = reg_key(ci - 1, cj + dj, ck);
-            at = reg_lower_bound(res_keys, n_res, k0);
-#pragma unroll
-            for (int di = 0; di < 3; ++di)
-                if (at < n_res && res_keys[at] == k0 + (uint64_t)di) {
-                    const float4 a = res_acc[at++];
-                    if (__float_as_uint(a.w) >= P.min_points) {
-                        const float4 c = acc_centroid(a, make_uint4(0u, 0u, 0u, 0u));
-                        add(c.x, c.y, c.z);
-                    }
-                }
-        }
-        if (S1 < 3.0) continue;
-        const double c00 = Sww * S1 - Sw * Sw, c01 = Sw * Su - Suw * S1, c02 = Suw * Sw - Sww * Su;
-        const double c11 = Suu * S1 - Su * Su, c12 = Su * Suw - Suu * Sw;
-        const double det = Suu * c00 + Suw * c01 + Su * c02;
-        if (!(det > kRegFitCond * Suu * Sww * S1)) continue;
-        const double a = (c00 * Suh + c01 * Swh + c02 * Sh) / det;
-        const double b = (c01 * Suh + c11 * Swh + c12 * Sh) / det;
-        const double nn = sqrt(a * a + b * b + 1.0);
-        const double nx = -a / nn, ny = -b / nn, nz = 1.0 / nn;
+        // the hit cell's plane; without the hit cell in the map, or without a plane, the point has no correspondence
+        double x0, y0, z0, nx, ny, nz;
+        if (!reg_fit(res_keys, res_acc, n_res, P.min_points, ci, cj, ck, x0, y0, z0, nx, ny, nz)) continue;
         const double r = nx * (x - x0) + ny * (y - y0) + nz * (z - z0);
         if (!(fabs(r) <= P.max_distance)) continue;
         const double qx = x - piv[0], qy = y - piv[1], qz = z - piv[2];

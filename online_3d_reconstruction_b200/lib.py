@@ -17,6 +17,7 @@ SYMBOLS = [
     "o3r_cloud_transform", "o3r_cloud_append", "o3r_cloud_downsample", "o3r_cloud_downsample_dev", "o3r_cloud_size",
     "o3r_cloud_clear", "o3r_cloud_track_changes", "o3r_cloud_changes", "o3r_cloud_changes_dev",
     "o3r_cloud_export_cells", "o3r_cloud_import_cells", "o3r_cloud_export_points", "o3r_cloud_register", "o3r_cloud_register_dev",
+    "o3r_cloud_mesh", "o3r_cloud_mesh_dev",
     "o3r_voxel_grid", "o3r_blur_u8", "o3r_frame_mask", "o3r_disp_variance", "o3r_plane_fit", "o3r_sor", "o3r_last_batch_partials",
     "o3r_set_keep_frame_voxels", "o3r_last_batch_engine",
     "o3r_comm_unique_id", "o3r_comm_init", "o3r_comm_attach", "o3r_comm_destroy", "o3r_exchange_cycle",
@@ -74,6 +75,8 @@ def load():
     RP, RS, F16 = C.POINTER(abi.RegisterParams), C.POINTER(abi.RegisterStats), C.POINTER(C.c_float)
     L.o3r_cloud_register.argtypes = [vp, vp, sz, F16, RP, F16, RS]
     L.o3r_cloud_register_dev.argtypes = [vp, vp, sz, F16, RP, F16, RS]
+    L.o3r_cloud_mesh.argtypes = [vp, C.c_double, vp, vp, sz, szp, vp, sz, szp]
+    L.o3r_cloud_mesh_dev.argtypes = [vp, C.c_double, C.POINTER(vp), C.POINTER(vp), szp, C.POINTER(vp), szp]
     L.o3r_voxel_grid.argtypes = [vp, vp, sz, C.c_float, C.c_float, C.c_float, C.c_uint, vp, sz, szp, vp, vp,
                                  C.POINTER(C.c_int)]
     L.o3r_blur_u8.argtypes = [vp, vp, sz, C.c_int, C.c_int, C.c_int, C.c_int, vp, sz]

@@ -251,6 +251,28 @@ class Pose:
                      info=np.array(st.info[:]).reshape(6, 6))
         return np.array(Tout[:], dtype=np.float32).reshape(4, 4), stats
 
+    def meshCloud(self, max_step=float("inf")):
+        """o3r_cloud_mesh: the resident map's height field as triangles (accumulate modes) -> (vertices as abi.POINT,
+        exactly downsamplePtCloud(); normals (n, 3) float32, (0, 0, 0) where no plane fits; triangles (m, 3) uint32
+        vertex indices, counter-clockwise seen from above).  A triangle is kept iff its largest |dz| is <= max_step."""
+        nv, nt = C.c_size_t(0), C.c_size_t(0)
+        self._check(self._L.o3r_cloud_mesh(self._h, float(max_step), None, None, 0, C.byref(nv), None, 0, C.byref(nt)))
+        verts = np.empty(max(1, nv.value), dtype=abi.POINT)
+        normals = np.empty((max(1, nv.value), 3), dtype=np.float32)
+        tris = np.empty((max(1, nt.value), 3), dtype=np.uint32)
+        self._check(self._L.o3r_cloud_mesh(self._h, float(max_step), verts.ctypes.data, normals.ctypes.data, nv.value,
+                                           C.byref(nv), tris.ctypes.data, nt.value, C.byref(nt)))
+        return verts[:nv.value], normals[:nv.value], tris[:nt.value]
+
+    def meshCloudDevice(self, max_step=float("inf")):
+        """Same as meshCloud but the result stays in device memory owned by the context (valid until the next call on it)
+        -> (vertices pointer, normals pointer, n vertices, triangles pointer, n triangles)."""
+        v, nrm, t = C.c_void_p(), C.c_void_p(), C.c_void_p()
+        nv, nt = C.c_size_t(0), C.c_size_t(0)
+        self._check(self._L.o3r_cloud_mesh_dev(self._h, float(max_step), C.byref(v), C.byref(nrm), C.byref(nv), C.byref(t),
+                                               C.byref(nt)))
+        return v.value, nrm.value, nv.value, t.value, nt.value
+
     # -- stand-alone stages --------------------------------------------------------------------------------
     def voxelGrid(self, pts, leaf, min_points=0):
         """pcl::VoxelGrid on a host cloud -> (points, keys u64, counts u32, passthrough)."""
